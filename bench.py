@@ -17,6 +17,7 @@ batch (weak scaling, no data-path collective: SURVEY.md section 8(e)).
             be built in this image) on the box's host cores, bounded sample
 
 `--impl reference` times that CPU restatement alone (the reference arm of the contract).
+`--dump-outputs DIR` writes a fixed sample of the last timed step's outputs to DIR (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -58,6 +59,8 @@ def parse():
     ap.add_argument("--check", type=int, default=512, help="outputs decrypted with the oracle after the run, spread over every PBS wave (checker only)")
     ap.add_argument("--no-sweep", action="store_true", help="skip the 3-point batch-size sweep (BASELINE config 5)")
     ap.add_argument("--no-sharded-graph", action="store_true", help="N > 1: skip the sharded mul32+compare graph (BASELINE config 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of the last step's "
+                    "GGSW outputs to DIR/cbs_ggsw_fft.npy (float64, at most 32 MiB)")
     return ap.parse_args()
 
 
@@ -662,6 +665,20 @@ def measure_sharded_graph(ev, keys, args, world, rank, dev):
     return res
 
 
+def dump_outputs(d_out, B: int, len_ggsw: int, out_dir: str) -> None:
+    """What a caller of the timed path receives from one step: B GGSW ciphertexts in the FFT domain at the device scale
+    (reference_scale=False), len_ggsw complex128 each, stored as (real, imag) float64 pairs.  A whole step is 256 KiB per
+    bootstrap at DEFAULT_128, so only a fixed seeded sample of the batch is written, in ascending batch order: two builds
+    run with the same arguments see the same inputs and can be compared output for output."""
+    import torch
+
+    n = min(B, max(1, (32 << 20) // (len_ggsw * 16)))
+    rows = np.sort(np.random.default_rng(0xD0).choice(B, n, replace=False))
+    ggsw = d_out.view(B, len_ggsw, 2)[torch.from_numpy(rows).to(d_out.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "cbs_ggsw_fft.npy"), ggsw)
+
+
 # ---------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------
@@ -766,6 +783,8 @@ def run_gpu(args):
     dev_ms = float(t.item())
     clocks = sampler.stop() if sampler else None
     value = world * B * args.steps / (dev_ms * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(d_out, B, ev.len_ggsw, args.dump_outputs)
 
     # ---- roofline of the dominant kernel (pbs_kernel), timed alone with CUDA events ------------
     roofline = None
