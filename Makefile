@@ -6,7 +6,7 @@ NVCC ?= nvcc
 CXX ?= g++
 NVFLAGS ?= -std=c++17 -O3 -fmad=false -gencode arch=compute_100a,code=sm_100a -lineinfo -Xcompiler -fPIC -Xptxas -v
 CSRC := spf_b200/csrc
-HDRS := $(CSRC)/fft16.cuh $(CSRC)/fft_consts.h $(CSRC)/team_ops.cuh $(CSRC)/kernels.cuh $(CSRC)/tables.h $(CSRC)/graph.cuh $(CSRC)/serial.inl include/spf_b200.h
+HDRS := $(CSRC)/fft16.cuh $(CSRC)/fft_consts.h $(CSRC)/team_ops.cuh $(CSRC)/kernels.cuh $(CSRC)/tables.h $(CSRC)/graph.cuh $(CSRC)/box.cuh $(CSRC)/serial.inl include/spf_b200.h
 
 all: spf_b200/libspf_b200.so $(CSRC)/libspf_emu.so oracle
 

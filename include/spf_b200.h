@@ -297,6 +297,72 @@ int spf_b200_graph_plan(const spf_params *params, const spf_node *nodes, size_t 
 /* Rank that writes Output* node `node` in a sharded run; -1 = every rank; -2 = not an Output* node. */
 int spf_b200_graph_output_rank(const spf_b200_graph *graph, size_t node);
 
+/* ---- one process, every GPU of a box: spf_b200_box ---------------------------------------------------
+ * A box is N ranks (1 <= N <= 8), each a context on its own device, owned by ONE handle and driven from ONE thread --
+ * the shape of parasol_runtime's CircuitProcessor (one dispatching thread, &mut self).  The same device may appear
+ * more than once (several ranks on one GPU).  Distinct devices must reach each other as peers (cudaDeviceCanAccessPeer
+ * both ways, else SPF_E_UNSUPPORTED); peer access is enabled for every pair.  The compute key is uploaded once, to
+ * rank 0's device, and replicated device to device over NVLink in a fan-out tree (0 -> 1, {0,1} -> {2,3}, ...); each
+ * rank's context is then made as spf_b200_create_from_device makes it.  Errors of box calls: spf_b200_box_last_error
+ * (box NULL: the last failing spf_b200_box_create* of this thread). */
+typedef struct spf_b200_box spf_b200_box;
+typedef struct spf_b200_box_graph spf_b200_box_graph;
+int spf_b200_box_create(const spf_params *params, const double *bsk_fft, size_t bsk_len, const uint64_t *ksk,
+                        size_t ksk_len, const double *ssk_fft, size_t ssk_len, const double *ak_fft, size_t ak_len,
+                        const int *devices, int n, spf_b200_box **out);
+int spf_b200_box_create_from_serialized(const spf_params *params, const uint8_t *buf, size_t len, const int *devices,
+                                        int n, spf_b200_box **out);
+/* Joins the box's worker threads and drops its contexts; box graphs still alive keep what they use. */
+void spf_b200_box_destroy(spf_b200_box *box);
+const char *spf_b200_box_last_error(const spf_b200_box *box);
+int spf_b200_box_size(const spf_b200_box *box);
+int spf_b200_box_device(const spf_b200_box *box, int rank);
+/* Rank `rank`'s context, for spf_b200_dev_* calls on that rank's device.  Owned by the box: do not destroy it. */
+spf_b200_ctx *spf_b200_box_context(spf_b200_box *box, int rank);
+/* Wall time of the device-to-device replication of the compute key at creation, milliseconds. */
+double spf_b200_box_key_replication_ms(const spf_b200_box *box);
+/* Elements [offset, offset + count) of key array `which` (0 bs_key, 1 ks_key, 2 ss_key, 3 auto_key) as resident on
+ * rank `rank`'s device, copied to `out` in the reference layout and scale (to check a replica against the host key). */
+int spf_b200_box_key_slice(spf_b200_box *box, int rank, int which, size_t offset, size_t count, void *out);
+/* The split of a batch over n ranks used by the box ops: contiguous ranges, the first batch % n ranks get one extra
+ * item (spf_b200/multi.py shard).  Host only. */
+void spf_b200_box_shard(size_t batch, int n, int rank, size_t *start, size_t *count);
+
+/* Host-pointer ops over the box: the batch is split by spf_b200_box_shard, every rank runs its slice of the
+ * single-context op at the same time (one worker thread per rank, created with the box), the call returns when every
+ * output is valid.  Outputs are bit-identical to the single-context op on the same slices. */
+int spf_b200_box_circuit_bootstrap(spf_b200_box *box, double *ggsw_out, const uint64_t *lwe0_in, size_t batch);
+int spf_b200_box_programmable_bootstrap(spf_b200_box *box, uint64_t *glwe_out, const uint64_t *lwe0_in,
+                                        const uint64_t *lut_glwe, uint32_t log_chi, uint32_t log_v, size_t batch);
+int spf_b200_box_keyswitch_lwe_l1_lwe_l0(spf_b200_box *box, uint64_t *lwe0_out, const uint64_t *lwe1_in, size_t batch);
+int spf_b200_box_cmux(spf_b200_box *box, uint64_t *glwe_out, const double *sel_ggsw, const uint64_t *a,
+                      const uint64_t *b, size_t batch);
+
+/* Graphs over the box: spf_b200_graph_build_sharded on every rank with world = N, wired to each other's arenas in
+ * this process (the peer-memory exchange of spf_b200_graph_run_sharded: fused GGSW stores, keyswitch broadcast, flag
+ * barriers between levels).  Every rank's run is enqueued from the calling thread, level-interleaved across the ranks;
+ * everything that could make the host wait on a device is done before the first enqueue, so no rank waits at a barrier
+ * for a rank that has not been enqueued.
+ * Output* nodes are written by their owner rank (spf_b200_graph_output_rank; rank 0 for nodes every rank holds) into
+ * the caller's host buffers.  io buffers are host memory only: device-memory handles are refused with SPF_E_INVALID.
+ * Spawn semantics are those of spf_b200_graph_spawn: on_complete fires exactly once per run, after every rank has
+ * retired, with the first error of any rank; `after` orders on the device (every rank behind every rank of the
+ * dependency); a run whose dependency failed
+ * retires as a no-op with that error; at most spf_b200_box_set_max_in_flight (default 4) runs per box are in flight,
+ * further spawns block the caller.  A failed run with N > 1 poisons the box graph (rebuild it).  Destroying a box
+ * graph waits for its run in flight. */
+int spf_b200_box_graph_build(spf_b200_box *box, const spf_node *nodes, size_t n_nodes, spf_b200_box_graph **out);
+int spf_b200_box_graph_run(spf_b200_box_graph *graph);
+int spf_b200_box_graph_spawn(spf_b200_box_graph *graph, spf_b200_box_graph *const *after, size_t n_after,
+                             spf_completion_fn on_complete, void *user);
+int spf_b200_box_graph_wait(spf_b200_box_graph *graph);
+const char *spf_b200_box_graph_status_message(const spf_b200_box_graph *graph);
+int spf_b200_box_graph_set_io(spf_b200_box_graph *graph, size_t node, void *io);
+void spf_b200_box_graph_destroy(spf_b200_box_graph *graph);
+int spf_b200_box_graph_levels(const spf_b200_box_graph *graph);
+uint64_t spf_b200_box_graph_launches(const spf_b200_box_graph *graph); /* kernel launches of the last run, all ranks */
+int spf_b200_box_set_max_in_flight(spf_b200_box *box, int n);
+
 /* ---- serialized keys and ciphertexts (SURVEY.md 8(f).1) ------------------------------------------
  * The reference serialises with bincode 1.3.3 (Cargo.lock:244-245), fixed-width little-endian
  * integers: every sunscreen_tfhe entity is one sequence `u64 length || elements`

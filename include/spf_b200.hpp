@@ -236,6 +236,116 @@ class CircuitProcessor {
   const Evaluation& ev_;
 };
 
+inline void check_box(int rc, const spf_b200_box* box) {
+  if (rc == SPF_OK) return;
+  const char* msg = spf_b200_box_last_error(box);
+  throw Error(rc, msg && *msg ? msg : "spf_b200 error " + std::to_string(rc));
+}
+
+// Evaluation over several GPUs of one box, from one thread (spf_b200_box_*): rank r is a context on devices[r]; the
+// compute key crosses PCIe once and is replicated device to device.  Batched ops split the batch over the ranks.
+class BoxEvaluation {
+ public:
+  BoxEvaluation(const spf_params& params, const std::vector<Complex>& bsk_fft, const std::vector<Torus>& ksk,
+                const std::vector<Complex>& ssk_fft, const std::vector<Complex>& ak_fft, const std::vector<int>& devices)
+      : p_(params) {
+    check_box(spf_b200_box_create(&p_, bsk_fft.data(), bsk_fft.size() / 2, ksk.data(), ksk.size(), ssk_fft.data(), ssk_fft.size() / 2,
+                                  ak_fft.data(), ak_fft.size() / 2, devices.data(), static_cast<int>(devices.size()), &box_),
+              nullptr);
+  }
+  static BoxEvaluation from_serialized(const spf_params& params, const std::uint8_t* buf, std::size_t len, const std::vector<int>& devices) {
+    BoxEvaluation e(params);
+    check_box(spf_b200_box_create_from_serialized(&e.p_, buf, len, devices.data(), static_cast<int>(devices.size()), &e.box_), nullptr);
+    return e;
+  }
+  BoxEvaluation(BoxEvaluation&& o) noexcept : p_(o.p_), box_(std::exchange(o.box_, nullptr)) {}
+  BoxEvaluation(const BoxEvaluation&) = delete;
+  BoxEvaluation& operator=(const BoxEvaluation&) = delete;
+  ~BoxEvaluation() { if (box_) spf_b200_box_destroy(box_); }
+
+  const spf_params& params() const { return p_; }
+  spf_b200_box* handle() const { return box_; }
+  int size() const { return spf_b200_box_size(box_); }
+  spf_b200_ctx* context(int rank) const { return spf_b200_box_context(box_, rank); }
+  double key_replication_ms() const { return spf_b200_box_key_replication_ms(box_); }
+
+  void circuit_bootstrap(std::vector<Complex>& ggsw_out, const std::vector<Torus>& lwe0_in) const {
+    const std::size_t batch = batch_of(lwe0_in.size(), spf_b200_len_lwe_l0(&p_), "circuit_bootstrap");
+    ggsw_out.resize(batch * spf_b200_len_ggsw_l1(&p_) * 2);
+    check_box(spf_b200_box_circuit_bootstrap(box_, ggsw_out.data(), lwe0_in.data(), batch), box_);
+  }
+  void programmable_bootstrap(std::vector<Torus>& glwe_out, const std::vector<Torus>& lwe0_in, const std::vector<Torus>& lut_glwe,
+                              std::uint32_t log_chi, std::uint32_t log_v) const {
+    const std::size_t batch = batch_of(lwe0_in.size(), spf_b200_len_lwe_l0(&p_), "programmable_bootstrap");
+    if (lut_glwe.size() != spf_b200_len_glwe_l1(&p_)) throw Error(SPF_E_INVALID, "programmable_bootstrap: LUT has the wrong length");
+    glwe_out.resize(batch * spf_b200_len_glwe_l1(&p_));
+    check_box(spf_b200_box_programmable_bootstrap(box_, glwe_out.data(), lwe0_in.data(), lut_glwe.data(), log_chi, log_v, batch), box_);
+  }
+  void keyswitch_lwe_l1_lwe_l0(std::vector<Torus>& lwe0_out, const std::vector<Torus>& lwe1_in) const {
+    const std::size_t batch = batch_of(lwe1_in.size(), spf_b200_len_lwe_l1(&p_), "keyswitch_lwe_l1_lwe_l0");
+    lwe0_out.resize(batch * spf_b200_len_lwe_l0(&p_));
+    check_box(spf_b200_box_keyswitch_lwe_l1_lwe_l0(box_, lwe0_out.data(), lwe1_in.data(), batch), box_);
+  }
+  void cmux(std::vector<Torus>& out, const std::vector<Complex>& sel, const std::vector<Torus>& a, const std::vector<Torus>& b) const {
+    const std::size_t batch = batch_of(a.size(), spf_b200_len_glwe_l1(&p_), "cmux");
+    if (b.size() != a.size() || sel.size() != batch * spf_b200_len_ggsw_l1(&p_) * 2) throw Error(SPF_E_INVALID, "cmux: operand sizes differ");
+    out.resize(a.size());
+    check_box(spf_b200_box_cmux(box_, out.data(), sel.data(), a.data(), b.data(), batch), box_);
+  }
+  void set_max_in_flight(int n) const { check_box(spf_b200_box_set_max_in_flight(box_, n), box_); }
+
+ private:
+  explicit BoxEvaluation(const spf_params& params) : p_(params) {}
+  static std::size_t batch_of(std::size_t len, std::size_t item, const char* what) {
+    if (item == 0 || len % item) throw Error(SPF_E_INVALID, std::string(what) + ": length is not a whole number of ciphertexts");
+    return len / item;
+  }
+  spf_params p_;
+  spf_b200_box* box_ = nullptr;
+};
+
+// A levelised graph over every rank of a box; host io buffers only.
+class BoxGraph {
+ public:
+  BoxGraph(const BoxEvaluation& ev, const FheCircuit& c) : box_(ev.handle()) {
+    check_box(spf_b200_box_graph_build(box_, c.nodes().data(), c.size(), &g_), box_);
+  }
+  BoxGraph(BoxGraph&& o) noexcept : box_(o.box_), g_(std::exchange(o.g_, nullptr)) {}
+  BoxGraph(const BoxGraph&) = delete;
+  BoxGraph& operator=(const BoxGraph&) = delete;
+  ~BoxGraph() { if (g_) spf_b200_box_graph_destroy(g_); }
+  void run() { check_box(spf_b200_box_graph_run(g_), box_); }
+  // spawn_graph: on_complete(user, status, message) fires once, after every rank has retired, on a CUDA thread
+  void spawn(const std::vector<const BoxGraph*>& after, spf_completion_fn on_complete, void* user) {
+    std::vector<spf_b200_box_graph*> deps;
+    for (const BoxGraph* d : after) deps.push_back(d->g_);
+    check_box(spf_b200_box_graph_spawn(g_, deps.data(), deps.size(), on_complete, user), box_);
+  }
+  void wait() {
+    const int rc = spf_b200_box_graph_wait(g_);
+    if (rc != SPF_OK) throw Error(rc, spf_b200_box_graph_status_message(g_));
+  }
+  void set_io(std::size_t node, void* io) { check_box(spf_b200_box_graph_set_io(g_, node, io), box_); }
+  int levels() const { return spf_b200_box_graph_levels(g_); }
+  std::uint64_t launches() const { return spf_b200_box_graph_launches(g_); }
+  spf_b200_box_graph* handle() const { return g_; }
+
+ private:
+  spf_b200_box* box_;
+  spf_b200_box_graph* g_ = nullptr;
+};
+
+// CircuitProcessor (circuit_processor/mod.rs:62-655) over every GPU of a box.
+class BoxCircuitProcessor {
+ public:
+  explicit BoxCircuitProcessor(const BoxEvaluation& ev) : ev_(ev) {}
+  BoxGraph compile(const FheCircuit& c) const { return BoxGraph(ev_, c); }
+  void run_graph_blocking(const FheCircuit& c) const { compile(c).run(); }
+
+ private:
+  const BoxEvaluation& ev_;
+};
+
 // MuxCircuit (mux_circuits/src/lib.rs:153-163) as the C ABI's flat, topologically ordered node list.
 class MuxCircuit {
  public:

@@ -9,6 +9,7 @@
 //!   (`circuit_processor/mod.rs:573-655`): [`Graph::spawn`] returns at once and calls the completion handler with the
 //!   first error (`completion_handler.rs:14-56`); [`DeviceCiphertext`] handles keep task outputs in HBM between graphs
 //!   (`circuit_processor/task.rs:10-16`).
+//! * [`BoxEvaluation`] / [`BoxGraph`]: the same over every GPU of a box, from one thread (one handle, one key upload).
 //! * module [`parasol`] (feature `parasol`): the glue a maintainer pastes into `parasol_runtime` so that
 //!   `CircuitProcessor::exec_op` (`circuit_processor/mod.rs:255-546`) dispatches to the GPU.
 //!
@@ -20,6 +21,7 @@ use std::os::raw::{c_char, c_int};
 use std::ptr::{self, NonNull};
 use std::sync::Arc;
 
+use spf_b200_sys::{spf_b200_box as RawBox, spf_b200_box_graph as RawBoxGraph};
 pub use sys::{spf_node, spf_params, spf_radix};
 
 /// `RuntimeError` of the GPU path: the library's status code and message.
@@ -298,6 +300,167 @@ impl Drop for Graph {
     }
 }
 
+/// `Evaluation` over several GPUs of one box, driven from one thread (`spf_b200_box_*`): rank `r` is a context on
+/// `devices[r]`; the compute key crosses PCIe once and is replicated device to device.  The batched ops split the batch
+/// contiguously over the ranks and run them concurrently; [`BoxGraph`] runs a whole `FheCircuit` over every rank.
+#[derive(Clone)]
+pub struct BoxEvaluation {
+    boxed: Arc<BoxHandle>,
+    pub params: spf_params,
+}
+
+struct BoxHandle(NonNull<RawBox>);
+unsafe impl Send for BoxHandle {}
+unsafe impl Sync for BoxHandle {} // one call at a time per box, as for a context
+impl Drop for BoxHandle {
+    fn drop(&mut self) {
+        unsafe { sys::spf_b200_box_destroy(self.0.as_ptr()) }
+    }
+}
+
+fn box_error(b: *const RawBox) -> String {
+    let p = unsafe { sys::spf_b200_box_last_error(b) };
+    if p.is_null() { String::new() } else { unsafe { CStr::from_ptr(p) }.to_string_lossy().into_owned() }
+}
+
+macro_rules! box_check {
+    ($self:expr, $rc:expr) => {{
+        let rc = $rc;
+        if rc == 0 { Ok(()) } else { Err(Error { code: rc, message: box_error($self.raw()) }) }
+    }};
+}
+
+impl BoxEvaluation {
+    /// `Evaluation::new` for every rank of the box; `devices` may repeat a device (several ranks on one GPU).
+    #[allow(clippy::too_many_arguments)]
+    pub fn new(params: &spf_params, bs_key: &[f64], ks_key: &[u64], ss_key: &[f64], auto_key: &[f64], devices: &[i32]) -> Result<Self> {
+        let devs: Vec<c_int> = devices.iter().map(|&d| d as c_int).collect();
+        let mut raw = ptr::null_mut();
+        let rc = unsafe {
+            sys::spf_b200_box_create(params, bs_key.as_ptr(), bs_key.len() / 2, ks_key.as_ptr(), ks_key.len(), ss_key.as_ptr(),
+                                     ss_key.len() / 2, auto_key.as_ptr(), auto_key.len() / 2, devs.as_ptr(), devs.len() as c_int, &mut raw)
+        };
+        match NonNull::new(raw) {
+            Some(p) if rc == 0 => Ok(Self { boxed: Arc::new(BoxHandle(p)), params: *params }),
+            _ => Err(Error { code: rc, message: box_error(ptr::null()) }),
+        }
+    }
+    /// `safe_bincode::deserialize::<ComputeKey>` + [`BoxEvaluation::new`].
+    pub fn from_serialized(params: &spf_params, compute_key_bincode: &[u8], devices: &[i32]) -> Result<Self> {
+        let devs: Vec<c_int> = devices.iter().map(|&d| d as c_int).collect();
+        let mut raw = ptr::null_mut();
+        let rc = unsafe {
+            sys::spf_b200_box_create_from_serialized(params, compute_key_bincode.as_ptr(), compute_key_bincode.len(), devs.as_ptr(),
+                                                     devs.len() as c_int, &mut raw)
+        };
+        match NonNull::new(raw) {
+            Some(p) if rc == 0 => Ok(Self { boxed: Arc::new(BoxHandle(p)), params: *params }),
+            _ => Err(Error { code: rc, message: box_error(ptr::null()) }),
+        }
+    }
+    fn raw(&self) -> *mut RawBox {
+        self.boxed.0.as_ptr()
+    }
+    fn len(&self, f: unsafe extern "C" fn(*const spf_params) -> usize) -> usize {
+        unsafe { f(&self.params) }
+    }
+    fn expect(&self, what: &str, got: usize, want: usize) -> Result<()> {
+        if got == want { Ok(()) } else { Err(Error { code: sys::SPF_E_INVALID, message: format!("{what}: {got} elements, expected {want}") }) }
+    }
+    /// Number of ranks.
+    pub fn size(&self) -> usize {
+        unsafe { sys::spf_b200_box_size(self.raw()) as usize }
+    }
+    /// `Evaluation::circuit_bootstrap` over the box.
+    pub fn circuit_bootstrap(&self, output: &mut [f64], input: &[u64]) -> Result<()> {
+        let batch = input.len() / self.len(sys::spf_b200_len_lwe_l0);
+        self.expect("circuit_bootstrap output", output.len(), 2 * batch * self.len(sys::spf_b200_len_ggsw_l1))?;
+        box_check!(self, unsafe { sys::spf_b200_box_circuit_bootstrap(self.raw(), output.as_mut_ptr(), input.as_ptr(), batch) })
+    }
+    /// `generalized_programmable_bootstrap` over the box.
+    pub fn programmable_bootstrap(&self, output: &mut [u64], input: &[u64], lut: &[u64], log_chi: u32, log_v: u32) -> Result<()> {
+        let batch = input.len() / self.len(sys::spf_b200_len_lwe_l0);
+        self.expect("programmable_bootstrap output", output.len(), batch * self.len(sys::spf_b200_len_glwe_l1))?;
+        box_check!(self, unsafe { sys::spf_b200_box_programmable_bootstrap(self.raw(), output.as_mut_ptr(), input.as_ptr(), lut.as_ptr(), log_chi, log_v, batch) })
+    }
+    /// `Evaluation::keyswitch_lwe_l1_lwe_l0` over the box.
+    pub fn keyswitch_lwe_l1_lwe_l0(&self, output: &mut [u64], input: &[u64]) -> Result<()> {
+        let batch = input.len() / self.len(sys::spf_b200_len_lwe_l1);
+        self.expect("keyswitch output", output.len(), batch * self.len(sys::spf_b200_len_lwe_l0))?;
+        box_check!(self, unsafe { sys::spf_b200_box_keyswitch_lwe_l1_lwe_l0(self.raw(), output.as_mut_ptr(), input.as_ptr(), batch) })
+    }
+    /// `KeylessEvaluation::cmux` over the box: `output = sel ? b : a`.
+    pub fn cmux(&self, output: &mut [u64], sel: &[f64], a: &[u64], b: &[u64]) -> Result<()> {
+        let batch = a.len() / self.len(sys::spf_b200_len_glwe_l1);
+        self.expect("cmux output", output.len(), a.len())?;
+        box_check!(self, unsafe { sys::spf_b200_box_cmux(self.raw(), output.as_mut_ptr(), sel.as_ptr(), a.as_ptr(), b.as_ptr(), batch) })
+    }
+    /// Flow control of spawned box graphs (runs in flight per box).
+    pub fn set_max_in_flight(&self, n: usize) -> Result<()> {
+        box_check!(self, unsafe { sys::spf_b200_box_set_max_in_flight(self.raw(), n as c_int) })
+    }
+}
+
+/// A validated, levelised `FheCircuit` over every rank of a [`BoxEvaluation`] (`spf_b200_box_graph_build`).  io buffers
+/// are host memory.
+pub struct BoxGraph {
+    raw: NonNull<RawBoxGraph>,
+    ev: BoxEvaluation,
+}
+unsafe impl Send for BoxGraph {}
+
+impl BoxGraph {
+    pub fn build(ev: &BoxEvaluation, nodes: &[spf_node]) -> Result<Self> {
+        let mut raw = ptr::null_mut();
+        let rc = unsafe { sys::spf_b200_box_graph_build(ev.raw(), nodes.as_ptr(), nodes.len(), &mut raw) };
+        match NonNull::new(raw) {
+            Some(p) if rc == 0 => Ok(Self { raw: p, ev: ev.clone() }),
+            _ => Err(Error { code: rc, message: box_error(ev.raw()) }),
+        }
+    }
+    /// `CircuitProcessor::run_graph_blocking` over the box.
+    pub fn run_blocking(&mut self) -> Result<()> {
+        let rc = unsafe { sys::spf_b200_box_graph_run(self.raw.as_ptr()) };
+        if rc == 0 { Ok(()) } else { Err(Error { code: rc, message: box_error(self.ev.raw()) }) }
+    }
+    /// `CircuitProcessor::spawn_graph` over the box: the handler fires once, after every rank has retired.
+    pub fn spawn<F: FnOnce(Option<Error>) + Send + 'static>(&mut self, after: &[&BoxGraph], on_completion: F) -> Result<()> {
+        let deps: Vec<*mut RawBoxGraph> = after.iter().map(|g| g.raw.as_ptr()).collect();
+        let handler: Box<Handler> = Box::new(Box::new(on_completion));
+        let user = Box::into_raw(handler) as *mut c_void;
+        let rc = unsafe { sys::spf_b200_box_graph_spawn(self.raw.as_ptr(), deps.as_ptr(), deps.len(), Some(completion_trampoline), user) };
+        if rc == 0 {
+            Ok(())
+        } else {
+            drop(unsafe { Box::from_raw(user as *mut Handler) });
+            Err(Error { code: rc, message: box_error(self.ev.raw()) })
+        }
+    }
+    /// Blocks until the last run (callback included) is over and returns its status.
+    pub fn wait(&self) -> Result<()> {
+        let rc = unsafe { sys::spf_b200_box_graph_wait(self.raw.as_ptr()) };
+        if rc == 0 {
+            Ok(())
+        } else {
+            let m = unsafe { CStr::from_ptr(sys::spf_b200_box_graph_status_message(self.raw.as_ptr())) }.to_string_lossy().into_owned();
+            Err(Error { code: rc, message: m })
+        }
+    }
+    /// Re-point an `Input*` / `Output*` node at another host buffer.
+    ///
+    /// # Safety
+    /// `io` must stay valid, and large enough for the node's ciphertext, until the graph has run.
+    pub unsafe fn set_io(&mut self, node: usize, io: *mut c_void) -> Result<()> {
+        let rc = sys::spf_b200_box_graph_set_io(self.raw.as_ptr(), node, io);
+        if rc == 0 { Ok(()) } else { Err(Error { code: rc, message: box_error(self.ev.raw()) }) }
+    }
+}
+impl Drop for BoxGraph {
+    fn drop(&mut self) {
+        unsafe { sys::spf_b200_box_graph_destroy(self.raw.as_ptr()) }
+    }
+}
+
 /// Glue for the reference workspace (feature `parasol`): what `parasol_runtime` needs so that
 /// `CircuitProcessor::exec_op` runs on the GPU.  Written against spf v0.9.0.
 #[cfg(feature = "parasol")]
@@ -430,19 +593,47 @@ pub mod parasol {
             .collect()
     }
 
+    /// The evaluator a `CircuitProcessor` dispatches to: one GPU, or every GPU of a box.
+    pub enum Evaluator<'a> {
+        Single(&'a Evaluation),
+        Box(&'a BoxEvaluation),
+    }
+    /// The graph [`spawn_graph`] returns, on the evaluator it was built for.
+    pub enum SpawnedGraph {
+        Single(Graph),
+        Box(BoxGraph),
+    }
+    impl SpawnedGraph {
+        pub fn wait(&self) -> Result<()> {
+            match self {
+                SpawnedGraph::Single(g) => g.wait(),
+                SpawnedGraph::Box(g) => g.wait(),
+            }
+        }
+    }
+
     /// `CircuitProcessor::spawn_graph` on the GPU: lower, build, spawn.  Validation errors reach the handler, as in
     /// the reference where they surface through `CompletionHandler::error`.
-    pub fn spawn_graph<F>(ev: &Evaluation, circuit: &parasol_runtime::FheCircuit, on_completion: F) -> Option<Graph>
+    pub fn spawn_graph<F>(ev: Evaluator<'_>, circuit: &parasol_runtime::FheCircuit, on_completion: F) -> Option<SpawnedGraph>
     where
         F: FnOnce(Option<Error>) + Send + 'static,
     {
-        match Graph::build(ev, &lower(circuit)) {
+        let nodes = lower(circuit);
+        let built = match ev {
+            Evaluator::Single(e) => Graph::build(e, &nodes).map(SpawnedGraph::Single),
+            Evaluator::Box(b) => BoxGraph::build(b, &nodes).map(SpawnedGraph::Box),
+        };
+        match built {
             Err(e) => {
                 on_completion(Some(e));
                 None
             }
             Ok(mut g) => {
-                if let Err(e) = g.spawn(&[], on_completion) {
+                let spawned = match &mut g {
+                    SpawnedGraph::Single(s) => s.spawn(&[], on_completion),
+                    SpawnedGraph::Box(b) => b.spawn(&[], on_completion),
+                };
+                if let Err(e) = spawned {
                     panic!("spf_b200: could not spawn a validated graph: {e}");
                 }
                 Some(g)

@@ -456,6 +456,39 @@ EXCHANGE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, 
 _RESTYPES.update({"spf_b200_graph_destroy": None, "spf_b200_graph_launches": C.c_uint64, "spf_b200_graph_arena": _vp,
                   "spf_b200_graph_status_message": C.c_char_p})
 
+# one process, every GPU of a box (spf_b200_box_*)
+ABI.update({
+    "spf_b200_box_create": [C.POINTER(Params), _vp, _sz, _vp, _sz, _vp, _sz, _vp, _sz, C.POINTER(C.c_int), C.c_int,
+                            C.POINTER(_vp)],
+    "spf_b200_box_create_from_serialized": [C.POINTER(Params), _vp, _sz, C.POINTER(C.c_int), C.c_int, C.POINTER(_vp)],
+    "spf_b200_box_destroy": [_vp],
+    "spf_b200_box_last_error": [_vp],
+    "spf_b200_box_size": [_vp],
+    "spf_b200_box_device": [_vp, C.c_int],
+    "spf_b200_box_context": [_vp, C.c_int],
+    "spf_b200_box_key_replication_ms": [_vp],
+    "spf_b200_box_key_slice": [_vp, C.c_int, C.c_int, _sz, _sz, _vp],
+    "spf_b200_box_shard": [_sz, C.c_int, C.c_int, C.POINTER(_sz), C.POINTER(_sz)],
+    "spf_b200_box_circuit_bootstrap": [_vp, _vp, _vp, _sz],
+    "spf_b200_box_programmable_bootstrap": [_vp, _vp, _vp, _vp, C.c_uint32, C.c_uint32, _sz],
+    "spf_b200_box_keyswitch_lwe_l1_lwe_l0": [_vp, _vp, _vp, _sz],
+    "spf_b200_box_cmux": [_vp, _vp, _vp, _vp, _vp, _sz],
+    "spf_b200_box_graph_build": [_vp, C.POINTER(_Node), _sz, C.POINTER(_vp)],
+    "spf_b200_box_graph_run": [_vp],
+    "spf_b200_box_graph_spawn": [_vp, C.POINTER(_vp), _sz, _vp, _vp],
+    "spf_b200_box_graph_wait": [_vp],
+    "spf_b200_box_graph_status_message": [_vp],
+    "spf_b200_box_graph_set_io": [_vp, _sz, _vp],
+    "spf_b200_box_graph_destroy": [_vp],
+    "spf_b200_box_graph_levels": [_vp],
+    "spf_b200_box_graph_launches": [_vp],
+    "spf_b200_box_set_max_in_flight": [_vp, C.c_int],
+})
+_RESTYPES.update({"spf_b200_box_destroy": None, "spf_b200_box_last_error": C.c_char_p, "spf_b200_box_context": _vp,
+                  "spf_b200_box_key_replication_ms": C.c_double, "spf_b200_box_shard": None,
+                  "spf_b200_box_graph_status_message": C.c_char_p, "spf_b200_box_graph_destroy": None,
+                  "spf_b200_box_graph_launches": C.c_uint64})
+
 
 class DeviceCiphertext:
     """A ciphertext HANDLE: `nbytes` of device memory holding one ciphertext that never leaves HBM (the role of the
@@ -653,12 +686,17 @@ def plan_graph(circuit: "FheCircuit", world: int = 1, params: Params | None = No
 
 class CircuitProcessor:
     """CircuitProcessor (parasol_runtime/src/circuit_processor/mod.rs:62-655) on the GPU: a graph is
-    compiled once into per-level batched launches and can be run repeatedly."""
+    compiled once into per-level batched launches and can be run repeatedly.  On a BoxEvaluation every graph runs
+    over all GPUs of the box (BoxGraph) from the calling thread."""
 
-    def __init__(self, evaluation: Evaluation):
+    def __init__(self, evaluation: "Evaluation | BoxEvaluation"):
         self.ev = evaluation
 
-    def compile(self, circuit: FheCircuit, world: int = 1, rank: int = 0, exchange=None) -> "CompiledGraph":
+    def compile(self, circuit: FheCircuit, world: int = 1, rank: int = 0, exchange=None) -> "CompiledGraph | BoxGraph":
+        if isinstance(self.ev, BoxEvaluation):
+            if world != 1 or rank != 0 or exchange is not None:
+                raise SpfError(-1, "a box graph is sharded over the box's ranks: world / rank / exchange do not apply")
+            return BoxGraph(self.ev, circuit)
         return CompiledGraph(self.ev, circuit, world=world, rank=rank, exchange=exchange)
 
     def run_graph_blocking(self, circuit: FheCircuit) -> None:
@@ -810,6 +848,225 @@ class CompiledGraph:
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
             lib().spf_b200_graph_destroy(self._h)
+            self._h = _vp()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+# ---------------------------------------------------------------------------------------------
+# One process, every GPU of a box: BoxEvaluation + BoxGraph (spf_b200_box_*)
+# ---------------------------------------------------------------------------------------------
+def box_shard(batch: int, n: int, rank: int) -> tuple[int, int]:
+    """(start, count) of rank `rank`'s slice of a batch in the box ops (spf_b200_box_shard; multi.shard's rule)."""
+    start, count = _sz(), _sz()
+    lib().spf_b200_box_shard(int(batch), int(n), int(rank), C.byref(start), C.byref(count))
+    return int(start.value), int(count.value)
+
+
+class BoxEvaluation:
+    """`Evaluation` over several GPUs of one box, from one thread: rank r is a context on devices[r] (a device may
+    repeat).  The compute key is uploaded once and replicated device to device.  The batched ops split the batch
+    contiguously over the ranks (box_shard) and run every rank at once; CircuitProcessor(box) runs graphs over all
+    ranks.  Single-device work goes through the rank contexts (`contexts`)."""
+
+    _in = staticmethod(Evaluation._in)
+
+    def __init__(self, bsk_fft, ksk, ssk_fft, ak_fft, devices=(0,), params: Params | None = None):
+        l = lib()
+        self.params = params if params is not None else default_128()
+        p = self.params
+        self._h = _vp()
+        lens = (l.spf_b200_len_bsk(C.byref(p)), l.spf_b200_len_ksk(C.byref(p)), l.spf_b200_len_ssk(C.byref(p)),
+                l.spf_b200_len_ak(C.byref(p)))
+        arrs = []
+        for a, dt, n, name in ((bsk_fft, np.complex128, lens[0], "bs_key"), (ksk, np.uint64, lens[1], "ks_key"),
+                               (ssk_fft, np.complex128, lens[2], "ss_key"), (ak_fft, np.complex128, lens[3], "auto_key")):
+            a = np.ascontiguousarray(a, dtype=dt).reshape(-1)
+            if a.size != n:
+                raise SpfError(-1, f"{name} has {a.size} elements, params require {n}")
+            arrs.append(a)
+        devs = self._devices(devices)
+        self._check_create(l.spf_b200_box_create(C.byref(p), arrs[0].ctypes.data, lens[0], arrs[1].ctypes.data, lens[1],
+                                                 arrs[2].ctypes.data, lens[2], arrs[3].ctypes.data, lens[3], devs,
+                                                 len(devs), C.byref(self._h)))
+        self._init_lengths()
+
+    @staticmethod
+    def _devices(devices):
+        devices = [int(d) for d in devices]
+        return (C.c_int * max(len(devices), 1))(*devices)
+
+    def _check_create(self, rc):
+        if rc != 0:
+            raise SpfError(rc, (lib().spf_b200_box_last_error(None) or b"").decode())
+
+    def _init_lengths(self):
+        l, p = lib(), self.params
+        self.len_lwe_l0 = l.spf_b200_len_lwe_l0(C.byref(p))
+        self.len_lwe_l1 = l.spf_b200_len_lwe_l1(C.byref(p))
+        self.len_glwe = l.spf_b200_len_glwe_l1(C.byref(p))
+        self.len_glev = l.spf_b200_len_glev_l1(C.byref(p))
+        self.len_ggsw = l.spf_b200_len_ggsw_l1(C.byref(p))
+
+    @classmethod
+    def from_serialized(cls, data: bytes, params: Params | None = None, devices=(0,)) -> "BoxEvaluation":
+        """safe_bincode::deserialize::<ComputeKey> + a box over `devices` (spf_b200_box_create_from_serialized)."""
+        self = cls.__new__(cls)
+        self.params = params if params is not None else default_128()
+        self._h = _vp()
+        buf = np.frombuffer(bytes(data), dtype=np.uint8)
+        devs = cls._devices(devices)
+        self._check_create(lib().spf_b200_box_create_from_serialized(C.byref(self.params), buf.ctypes.data, buf.size, devs,
+                                                                     len(devs), C.byref(self._h)))
+        self._init_lengths()
+        return self
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            lib().spf_b200_box_destroy(self._h)
+            self._h = _vp()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _check(self, rc: int):
+        if rc != 0:
+            raise SpfError(rc, (lib().spf_b200_box_last_error(self._h) or b"").decode())
+
+    @property
+    def handle(self):
+        return self._h
+
+    @property
+    def size(self) -> int:
+        return int(lib().spf_b200_box_size(self._h))
+
+    @property
+    def devices(self) -> list[int]:
+        return [int(lib().spf_b200_box_device(self._h, r)) for r in range(self.size)]
+
+    @property
+    def contexts(self) -> list[int]:
+        """spf_b200_ctx* of every rank (owned by the box), for the dev_* entry points of that rank's device."""
+        return [int(lib().spf_b200_box_context(self._h, r) or 0) for r in range(self.size)]
+
+    @property
+    def key_replication_ms(self) -> float:
+        return float(lib().spf_b200_box_key_replication_ms(self._h))
+
+    @property
+    def kernel_launches(self) -> int:
+        return sum(int(lib().spf_b200_kernel_launches(c)) for c in self.contexts)
+
+    def key_slice(self, rank: int, which: int, offset: int, count: int) -> np.ndarray:
+        """Elements [offset, offset + count) of key array `which` (0 bs_key, 1 ks_key, 2 ss_key, 3 auto_key) as resident
+        on rank `rank`'s device, in the reference layout and scale."""
+        out = np.empty(int(count), dtype=np.uint64 if which == 1 else np.complex128)
+        self._check(lib().spf_b200_box_key_slice(self._h, int(rank), int(which), int(offset), int(count), out.ctypes.data))
+        return out
+
+    def synchronize(self):
+        for c in self.contexts:
+            rc = lib().spf_b200_synchronize(c)
+            if rc:
+                raise SpfError(rc, (lib().spf_b200_last_error(c) or b"").decode())
+
+    def set_max_in_flight(self, n: int) -> None:
+        """Flow control of spawned box graphs: at most n runs per box between dispatch and completion."""
+        self._check(lib().spf_b200_box_set_max_in_flight(self._h, int(n)))
+
+    def circuit_bootstrap(self, lwe0) -> np.ndarray:
+        x = self._in(lwe0, np.uint64, self.len_lwe_l0, "lwe0")
+        out = np.empty((x.shape[0], self.len_ggsw), dtype=np.complex128)
+        self._check(lib().spf_b200_box_circuit_bootstrap(self._h, out.ctypes.data, x.ctypes.data, x.shape[0]))
+        return out
+
+    def programmable_bootstrap(self, lwe0, lut_glwe, log_chi: int = 0, log_v: int = 0) -> np.ndarray:
+        x = self._in(lwe0, np.uint64, self.len_lwe_l0, "lwe0")
+        lut = self._in(lut_glwe, np.uint64, self.len_glwe, "lut")
+        out = np.empty((x.shape[0], self.len_glwe), dtype=np.uint64)
+        self._check(lib().spf_b200_box_programmable_bootstrap(self._h, out.ctypes.data, x.ctypes.data, lut.ctypes.data,
+                                                              log_chi, log_v, x.shape[0]))
+        return out
+
+    def keyswitch_lwe_l1_lwe_l0(self, lwe1) -> np.ndarray:
+        x = self._in(lwe1, np.uint64, self.len_lwe_l1, "lwe1")
+        out = np.empty((x.shape[0], self.len_lwe_l0), dtype=np.uint64)
+        self._check(lib().spf_b200_box_keyswitch_lwe_l1_lwe_l0(self._h, out.ctypes.data, x.ctypes.data, x.shape[0]))
+        return out
+
+    def cmux(self, sel, a, b) -> np.ndarray:
+        s = self._in(sel, np.complex128, self.len_ggsw, "sel")
+        a = self._in(a, np.uint64, self.len_glwe, "a")
+        b = self._in(b, np.uint64, self.len_glwe, "b")
+        if not (s.shape[0] == a.shape[0] == b.shape[0]):
+            raise SpfError(-1, "cmux: batch sizes differ")
+        out = np.empty_like(a)
+        self._check(lib().spf_b200_box_cmux(self._h, out.ctypes.data, s.ctypes.data, a.ctypes.data, b.ctypes.data, a.shape[0]))
+        return out
+
+
+
+class BoxGraph:
+    """A graph over every rank of a BoxEvaluation (spf_b200_box_graph_*), with the CompiledGraph surface: run, spawn,
+    wait, set_io, levels, launches, close.  io buffers are host numpy arrays (DeviceCiphertext handles are refused)."""
+
+    def __init__(self, box: BoxEvaluation, circuit: FheCircuit):
+        self.ev = box
+        self._keep = circuit
+        self._h = _vp()
+        box._check(lib().spf_b200_box_graph_build(box.handle, circuit._pack(), len(circuit.nodes), C.byref(self._h)))
+
+    def run(self) -> None:
+        self.ev._check(lib().spf_b200_box_graph_run(self._h))
+
+    def set_io(self, node: int, buf) -> None:
+        if not 0 <= node < len(self._keep):
+            raise SpfError(-1, f"set_io: node {node} out of range")
+        self._keep._check_io(int(self._keep.ops[node]), buf)
+        self.ev._check(lib().spf_b200_box_graph_set_io(self._h, node, _io_ptr(buf)))
+        self._bound = getattr(self, "_bound", {})
+        self._bound[node] = buf
+
+    def spawn(self, after=(), on_complete=None) -> None:
+        """One asynchronous run over all ranks; on_complete(error) fires once, after every rank has retired, from a CUDA
+        callback thread (it must not call into spf_b200 or CUDA).  `after`: BoxGraphs of the same box."""
+        deps = [d for d in after if d is not None]
+        arr = (_vp * max(len(deps), 1))(*[d._h for d in deps])
+
+        def _done(user, status, message):
+            try:
+                if on_complete is not None:
+                    on_complete(None if status == 0 else SpfError(int(status), (message or b"").decode()))
+            except Exception:  # never let an exception cross the C ABI
+                pass
+
+        self._spawn_cb = COMPLETION_FN(_done)
+        self.ev._check(lib().spf_b200_box_graph_spawn(self._h, arr, len(deps), C.cast(self._spawn_cb, _vp), None))
+
+    def wait(self) -> None:
+        rc = lib().spf_b200_box_graph_wait(self._h)
+        if rc:
+            raise SpfError(int(rc), (lib().spf_b200_box_graph_status_message(self._h) or b"").decode() or "the graph's last run failed")
+
+    @property
+    def levels(self) -> int:
+        return int(lib().spf_b200_box_graph_levels(self._h))
+
+    @property
+    def launches(self) -> int:
+        return int(lib().spf_b200_box_graph_launches(self._h))
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            lib().spf_b200_box_graph_destroy(self._h)
             self._h = _vp()
 
     def __del__(self):

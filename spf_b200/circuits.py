@@ -164,9 +164,10 @@ class InstructionCache:
     FheCircuit::insert_mux_circuit_and_connect_inputs (fhe_circuit.rs:473-494) does."""
 
     def __init__(self, evaluation):
-        from . import CompiledGraph
+        from . import BoxEvaluation, BoxGraph, CompiledGraph
 
-        self._ev, self._compile, self._cache = evaluation, CompiledGraph, {}
+        self._compile = BoxGraph if isinstance(evaluation, BoxEvaluation) else CompiledGraph
+        self._ev, self._cache = evaluation, {}
         self.hits = self.misses = 0
 
     def _run(self, key, build, in_bufs, out_bufs):

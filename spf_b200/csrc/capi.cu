@@ -1020,3 +1020,4 @@ int spf_b200_fp64_peak(spf_b200_ctx* ctx, double* tflops_out) {
 
 #include "graph.cuh"
 #include "serial.inl"
+#include "box.cuh"

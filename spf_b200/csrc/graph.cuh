@@ -141,6 +141,9 @@ struct spf_b200_graph {
   ChainStage* d_chain = nullptr;
   unsigned long long* d_chain_bar = nullptr;
   bool poisoned = false;  // a failed peer-mode run leaves the ranks' barrier epochs out of step: rebuild the graphs
+  // rank that writes the Output* nodes every rank holds (output rank -1); -1 = every rank writes them (one process per
+  // rank: each has its own host buffers).  A box (box.cuh) runs all ranks into the same host buffers: rank 0 only.
+  int replicated_writer = -1;
 };
 
 // one spawned run between dispatch and completion
@@ -202,7 +205,7 @@ int graph_fail(spf_b200_ctx* ctx, const std::string& msg) { return fail(ctx, SPF
 // allocation known to the driver (pageable memory, a range registered piecemeal).  Copies are only ever merged between
 // buffers of the same allocation: a cudaMemcpyAsync that runs over the end of an allocation or registration is refused
 // by the driver, and two numpy rows or two 32 KiB cudaMallocs are routinely adjacent.
-unsigned long long alloc_base_of(const void* p) {
+unsigned long long alloc_base_of(const void* p, size_t* size_out = nullptr) {
   typedef int (*range_fn)(unsigned long long*, size_t*, unsigned long long);
   static range_fn fn = [] {
     void* f = nullptr;
@@ -215,6 +218,7 @@ unsigned long long alloc_base_of(const void* p) {
   unsigned long long base = 0;
   size_t size = 0;
   if (fn(&base, &size, (unsigned long long)(uintptr_t)p) != 0) return 0;
+  if (size_out) *size_out = size;
   return base;
 }
 
@@ -839,13 +843,18 @@ int launch_chain(spf_b200_graph* g, const spf_b200_graph::Chain& c, cudaStream_t
   return check_launch(ctx, "cmux_chain_kernel");
 }
 
-// Everything of one run that is ENQUEUED on stream s: input copies, all levels, exchanges, output copies.  Returns the
-// first error (message in ctx->err); work already enqueued keeps running -- the caller drains the stream.
-int enqueue_run(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange, void* user, cudaStream_t s,
-                std::vector<cudaEvent_t>* timing_events) {
+// Whether `rank` writes Output* node `id` into its io buffer: outputs of a MUX tree live on the tree's owner.
+bool writes_output(const spf_b200_graph* g, size_t id, int rank) {
+  const int r = spf_b200_graph_output_rank(g, id);
+  return r == rank || (r < 0 && (g->replicated_writer < 0 || g->replicated_writer == rank));
+}
+
+// The parts of one run that are ENQUEUED on stream s (enqueue_run: inputs, every group in order, outputs).  Each
+// returns the first error (message in ctx->err); work already enqueued keeps running -- the caller drains the stream.
+// Input copies (and, in peer mode, the start-of-run barrier).
+int enqueue_inputs(spf_b200_graph* g, bool peer_mode, cudaStream_t s) {
   spf_b200_ctx* ctx = g->ctx;
   const spf_params* p = &ctx->p;
-  const bool peer_mode = world > 1 && !exchange;
   // every rank has finished its previous run before anyone stores into its arena again
   if (peer_mode) if (int rc = peer_barrier(g, s)) return rc;
   // inputs whose host buffers AND device buffers are consecutive (rows of one host slab, in node order) go up as one copy
@@ -877,6 +886,40 @@ int enqueue_run(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange
                                 spf_b200_len_ggsw_l1(p), 1.0 / 1024.0, s))
         return rc;
   }
+  return 0;
+}
+
+// One group of this rank, then its exchange (circuit-bootstrap outputs (GGSW) and keyswitch outputs (L0 LWE)).
+int enqueue_group(spf_b200_graph* g, const Group& G, int rank, int world, spf_exchange_fn exchange, void* user, cudaStream_t s,
+                  cudaEvent_t after_group) {
+  spf_b200_ctx* ctx = g->ctx;
+  const bool peer_mode = world > 1 && !exchange;
+  // peer mode: the scheme-switch kernel stores its GGSWs into every rank's arena while it computes them
+  if (int rc = run_group(g, G, s, rank, peer_mode && G.op == SPF_OP_CIRCUIT_BOOTSTRAP ? &g->peers : nullptr)) return rc;
+  if (after_group) cudaEventRecord(after_group, s);
+  if (world > 1 && G.gather_chunk > 0) {
+    const size_t item_bytes = ct_bytes(&ctx->p, op_info(G.op).out);
+    if (!peer_mode) {
+      if (int rc = exchange(user, G.out_base, G.gather_chunk * item_bytes, world, s))
+        return fail(ctx, SPF_E_GRAPH, "exchange callback failed with status " + std::to_string(rc));
+    } else {
+      if (G.op == SPF_OP_KEYSWITCH_L1_TO_L0 && G.r_cnt[rank] > 0) {
+        const size_t n16 = G.r_cnt[rank] * item_bytes / 16;
+        peer_bcast_kernel<<<(unsigned)std::min<size_t>((n16 + 255) / 256, 4 * (size_t)ctx->sm_count), 256, 0, s>>>(
+            reinterpret_cast<const uint4*>(G.out_base + G.r_start[rank] * item_bytes), n16, g->peers);
+        if (int rc = check_launch(ctx, "peer_bcast_kernel")) return rc;
+      }
+      if (int rc = peer_barrier(g, s)) return rc;
+    }
+  }
+  return 0;
+}
+
+int enqueue_outputs(spf_b200_graph* g, int rank, cudaStream_t s);
+
+int enqueue_run(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange, void* user, cudaStream_t s,
+                std::vector<cudaEvent_t>* timing_events) {
+  if (int rc = enqueue_inputs(g, world > 1 && !exchange, s)) return rc;
   if (timing_events) cudaEventRecord((*timing_events)[0], s);
   // SPF_B200_CHAIN=1: runs of narrow CMux levels as one cooperative launch each (cmux_chain_kernel; measured slower than
   // programmatic dependent launches, so opt-in)
@@ -894,25 +937,15 @@ int enqueue_run(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange
       gidx = c.last;  // the groups in between launch nothing or were part of the run
       continue;
     }
-    // peer mode: the scheme-switch kernel stores its GGSWs into every rank's arena while it computes them
-    if (int rc = run_group(g, G, s, rank, peer_mode && G.op == SPF_OP_CIRCUIT_BOOTSTRAP ? &g->peers : nullptr)) return rc;
-    if (timing_events) cudaEventRecord((*timing_events)[++gi], s);
-    if (world > 1 && G.gather_chunk > 0) {  // circuit-bootstrap outputs (GGSW) and keyswitch outputs (L0 LWE)
-      const size_t item_bytes = ct_bytes(p, op_info(G.op).out);
-      if (!peer_mode) {
-        if (int rc = exchange(user, G.out_base, G.gather_chunk * item_bytes, world, s))
-          return fail(ctx, SPF_E_GRAPH, "exchange callback failed with status " + std::to_string(rc));
-      } else {
-        if (G.op == SPF_OP_KEYSWITCH_L1_TO_L0 && G.r_cnt[rank] > 0) {
-          const size_t n16 = G.r_cnt[rank] * item_bytes / 16;
-          peer_bcast_kernel<<<(unsigned)std::min<size_t>((n16 + 255) / 256, 4 * (size_t)ctx->sm_count), 256, 0, s>>>(
-              reinterpret_cast<const uint4*>(G.out_base + G.r_start[rank] * item_bytes), n16, g->peers);
-          if (int rc = check_launch(ctx, "peer_bcast_kernel")) return rc;
-        }
-        if (int rc = peer_barrier(g, s)) return rc;
-      }
-    }
+    if (int rc = enqueue_group(g, G, rank, world, exchange, user, s, timing_events ? (*timing_events)[++gi] : nullptr)) return rc;
   }
+  return enqueue_outputs(g, rank, s);
+}
+
+// Gathered and GGSW output copies of this rank.
+int enqueue_outputs(spf_b200_graph* g, int rank, cudaStream_t s) {
+  spf_b200_ctx* ctx = g->ctx;
+  const spf_params* p = &ctx->p;
   if (g->gather_items) {
     const size_t n_it = g->gather_items;
     const char* t = static_cast<const char*>(g->d_gather_tab);
@@ -922,10 +955,7 @@ int enqueue_run(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange
         reinterpret_cast<const unsigned*>(t + n_it * (sizeof(void*) + sizeof(unsigned long long))));
     if (int rc = check_launch(ctx, "gather_outputs_kernel")) return rc;
   }
-  auto mine = [&](size_t k) {  // outputs of a MUX tree live on the tree's owner
-    const int r = spf_b200_graph_output_rank(g, (size_t)g->outputs[k]);
-    return r < 0 || r == rank;
-  };
+  auto mine = [&](size_t k) { return writes_output(g, (size_t)g->outputs[k], rank); };
   size_t stage = 0;
   for (size_t k = 0; k < g->outputs.size();) {
     const int id = g->outputs[k];
@@ -972,8 +1002,7 @@ void copy_out_staged(spf_b200_graph* g, int rank) {
   for (size_t k = 0; k < g->outputs.size(); k++) {
     const int id = g->outputs[k];
     if (g->io_kind[id] != 1 || g->stage_off[id] == (size_t)-1) continue;
-    const int r = spf_b200_graph_output_rank(g, (size_t)id);
-    if (!(r < 0 || r == rank)) continue;
+    if (!writes_output(g, (size_t)id, rank)) continue;
     memcpy(g->nodes[id].io, g->h_stage + g->stage_off[id], ct_host_bytes(p, g->type[g->nodes[id].in[0]]));
   }
 }

@@ -1,0 +1,205 @@
+"""One process over the GPUs of a box (spf_b200.BoxEvaluation): key replication, device-resident and end-to-end circuit
+bootstrapping, and N x (mul32 then greater-than) in one box graph, blocking and spawned.  Prints one JSON line and
+records it under profiles/ (--out).  The same measurements as bench.py's multi-process line, so the two compare.
+
+usage: python tools/box_bench.py [--devices 0,1,...] [--batch 4096] [--steps 10] [--out profiles/box_bench_n8.json]"""
+import argparse
+import ctypes as C
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def gpu_identity(devices):
+    """Name and power limit of every GPU of the box, read by the same process that measures."""
+    q = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit", "--format=csv,noheader"], capture_output=True,
+                       text=True, timeout=60)
+    rows = {}
+    for line in q.stdout.strip().splitlines():
+        idx, name, limit = [x.strip() for x in line.split(",")]
+        rows[int(idx)] = {"name": name, "power_limit": limit}
+    return [rows.get(d, {"name": None, "power_limit": None}) for d in sorted(set(devices))]
+
+
+def encrypt_lwe0(sk, bits, std, seed):
+    """b = <a,s> + m + e, vectorised (client-side input generation only)."""
+    rng = np.random.default_rng(seed)
+    a = rng.integers(0, 1 << 64, (len(bits), sk.shape[0]), dtype=np.uint64)
+    e = np.round(rng.normal(0.0, std, len(bits)) * 2.0 ** 64).astype(np.int64).astype(np.uint64)
+    b = (a * sk[None, :]).sum(axis=1, dtype=np.uint64) + (bits.astype(np.uint64) << np.uint64(63)) + e
+    return np.ascontiguousarray(np.concatenate([a, b[:, None]], axis=1))
+
+
+def device_resident(box, cts, batch, steps, warmup):
+    """batch CBS per rank per step from device memory through each rank's context, every rank enqueued from this
+    thread; CUDA events per device; a step's time is the slowest rank's."""
+    import torch
+
+    import spf_b200
+
+    l = spf_b200.lib()
+    ranks = []
+    for r, (dev, ctx) in enumerate(zip(box.devices, box.contexts)):
+        d = torch.device("cuda", dev)
+        with torch.cuda.device(d):
+            s = torch.cuda.Stream(device=d)
+            d_in = torch.from_numpy(cts[r * batch:(r + 1) * batch].view(np.int64)).to(d)
+            d_out = torch.empty(batch * box.len_ggsw * 2, dtype=torch.float64, device=d)
+            flush = torch.empty(256 << 20, dtype=torch.uint8, device=d)
+        ranks.append((d, ctx, s, d_in, d_out, flush))
+
+    def step(events=None):
+        for r, (d, ctx, s, d_in, d_out, flush) in enumerate(ranks):
+            with torch.cuda.device(d), torch.cuda.stream(s):
+                flush.zero_()
+                if events:
+                    events[r][0].record(s)
+                rc = l.spf_b200_dev_circuit_bootstrap(ctx, d_out.data_ptr(), d_in.data_ptr(), batch, 0, s.cuda_stream)
+                if rc:
+                    raise spf_b200.SpfError(rc, (l.spf_b200_last_error(ctx) or b"").decode())
+                if events:
+                    events[r][1].record(s)
+
+    for _ in range(max(warmup, 2)):
+        step()
+    for d, *_ in ranks:
+        torch.cuda.synchronize(d)
+    per_step = []
+    for _ in range(steps):
+        ev = []
+        for d, *_ in ranks:
+            with torch.cuda.device(d):
+                ev.append((torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)))
+        step(ev)
+        for d, *_ in ranks:
+            torch.cuda.synchronize(d)
+        per_step.append(max(a.elapsed_time(b) for a, b in ev))
+    ms = float(np.median(per_step))
+    return {"ms_per_step": ms, "cbs_per_s": len(ranks) * batch / (ms * 1e-3)}
+
+
+def end_to_end(box, cts, steps, warmup):
+    """spf_b200_box_circuit_bootstrap from and to page-locked host buffers: host wall clock per call."""
+    import spf_b200
+
+    h_in = spf_b200.pinned_zeros(cts.shape)
+    h_in[:] = cts
+    h_out = spf_b200.pinned_zeros((cts.shape[0], box.len_ggsw), dtype=np.complex128)
+    l = spf_b200.lib()
+
+    def call():
+        box._check(l.spf_b200_box_circuit_bootstrap(box.handle, h_out.ctypes.data, h_in.ctypes.data, cts.shape[0]))
+
+    for _ in range(max(warmup, 1)):
+        call()
+    ts = []
+    for _ in range(steps):
+        t0 = time.perf_counter()
+        call()
+        ts.append(time.perf_counter() - t0)
+    s = float(np.median(ts))
+    return {"ms_per_call": 1e3 * s, "cbs_per_s": cts.shape[0] / s}, h_out
+
+
+def programs(box, keys, n_programs, reps):
+    """n_programs x (32-bit multiply, low word, then greater-than) in ONE box graph."""
+    import oracle as O
+    import spf_b200
+    from spf_b200.circuits import multiply_then_greater_than
+
+    client = O.Client(keys)
+    w = 32
+    rng = np.random.default_rng(0xB0C5)
+    vals = [tuple(int(x) for x in rng.integers(0, 1 << w, 3)) for _ in range(n_programs)]
+    slab = iter(spf_b200.pinned_zeros((n_programs * (3 * w + w + 1), keys.glwe_len)))
+
+    def enc(v):
+        out = [next(slab) for _ in range(w)]
+        for i, r in enumerate(out):
+            r[:] = client.encrypt_glwe_l1([(v >> i) & 1])
+        return out
+
+    a, b, c = ([enc(v[k]) for v in vals] for k in range(3))
+    out_prod = [[next(slab) for _ in range(w)] for _ in vals]
+    out_gt = [next(slab) for _ in vals]
+    circ = multiply_then_greater_than(a, b, c, out_prod, out_gt, n_programs)
+    g = spf_b200.CircuitProcessor(box).compile(circ)
+    g.run()
+
+    def correct():
+        ok = True
+        for (x, y, z), pb, gt in zip(vals, out_prod, out_gt):
+            p = sum(int(client.decrypt_glwe_l1(o)[0]) << i for i, o in enumerate(pb))
+            ok &= p == (x * y) % (1 << w) and int(client.decrypt_glwe_l1(gt)[0]) == int(p > z)
+        return bool(ok)
+
+    blocking = []
+    for _ in range(reps):
+        t0 = time.perf_counter()
+        g.run()
+        blocking.append(time.perf_counter() - t0)
+    ok_blocking = correct()
+    spawned = []
+    for _ in range(reps):
+        t0 = time.perf_counter()
+        g.spawn()
+        g.wait()
+        spawned.append(time.perf_counter() - t0)
+    res = {"programs": n_programs, "levels": g.levels, "launches": g.launches, "blocking_ms": 1e3 * float(np.median(blocking)),
+           "spawned_ms": 1e3 * float(np.median(spawned)), "correct": ok_blocking and correct()}
+    g.close()
+    return res
+
+
+def main():
+    ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
+    ap.add_argument("--devices", default=None, help="comma-separated device list (default: every visible GPU)")
+    ap.add_argument("--batch", type=int, default=4096, help="CBS per GPU per step")
+    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--reps", type=int, default=5, help="runs of the program graph per mode")
+    ap.add_argument("--out", default=None, help="also write the JSON line to this file")
+    args = ap.parse_args()
+
+    import torch
+
+    import oracle as O
+    import spf_b200
+
+    if not torch.cuda.is_available():
+        raise SystemExit("box_bench.py: no CUDA device; spf_b200 has no CPU fallback")
+    devices = [int(x) for x in args.devices.split(",")] if args.devices else list(range(torch.cuda.device_count()))
+    line = {"metric": "box_bench", "devices": devices, "gpus": gpu_identity(devices)}
+    keys = O.Keys()
+    t0 = time.perf_counter()
+    box = spf_b200.BoxEvaluation(keys.bsk_fft, keys.ksk, keys.ssk_fft, keys.ak_fft, devices=devices)
+    line["box_create_ms"] = 1e3 * (time.perf_counter() - t0)
+    line["key_replication_ms"] = box.key_replication_ms
+    n = box.size
+    p = keys.params
+    bits = np.random.default_rng(0xB0C4).integers(0, 2, n * args.batch)
+    cts = encrypt_lwe0(keys.lwe0_sk.astype(np.uint64), bits, p.lwe_std, 0xB0C4)
+    line["device_resident"] = {"batch_per_gpu": args.batch, **device_resident(box, cts, args.batch, args.steps, args.warmup)}
+    e2e, h_out = end_to_end(box, cts, args.steps, args.warmup)
+    client = O.Client(keys)
+    idx = np.linspace(0, len(bits) - 1, 16).astype(int)
+    e2e["correct"] = bool(all(client.decrypt_ggsw_l1(h_out[i]) == int(bits[i]) for i in idx))
+    line["end_to_end"] = {"batch_per_gpu": args.batch, **e2e}
+    line["mul32_then_gt"] = programs(box, keys, n, args.reps)
+    box.close()
+    text = json.dumps(line)
+    print(text)
+    if args.out:
+        with open(args.out, "w") as f:
+            f.write(text + "\n")
+
+
+if __name__ == "__main__":
+    main()
