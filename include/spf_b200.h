@@ -343,8 +343,13 @@ int spf_b200_box_cmux(spf_b200_box *box, uint64_t *glwe_out, const double *sel_g
  * barriers between levels).  Every rank's run is enqueued from the calling thread, level-interleaved across the ranks;
  * everything that could make the host wait on a device is done before the first enqueue, so no rank waits at a barrier
  * for a rank that has not been enqueued.
- * Output* nodes are written by their owner rank (spf_b200_graph_output_rank; rank 0 for nodes every rank holds) into
- * the caller's host buffers.  io buffers are host memory only: device-memory handles are refused with SPF_E_INVALID.
+ * io buffers are host memory or BOX CIPHERTEXT HANDLES (below); one graph may mix both.  Raw device pointers are
+ * refused with SPF_E_INVALID (a box needs one copy per rank, and which rank computes an output is known only after
+ * sharding).  Output* nodes with a host buffer are written by their owner rank (spf_b200_graph_output_rank; rank 0 for
+ * nodes every rank holds).  A handle-bound Output* node is written into every rank's replica: by each rank itself when
+ * every rank holds the ciphertext, by the owner over NVLink when one rank computes it (after a barrier that every rank
+ * reaches once it has read its handle inputs).  A handle-bound Input* node is read by each rank from its own replica.
+ * All handle copies of a rank go through one table-driven copy kernel for the inputs and one for the outputs.
  * Spawn semantics are those of spf_b200_graph_spawn: on_complete fires exactly once per run, after every rank has
  * retired, with the first error of any rank; `after` orders on the device (every rank behind every rank of the
  * dependency); a run whose dependency failed
@@ -362,6 +367,25 @@ void spf_b200_box_graph_destroy(spf_b200_box_graph *graph);
 int spf_b200_box_graph_levels(const spf_b200_box_graph *graph);
 uint64_t spf_b200_box_graph_launches(const spf_b200_box_graph *graph); /* kernel launches of the last run, all ranks */
 int spf_b200_box_set_max_in_flight(spf_b200_box *box, int n);
+
+/* Box ciphertext handles: one ciphertext kept in HBM between box graphs -- the box's DeviceCiphertext.  A handle holds
+ * one replica per rank, on that rank's device (a device that appears twice in the box gets two).  Pass the handle
+ * pointer itself as spf_node.io or to spf_b200_box_graph_set_io: graph k's Output* node and graph k + 1's Input* node
+ * name the same handle, nothing crosses PCIe, and `after` orders the two graphs on the devices.  Errors
+ * (SPF_E_INVALID): a handle of another box, a handle whose kind is not the node's ciphertext type, a handle on a node
+ * that is not Input* / Output*; single-context graphs (spf_b200_graph_build*, spf_b200_graph_set_io) refuse handles.
+ * `kind` is the Input* op code of the ciphertext type (SPF_OP_INPUT_LWE0 .. SPF_OP_INPUT_GLEV1).  alloc zero-fills.
+ * GGSWs stay in the device scale (x 2^-10) in every replica: write takes and read returns the reference scale.
+ * Handles are reference-counted: a box graph holds a reference for every node bound to the handle (dropped on rebind
+ * and destroy), free drops the caller's; the memory goes with the last reference.  A handle keeps its box alive.
+ * write and read are synchronous; order them against spawned runs with spf_b200_box_graph_wait. */
+typedef struct spf_b200_box_ciphertext spf_b200_box_ciphertext;
+int spf_b200_box_ciphertext_alloc(spf_b200_box *box, uint32_t kind, spf_b200_box_ciphertext **out);
+void spf_b200_box_ciphertext_free(spf_b200_box_ciphertext *h);
+/* host -> every replica */
+int spf_b200_box_ciphertext_write(spf_b200_box_ciphertext *h, const void *host_src);
+/* rank `rank`'s replica -> host */
+int spf_b200_box_ciphertext_read(spf_b200_box_ciphertext *h, int rank, void *host_dst);
 
 /* ---- serialized keys and ciphertexts (SURVEY.md 8(f).1) ------------------------------------------
  * The reference serialises with bincode 1.3.3 (Cargo.lock:244-245), fixed-width little-endian

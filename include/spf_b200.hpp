@@ -304,7 +304,30 @@ class BoxEvaluation {
   spf_b200_box* box_ = nullptr;
 };
 
-// A levelised graph over every rank of a box; host io buffers only.
+// A box ciphertext handle (spf_b200_box_ciphertext_*): one ciphertext in HBM, one replica per rank.  Bind handle()
+// as the io of box graph Input* / Output* nodes; box graphs hold their own references, so the handle may go out of
+// scope while a graph still binds it.  kind: SPF_OP_INPUT_LWE0 .. SPF_OP_INPUT_GLEV1.
+class BoxCiphertext {
+ public:
+  BoxCiphertext(const BoxEvaluation& ev, spf_op kind) : box_(ev.handle()) {
+    check_box(spf_b200_box_ciphertext_alloc(box_, static_cast<std::uint32_t>(kind), &h_), box_);
+  }
+  BoxCiphertext(BoxCiphertext&& o) noexcept : box_(o.box_), h_(std::exchange(o.h_, nullptr)) {}
+  BoxCiphertext(const BoxCiphertext&) = delete;
+  BoxCiphertext& operator=(const BoxCiphertext&) = delete;
+  ~BoxCiphertext() { spf_b200_box_ciphertext_free(h_); }
+  // host -> every replica (reference layout and scale); host_src holds one whole ciphertext
+  void write(const void* host_src) { check_box(spf_b200_box_ciphertext_write(h_, host_src), box_); }
+  // rank's replica -> host (reference layout and scale)
+  void read(void* host_dst, int rank = 0) const { check_box(spf_b200_box_ciphertext_read(h_, rank, host_dst), box_); }
+  spf_b200_box_ciphertext* handle() const { return h_; }
+
+ private:
+  spf_b200_box* box_;
+  spf_b200_box_ciphertext* h_ = nullptr;
+};
+
+// A levelised graph over every rank of a box; io buffers are host memory or BoxCiphertext handles.
 class BoxGraph {
  public:
   BoxGraph(const BoxEvaluation& ev, const FheCircuit& c) : box_(ev.handle()) {

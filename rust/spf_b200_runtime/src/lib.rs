@@ -9,7 +9,8 @@
 //!   (`circuit_processor/mod.rs:573-655`): [`Graph::spawn`] returns at once and calls the completion handler with the
 //!   first error (`completion_handler.rs:14-56`); [`DeviceCiphertext`] handles keep task outputs in HBM between graphs
 //!   (`circuit_processor/task.rs:10-16`).
-//! * [`BoxEvaluation`] / [`BoxGraph`]: the same over every GPU of a box, from one thread (one handle, one key upload).
+//! * [`BoxEvaluation`] / [`BoxGraph`]: the same over every GPU of a box, from one thread (one handle, one key upload);
+//!   [`BoxCiphertext`] handles keep task outputs in HBM between box graphs, one replica per rank.
 //! * module [`parasol`] (feature `parasol`): the glue a maintainer pastes into `parasol_runtime` so that
 //!   `CircuitProcessor::exec_op` (`circuit_processor/mod.rs:255-546`) dispatches to the GPU.
 //!
@@ -21,7 +22,7 @@ use std::os::raw::{c_char, c_int};
 use std::ptr::{self, NonNull};
 use std::sync::Arc;
 
-use spf_b200_sys::{spf_b200_box as RawBox, spf_b200_box_graph as RawBoxGraph};
+use spf_b200_sys::{spf_b200_box as RawBox, spf_b200_box_ciphertext as RawBoxCiphertext, spf_b200_box_graph as RawBoxGraph};
 pub use sys::{spf_node, spf_params, spf_radix};
 
 /// `RuntimeError` of the GPU path: the library's status code and message.
@@ -401,8 +402,57 @@ impl BoxEvaluation {
     }
 }
 
+/// A ciphertext kept in HBM with one replica per rank of a box (`spf_b200_box_ciphertext_*`): the box's
+/// [`DeviceCiphertext`].  Pass `as_io()` as the `io` of an `Output*` node of one box graph and of an `Input*` node of the
+/// next.  Box graphs hold their own references, so the handle may be dropped while a graph still binds it.  GGSWs stay
+/// in the device scale in the replicas; `write` takes and `read` returns the reference scale.
+pub struct BoxCiphertext {
+    raw: NonNull<RawBoxCiphertext>,
+    ev: BoxEvaluation,
+    pub bytes: usize,
+}
+unsafe impl Send for BoxCiphertext {}
+impl BoxCiphertext {
+    /// A zero-filled handle; `kind` is the `Input*` op code of the ciphertext type (`SPF_OP_INPUT_LWE0` ..
+    /// `SPF_OP_INPUT_GLEV1`).
+    pub fn alloc(ev: &BoxEvaluation, kind: u32) -> Result<Self> {
+        let mut raw = ptr::null_mut();
+        let rc = unsafe { sys::spf_b200_box_ciphertext_alloc(ev.raw(), kind, &mut raw) };
+        let p = match NonNull::new(raw) {
+            Some(p) if rc == 0 => p,
+            _ => return Err(Error { code: rc, message: box_error(ev.raw()) }),
+        };
+        let bytes = match kind {
+            sys::SPF_OP_INPUT_LWE0 => ev.len(sys::spf_b200_len_lwe_l0) * 8,
+            sys::SPF_OP_INPUT_LWE1 => ev.len(sys::spf_b200_len_lwe_l1) * 8,
+            sys::SPF_OP_INPUT_GLWE1 => ev.len(sys::spf_b200_len_glwe_l1) * 8,
+            sys::SPF_OP_INPUT_GGSW1 => ev.len(sys::spf_b200_len_ggsw_l1) * 16,
+            _ => ev.len(sys::spf_b200_len_glev_l1) * 8,
+        };
+        Ok(Self { raw: p, ev: ev.clone(), bytes })
+    }
+    pub fn as_io(&self) -> *mut c_void {
+        self.raw.as_ptr() as *mut c_void
+    }
+    /// One host ciphertext (reference layout and scale) to every rank's replica.
+    pub fn write<T: Copy>(&self, src: &[T]) -> Result<()> {
+        self.ev.expect("BoxCiphertext::write bytes", std::mem::size_of_val(src), self.bytes)?;
+        box_check!(self.ev, unsafe { sys::spf_b200_box_ciphertext_write(self.raw.as_ptr(), src.as_ptr() as *const c_void) })
+    }
+    /// Rank `rank`'s replica to the host (reference layout and scale).
+    pub fn read<T: Copy>(&self, rank: usize, dst: &mut [T]) -> Result<()> {
+        self.ev.expect("BoxCiphertext::read bytes", std::mem::size_of_val(dst), self.bytes)?;
+        box_check!(self.ev, unsafe { sys::spf_b200_box_ciphertext_read(self.raw.as_ptr(), rank as c_int, dst.as_mut_ptr() as *mut c_void) })
+    }
+}
+impl Drop for BoxCiphertext {
+    fn drop(&mut self) {
+        unsafe { sys::spf_b200_box_ciphertext_free(self.raw.as_ptr()) }
+    }
+}
+
 /// A validated, levelised `FheCircuit` over every rank of a [`BoxEvaluation`] (`spf_b200_box_graph_build`).  io buffers
-/// are host memory.
+/// are host memory or [`BoxCiphertext::as_io`].
 pub struct BoxGraph {
     raw: NonNull<RawBoxGraph>,
     ev: BoxEvaluation,
@@ -446,7 +496,7 @@ impl BoxGraph {
             Err(Error { code: rc, message: m })
         }
     }
-    /// Re-point an `Input*` / `Output*` node at another host buffer.
+    /// Re-point an `Input*` / `Output*` node at another host buffer or [`BoxCiphertext::as_io`].
     ///
     /// # Safety
     /// `io` must stay valid, and large enough for the node's ciphertext, until the graph has run.
@@ -612,6 +662,22 @@ pub mod parasol {
         }
     }
 
+    /// Task outputs kept in HBM on a box: the address of a task's ciphertext buffer (the `io` that [`lower`] gives its
+    /// `Input*` / `Output*` nodes) -> the [`BoxCiphertext`] that stands for it.  Instruction k's output task and
+    /// instruction k + 1's input task then name the same handle, and the hand-off never leaves the devices.
+    pub type BoxResident<'a> = std::collections::HashMap<*mut c_void, &'a BoxCiphertext>;
+
+    /// [`lower`], with the io buffers found in `resident` replaced by their box ciphertext handles.
+    pub fn lower_resident(circuit: &parasol_runtime::FheCircuit, resident: &BoxResident<'_>) -> Vec<spf_node> {
+        let mut nodes = lower(circuit);
+        for n in nodes.iter_mut() {
+            if let Some(h) = resident.get(&n.io) {
+                n.io = h.as_io();
+            }
+        }
+        nodes
+    }
+
     /// `CircuitProcessor::spawn_graph` on the GPU: lower, build, spawn.  Validation errors reach the handler, as in
     /// the reference where they surface through `CompletionHandler::error`.
     pub fn spawn_graph<F>(ev: Evaluator<'_>, circuit: &parasol_runtime::FheCircuit, on_completion: F) -> Option<SpawnedGraph>
@@ -634,6 +700,28 @@ pub mod parasol {
                     SpawnedGraph::Box(b) => b.spawn(&[], on_completion),
                 };
                 if let Err(e) = spawned {
+                    panic!("spf_b200: could not spawn a validated graph: {e}");
+                }
+                Some(g)
+            }
+        }
+    }
+
+    /// [`spawn_graph`] on a box with task outputs in HBM: the io buffers in `resident` are mapped to their
+    /// [`BoxCiphertext`]s, and the run is ordered on the devices behind the last runs of `after` (the graphs of the
+    /// instructions whose outputs it reads).
+    pub fn spawn_box_graph<F>(b: &BoxEvaluation, circuit: &parasol_runtime::FheCircuit, resident: &BoxResident<'_>, after: &[&BoxGraph],
+                              on_completion: F) -> Option<BoxGraph>
+    where
+        F: FnOnce(Option<Error>) + Send + 'static,
+    {
+        match BoxGraph::build(b, &lower_resident(circuit, resident)) {
+            Err(e) => {
+                on_completion(Some(e));
+                None
+            }
+            Ok(mut g) => {
+                if let Err(e) = g.spawn(after, on_completion) {
                     panic!("spf_b200: could not spawn a validated graph: {e}");
                 }
                 Some(g)

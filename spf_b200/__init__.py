@@ -483,11 +483,15 @@ ABI.update({
     "spf_b200_box_graph_levels": [_vp],
     "spf_b200_box_graph_launches": [_vp],
     "spf_b200_box_set_max_in_flight": [_vp, C.c_int],
+    "spf_b200_box_ciphertext_alloc": [_vp, C.c_uint32, C.POINTER(_vp)],
+    "spf_b200_box_ciphertext_free": [_vp],
+    "spf_b200_box_ciphertext_write": [_vp, _vp],
+    "spf_b200_box_ciphertext_read": [_vp, C.c_int, _vp],
 })
 _RESTYPES.update({"spf_b200_box_destroy": None, "spf_b200_box_last_error": C.c_char_p, "spf_b200_box_context": _vp,
                   "spf_b200_box_key_replication_ms": C.c_double, "spf_b200_box_shard": None,
                   "spf_b200_box_graph_status_message": C.c_char_p, "spf_b200_box_graph_destroy": None,
-                  "spf_b200_box_graph_launches": C.c_uint64})
+                  "spf_b200_box_graph_launches": C.c_uint64, "spf_b200_box_ciphertext_free": None})
 
 
 class DeviceCiphertext:
@@ -512,8 +516,63 @@ class DeviceCiphertext:
         return h
 
 
+class BoxCiphertext:
+    """A box ciphertext HANDLE (spf_b200_box_ciphertext_*): one ciphertext kept in HBM with one replica per rank of a
+    BoxEvaluation -- the box's DeviceCiphertext.  Pass it as the `io` of an Output* node of one box graph and of an
+    Input* node of the next; `ptr` is the handle address, `nbytes` the ciphertext size.  GGSWs stay in the device scale
+    in the replicas; write() takes and read() returns the reference scale.  close() (or garbage collection) drops this
+    reference: box graphs that still bind the handle keep its memory until they are closed or rebound."""
+
+    def __init__(self, box: "BoxEvaluation", kind: str, ptr: int):
+        import weakref
+
+        self.box, self.kind, self.ptr = box, kind, int(ptr)
+        self._box_ptr = box.handle.value  # the handle keeps the box's error slot alive, also after box.close()
+        self.nbytes = io_bytes(kind, box.params)
+        self._free = weakref.finalize(self, lib().spf_b200_box_ciphertext_free, self.ptr)
+
+    @classmethod
+    def alloc(cls, box: "BoxEvaluation", kind: str) -> "BoxCiphertext":
+        """A zero-filled handle for a ciphertext of `kind` ("Lwe0", "Lwe1", "Glwe1", "Ggsw1" or "Glev1")."""
+        if kind not in _IO_KIND:
+            raise SpfError(-1, f"BoxCiphertext: unknown kind {kind!r}, expected one of {sorted(_IO_KIND)}")
+        h = _vp()
+        box._check(lib().spf_b200_box_ciphertext_alloc(box.handle, OP["Input" + kind], C.byref(h)))
+        return cls(box, kind, h.value)
+
+    def _array(self):
+        return np.empty(self.nbytes // 16, np.complex128) if self.kind == "Ggsw1" else np.empty(self.nbytes // 8, np.uint64)
+
+    def _check(self, rc: int):
+        if rc != 0:
+            raise SpfError(rc, (lib().spf_b200_box_last_error(self._box_ptr) or b"").decode())
+
+    def _live(self):
+        if not self._free.alive:
+            raise SpfError(-1, "BoxCiphertext is closed")
+        return self.ptr
+
+    def write(self, arr) -> None:
+        """Host ciphertext (reference layout and scale) -> every rank's replica."""
+        a = np.ascontiguousarray(arr)
+        dtypes = (np.dtype(np.complex128), np.dtype(np.float64)) if self.kind == "Ggsw1" else (np.dtype(np.uint64),)
+        if a.dtype not in dtypes or a.nbytes != self.nbytes:
+            raise SpfError(-1, f"BoxCiphertext.write: a {self.kind} ciphertext is {self.nbytes} bytes of {dtypes[0]}, "
+                               f"got {a.nbytes} bytes of {a.dtype}")
+        self._check(lib().spf_b200_box_ciphertext_write(self._live(), a.ctypes.data))
+
+    def read(self, rank: int = 0) -> np.ndarray:
+        """Rank `rank`'s replica, in the reference layout and scale."""
+        out = self._array()
+        self._check(lib().spf_b200_box_ciphertext_read(self._live(), int(rank), out.ctypes.data))
+        return out
+
+    def close(self) -> None:
+        self._free()
+
+
 def _io_ptr(io) -> int:
-    return io.ptr if isinstance(io, DeviceCiphertext) else io.ctypes.data
+    return io.ptr if isinstance(io, (DeviceCiphertext, BoxCiphertext)) else io.ctypes.data
 
 
 def _io_nbytes(io) -> int:
@@ -565,12 +624,14 @@ class FheCircuit:
     def _check_io(self, opc: int, io) -> None:
         """An io buffer must hold exactly one ciphertext of the node's kind: the executor copies that many bytes
         through the raw pointer whatever the array's size (the reference is type-safe at this seam)."""
-        if not isinstance(io, DeviceCiphertext):
+        if not isinstance(io, (DeviceCiphertext, BoxCiphertext)):
             if not isinstance(io, np.ndarray) or not io.flags["C_CONTIGUOUS"]:
-                raise SpfError(-1, "io buffers must be C-contiguous numpy arrays or DeviceCiphertext handles")
+                raise SpfError(-1, "io buffers must be C-contiguous numpy arrays, DeviceCiphertext or BoxCiphertext handles")
         name = OPS[opc]
         if not (name.startswith("Input") or name.startswith("Output")):
             raise SpfError(-1, f"{name} takes no io buffer")
+        if isinstance(io, BoxCiphertext) and name.replace("Input", "").replace("Output", "") != io.kind:
+            raise SpfError(-1, f"{name}: the BoxCiphertext holds a {io.kind} ciphertext")
         want = io_bytes(name, self.params)
         if _io_nbytes(io) != want:
             raise SpfError(-1, f"{name}: io buffer has {_io_nbytes(io)} bytes, the ciphertext has {want}")
@@ -773,6 +834,8 @@ class CompiledGraph:
         instruction shape."""
         if not 0 <= node < len(self._keep):
             raise SpfError(-1, f"set_io: node {node} out of range")
+        if isinstance(buf, BoxCiphertext):
+            raise SpfError(-1, "set_io: a BoxCiphertext is the io of box graphs only (BoxGraph)")
         self._keep._check_io(int(self._keep.ops[node]), buf)
         self.ev._check(lib().spf_b200_graph_set_io(self._h, node, _io_ptr(buf)))
         self._bound = getattr(self, "_bound", {})
@@ -1016,7 +1079,8 @@ class BoxEvaluation:
 
 class BoxGraph:
     """A graph over every rank of a BoxEvaluation (spf_b200_box_graph_*), with the CompiledGraph surface: run, spawn,
-    wait, set_io, levels, launches, close.  io buffers are host numpy arrays (DeviceCiphertext handles are refused)."""
+    wait, set_io, levels, launches, close.  io buffers are host numpy arrays or BoxCiphertext handles of the same box
+    (DeviceCiphertext handles are refused)."""
 
     def __init__(self, box: BoxEvaluation, circuit: FheCircuit):
         self.ev = box

@@ -2,7 +2,8 @@
 // graph.cuh.  One process, one dispatching thread: a rank is a context on its own device; the compute key is uploaded
 // once and replicated device to device; host-pointer ops split the batch over the ranks and run them concurrently on
 // one worker thread per rank; a box graph is a sharded graph per rank, wired to the other ranks' arenas in-process,
-// and every rank's run is enqueued from the calling thread, level by level across the ranks.
+// and every rank's run is enqueued from the calling thread, level by level across the ranks.  A box ciphertext handle
+// holds one replica of a ciphertext per rank, so that box graphs hand their outputs to the next graph in HBM.
 #include <array>
 #include <functional>
 #include <thread>
@@ -29,9 +30,21 @@ struct spf_b200_box {
   bool stop = false;
 };
 
+// One ciphertext kept in HBM, one replica per rank on that rank's device (a device that appears twice gets two).
+// GGSWs are stored in the device scale (2^-10).  Reference-counted: the caller's reference and one per box graph node
+// bound to it; the handle holds a reference on its box.
+struct spf_b200_box_ciphertext {
+  spf_b200_box* box = nullptr;
+  uint32_t kind = 0;  // the Input* op code of the ciphertext type
+  size_t bytes = 0;
+  std::vector<char*> rep;  // rank r's replica
+  std::atomic<int> refs{1};
+};
+
 struct spf_b200_box_graph {
   spf_b200_box* box = nullptr;
   std::vector<spf_b200_graph*> g;  // rank r's sharded graph, on rank r's context
+  std::vector<spf_b200_box_ciphertext*> bound;  // per node: the box ciphertext handle bound to it (a reference), or NULL
   std::vector<void*> pinned;       // host io buffers page-locked (portable: every device DMAs them) by this box graph
   int* h_err = nullptr;            // page-locked copy of every rank's barrier error word, read by the completion
   std::atomic<int> status{0};
@@ -101,6 +114,107 @@ int box_each(spf_b200_box* b, size_t batch, const std::function<int(spf_b200_ctx
 
 void box_release(spf_b200_box* b) {
   if (b->refs.fetch_sub(1) == 1) delete b;
+}
+
+void box_ciphertext_delete(spf_b200_box_ciphertext* h) {
+  for (size_t r = 0; r < h->rep.size(); r++) {
+    if (!h->rep[r]) continue;
+    cudaSetDevice(h->box->device[r]);
+    cudaFree(h->rep[r]);
+  }
+  box_release(h->box);
+  delete h;
+}
+
+// Drops one reference; the last one unregisters the handle and frees its replicas.  A spawned run of a graph that was
+// rebound to another buffer may still read or write a replica (owners write the replicas of every rank), so every
+// device of the box finishes its work first.
+void box_ciphertext_release(spf_b200_box_ciphertext* h) {
+  if (!h || h->refs.fetch_sub(1) != 1) return;
+  {
+    std::lock_guard<std::mutex> lk(g_box_handles_mu);
+    g_box_handles.erase(h);
+  }
+  std::vector<int> devs = h->box->device;
+  std::sort(devs.begin(), devs.end());
+  devs.erase(std::unique(devs.begin(), devs.end()), devs.end());
+  for (int d : devs) {
+    cudaSetDevice(d);
+    cudaDeviceSynchronize();
+  }
+  box_ciphertext_delete(h);
+}
+
+// A box ciphertext handle named by io node `node` (op `op`) of a box graph on box b: SPF_E_INVALID unless it belongs to
+// b, the node is an Input* / Output* node and the handle holds the node's ciphertext type.
+int check_box_handle(spf_b200_box* b, const spf_b200_box_ciphertext* h, size_t node, uint32_t op) {
+  const std::string at = "box graph: node " + std::to_string(node);
+  if (op > SPF_OP_OUTPUT_GLEV1)
+    return box_fail(b, SPF_E_INVALID, at + " (" + (op <= SPF_OP_MUL_XN ? kOpNames[op] : "unknown op") +
+                                          ") takes no io; box ciphertext handles bind Input* and Output* nodes");
+  if (h->box != b) return box_fail(b, SPF_E_INVALID, at + ": the box ciphertext handle belongs to another box");
+  if (op % 5 != h->kind)
+    return box_fail(b, SPF_E_INVALID, at + " (" + kOpNames[op] + "): the box ciphertext handle holds a " +
+                                          (kOpNames[h->kind] + 5) + " ciphertext, a kind mismatch");
+  return 0;
+}
+
+// One or more box_copy_kernel launches over `items` (at most kBoxCopyLarge per launch).
+template <int N>
+int launch_box_copy_chunk(spf_b200_ctx* ctx, const BoxCopyItem* items, size_t cnt, cudaStream_t s) {
+  BoxCopyTable<N> t{};
+  unsigned widest = 0;
+  for (size_t i = 0; i < cnt; i++) {
+    t.item[i] = items[i];
+    widest = std::max(widest, items[i].n8);
+  }
+  const unsigned gx = std::min(32u, std::max(1u, (widest / 2 + 255) / 256));
+  box_copy_kernel<N><<<dim3(gx, (unsigned)cnt), 256, 0, s>>>(t);
+  return check_launch(ctx, "box_copy_kernel");
+}
+
+int launch_box_copy(spf_b200_ctx* ctx, const std::vector<BoxCopyItem>& items, cudaStream_t s) {
+  for (size_t i = 0; i < items.size(); i += kBoxCopyLarge) {
+    const size_t cnt = std::min(items.size() - i, (size_t)kBoxCopyLarge);
+    if (int rc = cnt <= (size_t)kBoxCopySmall ? launch_box_copy_chunk<kBoxCopySmall>(ctx, items.data() + i, cnt, s)
+                                              : launch_box_copy_chunk<kBoxCopyLarge>(ctx, items.data() + i, cnt, s))
+      return rc;
+  }
+  return 0;
+}
+
+// Rank r's handle traffic of one run, enqueued on its stream: inputs copy the rank's own replica into its arena;
+// outputs every rank holds (output rank -1) go to the rank's own replica; outputs of a MUX tree go from the owner to
+// the replicas of every rank.
+int enqueue_handle_copies(spf_b200_box_graph* bg, int r, bool outputs) {
+  spf_b200_graph* g = bg->g[r];
+  std::vector<BoxCopyItem> items;
+  for (int id : outputs ? g->outputs : g->inputs) {
+    if (g->io_kind[id] != 3) continue;
+    const spf_b200_box_ciphertext* h = static_cast<const spf_b200_box_ciphertext*>(g->nodes[id].io);
+    BoxCopyItem it{};
+    it.n8 = (unsigned)(h->bytes / 8);
+    if (!outputs) {
+      it.src = reinterpret_cast<const unsigned long long*>(h->rep[r]);
+      it.dst[it.n_dst++] = reinterpret_cast<unsigned long long*>(g->dptr[id]);
+    } else {
+      const int owner = spf_b200_graph_output_rank(g, id);
+      if (owner >= 0 && owner != r) continue;
+      it.src = reinterpret_cast<const unsigned long long*>(g->dptr[g->nodes[id].in[0]]);
+      for (size_t q = 0; q < h->rep.size(); q++)
+        if (owner >= 0 || (int)q == r) it.dst[it.n_dst++] = reinterpret_cast<unsigned long long*>(h->rep[q]);
+    }
+    items.push_back(it);
+  }
+  if (items.empty()) return 0;
+  return launch_box_copy(g->ctx, items, g->stream);
+}
+
+// Whether some handle-bound output is written by one rank into the replicas of the others.
+bool has_owned_handle_outputs(const spf_b200_graph* g) {
+  for (int id : g->outputs)
+    if (g->io_kind[id] == 3 && spf_b200_graph_output_rank(g, id) >= 0) return true;
+  return false;
 }
 
 int box_create_impl(const spf_params* params, const double* bsk, size_t bsk_len, const uint64_t* ksk, size_t ksk_len,
@@ -298,6 +412,10 @@ void CUDART_CB box_rank_done(void* arg) {
 // every rank for k = 0, 1, ..., then the outputs of every rank.  So when the host has to wait for a rank's stream (its
 // launch queue is full), every other rank's work up to the same level -- and so to the same peer barrier -- is
 // enqueued already, and the wait ends.  Returns the first error; ranks after a failed one are not enqueued further.
+// Box ciphertext handles: each rank reads its own replica right after its other inputs.  When an owner writes the
+// replicas of other ranks at the end, a barrier after the inputs first makes sure that every rank has read its
+// replica (a graph may read and write the same handle, and need not have a bootstrap level, whose barrier would do);
+// the start-of-run barrier keeps these writes ahead of the next run's reads.
 int box_enqueue(spf_b200_box_graph* bg) {
   spf_b200_box* b = bg->box;
   const int n = (int)bg->g.size();
@@ -307,7 +425,13 @@ int box_enqueue(spf_b200_box_graph* bg) {
   for (int r = 0; r < n; r++) {
     BCU(b, cudaSetDevice(bg->g[r]->ctx->device));
     if (int rc = enqueue_inputs(bg->g[r], n > 1, bg->g[r]->stream)) return rank_fail(r, rc);
+    if (int rc = enqueue_handle_copies(bg, r, false)) return rank_fail(r, rc);
   }
+  if (n > 1 && has_owned_handle_outputs(bg->g[0]))
+    for (int r = 0; r < n; r++) {
+      BCU(b, cudaSetDevice(bg->g[r]->ctx->device));
+      if (int rc = peer_barrier(bg->g[r], bg->g[r]->stream)) return rank_fail(r, rc);
+    }
   for (size_t k = 0; k < bg->g[0]->groups.size(); k++)
     for (int r = 0; r < n; r++) {
       spf_b200_graph* g = bg->g[r];
@@ -317,6 +441,7 @@ int box_enqueue(spf_b200_box_graph* bg) {
   for (int r = 0; r < n; r++) {
     BCU(b, cudaSetDevice(bg->g[r]->ctx->device));
     if (int rc = enqueue_outputs(bg->g[r], r, bg->g[r]->stream)) return rank_fail(r, rc);
+    if (int rc = enqueue_handle_copies(bg, r, true)) return rank_fail(r, rc);
   }
   return 0;
 }
@@ -475,6 +600,7 @@ void spf_b200_box_graph_destroy(spf_b200_box_graph* bg) {
   for (spf_b200_graph* g : bg->g) spf_b200_graph_destroy(g);
   for (void* q : bg->pinned) cudaHostUnregister(q);
   if (bg->h_err) cudaFreeHost(bg->h_err);
+  for (spf_b200_box_ciphertext* h : bg->bound) box_ciphertext_release(h);
   spf_b200_box* b = bg->box;
   delete bg;
   box_release(b);
@@ -486,21 +612,30 @@ int spf_b200_box_graph_build(spf_b200_box* b, const spf_node* nodes, size_t n_no
   *out = nullptr;
   const spf_params* p = &b->ctx[0]->p;
   BCU(b, cudaSetDevice(b->device[0]));
-  // io buffers: host memory only.  Unpinned ones are page-locked here as PORTABLE memory, so that every rank's device
-  // copies them by DMA (a plain registration is page-locked for one device only).
+  // io buffers: box ciphertext handles or host memory.  Unpinned host buffers are page-locked here as PORTABLE memory,
+  // so that every rank's device copies them by DMA (a plain registration is page-locked for one device only).
   std::unique_ptr<spf_b200_box_graph, void (*)(spf_b200_box_graph*)> bg(new spf_b200_box_graph(), spf_b200_box_graph_destroy);
   bg->box = b;
   b->refs.fetch_add(1);
+  bg->bound.assign(n_nodes, nullptr);
+  for (size_t i = 0; i < n_nodes; i++) {
+    if (!is_box_handle(nodes[i].io)) continue;
+    spf_b200_box_ciphertext* h = static_cast<spf_b200_box_ciphertext*>(nodes[i].io);
+    if (int rc = check_box_handle(b, h, i, nodes[i].op)) return rc;
+    h->refs.fetch_add(1);
+    bg->bound[i] = h;
+  }
   for (size_t i = 0; i < n_nodes; i++) {
     const uint32_t op = nodes[i].op;
-    if (op > SPF_OP_OUTPUT_GLEV1 || !nodes[i].io) continue;
+    if (op > SPF_OP_OUTPUT_GLEV1 || !nodes[i].io || bg->bound[i]) continue;
     const size_t bytes = ct_host_bytes(p, (CtType)(T_LWE0 + op % 5));
     cudaPointerAttributes a0, a1;
     if (cudaPointerGetAttributes(&a0, nodes[i].io) == cudaSuccess &&
         cudaPointerGetAttributes(&a1, static_cast<char*>(nodes[i].io) + bytes - 1) == cudaSuccess) {
       if (a0.type == cudaMemoryTypeDevice || a0.type == cudaMemoryTypeManaged)
         return box_fail(b, SPF_E_INVALID, "box graph: node " + std::to_string(i) +
-                                              " has a device-memory io buffer; box graphs take host buffers only");
+                                              " has a device-memory io buffer; box graphs take host buffers or box "
+                                              "ciphertext handles (spf_b200_box_ciphertext_alloc)");
       if (a0.type == cudaMemoryTypeHost && a1.type == cudaMemoryTypeHost) continue;
     }
     cudaGetLastError();
@@ -510,7 +645,7 @@ int spf_b200_box_graph_build(spf_b200_box* b, const spf_node* nodes, size_t n_no
   const int n = b->n;
   bg->g.assign(n, nullptr);
   for (int r = 0; r < n; r++) {
-    if (int rc = spf_b200_graph_build_sharded(b->ctx[r], nodes, n_nodes, n, &bg->g[r]))
+    if (int rc = graph_build_checked(b->ctx[r], nodes, n_nodes, n, &bg->g[r], true))
       return box_fail(b, rc, (r ? "rank " + std::to_string(r) + ": " : std::string()) + b->ctx[r]->err);
     bg->g[r]->replicated_writer = 0;
     settle_all_io(bg->g[r]);
@@ -656,13 +791,103 @@ int spf_b200_box_graph_set_io(spf_b200_box_graph* bg, size_t node, void* io) {
   if (!bg) return SPF_E_INVALID;
   spf_b200_box* b = bg->box;
   if (!io) return box_fail(b, SPF_E_INVALID, "set_io: io pointer is NULL");
+  if (node >= bg->bound.size())
+    return box_fail(b, SPF_E_INVALID, "set_io: node " + std::to_string(node) + " is not an Input*/Output* node");
+  spf_b200_box_ciphertext* const old = bg->bound[node];
+  if (is_box_handle(io)) {
+    spf_b200_box_ciphertext* h = static_cast<spf_b200_box_ciphertext*>(io);
+    if (int rc = check_box_handle(b, h, node, bg->g[0]->nodes[node].op)) return rc;
+    h->refs.fetch_add(1);
+    for (spf_b200_graph* g : bg->g) {
+      g->nodes[node].io = h;
+      g->io_kind[node] = 3;
+      g->io_alloc[node] = 0;
+    }
+    bg->bound[node] = h;
+    box_ciphertext_release(old);
+    return 0;
+  }
   cudaPointerAttributes a;
   if (cudaPointerGetAttributes(&a, io) == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged))
-    return box_fail(b, SPF_E_INVALID, "box graph: device-memory io buffers are not supported; box graphs take host buffers only");
+    return box_fail(b, SPF_E_INVALID, "box graph: device-memory io buffers are not supported; box graphs take host buffers "
+                                      "or box ciphertext handles (spf_b200_box_ciphertext_alloc)");
   cudaGetLastError();
   for (size_t r = 0; r < bg->g.size(); r++) {
     if (int rc = spf_b200_graph_set_io(bg->g[r], node, io)) return box_fail(b, rc, bg->g[r]->ctx->err);
     settle_io(bg->g[r], node);
+  }
+  bg->bound[node] = nullptr;
+  box_ciphertext_release(old);
+  return 0;
+}
+
+int spf_b200_box_ciphertext_alloc(spf_b200_box* b, uint32_t kind, spf_b200_box_ciphertext** out) {
+  if (out) *out = nullptr;
+  if (kind > SPF_OP_INPUT_GLEV1)
+    return box_fail(b, SPF_E_INVALID, "box ciphertext: unknown kind " + std::to_string(kind) +
+                                          " (the Input* op code of the ciphertext type: SPF_OP_INPUT_LWE0 .. SPF_OP_INPUT_GLEV1)");
+  if (!b) return box_fail(nullptr, SPF_E_INVALID, "box ciphertext: box is NULL");
+  if (!out) return box_fail(b, SPF_E_INVALID, "box ciphertext: out is NULL");
+  spf_b200_box_ciphertext* h = new spf_b200_box_ciphertext();
+  h->box = b;
+  b->refs.fetch_add(1);
+  h->kind = kind;
+  h->bytes = ct_bytes(&b->ctx[0]->p, (CtType)(T_LWE0 + kind));
+  h->rep.assign(b->n, nullptr);
+  // zero-filled, as the reference's enc.allocate_* (the legacy stream orders the fill before any later copy)
+  for (int r = 0; r < b->n; r++) {
+    cudaError_t e = cudaSetDevice(b->device[r]);
+    if (e == cudaSuccess) e = cudaMalloc(&h->rep[r], h->bytes);
+    if (e == cudaSuccess) e = cudaMemsetAsync(h->rep[r], 0, h->bytes, 0);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+    if (e != cudaSuccess) {
+      box_ciphertext_delete(h);
+      return box_fail(b, SPF_E_CUDA, std::string("box ciphertext alloc: ") + cudaGetErrorString(e));
+    }
+  }
+  {
+    std::lock_guard<std::mutex> lk(g_box_handles_mu);
+    g_box_handles.insert(h);
+  }
+  *out = h;
+  return 0;
+}
+
+void spf_b200_box_ciphertext_free(spf_b200_box_ciphertext* h) {
+  if (is_box_handle(h)) box_ciphertext_release(h);
+}
+
+int spf_b200_box_ciphertext_write(spf_b200_box_ciphertext* h, const void* host_src) {
+  if (!is_box_handle(h)) return box_fail(nullptr, SPF_E_INVALID, "box ciphertext: not a live handle");
+  spf_b200_box* b = h->box;
+  if (!host_src) return box_fail(b, SPF_E_INVALID, "box ciphertext write: NULL buffer");
+  const void* src = host_src;
+  std::vector<double> scaled;
+  if (h->kind == SPF_OP_INPUT_GGSW1) {  // reference scale -> device scale (exact: a power of two)
+    const double* d = static_cast<const double*>(host_src);
+    scaled.assign(d, d + h->bytes / 8);
+    for (double& x : scaled) x *= 1.0 / 1024.0;
+    src = scaled.data();
+  }
+  for (size_t r = 0; r < h->rep.size(); r++) {
+    BCU(b, cudaSetDevice(b->device[r]));
+    BCU(b, cudaMemcpyAsync(h->rep[r], src, h->bytes, cudaMemcpyHostToDevice, 0));
+    BCU(b, cudaStreamSynchronize(0));
+  }
+  return 0;
+}
+
+int spf_b200_box_ciphertext_read(spf_b200_box_ciphertext* h, int rank, void* host_dst) {
+  if (!is_box_handle(h)) return box_fail(nullptr, SPF_E_INVALID, "box ciphertext: not a live handle");
+  spf_b200_box* b = h->box;
+  if (rank < 0 || rank >= (int)h->rep.size()) return box_fail(b, SPF_E_INVALID, "box ciphertext read: rank out of range");
+  if (!host_dst) return box_fail(b, SPF_E_INVALID, "box ciphertext read: NULL buffer");
+  BCU(b, cudaSetDevice(b->device[rank]));
+  BCU(b, cudaMemcpyAsync(host_dst, h->rep[rank], h->bytes, cudaMemcpyDeviceToHost, 0));
+  BCU(b, cudaStreamSynchronize(0));
+  if (h->kind == SPF_OP_INPUT_GGSW1) {  // device scale -> reference scale
+    double* d = static_cast<double*>(host_dst);
+    for (size_t i = 0; i < h->bytes / 8; i++) d[i] *= 1024.0;
   }
   return 0;
 }

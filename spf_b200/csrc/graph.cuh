@@ -120,7 +120,8 @@ struct spf_b200_graph {
   // io kinds per node (Input* / Output* only): 0 = page-locked host memory (plain DMA), 1 = pageable host memory staged
   // through the graph's own page-locked slab (set_io on an unpinned buffer: registering costs 0.4 ms per buffer and call),
   // 2 = DEVICE memory: a ciphertext handle that never leaves HBM (another graph's output, a torch tensor, ...); GGSWs
-  // behind device handles keep the device scale (2^-10)
+  // behind device handles keep the device scale (2^-10), 3 = a box ciphertext handle (rank graphs of a box only: io is
+  // the spf_b200_box_ciphertext, whose copies box.cuh enqueues; the single-context parts below skip these nodes)
   std::vector<char> io_kind;
   std::vector<unsigned long long> io_alloc;  // allocation that holds the node's io buffer (alloc_base_of), 0 = do not merge copies
   char* h_stage = nullptr;        // page-locked staging slab for kind-1 buffers
@@ -158,6 +159,17 @@ struct SpawnRecord {
 namespace {
 
 constexpr size_t kArenaHeader = 4096;  // flags[world] at 0, error word at 2048
+
+// Addresses of the live box ciphertext handles (spf_b200_box_ciphertext_alloc .. _free).  A handle passed where a host
+// buffer is expected would otherwise be page-locked and DMA'd as if its bytes were a ciphertext.
+std::mutex g_box_handles_mu;
+std::unordered_set<const void*> g_box_handles;
+
+bool is_box_handle(const void* p) {
+  if (!p) return false;
+  std::lock_guard<std::mutex> lk(g_box_handles_mu);
+  return g_box_handles.count(p) != 0;
+}
 
 // Device constants for Zero*/One* nodes (mod.rs:95-105,475-506).  ZeroGgsw1/OneGgsw1 are real CBS
 // outputs of the trivial LWE 0/1, exactly as Evaluation::new computes them (evaluation.rs:161-197).
@@ -487,22 +499,33 @@ int spf_b200_graph_run_sharded(spf_b200_graph* g, int rank, int world, spf_excha
 int spf_b200_graph_set_io(spf_b200_graph* g, size_t node, void* io);
 int spf_b200_graph_output_rank(const spf_b200_graph* g, size_t node);
 
-static int graph_build_sharded_impl(spf_b200_ctx* ctx, const spf_node* nodes, size_t n, int world, spf_b200_graph** out);
-// C++ exceptions (std::bad_alloc / length_error on a huge graph) never cross the C ABI
-int spf_b200_graph_build_sharded(spf_b200_ctx* ctx, const spf_node* nodes, size_t n, int world, spf_b200_graph** out) {
+static int graph_build_sharded_impl(spf_b200_ctx* ctx, const spf_node* nodes, size_t n, int world, spf_b200_graph** out,
+                                    bool box_handles);
+// C++ exceptions (std::bad_alloc / length_error on a huge graph) never cross the C ABI.  `box_handles`: the rank graph
+// of a box graph, whose io nodes may name box ciphertext handles (io kind 3); every other graph refuses them.
+static int graph_build_checked(spf_b200_ctx* ctx, const spf_node* nodes, size_t n, int world, spf_b200_graph** out,
+                               bool box_handles) {
   try {
-    return graph_build_sharded_impl(ctx, nodes, n, world, out);
+    return graph_build_sharded_impl(ctx, nodes, n, world, out, box_handles);
   } catch (const std::exception& e) {
     return fail(ctx, SPF_E_GRAPH, std::string("graph build: ") + e.what());
   } catch (...) {
     return fail(ctx, SPF_E_GRAPH, "graph build: unknown exception");
   }
 }
-static int graph_build_sharded_impl(spf_b200_ctx* ctx, const spf_node* nodes, size_t n, int world, spf_b200_graph** out) {
+int spf_b200_graph_build_sharded(spf_b200_ctx* ctx, const spf_node* nodes, size_t n, int world, spf_b200_graph** out) {
+  return graph_build_checked(ctx, nodes, n, world, out, false);
+}
+static int graph_build_sharded_impl(spf_b200_ctx* ctx, const spf_node* nodes, size_t n, int world, spf_b200_graph** out,
+                                    bool box_handles) {
   if (!ctx) return SPF_E_INVALID;
   if (!out || (!nodes && n)) return fail(ctx, SPF_E_INVALID, "NULL argument");
   if (world < 1 || world > 1024) return fail(ctx, SPF_E_INVALID, "world must be in 1..1024");
   *out = nullptr;
+  if (!box_handles)
+    for (size_t i = 0; i < n; i++)
+      if (is_box_handle(nodes[i].io))
+        return fail(ctx, SPF_E_INVALID, "node " + std::to_string(i) + ": a box ciphertext handle is the io of box graphs only (spf_b200_box_graph_build)");
   const spf_params* p = &ctx->p;
   std::unique_ptr<spf_b200_graph, void (*)(spf_b200_graph*)> g(new spf_b200_graph(), spf_b200_graph_destroy);
   g->ctx = ctx;
@@ -651,15 +674,16 @@ static int graph_build_sharded_impl(spf_b200_ctx* ctx, const spf_node* nodes, si
           if (G.slot_outputs) g->dptr[id] = g->arena + pool_off + (size_t)g->slot[id] * ct_bytes(p, T_GLWE1);
           else if (G.out_base) g->dptr[id] = G.out_base + k * ct_bytes(p, oi.out);
       }
+      const bool handle = box_handles && G.op <= SPF_OP_OUTPUT_GLEV1 && is_box_handle(g->nodes[id].io);
       if (G.op <= SPF_OP_INPUT_GLEV1) {
         g->inputs.push_back(id);
-        g->io_kind[id] = (char)pin_io(g.get(), g->nodes[id].io, ct_host_bytes(p, g->type[id]));
-        g->io_alloc[id] = alloc_base_of(g->nodes[id].io);
+        g->io_kind[id] = handle ? 3 : (char)pin_io(g.get(), g->nodes[id].io, ct_host_bytes(p, g->type[id]));
+        g->io_alloc[id] = handle ? 0 : alloc_base_of(g->nodes[id].io);
       }
       if (G.op >= SPF_OP_OUTPUT_LWE0 && G.op <= SPF_OP_OUTPUT_GLEV1) {
         g->outputs.push_back(id);
-        g->io_kind[id] = (char)pin_io(g.get(), g->nodes[id].io, ct_host_bytes(p, g->type[g->nodes[id].in[0]]));
-        g->io_alloc[id] = alloc_base_of(g->nodes[id].io);
+        g->io_kind[id] = handle ? 3 : (char)pin_io(g.get(), g->nodes[id].io, ct_host_bytes(p, g->type[g->nodes[id].in[0]]));
+        g->io_alloc[id] = handle ? 0 : alloc_base_of(g->nodes[id].io);
       }
     }
   }
@@ -862,6 +886,10 @@ int enqueue_inputs(spf_b200_graph* g, bool peer_mode, cudaStream_t s) {
     const int id0 = g->inputs[i];
     const int kind = g->io_kind[id0];
     size_t bytes = ct_host_bytes(p, g->type[id0]), j = i + 1;
+    if (kind == 3) {  // box ciphertext handle: box.cuh copies it
+      i = j;
+      continue;
+    }
     if (kind == 1) {  // pageable host buffer: through the page-locked slab
       char* st = nullptr;
       if (int rc = stage_slot(g, id0, bytes, &st)) return rc;
@@ -881,7 +909,7 @@ int enqueue_inputs(spf_b200_graph* g, bool peer_mode, cudaStream_t s) {
   }
   for (int id : g->inputs) {
     const CtType t = g->type[id];
-    if (t == T_GGSW1 && g->io_kind[id] != 2)  // device handles carry GGSWs in the device scale already
+    if (t == T_GGSW1 && g->io_kind[id] < 2)  // device and box handles carry GGSWs in the device scale already
       if (int rc = launch_scale(ctx, reinterpret_cast<C2*>(g->dptr[id]), reinterpret_cast<const C2*>(g->dptr[id]),
                                 spf_b200_len_ggsw_l1(p), 1.0 / 1024.0, s))
         return rc;
@@ -962,6 +990,10 @@ int enqueue_outputs(spf_b200_graph* g, int rank, cudaStream_t s) {
     const int src = g->nodes[id].in[0];
     const CtType t = g->type[src];
     const int kind = g->io_kind[id];
+    if (kind == 3) {  // box ciphertext handle: box.cuh copies it
+      k++;
+      continue;
+    }
     char* dst = static_cast<char*>(g->nodes[id].io);
     if (kind == 1 && mine(k))
       if (int rc = stage_slot(g, id, ct_host_bytes(p, t), &dst)) return rc;
@@ -1209,6 +1241,8 @@ int spf_b200_graph_set_io(spf_b200_graph* g, size_t node, void* io) {
   if (node >= g->nodes.size() || g->nodes[node].op > SPF_OP_OUTPUT_GLEV1)
     return fail(g->ctx, SPF_E_INVALID, "set_io: node " + std::to_string(node) + " is not an Input*/Output* node");
   if (!io) return fail(g->ctx, SPF_E_INVALID, "set_io: io pointer is NULL");
+  if (is_box_handle(io))
+    return fail(g->ctx, SPF_E_INVALID, "set_io: a box ciphertext handle is the io of box graphs only (spf_b200_box_graph_set_io)");
   void* old = g->nodes[node].io;
   if (old == io) return 0;
   cudaSetDevice(g->ctx->device);

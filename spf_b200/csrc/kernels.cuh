@@ -1276,6 +1276,44 @@ __global__ void peer_bcast_kernel(const uint4* src, size_t n16, PeerOffsets peer
   }
 }
 
+// All box-ciphertext-handle traffic of one rank in one run phase (box.cuh): item k copies n8 u64 words from src to
+// each of its n_dst destinations -- this rank's arena, its own replica, or the replicas of the other ranks (peer
+// stores over NVLink).  The table travels as a __grid_constant__ parameter, so every launch works on its own snapshot
+// of the bindings.  Items whose pointers are all 16-byte aligned move 16-byte words (an L1 LWE is 2049 u64 words:
+// the odd word goes in the tail loop); the others move u64 words.
+constexpr int kBoxCopyMaxDst = 8;
+struct BoxCopyItem {
+  const unsigned long long* src;
+  unsigned long long* dst[kBoxCopyMaxDst];
+  unsigned n8;
+  int n_dst;
+};
+template <int N>
+struct BoxCopyTable {
+  BoxCopyItem item[N];
+};
+constexpr int kBoxCopySmall = 32;   // 2.6 KB of parameters
+constexpr int kBoxCopyLarge = 400;  // 32 000 bytes: within the 32 764-byte kernel parameter limit (CUDA >= 12.1)
+static_assert(sizeof(BoxCopyTable<kBoxCopyLarge>) <= 32764, "box copy table exceeds the kernel parameter limit");
+
+template <int N>
+__global__ void __launch_bounds__(256) box_copy_kernel(const __grid_constant__ BoxCopyTable<N> t) {
+  const BoxCopyItem& it = t.item[blockIdx.y];
+  const int nd = it.n_dst;
+  bool v16 = (reinterpret_cast<uintptr_t>(it.src) & 15) == 0;
+  for (int d = 0; d < nd; d++) v16 &= (reinterpret_cast<uintptr_t>(it.dst[d]) & 15) == 0;
+  const size_t n16 = v16 ? it.n8 / 2 : 0;
+  const size_t stride = (size_t)gridDim.x * blockDim.x, first = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+  for (size_t i = first; i < n16; i += stride) {
+    const uint4 v = reinterpret_cast<const uint4*>(it.src)[i];
+    for (int d = 0; d < nd; d++) reinterpret_cast<uint4*>(it.dst[d])[i] = v;
+  }
+  for (size_t i = 2 * n16 + first; i < it.n8; i += stride) {
+    const unsigned long long v = it.src[i];
+    for (int d = 0; d < nd; d++) it.dst[d][i] = v;
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // K2: runtime CMUX / external product, one team per GLWE output.
 // ------------------------------------------------------------------------------------------

@@ -1,8 +1,11 @@
 """One process over the GPUs of a box (spf_b200.BoxEvaluation): key replication, device-resident and end-to-end circuit
 bootstrapping, and N x (mul32 then greater-than) in one box graph, blocking and spawned.  Prints one JSON line and
 records it under profiles/ (--out).  The same measurements as bench.py's multi-process line, so the two compare.
+--chain measures instead a two-instruction program run as two box graphs (mul32, then greater-than on the product),
+with the 32 product bits handed over through host buffers or through box ciphertext handles.
 
-usage: python tools/box_bench.py [--devices 0,1,...] [--batch 4096] [--steps 10] [--out profiles/box_bench_n8.json]"""
+usage: python tools/box_bench.py [--devices 0,1,...] [--batch 4096] [--steps 10] [--out profiles/box_bench_n8.json]
+       python tools/box_bench.py --chain [--devices 0,0] [--reps 20] [--out profiles/box_chain_n1.json]"""
 import argparse
 import ctypes as C
 import json
@@ -158,6 +161,104 @@ def programs(box, keys, n_programs, reps):
     return res
 
 
+def chain(box, keys, n_programs, reps, warmup):
+    """n_programs x (mul32 | greater-than on the product) as TWO box graphs, the 32 product bits of every program handed
+    from the first to the second through page-locked host buffers ("host") or box ciphertext handles ("handle"), each
+    run blocking (run, run) and spawned (spawn, spawn after the first, wait).  Times are host clocks around the whole
+    program pair up to the end of the second graph (median over reps, rounds of the four ways interleaved); enqueue_ms
+    is the host time of the two spawn calls.  PCIe bytes per run follow from the shapes: every rank copies every host
+    input, the owner of a product bit copies it out, and the host-buffer hand-off is read back by every rank."""
+    import oracle as O
+    import spf_b200
+    from spf_b200 import FheCircuit
+    from spf_b200 import mux_circuits as M
+    from spf_b200.circuits import _front
+
+    client = O.Client(keys)
+    w = 32
+    rng = np.random.default_rng(0xB0C6)
+    vals = [tuple(int(x) for x in rng.integers(0, 1 << w, 3)) for _ in range(n_programs)]
+    slab = iter(spf_b200.pinned_zeros((n_programs * (3 * w + w + 1), keys.glwe_len)))
+
+    def enc(v):
+        out = [next(slab) for _ in range(w)]
+        for i, r in enumerate(out):
+            r[:] = client.encrypt_glwe_l1([(v >> i) & 1])
+        return out
+
+    a, b, c = ([enc(v[k]) for v in vals] for k in range(3))
+    mid_host = [[next(slab) for _ in range(w)] for _ in vals]
+    out_gt = [next(slab) for _ in vals]
+    mid_handle = [[spf_b200.BoxCiphertext.alloc(box, "Glwe1") for _ in range(w)] for _ in vals]
+
+    def graphs(mid):
+        c1, c2 = FheCircuit(), FheCircuit()
+        keep1, keep2 = [], []
+        for p in range(n_programs):
+            lo, _hi = M.append_uint_multiply(c1, [_front(c1, x) for x in a[p]], [_front(c1, x) for x in b[p]])
+            keep1 += [c1.add("OutputGlwe1", lo[i], io=mid[p][i]) for i in range(w)]
+            pairs = [x for pr in zip([_front(c2, x) for x in mid[p]], [_front(c2, x) for x in c[p]]) for x in pr]
+            (gt,) = M.insert_mux_circuit(c2, M.compare_or_maybe_equal(w, True, False), pairs)
+            keep2.append(c2.add("OutputGlwe1", gt, io=out_gt[p]))
+        return spf_b200.BoxGraph(box, M.prune(c1, keep1)[0]), spf_b200.BoxGraph(box, M.prune(c2, keep2)[0])
+
+    pairs = {"host": graphs(mid_host), "handle": graphs(mid_handle)}
+
+    def correct(mode):
+        ok = True
+        for p, (x, y, z) in enumerate(vals):
+            bits = [m if mode == "host" else m.read() for m in (mid_host if mode == "host" else mid_handle)[p]]
+            prod = sum(int(client.decrypt_glwe_l1(o)[0]) << i for i, o in enumerate(bits))
+            ok &= prod == (x * y) % (1 << w) and int(client.decrypt_glwe_l1(out_gt[p])[0]) == int(prod > z)
+        return bool(ok)
+
+    def once(mode, spawned):
+        g1, g2 = pairs[mode]
+        for o in out_gt:
+            o[:] = 0
+        t0 = time.perf_counter()
+        if spawned:
+            g1.spawn()
+            g2.spawn(after=[g1])
+            t_enq = time.perf_counter() - t0
+            g2.wait()
+            g1.wait()
+        else:
+            g1.run()
+            g2.run()
+            t_enq = None
+        return time.perf_counter() - t0, t_enq
+
+    ways = [(m, s) for m in ("host", "handle") for s in (False, True)]
+    for _ in range(max(warmup, 2)):
+        for m, s in ways:
+            once(m, s)
+    times = {k: [] for k in ways}
+    enq = {k: [] for k in ways}
+    ok = {m: True for m in pairs}
+    for _ in range(reps):
+        for m, s in ways:
+            t, e = once(m, s)
+            times[(m, s)].append(t)
+            if e is not None:
+                enq[(m, s)].append(e)
+            ok[m] &= correct(m)
+    glwe, n = keys.glwe_len * 8, box.size
+    pcie_in = n * 3 * w * glwe * n_programs + 1 * glwe * n_programs  # operand inputs on every rank, the verdict out
+    res = {"programs": n_programs, "ranks": n, "levels": [pairs["host"][0].levels, pairs["host"][1].levels],
+           "launches_handle": [g.launches for g in pairs["handle"]], "launches_host": [g.launches for g in pairs["host"]]}
+    for m in pairs:
+        res[m] = {"pcie_bytes_per_run": pcie_in + (w * glwe + n * w * glwe) * n_programs * (m == "host"), "correct": ok[m]}
+        for s in (False, True):
+            key = "spawned" if s else "blocking"
+            res[m][key + "_ms"] = 1e3 * float(np.median(times[(m, s)]))
+            if s:
+                res[m]["spawned_enqueue_ms"] = 1e3 * float(np.median(enq[(m, s)]))
+    for g in [g for pr in pairs.values() for g in pr]:
+        g.close()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--devices", default=None, help="comma-separated device list (default: every visible GPU)")
@@ -166,6 +267,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--reps", type=int, default=5, help="runs of the program graph per mode")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
+    ap.add_argument("--chain", action="store_true", help="measure the two-graph mul32 | greater-than hand-off only")
+    ap.add_argument("--programs", type=int, default=1, help="--chain: programs per graph")
     args = ap.parse_args()
 
     import torch
@@ -176,13 +279,18 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("box_bench.py: no CUDA device; spf_b200 has no CPU fallback")
     devices = [int(x) for x in args.devices.split(",")] if args.devices else list(range(torch.cuda.device_count()))
-    line = {"metric": "box_bench", "devices": devices, "gpus": gpu_identity(devices)}
+    line = {"metric": "box_chain" if args.chain else "box_bench", "devices": devices, "gpus": gpu_identity(devices)}
     keys = O.Keys()
     t0 = time.perf_counter()
     box = spf_b200.BoxEvaluation(keys.bsk_fft, keys.ksk, keys.ssk_fft, keys.ak_fft, devices=devices)
     line["box_create_ms"] = 1e3 * (time.perf_counter() - t0)
     line["key_replication_ms"] = box.key_replication_ms
     n = box.size
+    if args.chain:
+        line["chain"] = chain(box, keys, args.programs, max(args.reps, 20), args.warmup)
+        box.close()
+        emit(line, args.out)
+        return
     p = keys.params
     bits = np.random.default_rng(0xB0C4).integers(0, 2, n * args.batch)
     cts = encrypt_lwe0(keys.lwe0_sk.astype(np.uint64), bits, p.lwe_std, 0xB0C4)
@@ -194,10 +302,14 @@ def main():
     line["end_to_end"] = {"batch_per_gpu": args.batch, **e2e}
     line["mul32_then_gt"] = programs(box, keys, n, args.reps)
     box.close()
+    emit(line, args.out)
+
+
+def emit(line, out):
     text = json.dumps(line)
     print(text)
-    if args.out:
-        with open(args.out, "w") as f:
+    if out:
+        with open(out, "w") as f:
             f.write(text + "\n")
 
 
