@@ -355,8 +355,26 @@ int spf_b200_box_cmux(spf_b200_box *box, uint64_t *glwe_out, const double *sel_g
  * dependency); a run whose dependency failed
  * retires as a no-op with that error; at most spf_b200_box_set_max_in_flight (default 4) runs per box are in flight,
  * further spawns block the caller.  A failed run with N > 1 poisons the box graph (rebuild it).  Destroying a box
- * graph waits for its run in flight. */
+ * graph waits for its run in flight.
+ * PLACEMENT: spf_b200_box_graph_build_on runs the graph on an ordered subset of the box's ranks, its members:
+ * ranks[i] is the box rank that runs member i, and the graph is sharded over the n_ranks members exactly as a box graph
+ * over a box of n_ranks ranks would be ("rank" above then means member; member 0 writes the host outputs every member
+ * holds).  spf_b200_box_graph_build is build_on with ranks 0 .. N - 1.  Independent graphs placed on different ranks
+ * run at the same time.  A one-member graph has no peer barriers and runs as a one-rank box does (a failed run does
+ * not poison it).  Handle-bound inputs are read from the members' own replicas; handle-bound outputs are written into
+ * the replicas of EVERY rank of the box, members or not (a MUX-tree output by its owner member, an output every member
+ * holds by each member into its own replica and by member 0 into the replicas of the other ranks), so the next graph
+ * reads it wherever it is placed.  `after` may name graphs placed on other ranks: every member waits for every member
+ * of the dependency.  Errors (SPF_E_INVALID, the box stays usable): ranks NULL, n_ranks outside 1 .. N, a rank outside
+ * 0 .. N - 1, a rank named twice.  spf_b200_box_graph_ranks returns the member count and, if ranks_out is not NULL,
+ * stores the members' box ranks in it.
+ * HAZARD RULE: a run writes a handle-bound output into every replica, on every rank.  So a graph that writes a handle
+ * which another graph reads -- on any rank -- must be spawned with that reader in `after` (and a graph that reads a
+ * handle with its writer in `after`), as for DeviceCiphertext handles on one context. */
 int spf_b200_box_graph_build(spf_b200_box *box, const spf_node *nodes, size_t n_nodes, spf_b200_box_graph **out);
+int spf_b200_box_graph_build_on(spf_b200_box *box, const spf_node *nodes, size_t n_nodes, const int *ranks, int n_ranks,
+                                spf_b200_box_graph **out);
+int spf_b200_box_graph_ranks(const spf_b200_box_graph *graph, int *ranks_out);
 int spf_b200_box_graph_run(spf_b200_box_graph *graph);
 int spf_b200_box_graph_spawn(spf_b200_box_graph *graph, spf_b200_box_graph *const *after, size_t n_after,
                              spf_completion_fn on_complete, void *user);
@@ -369,7 +387,8 @@ uint64_t spf_b200_box_graph_launches(const spf_b200_box_graph *graph); /* kernel
 int spf_b200_box_set_max_in_flight(spf_b200_box *box, int n);
 
 /* Box ciphertext handles: one ciphertext kept in HBM between box graphs -- the box's DeviceCiphertext.  A handle holds
- * one replica per rank, on that rank's device (a device that appears twice in the box gets two).  Pass the handle
+ * one replica per rank of the box, on that rank's device (a device that appears twice in the box gets two), whatever
+ * ranks the graphs that use it are placed on (see PLACEMENT and the HAZARD RULE above).  Pass the handle
  * pointer itself as spf_node.io or to spf_b200_box_graph_set_io: graph k's Output* node and graph k + 1's Input* node
  * name the same handle, nothing crosses PCIe, and `after` orders the two graphs on the devices.  Errors
  * (SPF_E_INVALID): a handle of another box, a handle whose kind is not the node's ciphertext type, a handle on a node

@@ -327,11 +327,23 @@ class BoxCiphertext {
   spf_b200_box_ciphertext* h_ = nullptr;
 };
 
-// A levelised graph over every rank of a box; io buffers are host memory or BoxCiphertext handles.
+// A levelised graph over every rank of a box, or over the ranks named in `ranks` (member i runs on box rank ranks[i]);
+// io buffers are host memory or BoxCiphertext handles.
 class BoxGraph {
  public:
   BoxGraph(const BoxEvaluation& ev, const FheCircuit& c) : box_(ev.handle()) {
     check_box(spf_b200_box_graph_build(box_, c.nodes().data(), c.size(), &g_), box_);
+  }
+  BoxGraph(const BoxEvaluation& ev, const FheCircuit& c, const std::vector<int>& ranks) : box_(ev.handle()) {
+    check_box(spf_b200_box_graph_build_on(box_, c.nodes().data(), c.size(), ranks.data(), static_cast<int>(ranks.size()), &g_),
+              box_);
+  }
+  // the box ranks the graph runs on, in member order
+  std::vector<int> ranks() const {
+    const int n = spf_b200_box_graph_ranks(g_, nullptr);
+    std::vector<int> r(static_cast<std::size_t>(n > 0 ? n : 0));
+    if (n > 0) spf_b200_box_graph_ranks(g_, r.data());
+    return r;
   }
   BoxGraph(BoxGraph&& o) noexcept : box_(o.box_), g_(std::exchange(o.g_, nullptr)) {}
   BoxGraph(const BoxGraph&) = delete;
@@ -363,6 +375,7 @@ class BoxCircuitProcessor {
  public:
   explicit BoxCircuitProcessor(const BoxEvaluation& ev) : ev_(ev) {}
   BoxGraph compile(const FheCircuit& c) const { return BoxGraph(ev_, c); }
+  BoxGraph compile(const FheCircuit& c, const std::vector<int>& ranks) const { return BoxGraph(ev_, c, ranks); }
   void run_graph_blocking(const FheCircuit& c) const { compile(c).run(); }
 
  private:

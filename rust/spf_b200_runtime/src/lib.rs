@@ -9,8 +9,9 @@
 //!   (`circuit_processor/mod.rs:573-655`): [`Graph::spawn`] returns at once and calls the completion handler with the
 //!   first error (`completion_handler.rs:14-56`); [`DeviceCiphertext`] handles keep task outputs in HBM between graphs
 //!   (`circuit_processor/task.rs:10-16`).
-//! * [`BoxEvaluation`] / [`BoxGraph`]: the same over every GPU of a box, from one thread (one handle, one key upload);
-//!   [`BoxCiphertext`] handles keep task outputs in HBM between box graphs, one replica per rank.
+//! * [`BoxEvaluation`] / [`BoxGraph`]: the same over every GPU of a box, from one thread (one handle, one key upload),
+//!   or over chosen ranks of it ([`BoxGraph::build_on`]); [`BoxCiphertext`] handles keep task outputs in HBM between
+//!   box graphs, one replica per rank.
 //! * module [`parasol`] (feature `parasol`): the glue a maintainer pastes into `parasol_runtime` so that
 //!   `CircuitProcessor::exec_op` (`circuit_processor/mod.rs:255-546`) dispatches to the GPU.
 //!
@@ -451,8 +452,8 @@ impl Drop for BoxCiphertext {
     }
 }
 
-/// A validated, levelised `FheCircuit` over every rank of a [`BoxEvaluation`] (`spf_b200_box_graph_build`).  io buffers
-/// are host memory or [`BoxCiphertext::as_io`].
+/// A validated, levelised `FheCircuit` over every rank of a [`BoxEvaluation`] (`spf_b200_box_graph_build`), or over the
+/// ranks chosen with [`BoxGraph::build_on`].  io buffers are host memory or [`BoxCiphertext::as_io`].
 pub struct BoxGraph {
     raw: NonNull<RawBoxGraph>,
     ev: BoxEvaluation,
@@ -467,6 +468,26 @@ impl BoxGraph {
             Some(p) if rc == 0 => Ok(Self { raw: p, ev: ev.clone() }),
             _ => Err(Error { code: rc, message: box_error(ev.raw()) }),
         }
+    }
+    /// The graph on the box ranks `ranks` only (`spf_b200_box_graph_build_on`): member `i` runs on box rank `ranks[i]`,
+    /// and the graph is sharded over the members as over a box of `ranks.len()` ranks.  Handle outputs still reach the
+    /// replica of every rank.  A graph that writes a handle another graph reads, on any rank, must be named in that
+    /// reader's `after`.
+    pub fn build_on(ev: &BoxEvaluation, nodes: &[spf_node], ranks: &[i32]) -> Result<Self> {
+        let mut raw = ptr::null_mut();
+        let n = c_int::try_from(ranks.len()).unwrap_or(c_int::MAX);  // the library refuses more ranks than the box has
+        let rc = unsafe { sys::spf_b200_box_graph_build_on(ev.raw(), nodes.as_ptr(), nodes.len(), ranks.as_ptr(), n, &mut raw) };
+        match NonNull::new(raw) {
+            Some(p) if rc == 0 => Ok(Self { raw: p, ev: ev.clone() }),
+            _ => Err(Error { code: rc, message: box_error(ev.raw()) }),
+        }
+    }
+    /// The box ranks the graph runs on, in member order.
+    pub fn ranks(&self) -> Vec<i32> {
+        let n = unsafe { sys::spf_b200_box_graph_ranks(self.raw.as_ptr(), ptr::null_mut()) };
+        let mut out = vec![0; n.max(0) as usize];
+        unsafe { sys::spf_b200_box_graph_ranks(self.raw.as_ptr(), out.as_mut_ptr()) };
+        out
     }
     /// `CircuitProcessor::run_graph_blocking` over the box.
     pub fn run_blocking(&mut self) -> Result<()> {
@@ -709,13 +730,19 @@ pub mod parasol {
 
     /// [`spawn_graph`] on a box with task outputs in HBM: the io buffers in `resident` are mapped to their
     /// [`BoxCiphertext`]s, and the run is ordered on the devices behind the last runs of `after` (the graphs of the
-    /// instructions whose outputs it reads).
+    /// instructions whose outputs it reads, and of those that read what it writes).  `ranks`: the box ranks the graph
+    /// runs on ([`BoxGraph::build_on`]; `None` = every rank), so that independent instructions run on different GPUs.
     pub fn spawn_box_graph<F>(b: &BoxEvaluation, circuit: &parasol_runtime::FheCircuit, resident: &BoxResident<'_>, after: &[&BoxGraph],
-                              on_completion: F) -> Option<BoxGraph>
+                              ranks: Option<&[i32]>, on_completion: F) -> Option<BoxGraph>
     where
         F: FnOnce(Option<Error>) + Send + 'static,
     {
-        match BoxGraph::build(b, &lower_resident(circuit, resident)) {
+        let nodes = lower_resident(circuit, resident);
+        let built = match ranks {
+            None => BoxGraph::build(b, &nodes),
+            Some(r) => BoxGraph::build_on(b, &nodes, r),
+        };
+        match built {
             Err(e) => {
                 on_completion(Some(e));
                 None

@@ -9,6 +9,7 @@ entry point raises.  Nothing here imports the test oracle.
 from __future__ import annotations
 
 import ctypes as C
+import operator
 import os
 
 import numpy as np
@@ -474,6 +475,8 @@ ABI.update({
     "spf_b200_box_keyswitch_lwe_l1_lwe_l0": [_vp, _vp, _vp, _sz],
     "spf_b200_box_cmux": [_vp, _vp, _vp, _vp, _vp, _sz],
     "spf_b200_box_graph_build": [_vp, C.POINTER(_Node), _sz, C.POINTER(_vp)],
+    "spf_b200_box_graph_build_on": [_vp, C.POINTER(_Node), _sz, C.POINTER(C.c_int), C.c_int, C.POINTER(_vp)],
+    "spf_b200_box_graph_ranks": [_vp, C.POINTER(C.c_int)],
     "spf_b200_box_graph_run": [_vp],
     "spf_b200_box_graph_spawn": [_vp, C.POINTER(_vp), _sz, _vp, _vp],
     "spf_b200_box_graph_wait": [_vp],
@@ -748,16 +751,19 @@ def plan_graph(circuit: "FheCircuit", world: int = 1, params: Params | None = No
 class CircuitProcessor:
     """CircuitProcessor (parasol_runtime/src/circuit_processor/mod.rs:62-655) on the GPU: a graph is
     compiled once into per-level batched launches and can be run repeatedly.  On a BoxEvaluation every graph runs
-    over all GPUs of the box (BoxGraph) from the calling thread."""
+    over all GPUs of the box (BoxGraph) from the calling thread, or over the box ranks named in `ranks`."""
 
     def __init__(self, evaluation: "Evaluation | BoxEvaluation"):
         self.ev = evaluation
 
-    def compile(self, circuit: FheCircuit, world: int = 1, rank: int = 0, exchange=None) -> "CompiledGraph | BoxGraph":
+    def compile(self, circuit: FheCircuit, world: int = 1, rank: int = 0, exchange=None,
+                ranks=None) -> "CompiledGraph | BoxGraph":
         if isinstance(self.ev, BoxEvaluation):
             if world != 1 or rank != 0 or exchange is not None:
                 raise SpfError(-1, "a box graph is sharded over the box's ranks: world / rank / exchange do not apply")
-            return BoxGraph(self.ev, circuit)
+            return BoxGraph(self.ev, circuit, ranks=ranks)
+        if ranks is not None:
+            raise SpfError(-1, "ranks place a graph on ranks of a BoxEvaluation; this evaluation is a single context")
         return CompiledGraph(self.ev, circuit, world=world, rank=rank, exchange=exchange)
 
     def run_graph_blocking(self, circuit: FheCircuit) -> None:
@@ -769,14 +775,14 @@ class CircuitProcessor:
         finally:
             g.close()
 
-    def spawn_graph(self, circuit: FheCircuit, on_completion=None, after=()) -> "CompiledGraph":
+    def spawn_graph(self, circuit: FheCircuit, on_completion=None, after=(), ranks=None) -> "CompiledGraph":
         """spawn_graph (mod.rs:573-623): dispatches the graph and returns; `on_completion(error)` is called once when all
         of its ops have retired, with None or the first SpfError (CompletionHandler, completion_handler.rs:14-56) --
         validation errors included, as in the reference.  Outputs must not be read before.  Returns the compiled graph:
         pass it in `after` of a later spawn that consumes this one's DeviceCiphertext outputs, and close() it after
-        wait()."""
+        wait().  `ranks` (BoxEvaluation only): the box ranks the graph runs on, as in BoxGraph."""
         try:
-            g = self.compile(circuit)
+            g = self.compile(circuit, ranks=ranks)
         except SpfError as e:
             if on_completion is None:
                 raise
@@ -1078,15 +1084,29 @@ class BoxEvaluation:
 
 
 class BoxGraph:
-    """A graph over every rank of a BoxEvaluation (spf_b200_box_graph_*), with the CompiledGraph surface: run, spawn,
+    """A graph over the ranks of a BoxEvaluation (spf_b200_box_graph_*), with the CompiledGraph surface: run, spawn,
     wait, set_io, levels, launches, close.  io buffers are host numpy arrays or BoxCiphertext handles of the same box
-    (DeviceCiphertext handles are refused)."""
+    (DeviceCiphertext handles are refused).  `ranks`: the box ranks the graph runs on, in member order (None: every
+    rank in order); the graph is sharded over them as over a box of len(ranks) ranks.  Handle outputs still reach the
+    replica of every rank of the box.  A graph that writes a handle another graph reads, on any rank, must be in that
+    reader's `after` (and the reader in the writer's, when the writer runs later)."""
 
-    def __init__(self, box: BoxEvaluation, circuit: FheCircuit):
+    def __init__(self, box: BoxEvaluation, circuit: FheCircuit, ranks=None):
         self.ev = box
         self._keep = circuit
         self._h = _vp()
-        box._check(lib().spf_b200_box_graph_build(box.handle, circuit._pack(), len(circuit.nodes), C.byref(self._h)))
+        if ranks is None:
+            box._check(lib().spf_b200_box_graph_build(box.handle, circuit._pack(), len(circuit.nodes), C.byref(self._h)))
+            return
+        try:
+            rs = [operator.index(r) for r in ranks]
+        except TypeError:
+            raise SpfError(-1, f"BoxGraph: ranks must be a sequence of box rank numbers, got {ranks!r}") from None
+        if any(not -2**31 <= r < 2**31 for r in rs):  # a C int each: no silent wrap-around into a valid rank
+            raise SpfError(-1, f"BoxGraph: ranks {rs} are not ranks of a box")
+        arr = (C.c_int * max(len(rs), 1))(*rs)
+        box._check(lib().spf_b200_box_graph_build_on(box.handle, circuit._pack(), len(circuit.nodes), arr, len(rs),
+                                                     C.byref(self._h)))
 
     def run(self) -> None:
         self.ev._check(lib().spf_b200_box_graph_run(self._h))
@@ -1127,6 +1147,14 @@ class BoxGraph:
     @property
     def launches(self) -> int:
         return int(lib().spf_b200_box_graph_launches(self._h))
+
+    @property
+    def ranks(self) -> list[int]:
+        """The box ranks the graph runs on, in member order."""
+        n = int(lib().spf_b200_box_graph_ranks(self._h, None))
+        out = (C.c_int * max(n, 1))()
+        lib().spf_b200_box_graph_ranks(self._h, out)
+        return list(out[:n])
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:

@@ -2,8 +2,10 @@
 // graph.cuh.  One process, one dispatching thread: a rank is a context on its own device; the compute key is uploaded
 // once and replicated device to device; host-pointer ops split the batch over the ranks and run them concurrently on
 // one worker thread per rank; a box graph is a sharded graph per rank, wired to the other ranks' arenas in-process,
-// and every rank's run is enqueued from the calling thread, level by level across the ranks.  A box ciphertext handle
-// holds one replica of a ciphertext per rank, so that box graphs hand their outputs to the next graph in HBM.
+// and every rank's run is enqueued from the calling thread, level by level across the ranks.  A box graph runs on an
+// ordered subset of the box's ranks, its MEMBERS (all ranks in order by default): member i runs shard i of the graph
+// sharded over the members.  A box ciphertext handle holds one replica of a ciphertext per rank of the box, so that box
+// graphs hand their outputs to the next graph in HBM, whichever ranks either graph runs on.
 #include <array>
 #include <functional>
 #include <thread>
@@ -43,10 +45,11 @@ struct spf_b200_box_ciphertext {
 
 struct spf_b200_box_graph {
   spf_b200_box* box = nullptr;
-  std::vector<spf_b200_graph*> g;  // rank r's sharded graph, on rank r's context
+  std::vector<int> rank;           // member i's box rank
+  std::vector<spf_b200_graph*> g;  // member i's sharded graph (shard i of rank.size()), on box rank rank[i]'s context
   std::vector<spf_b200_box_ciphertext*> bound;  // per node: the box ciphertext handle bound to it (a reference), or NULL
   std::vector<void*> pinned;       // host io buffers page-locked (portable: every device DMAs them) by this box graph
-  int* h_err = nullptr;            // page-locked copy of every rank's barrier error word, read by the completion
+  int* h_err = nullptr;            // page-locked copy of every member's barrier error word, read by the completion
   std::atomic<int> status{0};
   std::string status_msg;
   std::atomic<bool> poisoned{false};
@@ -183,11 +186,15 @@ int launch_box_copy(spf_b200_ctx* ctx, const std::vector<BoxCopyItem>& items, cu
   return 0;
 }
 
-// Rank r's handle traffic of one run, enqueued on its stream: inputs copy the rank's own replica into its arena;
-// outputs every rank holds (output rank -1) go to the rank's own replica; outputs of a MUX tree go from the owner to
-// the replicas of every rank.
-int enqueue_handle_copies(spf_b200_box_graph* bg, int r, bool outputs) {
-  spf_b200_graph* g = bg->g[r];
+// Member i's handle traffic of one run, enqueued on its stream: inputs copy the replica of the member's box rank into
+// its arena.  Outputs reach the replicas of EVERY rank of the box, members or not: an output every member holds
+// (output rank -1) goes from each member to its own replica, and from member 0 also to the replicas of the ranks
+// outside the graph; an output of a MUX tree goes from its owner member to every replica.
+int enqueue_handle_copies(spf_b200_box_graph* bg, int i, bool outputs) {
+  spf_b200_graph* g = bg->g[i];
+  const int n_box = bg->box->n;
+  std::vector<char> member(n_box, 0);
+  for (int r : bg->rank) member[r] = 1;
   std::vector<BoxCopyItem> items;
   for (int id : outputs ? g->outputs : g->inputs) {
     if (g->io_kind[id] != 3) continue;
@@ -195,14 +202,15 @@ int enqueue_handle_copies(spf_b200_box_graph* bg, int r, bool outputs) {
     BoxCopyItem it{};
     it.n8 = (unsigned)(h->bytes / 8);
     if (!outputs) {
-      it.src = reinterpret_cast<const unsigned long long*>(h->rep[r]);
+      it.src = reinterpret_cast<const unsigned long long*>(h->rep[bg->rank[i]]);
       it.dst[it.n_dst++] = reinterpret_cast<unsigned long long*>(g->dptr[id]);
     } else {
       const int owner = spf_b200_graph_output_rank(g, id);
-      if (owner >= 0 && owner != r) continue;
+      if (owner >= 0 && owner != i) continue;
       it.src = reinterpret_cast<const unsigned long long*>(g->dptr[g->nodes[id].in[0]]);
-      for (size_t q = 0; q < h->rep.size(); q++)
-        if (owner >= 0 || (int)q == r) it.dst[it.n_dst++] = reinterpret_cast<unsigned long long*>(h->rep[q]);
+      for (int q = 0; q < n_box; q++)
+        if (owner >= 0 || q == bg->rank[i] || (i == 0 && !member[q]))
+          it.dst[it.n_dst++] = reinterpret_cast<unsigned long long*>(h->rep[q]);
     }
     items.push_back(it);
   }
@@ -210,7 +218,8 @@ int enqueue_handle_copies(spf_b200_box_graph* bg, int r, bool outputs) {
   return launch_box_copy(g->ctx, items, g->stream);
 }
 
-// Whether some handle-bound output is written by one rank into the replicas of the others.
+// Whether some handle-bound output is written by one member into the replicas of the others (with two or more
+// members; the replicas of non-members written by member 0 are not read by this graph).
 bool has_owned_handle_outputs(const spf_b200_graph* g) {
   for (int id : g->outputs)
     if (g->io_kind[id] == 3 && spf_b200_graph_output_rank(g, id) >= 0) return true;
@@ -408,18 +417,18 @@ void CUDART_CB box_rank_done(void* arg) {
   delete rec;
 }
 
-// Enqueues one run on every rank from the calling thread, level-interleaved: the inputs of every rank, then group k of
-// every rank for k = 0, 1, ..., then the outputs of every rank.  So when the host has to wait for a rank's stream (its
-// launch queue is full), every other rank's work up to the same level -- and so to the same peer barrier -- is
-// enqueued already, and the wait ends.  Returns the first error; ranks after a failed one are not enqueued further.
-// Box ciphertext handles: each rank reads its own replica right after its other inputs.  When an owner writes the
-// replicas of other ranks at the end, a barrier after the inputs first makes sure that every rank has read its
-// replica (a graph may read and write the same handle, and need not have a bootstrap level, whose barrier would do);
-// the start-of-run barrier keeps these writes ahead of the next run's reads.
+// Enqueues one run on every member from the calling thread, level-interleaved: the inputs of every member, then group k
+// of every member for k = 0, 1, ..., then the outputs of every member.  So when the host has to wait for a member's
+// stream (its launch queue is full), every other member's work up to the same level -- and so to the same peer barrier
+// -- is enqueued already, and the wait ends.  Returns the first error; members after a failed one are not enqueued
+// further.  Box ciphertext handles: each member reads its own replica right after its other inputs.  When an owner
+// writes the replicas of other members at the end, a barrier after the inputs first makes sure that every member has
+// read its replica (a graph may read and write the same handle, and need not have a bootstrap level, whose barrier
+// would do); the start-of-run barrier keeps these writes ahead of the next run's reads.
 int box_enqueue(spf_b200_box_graph* bg) {
   spf_b200_box* b = bg->box;
   const int n = (int)bg->g.size();
-  auto rank_fail = [&](int r, int rc) { return box_fail(b, rc, "rank " + std::to_string(r) + ": " + bg->g[r]->ctx->err); };
+  auto rank_fail = [&](int r, int rc) { return box_fail(b, rc, "rank " + std::to_string(bg->rank[r]) + ": " + bg->g[r]->ctx->err); };
   for (int r = 0; r < n; r++)
     if (int rc = prepare_run(bg->g[r], r)) return rank_fail(r, rc);
   for (int r = 0; r < n; r++) {
@@ -606,10 +615,23 @@ void spf_b200_box_graph_destroy(spf_b200_box_graph* bg) {
   box_release(b);
 }
 
-int spf_b200_box_graph_build(spf_b200_box* b, const spf_node* nodes, size_t n_nodes, spf_b200_box_graph** out) {
+int spf_b200_box_graph_build_on(spf_b200_box* b, const spf_node* nodes, size_t n_nodes, const int* ranks, int n_ranks,
+                                spf_b200_box_graph** out) {
   if (!b) return SPF_E_INVALID;
   if (!out || (!nodes && n_nodes)) return box_fail(b, SPF_E_INVALID, "NULL argument");
   *out = nullptr;
+  if (!ranks) return box_fail(b, SPF_E_INVALID, "box graph: ranks is NULL");
+  if (n_ranks < 1 || n_ranks > b->n)
+    return box_fail(b, SPF_E_INVALID, "box graph: n_ranks is " + std::to_string(n_ranks) + ", must be in 1.." + std::to_string(b->n) +
+                                          " (the box size)");
+  std::vector<char> seen(b->n, 0);
+  for (int i = 0; i < n_ranks; i++) {
+    if (ranks[i] < 0 || ranks[i] >= b->n)
+      return box_fail(b, SPF_E_INVALID, "box graph: ranks[" + std::to_string(i) + "] = " + std::to_string(ranks[i]) +
+                                            " is not a rank of the box (0.." + std::to_string(b->n - 1) + ")");
+    if (seen[ranks[i]]++)
+      return box_fail(b, SPF_E_INVALID, "box graph: rank " + std::to_string(ranks[i]) + " is named twice in ranks");
+  }
   const spf_params* p = &b->ctx[0]->p;
   BCU(b, cudaSetDevice(b->device[0]));
   // io buffers: box ciphertext handles or host memory.  Unpinned host buffers are page-locked here as PORTABLE memory,
@@ -642,24 +664,40 @@ int spf_b200_box_graph_build(spf_b200_box* b, const spf_node* nodes, size_t n_no
     if (cudaHostRegister(nodes[i].io, bytes, cudaHostRegisterPortable) == cudaSuccess) bg->pinned.push_back(nodes[i].io);
     else cudaGetLastError();  // left pageable: the rank graphs stage it through their page-locked slabs
   }
-  const int n = b->n;
+  // member i runs shard i of the graph sharded over the members; member 0 writes the outputs every member holds
+  const int n = n_ranks;
+  bg->rank.assign(ranks, ranks + n);
   bg->g.assign(n, nullptr);
-  for (int r = 0; r < n; r++) {
-    if (int rc = graph_build_checked(b->ctx[r], nodes, n_nodes, n, &bg->g[r], true))
-      return box_fail(b, rc, (r ? "rank " + std::to_string(r) + ": " : std::string()) + b->ctx[r]->err);
-    bg->g[r]->replicated_writer = 0;
-    settle_all_io(bg->g[r]);
+  for (int i = 0; i < n; i++) {
+    spf_b200_ctx* c = b->ctx[bg->rank[i]];
+    if (int rc = graph_build_checked(c, nodes, n_nodes, n, &bg->g[i], true))
+      return box_fail(b, rc, (bg->rank[i] ? "rank " + std::to_string(bg->rank[i]) + ": " : std::string()) + c->err);
+    bg->g[i]->replicated_writer = 0;
+    settle_all_io(bg->g[i]);
   }
   if (n > 1) {
     std::vector<void*> arenas(n);
-    for (int r = 0; r < n; r++) arenas[r] = bg->g[r]->arena;
-    for (int r = 0; r < n; r++)
-      if (int rc = spf_b200_graph_set_peers(bg->g[r], r, n, arenas.data())) return box_fail(b, rc, b->ctx[r]->err);
+    for (int i = 0; i < n; i++) arenas[i] = bg->g[i]->arena;
+    for (int i = 0; i < n; i++)
+      if (int rc = spf_b200_graph_set_peers(bg->g[i], i, n, arenas.data())) return box_fail(b, rc, bg->g[i]->ctx->err);
   }
   BCU(b, cudaHostAlloc(reinterpret_cast<void**>(&bg->h_err), sizeof(int) * n, cudaHostAllocPortable));
   memset(bg->h_err, 0, sizeof(int) * n);
   *out = bg.release();
   return 0;
+}
+
+int spf_b200_box_graph_build(spf_b200_box* b, const spf_node* nodes, size_t n_nodes, spf_b200_box_graph** out) {
+  if (!b) return SPF_E_INVALID;
+  std::vector<int> all(b->n);
+  for (int r = 0; r < b->n; r++) all[r] = r;
+  return spf_b200_box_graph_build_on(b, nodes, n_nodes, all.data(), b->n, out);
+}
+
+int spf_b200_box_graph_ranks(const spf_b200_box_graph* bg, int* ranks_out) {
+  if (!bg) return SPF_E_INVALID;
+  if (ranks_out) std::copy(bg->rank.begin(), bg->rank.end(), ranks_out);
+  return (int)bg->rank.size();
 }
 
 int spf_b200_box_graph_run(spf_b200_box_graph* bg) {
@@ -729,17 +767,18 @@ int spf_b200_box_graph_spawn(spf_b200_box_graph* bg, spf_b200_box_graph* const* 
   for (size_t i = 0; i < n_after && rec->status == 0; i++) {
     spf_b200_box_graph* d = after[i];
     if (!d || d == bg) continue;
-    if (d->box != b || d->g.size() != bg->g.size()) {
+    if (d->box != b) {
       rec->status = SPF_E_INVALID;
       rec->msg = "spawn: a dependency belongs to another box";
     } else if (const int ds = d->status.load()) {
       rec->status = ds;
       rec->msg = "a dependency of this graph failed: " + d->status_msg;
     } else {
-      // every rank waits for every rank of the dependency: an output is written by one rank, read by all
+      // every member waits for every member of the dependency, whichever ranks either runs on (a cross-device wait
+      // when they differ): an output is written by one member into every replica, read by all
       for (int r = 0; r < n && rec->status == 0; r++) {
         cudaSetDevice(bg->g[r]->ctx->device);
-        for (int q = 0; q < n && rec->status == 0; q++)
+        for (size_t q = 0; q < d->g.size() && rec->status == 0; q++)
           if (cudaStreamWaitEvent(bg->g[r]->stream, d->g[q]->done, 0) != cudaSuccess) {
             rec->status = SPF_E_CUDA;
             rec->msg = "cudaStreamWaitEvent on a dependency failed";

@@ -3,9 +3,12 @@ bootstrapping, and N x (mul32 then greater-than) in one box graph, blocking and 
 records it under profiles/ (--out).  The same measurements as bench.py's multi-process line, so the two compare.
 --chain measures instead a two-instruction program run as two box graphs (mul32, then greater-than on the product),
 with the 32 product bits handed over through host buffers or through box ciphertext handles.
+--placed K measures K independent mul32-then-greater-than programs spawned as K box graphs, the way a Parasol
+processor issues instructions: every graph over all ranks, against program i placed on rank i mod N.
 
 usage: python tools/box_bench.py [--devices 0,1,...] [--batch 4096] [--steps 10] [--out profiles/box_bench_n8.json]
-       python tools/box_bench.py --chain [--devices 0,0] [--reps 20] [--out profiles/box_chain_n1.json]"""
+       python tools/box_bench.py --chain [--devices 0,0] [--reps 20] [--out profiles/box_chain_n1.json]
+       python tools/box_bench.py --placed 8 [--devices 0,0] [--reps 10] [--out profiles/box_place_n1.json]"""
 import argparse
 import ctypes as C
 import json
@@ -259,6 +262,82 @@ def chain(box, keys, n_programs, reps, warmup):
     return res
 
 
+def placed(box, keys, k, reps, warmup):
+    """k independent programs (32-bit multiply, low word, then greater-than), one box graph each as programs() builds
+    them, with max_in_flight = k: all k graphs spawned, then all k waited for.  Two modes, alternated round by round:
+    "all_ranks" builds every graph over the whole box (spf_b200_box_graph_build), "placed" puts program i on rank
+    i mod N alone (spf_b200_box_graph_build_on).  Times are host clocks around a batch of k, ending after the last
+    wait (median over reps); every output of every timed batch is zeroed before and decrypted after it."""
+    import oracle as O
+    import spf_b200
+    from spf_b200.circuits import multiply_then_greater_than
+
+    client = O.Client(keys)
+    w, n = 32, box.size
+    rng = np.random.default_rng(0xB0C7)
+    vals = [tuple(int(x) for x in rng.integers(0, 1 << w, 3)) for _ in range(k)]
+    modes = ("all_ranks", "placed")
+    slab = iter(spf_b200.pinned_zeros((k * 3 * w + len(modes) * k * (w + 1), keys.glwe_len)))
+
+    def enc(v):
+        out = [next(slab) for _ in range(w)]
+        for i, r in enumerate(out):
+            r[:] = client.encrypt_glwe_l1([(v >> i) & 1])
+        return out
+
+    a, b, c = ([enc(v[j]) for v in vals] for j in range(3))
+    outs, graphs = {}, {}
+    for m in modes:
+        out_prod = [[next(slab) for _ in range(w)] for _ in vals]
+        out_gt = [next(slab) for _ in vals]
+        outs[m] = (out_prod, out_gt)
+        graphs[m] = [spf_b200.BoxGraph(box, multiply_then_greater_than([a[i]], [b[i]], [c[i]], [out_prod[i]], [out_gt[i]], 1),
+                                       ranks=None if m == "all_ranks" else [i % n]) for i in range(k)]
+
+    def correct(m):
+        ok = True
+        out_prod, out_gt = outs[m]
+        for (x, y, z), pb, gt in zip(vals, out_prod, out_gt):
+            p = sum(int(client.decrypt_glwe_l1(o)[0]) << i for i, o in enumerate(pb))
+            ok &= p == (x * y) % (1 << w) and int(client.decrypt_glwe_l1(gt)[0]) == int(p > z)
+        return bool(ok)
+
+    def batch(m):
+        out_prod, out_gt = outs[m]
+        for o in [x for pb in out_prod for x in pb] + out_gt:
+            o[:] = 0
+        fired = []
+        t0 = time.perf_counter()
+        for g in graphs[m]:
+            g.spawn(on_complete=fired.append)
+        for g in graphs[m]:
+            g.wait()
+        t = time.perf_counter() - t0
+        return t, len(fired) == k and not any(fired) and correct(m)
+
+    box.set_max_in_flight(k)
+    for _ in range(max(warmup, 1)):
+        for m in modes:
+            batch(m)
+    times = {m: [] for m in modes}
+    ok = {m: True for m in modes}
+    for _ in range(reps):
+        for m in modes:
+            t, good = batch(m)
+            times[m].append(t)
+            ok[m] &= good
+    res = {"programs": k, "ranks": n, "levels": graphs["all_ranks"][0].levels,
+           "placement": [g.ranks for g in graphs["placed"]]}
+    for m in modes:
+        res[m] = {"batch_ms": 1e3 * float(np.median(times[m])), "batch_ms_min": 1e3 * float(np.min(times[m])),
+                  "batch_ms_max": 1e3 * float(np.max(times[m])), "launches": sum(g.launches for g in graphs[m]),
+                  "correct": ok[m]}
+    for g in [g for gs in graphs.values() for g in gs]:
+        g.close()
+    box.set_max_in_flight(4)
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--devices", default=None, help="comma-separated device list (default: every visible GPU)")
@@ -269,6 +348,8 @@ def main():
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     ap.add_argument("--chain", action="store_true", help="measure the two-graph mul32 | greater-than hand-off only")
     ap.add_argument("--programs", type=int, default=1, help="--chain: programs per graph")
+    ap.add_argument("--placed", type=int, default=0, metavar="K",
+                    help="measure K independent program graphs over all ranks against placed on rank i mod N")
     args = ap.parse_args()
 
     import torch
@@ -279,13 +360,19 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("box_bench.py: no CUDA device; spf_b200 has no CPU fallback")
     devices = [int(x) for x in args.devices.split(",")] if args.devices else list(range(torch.cuda.device_count()))
-    line = {"metric": "box_chain" if args.chain else "box_bench", "devices": devices, "gpus": gpu_identity(devices)}
+    metric = "box_chain" if args.chain else "box_place" if args.placed else "box_bench"
+    line = {"metric": metric, "devices": devices, "gpus": gpu_identity(devices)}
     keys = O.Keys()
     t0 = time.perf_counter()
     box = spf_b200.BoxEvaluation(keys.bsk_fft, keys.ksk, keys.ssk_fft, keys.ak_fft, devices=devices)
     line["box_create_ms"] = 1e3 * (time.perf_counter() - t0)
     line["key_replication_ms"] = box.key_replication_ms
     n = box.size
+    if args.placed:
+        line["placed"] = placed(box, keys, args.placed, args.reps, args.warmup)
+        box.close()
+        emit(line, args.out)
+        return
     if args.chain:
         line["chain"] = chain(box, keys, args.programs, max(args.reps, 20), args.warmup)
         box.close()
