@@ -40,9 +40,8 @@ struct spf_b200_ctx {
   C2 *bsk = nullptr, *ak = nullptr, *ssk = nullptr;
   uint64_t* ksk = nullptr;
   uint64_t* ksk_colsum = nullptr;  // keyswitch_kernel's per-block column sums of the KSK
-  uint4* ks_bfrag = nullptr;       // keyswitch_tc_kernel: KSK byte planes in mma B-fragment order (nullptr: shape unsupported)
-  uint64_t* ks_tc_colsum = nullptr;  // keyswitch_tc_kernel: per-(chunk, level) column sums
-  uint8_t* ks_btiles = nullptr;      // keyswitch_umma_kernel: KSK byte planes as canonical K-major UMMA tiles
+  uint64_t* ks_tc_colsum = nullptr;  // keyswitch_umma_kernel: per-(chunk, level) column sums
+  uint8_t* ks_btiles = nullptr;      // keyswitch_umma_kernel: KSK byte planes as canonical K-major UMMA tiles (nullptr: shape unsupported)
   C2 *T1 = nullptr, *T2 = nullptr;
   uint32_t* kinv = nullptr;
   cudaStream_t stream[2] = {nullptr, nullptr};
@@ -198,7 +197,6 @@ int create_common(const spf_params* params, const double* bsk, size_t bsk_len, c
   CUB(cudaFuncSetAttribute(trace_ss_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTrSmem));
   CUB(cudaFuncSetAttribute(cmux_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCmuxSmem));
   CUB(cudaFuncSetAttribute(cmux_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWideSmem));
-  CUB(cudaFuncSetAttribute(cmux_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWideSmem));
   {
     const int ks_smem = kKsBatch * (int)(params->glwe_k * params->glwe_n + kKsBlock) * 4;
     switch (params->ks.count) {
@@ -220,13 +218,6 @@ int create_common(const spf_params* params, const double* bsk, size_t bsk_len, c
     CUB(cudaMemcpy(ctx->T1, T1.data(), sizeof(C2) * kT1Elems, cudaMemcpyHostToDevice));
     CUB(cudaMemcpy(ctx->T2, T2.data(), sizeof(C2) * kT2Elems, cudaMemcpyHostToDevice));
     CUB(cudaMemcpy(ctx->kinv, kinv, sizeof(kinv), cudaMemcpyHostToDevice));
-    // constants of the in-register transforms, in the order the kernels consume them (fft16.cuh: constant pools)
-    static double pools[kPools][kPoolLen];
-    if (!fill_kpools(pools)) {
-      spf_b200_destroy(ctx);
-      return SPF_E_INVALID;
-    }
-    CUB(cudaMemcpyToSymbol(spf_kpool, pools, sizeof(pools)));
   }
   // keys: FFT-domain keys are rescaled by 2^-10 in place on the device (exact)
   const cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
@@ -249,21 +240,16 @@ int create_common(const spf_params* params, const double* bsk, size_t bsk_len, c
     ksk_colsum_kernel<<<dim3((cols + 127) / 128, nblk), 128, 0, ctx->stream[0]>>>(ctx->ksk_colsum, ctx->ksk, n1,
                                                                                    (int)params->ks.count, cols);
     CUB(cudaGetLastError());
-    // tensor-core keyswitch (kernels.cuh K4t): KSK byte planes in fragment order + per-chunk column sums
+    // tensor-core keyswitch (kernels.cuh K4u): per-chunk column sums + the KSK byte planes as UMMA tiles
     const int L = (int)params->ks.count, lb = (int)params->ks.radix_log;
     // byte-plane GEMMs accumulate in s32: (B - 1) * 255 per term, n1 * L terms
     const bool s32_ok = (uint64_t)n1 * L * ((1u << lb) - 1) * 255ull < (1ull << 31);
     if (n1 % kKtIC == 0 && L * lb + 1 <= 16 && lb <= 8 && s32_ok) {
-      const int n_tiles = (cols + kKtN - 1) / kKtN * (kKtN / 8), ks_total = n1 * L / 32, chunks = n1 / kKtIC * L;
-      const size_t slots = (size_t)n_tiles * ks_total * 32;
-      CUB(cudaMalloc(&ctx->ks_bfrag, slots * 4 * sizeof(uint4)));
+      const int ks_total = n1 * L / 32, chunks = n1 / kKtIC * L;
       CUB(cudaMalloc(&ctx->ks_tc_colsum, sizeof(uint64_t) * (size_t)chunks * cols));
-      ks_tc_prepare_kernel<<<(unsigned)((slots + 255) / 256), 256, 0, ctx->stream[0]>>>(ctx->ks_bfrag, ctx->ksk, n1, L, cols, n_tiles);
-      CUB(cudaGetLastError());
       ks_tc_colsum_kernel<<<dim3((cols + 127) / 128, chunks), 128, 0, ctx->stream[0]>>>(ctx->ks_tc_colsum, ctx->ksk, n1, L, cols);
       CUB(cudaGetLastError());
-      CUB(cudaFuncSetAttribute(keyswitch_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kKtSmem));
-      // tcgen05 keyswitch (K4u): the same planes as canonical K-major UMMA tiles, 16 KiB per (column block, k-step)
+      // the KSK byte planes as canonical K-major UMMA tiles, 16 KiB per (column block, k-step)
       const int n_blocks = (cols + kKuN - 1) / kKuN;
       const size_t tile_bytes = (size_t)n_blocks * ks_total * kKuBTile;
       CUB(cudaMalloc(&ctx->ks_btiles, tile_bytes));
@@ -312,11 +298,10 @@ int launch_pbs(spf_b200_ctx* ctx, uint64_t* d_glwe_out, const uint64_t* d_lwe_in
   // Tail wave: a batch is a whole number of waves (sm_count x kPbsPairs ciphertexts) plus a remainder.  A remainder of
   // at most one ciphertext per SM would run as one pair per SM after everything else has finished (5.1 ms for e.g. the
   // last 100 of 4096 ciphertexts); the four-team latency kernel does the same work in 3.5 ms, so the remainder goes
-  // there (same stream, right behind the full waves).  SPF_B200_PBS_TAIL=pair keeps everything on the pair kernel.
-  static const bool quad_tail = [] { const char* e = getenv("SPF_B200_PBS_TAIL"); return !(e && !strcmp(e, "pair")); }();
+  // there (same stream, right behind the full waves).
   const size_t wave = (size_t)ctx->sm_count * kPbsPairs;
   const size_t rem = batch % wave;
-  if (quad_tail && batch > wave && rem > 0 && rem <= (size_t)ctx->sm_count && !P.lut_stride) {
+  if (batch > wave && rem > 0 && rem <= (size_t)ctx->sm_count && !P.lut_stride) {
     const size_t full = batch - rem;
     P.batch = (int)full;
     pbs_kernel<<<ctx->sm_count, kPbsPairs * 2 * kTeam, kPbsSmem, s>>>(P, tabs(ctx));
@@ -375,11 +360,10 @@ int launch_trace_ss(spf_b200_ctx* ctx, const uint64_t* d_glwe_in, uint64_t* d_gl
 // side stream and runs CONCURRENTLY with the trace / scheme-switch kernel of the full waves, whose thousands of short
 // CTAs fill the remaining SMs: the step ends after (all work) / (all SMs) instead of after the sum of three under-filled
 // phases.  Only scheduling depends on the first event (the remainder reads nothing the full waves write); the second one
-// orders the remainder's trace kernel behind its blind rotation.  SPF_B200_CBS_OVERLAP=0 restores the serial form.
+// orders the remainder's trace kernel behind its blind rotation.
 int launch_cbs(spf_b200_ctx* ctx, C2* d_ggsw_out, uint64_t* d_glwe, const uint64_t* d_lwe_in, const void* const* ptrs,
                double out_scale, size_t batch, cudaStream_t s, const PeerOffsets* peers = nullptr) {
   if (batch == 0) return 0;
-  static const bool overlap = [] { const char* e = getenv("SPF_B200_CBS_OVERLAP"); return !(e && !strcmp(e, "0")); }();
   const int levels = (int)ctx->p.cbs.count;
   const size_t wave = (size_t)ctx->sm_count * kPbsPairs, rem = batch % wave, full = batch - rem;
   const size_t lwe = (size_t)ctx->p.lwe_n + 1, ggsw = len_ggsw(&ctx->p, ctx->p.cbs);
@@ -394,7 +378,7 @@ int launch_cbs(spf_b200_ctx* ctx, C2* d_ggsw_out, uint64_t* d_glwe, const uint64
     const double packed = std::max(1.0, ((double)full * c * sm + tail_sms) / sm) + (double)rem * c;
     pays = packed < serial;
   }
-  if (!overlap || !pays || s == ctx->aux) {
+  if (!pays || s == ctx->aux) {
     if (int rc = launch_pbs(ctx, d_glwe, d_lwe_in, nullptr, true, 0, cbs_log_v(&ctx->p), batch, s, ptrs)) return rc;
     return launch_trace_ss(ctx, d_glwe, nullptr, d_ggsw_out, 0, levels, out_scale, batch, s, nullptr, peers);
   }
@@ -435,19 +419,17 @@ int launch_cmux(spf_b200_ctx* ctx, uint64_t* d_out, const uint64_t* d_d0, const 
   // few outputs (a level of a MUX tree): one CTA of 8 teams per output, 3-5x lower latency
   // Programmatic dependent launch: consecutive levels of a MUX tree are back-to-back CMUX kernels; each
   // loads its tables (and prefetches its selector) while the previous level drains (kernels.cuh, pdl_wait).
-  static const bool pdl = !getenv("SPF_B200_NO_PDL");
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cudaLaunchConfig_t cfg = {};
   cfg.stream = s;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   const DevTables T = tabs(ctx);
-  static const char* wide_env = getenv("SPF_B200_CMUX_WIDE_MAX");  // A/B: largest batch served by the wide kernel
   // two waves of the wide kernel still beat one team per output (cold L2: 49 vs 59 us at 296 outputs; 4 x mul32 in one
   // graph 45.2 -> 42.2 ms); from three waves on the throughput kernel wins (profiles/r1_w_cmux_kernel_choice.json)
-  const size_t wide_max = wide_env ? (size_t)atoll(wide_env) : 2 * (size_t)ctx->sm_count;
+  const size_t wide_max = 2 * (size_t)ctx->sm_count;
   if (n_glwe <= wide_max && P.count == 4) {
     cfg.gridDim = dim3((unsigned)n_glwe);
     cfg.blockDim = dim3(kWideTeams * kTeam);
@@ -477,38 +459,24 @@ int launch_keyswitch(spf_b200_ctx* ctx, uint64_t* d_out, const uint64_t* d_in, s
   P.n0 = (int)ctx->p.lwe_n;
   P.radix_log = (int)ctx->p.ks.radix_log;
   P.count = (int)ctx->p.ks.count;
-  static const bool ks_no_tc = getenv("SPF_B200_KS_NO_TC") != nullptr;  // environment knobs are read once, not per launch
-  static const bool ks_mma = [] { const char* e = getenv("SPF_B200_KS_IMPL"); return e && !strcmp(e, "mma"); }();
-  if (ctx->ks_bfrag && !ks_no_tc) {  // dense contraction on the int8 tensor cores (K4t)
-    KsTcBatch T;
+  static const bool ks_no_tc = getenv("SPF_B200_KS_NO_TC") != nullptr;  // read once, not per launch
+  if (ctx->ks_btiles && !ks_no_tc) {  // dense contraction on the int8 tensor cores (K4u)
     DevBuf& st16 = states ? *states : ctx->scratch[s == ctx->stream[1] ? 1 : 0][6];
     if (int rc = ensure(ctx, st16, batch * (size_t)P.n1 * 2)) return rc;
     ks_tc_states_kernel<<<std::min<int>((int)((batch * (size_t)P.n1 + 255) / 256), ctx->sm_count * 8), 256, 0, s>>>(
         (uint16_t*)st16.p, d_in, ptrs, P.batch, P.n1, P.radix_log, P.count);
     if (int rc = check_launch(ctx, "ks_tc_states_kernel")) return rc;
-    if (!ks_mma) {  // SPF_B200_KS_IMPL=mma: legacy mma.sync kernel (K4t); default: tcgen05 (K4u)
-      KsUBatch U;
-      U.out = d_out; U.in = d_in; U.ptrs = ptrs; U.st16 = (const uint16_t*)st16.p; U.btiles = ctx->ks_btiles; U.colsum = ctx->ks_tc_colsum;
-      U.batch = P.batch; U.n1 = P.n1; U.n0 = P.n0; U.radix_log = P.radix_log; U.count = P.count;
-      const int ux = (int)((batch + kKuM - 1) / kKuM), uy = (P.n0 + 1 + kKuN - 1) / kKuN;
-      const int chunks = P.n1 / kKtIC * P.count;
-      int z = std::max(1, std::min(chunks, (ctx->sm_count + ux * uy - 1) / (ux * uy)));  // split K until every SM has a CTA
-      U.chunks_per_cta = (chunks + z - 1) / z;
-      z = (chunks + U.chunks_per_cta - 1) / U.chunks_per_cta;
-      if (z > 1) CU(cudaMemsetAsync(d_out, 0, batch * (size_t)(P.n0 + 1) * 8, s));
-      keyswitch_umma_kernel<<<dim3(ux, uy, z), 192, kKuSmem, s>>>(U);
-      return check_launch(ctx, "keyswitch_umma_kernel");
-    }
-    T.out = d_out; T.in = d_in; T.ptrs = ptrs; T.st16 = (const uint16_t*)st16.p; T.bfrag = ctx->ks_bfrag; T.colsum = ctx->ks_tc_colsum;
-    T.batch = P.batch; T.n1 = P.n1; T.n0 = P.n0; T.radix_log = P.radix_log; T.count = P.count;
-    const int gx = (int)((batch + kKtM - 1) / kKtM), gy = (P.n0 + 1 + kKtN - 1) / kKtN;
+    KsUBatch U;
+    U.out = d_out; U.in = d_in; U.ptrs = ptrs; U.st16 = (const uint16_t*)st16.p; U.btiles = ctx->ks_btiles; U.colsum = ctx->ks_tc_colsum;
+    U.batch = P.batch; U.n1 = P.n1; U.n0 = P.n0; U.radix_log = P.radix_log; U.count = P.count;
+    const int ux = (int)((batch + kKuM - 1) / kKuM), uy = (P.n0 + 1 + kKuN - 1) / kKuN;
     const int chunks = P.n1 / kKtIC * P.count;
-    int z = std::max(1, std::min(chunks, (2 * ctx->sm_count + gx * gy - 1) / (gx * gy)));  // split K until the GPU is full
-    T.chunks_per_cta = (chunks + z - 1) / z;
-    z = (chunks + T.chunks_per_cta - 1) / T.chunks_per_cta;
+    int z = std::max(1, std::min(chunks, (ctx->sm_count + ux * uy - 1) / (ux * uy)));  // split K until every SM has a CTA
+    U.chunks_per_cta = (chunks + z - 1) / z;
+    z = (chunks + U.chunks_per_cta - 1) / U.chunks_per_cta;
     if (z > 1) CU(cudaMemsetAsync(d_out, 0, batch * (size_t)(P.n0 + 1) * 8, s));
-    keyswitch_tc_kernel<<<dim3(gx, gy, z), 256, kKtSmem, s>>>(T);
-    return check_launch(ctx, "keyswitch_tc_kernel");
+    keyswitch_umma_kernel<<<dim3(ux, uy, z), 192, kKuSmem, s>>>(U);
+    return check_launch(ctx, "keyswitch_umma_kernel");
   }
   if (P.n0 + 1 > 2 * kKsThreads) return fail(ctx, SPF_E_UNSUPPORTED, "l0 dimension too large for the keyswitch kernel");
   if (P.count > kKsMaxLevels) return fail(ctx, SPF_E_UNSUPPORTED, "ks_radix.count too large for the keyswitch kernel");
@@ -572,16 +540,9 @@ int launch_rlwe_encrypt(spf_b200_ctx* ctx, uint64_t* d_out, const uint64_t* d_pk
   return 0;
 }
 
-// Largest chunk of a host-pointer batch processed per pipeline slot: a whole number of PBS
-// waves (148 SMs x 3 ciphertexts) so chunking costs no tail.
-size_t cbs_chunk(const spf_b200_ctx* ctx) {
-  static const long waves = [] {
-    const char* e = getenv("SPF_B200_CHUNK_WAVES");  // tuning knob for the host-pointer pipeline
-    const long w = e ? atol(e) : 0;
-    return w > 0 ? w : 1;
-  }();
-  return (size_t)ctx->sm_count * kPbsPairs * (size_t)waves;
-}
+// Largest chunk of a host-pointer batch processed per pipeline slot: one PBS
+// wave (148 SMs x 3 ciphertexts) so chunking costs no tail.
+size_t cbs_chunk(const spf_b200_ctx* ctx) { return (size_t)ctx->sm_count * kPbsPairs; }
 
 // ---- host-pointer ops: chunked, double-buffered over the context's two streams ---------------
 
@@ -706,7 +667,7 @@ void spf_b200_destroy(spf_b200_ctx* ctx) {
   if (ctx->refs.fetch_sub(1) > 1) return;  // graphs built on this context are still alive: the last one frees it
   cudaSetDevice(ctx->device);
   cudaDeviceSynchronize();
-  cudaFree(ctx->bsk); cudaFree(ctx->ak); cudaFree(ctx->ssk); cudaFree(ctx->ksk); cudaFree(ctx->ksk_colsum); cudaFree(ctx->ks_bfrag); cudaFree(ctx->ks_tc_colsum); cudaFree(ctx->ks_btiles);
+  cudaFree(ctx->bsk); cudaFree(ctx->ak); cudaFree(ctx->ssk); cudaFree(ctx->ksk); cudaFree(ctx->ksk_colsum); cudaFree(ctx->ks_tc_colsum); cudaFree(ctx->ks_btiles);
   cudaFree(ctx->T1); cudaFree(ctx->T2); cudaFree(ctx->kinv); cudaFree(ctx->consts);
   for (int i = 0; i < 2; i++) {
     for (DevBuf& b : ctx->scratch[i]) cudaFree(b.p);

@@ -28,21 +28,11 @@ struct HostCx {
   void rp_load(uint64_t (&rp)[32]) { memcpy(rp, rp_stash, sizeof(rp_stash)); }
 };
 
-// pair of teams (pbs_pair_team): 128 host threads, one barrier per half and one for the pair.  TR / CH select the
-// same code paths as the device builds (accumulator image in the exchange buffer; chunked own-coefficient access).
-template <bool TR, bool CH>
-struct HostPairCxT {
-  static constexpr bool kTransient = TR;
-  static constexpr bool kChunked = CH;
+// pair of teams (pbs_pair_team): 128 host threads, one barrier per half and one for the pair
+struct HostPairCx {
   int u, h;
   pthread_barrier_t* bar_half;
   pthread_barrier_t* bar_pair;
-  // the device runs the first exchange inside the warp through tensor memory (renumbering the threads in the time
-  // domain); the arithmetic per logical thread is the same, so the host keeps the plain numbering and shared buffers
-  static constexpr bool kTmemX1 = false;
-  int time_index() const { return u; }
-  void x1_fwd(C2 (&)[16]) {}
-  void x1_inv(C2 (&)[16]) {}
   void sync() { pthread_barrier_wait(bar_half); }
   void pair_sync() { pthread_barrier_wait(bar_pair); }
   // the device keeps the thread's 16 pass-1 twiddles in tensor memory; here they come from the table
@@ -50,53 +40,16 @@ struct HostPairCxT {
   void t1_mul(C2 (&v)[16], const C2* T1) {
     for (int k1 = 0; k1 < 16; k1++) v[k1] = CONJ ? cmul_conj(v[k1], T1[k1 * 64 + u]) : cmul(v[k1], T1[k1 * 64 + u]);
   }
-  template <bool CONJ>
-  void t2_mul(C2 (&v)[16], const C2* T2) {
-    const int q = u >> 4;
-    for (int k2 = 1; k2 < 16; k2++) v[k2] = CONJ ? cmul_conj(v[k2], T2[q * kT2Pad + k2]) : cmul(v[k2], T2[q * kT2Pad + k2]);
-  }
   // reader-side pass-2 twiddles (device: the thread's constants sit in tensor memory; here they are recomputed, same arithmetic)
-  static constexpr bool kReaderT2 = true;
-#ifndef SPF_PBS_TWOBUF
-#define SPF_PBS_TWOBUF 0
-#endif
-  static constexpr bool kTwoBuf = SPF_PBS_TWOBUF != 0 && !CH;  // the fused-store variant keeps the one-buffer form
-#ifndef SPF_PBS_INT_CONV
-#define SPF_PBS_INT_CONV 0
-#endif
-  static constexpr bool kIntConv = SPF_PBS_INT_CONV != 0;
-#ifndef SPF_PBS_FRND_CONV
-#define SPF_PBS_FRND_CONV 0
-#endif
-  static constexpr bool kFrndConv = SPF_PBS_FRND_CONV != 0;
   void rt2_fwd(double (&tw)[12], const C2* T2) { rt2_fwd_consts(T2, u >> 4, h, tw); }
   void rt2_inv(C2 (&w)[6], const C2* T2) { rt2_inv_consts(T2, u >> 4, h, w); }
-  static constexpr bool kBskRing = false;   // the ring is device machinery: the host reads the key in place
+  // the BSK ring is device machinery: the host reads the key in place
   const C2* bsk_acquire(int, const C2* g) { return g; }
   void bsk_release(int) {}
-  void bsk_release_early(int) {}
   void bsk_skip(int) {}
   C2 bsk_load(const C2* p) { return *p; }
-  static constexpr bool kFusedStores = CH;  // exercised together with the chunked variant
-  void sts(C2* p, C2 v) { *p = v; }
-  template <bool CONJ>
-  void t1_mul_store(C2 (&v)[16], const C2* T1, C2* buf) {
-    for (int k1 = 0; k1 < 16; k1++) {
-      v[k1] = CONJ ? cmul_conj(v[k1], T1[k1 * 64 + u]) : cmul(v[k1], T1[k1 * 64 + u]);
-      buf[k1 * kXPad + u] = v[k1];
-    }
-  }
-  template <bool CONJ>
-  void t2_mul_store(C2 (&v)[16], const C2* T2, C2* buf) {
-    const int k1 = u & 15, q = u >> 4;
-    for (int k2 = 0; k2 < 16; k2++) {
-      if (k2) v[k2] = CONJ ? cmul_conj(v[k2], T2[q * kT2Pad + k2]) : cmul(v[k2], T2[q * kT2Pad + k2]);
-      buf[k1 * kXPad + q + 4 * k2] = v[k2];
-    }
-  }
   // the device keeps a private copy of the thread's own accumulator coefficients in tensor memory
   uint64_t own_stash[32];
-  void own_load(uint64_t (&own)[32], const uint64_t*) { memcpy(own, own_stash, sizeof(own_stash)); }
   void own_store(const uint64_t (&own)[32]) { memcpy(own_stash, own, sizeof(own_stash)); }
   void own_ld8(uint64_t (&o)[8], int c) { memcpy(o, own_stash + 8 * c, 64); }
   void own_ld4x2(uint64_t (&o)[8], int m4) { memcpy(o, own_stash + m4, 32); memcpy(o + 4, own_stash + m4 + 16, 32); }
@@ -172,9 +125,6 @@ struct HostWideCx {
   pthread_barrier_t* bar_cta;
   void sync() { pthread_barrier_wait(bar_team); }
   void cta_sync() { pthread_barrier_wait(bar_cta); }
-  static constexpr bool kStageG = false;  // device: the selector GGSW is staged in tensor memory during the transforms
-  template <int I> void g_stage() {}
-  void g_read16(C2 (&)[4][4], int) {}
 };
 template <class Body>
 struct WideLaunch {
@@ -210,7 +160,6 @@ struct HostQuadCx {
   pthread_barrier_t* bar_team;
   pthread_barrier_t* bar_quad;
   // split gather: the two teams of a polynomial swap 16 packed digits per thread (device: through tensor memory)
-  static constexpr bool kSplitGather = true;
   pthread_barrier_t* bar_poly = nullptr;  // the 128 threads of teams (h, 0) and (h, 1)
   uint32_t* xchg = nullptr;               // [h][t][u][8]
   void digit_xchg(uint32_t (&pk)[8]) {
@@ -218,10 +167,6 @@ struct HostQuadCx {
     pthread_barrier_wait(bar_poly);
     memcpy(pk, xchg + ((size_t)(h * 2 + (1 - t)) * kTeam + u) * 8, sizeof(pk));
   }
-#ifndef SPF_QUAD_READER_T2
-#define SPF_QUAD_READER_T2 1
-#endif
-  static constexpr bool kReaderT2 = SPF_QUAD_READER_T2 != 0;
   void rt2(double (&tw)[6], C2 (&wi)[3], const C2* T2) { rt2_group_consts(T2, u >> 4, 2 * h + t, tw, wi); }
   void sync() { pthread_barrier_wait(bar_team); }
   void quad_sync() { pthread_barrier_wait(bar_quad); }
@@ -232,11 +177,6 @@ struct HostQuadCx {
   template <bool CONJ>
   void t1_mul(C2 (&v)[16], const C2* T1) {
     for (int k1 = 0; k1 < 16; k1++) v[k1] = CONJ ? cmul_conj(v[k1], T1[k1 * 64 + u]) : cmul(v[k1], T1[k1 * 64 + u]);
-  }
-  template <bool CONJ>
-  void t2_mul(C2 (&v)[16], const C2* T2) {
-    const int q = u >> 4;
-    for (int k2 = 1; k2 < 16; k2++) v[k2] = CONJ ? cmul_conj(v[k2], T2[q * kT2Pad + k2]) : cmul(v[k2], T2[q * kT2Pad + k2]);
   }
 };
 template <class Body>
@@ -280,21 +220,6 @@ const Tables& tables() {
   return t;
 }
 
-// generalized PBS; bsk in device scale (2^-10).  lut may be null (CBS mode).  transient / chunked select the code
-// paths of the device builds (SPF_PBS_TRANSIENT, 4 pairs per CTA); the arithmetic is the same in all four.
-template <bool TR, bool CH>
-void emu_pbs_t(uint64_t* glwe_out, const uint64_t* lwe_in, const uint64_t* lut, const C2* bsk_dev, int lwe_n,
-                      int log_chi, int log_v, int cbs_radix_log, int cbs_count) {
-  const Tables& t = tables();
-  std::vector<C2> xbuf(4 * kXBuf);  // two exchange buffers per half when Cx::kTwoBuf
-  std::vector<uint64_t> acc(2 * kN);
-  PbsArgs A{lwe_in, lut, glwe_out, bsk_dev, lwe_n, log_chi, log_v, cbs_radix_log, cbs_count};
-  using Cx = HostPairCxT<TR, CH>;
-  run_pair<Cx>([&](Cx& cx) {
-    int G = 0;
-    pbs_pair_team(cx, A, acc.data(), xbuf.data(), t.T1.data(), t.T2.data(), G);
-  });
-}
 }  // namespace
 
 extern "C" {
@@ -359,15 +284,22 @@ void emu_cmux_wide(uint64_t* out, const uint64_t* d0, const uint64_t* d1, const 
   });
 }
 
-void emu_pbs_variant(uint64_t* glwe_out, const uint64_t* lwe_in, const uint64_t* lut, const C2* bsk_dev, int lwe_n,
-                     int log_chi, int log_v, int cbs_radix_log, int cbs_count, int transient, int chunked) {
-  auto fn = transient ? (chunked ? emu_pbs_t<true, true> : emu_pbs_t<true, false>)
-                      : (chunked ? emu_pbs_t<false, true> : emu_pbs_t<false, false>);
-  fn(glwe_out, lwe_in, lut, bsk_dev, lwe_n, log_chi, log_v, cbs_radix_log, cbs_count);
-}
+// generalized PBS on the pair-team code the device runs; bsk in device scale (2^-10).  lut may be null (CBS mode).
 void emu_pbs(uint64_t* glwe_out, const uint64_t* lwe_in, const uint64_t* lut, const C2* bsk_dev, int lwe_n,
              int log_chi, int log_v, int cbs_radix_log, int cbs_count) {
-  emu_pbs_t<true, false>(glwe_out, lwe_in, lut, bsk_dev, lwe_n, log_chi, log_v, cbs_radix_log, cbs_count);
+  const Tables& t = tables();
+  std::vector<C2> xbuf(2 * kXBuf);
+  PbsArgs A{lwe_in, lut, glwe_out, bsk_dev, lwe_n, log_chi, log_v, cbs_radix_log, cbs_count};
+  run_pair<HostPairCx>([&](HostPairCx& cx) {
+    int G = 0;
+    pbs_pair_team(cx, A, xbuf.data(), t.T1.data(), t.T2.data(), G);
+  });
+}
+// Part of the library's interface that tests/emu_util.py binds.  The transient and chunked forms it used to select all
+// gave emu_pbs's output bit for bit; they are now the one form the device ships, so every flag pair runs emu_pbs.
+void emu_pbs_variant(uint64_t* glwe_out, const uint64_t* lwe_in, const uint64_t* lut, const C2* bsk_dev, int lwe_n,
+                     int log_chi, int log_v, int cbs_radix_log, int cbs_count, int /*transient*/, int /*chunked*/) {
+  emu_pbs(glwe_out, lwe_in, lut, bsk_dev, lwe_n, log_chi, log_v, cbs_radix_log, cbs_count);
 }
 
 // the latency-mode (four-team) blind rotation

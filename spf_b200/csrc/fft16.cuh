@@ -37,25 +37,6 @@ struct alignas(16) C2 {
   double x, y;
 };
 
-// SPF_ABL (experiment builds only, tools/ablate.sh): bit mask of kernel components replaced by no-ops to measure what the
-// blind-rotation kernel's time is sensitive to: 1 butterflies, 2 complex multiplies / MADs, 4 exchange-buffer traffic,
-// 8 barriers, 16 key loads, 32 accumulator gather, 64 f64 -> torus conversion.  Results are garbage by construction.
-#if defined(SPF_ABL) && defined(__CUDA_ARCH__)
-#define SPF_ABLATE(bit) ((SPF_ABL) & (bit))
-#else
-#define SPF_ABLATE(bit) 0
-#endif
-SPF_HD C2 abl_mix(C2 a, C2 b) {
-  C2 r;
-#if defined(__CUDA_ARCH__)
-  r.x = __longlong_as_double(__double_as_longlong(a.x) ^ __double_as_longlong(b.x));
-  r.y = __longlong_as_double(__double_as_longlong(a.y) ^ __double_as_longlong(b.y));
-#else
-  r = a; (void)b;
-#endif
-  return r;
-}
-
 constexpr int kN = 2048;        // polynomial degree (DEFAULT_128 l1_params)
 constexpr int kM = 1024;        // complex FFT length
 constexpr int kTeam = 64;       // threads per polynomial transform
@@ -88,17 +69,13 @@ SPF_HD double spf_fma(double a, double b, double c) {
 }
 // a * (c + i s)
 SPF_HD C2 cmul_cs(C2 a, double c, double s) {
-  if (SPF_ABLATE(2)) return abl_mix(a, C2{c, s});
   return C2{spf_fma(a.x, c, -(a.y * s)), spf_fma(a.x, s, a.y * c)}; }
 SPF_HD C2 cmul(C2 a, C2 b) {
-  if (SPF_ABLATE(2)) return abl_mix(a, b);
   return C2{spf_fma(a.x, b.x, -(a.y * b.y)), spf_fma(a.x, b.y, a.y * b.x)}; }
 SPF_HD C2 cmul_conj(C2 a, C2 b) {
-  if (SPF_ABLATE(2)) return abl_mix(a, b);
   return C2{spf_fma(a.x, b.x, a.y * b.y), spf_fma(a.y, b.x, -(a.x * b.y))}; }  // a * conj(b)
 // acc += a * b as four chained FMAs
 SPF_HD void cmad(C2& acc, C2 a, C2 b) {
-  if (SPF_ABLATE(2)) { acc = abl_mix(acc, abl_mix(a, b)); return; }
   acc.x = spf_fma(-a.y, b.y, spf_fma(a.x, b.x, acc.x));
   acc.y = spf_fma(a.y, b.x, spf_fma(a.x, b.y, acc.y));
 }
@@ -106,7 +83,6 @@ SPF_HD void cmad(C2& acc, C2 a, C2 b) {
 // 4-point DFT in place: (a,b,c,d) -> (X0,X1,X2,X3); INV uses e^{+...}
 template <bool INV>
 SPF_HD void bfly4(C2& a, C2& b, C2& c, C2& d) {
-  if (SPF_ABLATE(1)) return;
   C2 apc = cadd(a, c), amc = csub(a, c), bpd = cadd(b, d), bmd = csub(b, d);
   a = cadd(apc, bpd);
   c = csub(apc, bpd);
@@ -119,43 +95,14 @@ SPF_HD void bfly4(C2& a, C2& b, C2& c, C2& d) {
   }
 }
 
-// ---- constant pools --------------------------------------------------------------------------------------------------
-// The deferred-scale transforms below use ~40 distinct double constants per pass (tangents, scale ratios).  As literals every
-// one of them costs two UMOV instructions (32-bit immediates into a uniform register pair) each time it is materialised:
-// ~230 of the ~3 700 instructions of a blind-rotation step, in a kernel whose time follows its instruction count.  A constant
-// PROVIDER hands them out instead: KLit returns the literal (host emulator, -DSPF_KPOOL=0), KDev<P> reads pool P of a
-// __constant__ array in call order -- after unrolling every index is a compile-time constant and ptxas fetches two constants
-// per LDCU.128 -- and KRec (host, tables.h: fill_kpools) records the same call sequence once to fill the array.  Factors of
-// exactly 1 stay literals so that the compiler still folds fma(1, x, y) into an add; the sequence is data-independent.
+// ---- constant providers -----------------------------------------------------------------------------------------------
+// The deferred-scale transforms below take their ~40 distinct double constants per pass (tangents, scale ratios) from a
+// PROVIDER kp(v); KLit returns the literal, which the device code materialises as FMA immediates.  (Reading them from a
+// __constant__ pool instead was measured: no gain in pbs_kernel, 6.75 vs 6.73 ms per wave, and spills in the 255-register
+// trace_ss_kernel, 7.4 -> 9.0 ms.)
 struct KLit {
   SPF_HD double operator()(double v) { return v; }
 };
-constexpr int kPoolLen = 80;
-constexpr int kPools = 4;  // 0 forward pass 1, 1 inverse pass 1 (+ output scales), 2 / 3 forward / inverse unit-scale 16-point transform
-struct KRec {
-  double* out;
-  int i;
-  SPF_HD double operator()(double v) {
-    if (v == 1.0) return 1.0;
-    if (i < kPoolLen) out[i] = v;
-    i++;
-    return v;
-  }
-};
-#ifndef SPF_KPOOL
-#define SPF_KPOOL 0  // measured: no gain in pbs_kernel (UMOV pairs become LDCU.64 + R2UR, 6.75 vs 6.73 ms per wave) and 255-register kernels spill (trace_ss_kernel 7.4 -> 9.0 ms): off
-#endif
-#if defined(__CUDACC__)
-__constant__ double spf_kpool[kPools][kPoolLen];
-template <int P>
-struct KDev {
-  int i = 0;
-  __device__ __forceinline__ double operator()(double v) {
-    if (v == 1.0) return 1.0;
-    return spf_kpool[P][i++];
-  }
-};
-#endif
 
 // ---- deferred-scale arithmetic --------------------------------------------------------------
 // Inside the in-register transforms a value is a pair (v, s): the true value is s * v, where s is a
@@ -171,7 +118,6 @@ SPF_HD constexpr double spf_abs(double x) { return x < 0 ? -x : x; }
 // (v, s) *= e^{i pi e / 32}
 template <class KP>
 SPF_HD void rot_s(C2& v, double& s, int e, KP& kp) {
-  if (SPF_ABLATE(1)) return;
   e &= 63;
   if (e == 0) return;
   // quarter turns are sign changes and swaps (they fold into the operand modifiers of the next FMA); the tan / cot form
@@ -197,7 +143,6 @@ SPF_HD void rot_s(C2& v, double& s, int e) {
 // 4-point DFT of (a, sa) .. (d, sd); all four results carry scale sa.
 template <bool INV, class KP>
 SPF_HD void bfly4_s(C2& a, C2& b, C2& c, C2& d, double sa, double sb, double sc, double sd, KP& kp) {
-  if (SPF_ABLATE(1)) return;
   const double rc = kp(sc / sa), rd = kp(sd / sb), rb = kp(sb / sa);
   const C2 apc{spf_fma(rc, c.x, a.x), spf_fma(rc, c.y, a.y)}, amc{spf_fma(-rc, c.x, a.x), spf_fma(-rc, c.y, a.y)};
   const C2 bpd{spf_fma(rd, d.x, b.x), spf_fma(rd, d.y, b.y)}, bmd{spf_fma(-rd, d.x, b.x), spf_fma(-rd, d.y, b.y)};
@@ -221,7 +166,6 @@ SPF_HD void bfly4_s(C2& a, C2& b, C2& c, C2& d, double sa, double sb, double sc,
 // scale sa): the reader-side pass-2 twiddles of the pair kernel (team_ops.cuh: rt2_fwd_consts) arrive as per-thread constants.
 template <bool INV>
 SPF_HD void bfly4_r(C2& a, C2& b, C2& c, C2& d, double rb, double rc, double rd) {
-  if (SPF_ABLATE(1)) return;
   const C2 apc{spf_fma(rc, c.x, a.x), spf_fma(rc, c.y, a.y)}, amc{spf_fma(-rc, c.x, a.x), spf_fma(-rc, c.y, a.y)};
   const C2 bpd{spf_fma(rd, d.x, b.x), spf_fma(rd, d.y, b.y)}, bmd{spf_fma(-rd, d.x, b.x), spf_fma(-rd, d.y, b.y)};
   a = C2{spf_fma(rb, bpd.x, apc.x), spf_fma(rb, bpd.y, apc.y)};
@@ -271,34 +215,6 @@ SPF_HD void dft16_s(C2 (&v)[16], double (&s)[16], KP& kp) {
     for (int kh = 0; kh < 4; kh++) { v[kl + 4 * kh] = t[4 * kl + kh]; s[kl + 4 * kh] = ts[4 * kl + kh]; }
   }
 }
-// The same transform with unit input scales, handing every output to emit(k, X[k]) as soon as its last butterfly is
-// done (the caller stores it to the exchange buffer right there, so the stores interleave with the remaining
-// butterflies instead of queueing behind them); v is left in the internal order.
-template <bool INV, class Emit>
-SPF_HD void dft16_emit(C2 (&v)[16], Emit emit) {
-  double s[16];
-#pragma unroll
-  for (int i = 0; i < 16; i++) s[i] = 1.0;
-#pragma unroll
-  for (int m0 = 0; m0 < 4; m0++) {
-    bfly4_s<INV>(v[m0], v[m0 + 4], v[m0 + 8], v[m0 + 12], s[m0], s[m0 + 4], s[m0 + 8], s[m0 + 12]);
-    s[m0 + 4] = s[m0 + 8] = s[m0 + 12] = s[m0];
-  }
-#pragma unroll
-  for (int m0 = 1; m0 < 4; m0++) {
-#pragma unroll
-    for (int kl = 1; kl < 4; kl++) {
-      const int e = 4 * m0 * kl;
-      rot_s(v[m0 + 4 * kl], s[m0 + 4 * kl], INV ? e : 64 - e);
-    }
-  }
-#pragma unroll
-  for (int kl = 0; kl < 4; kl++) {
-    bfly4_s<INV>(v[4 * kl], v[4 * kl + 1], v[4 * kl + 2], v[4 * kl + 3], s[4 * kl], s[4 * kl + 1], s[4 * kl + 2], s[4 * kl + 3]);
-#pragma unroll
-    for (int kh = 0; kh < 4; kh++) emit(kl + 4 * kh, v[4 * kl + kh]);  // scale s[4 kl] == 1
-  }
-}
 template <bool INV>
 SPF_HD void dft16_s(C2 (&v)[16], double (&s)[16]) {
   KLit kp;
@@ -313,11 +229,7 @@ SPF_HD void dft16_k(C2 (&v)[16], KP& kp) {
 }
 template <bool INV>
 SPF_HD void dft16(C2 (&v)[16]) {
-#if defined(__CUDA_ARCH__) && SPF_KPOOL
-  KDev<INV ? 3 : 2> kp;
-#else
   KLit kp;
-#endif
   dft16_k<INV>(v, kp);
 }
 
@@ -335,11 +247,7 @@ SPF_HD void fwd_pass1_core_k(C2 (&v)[16], KP& kp) {
   dft16_s<false>(v, s, kp);  // the twist factors fold into the butterflies; outputs carry s[0] = 1
 }
 SPF_HD void fwd_pass1_core(C2 (&v)[16]) {
-#if defined(__CUDA_ARCH__) && SPF_KPOOL
-  KDev<0> kp;
-#else
   KLit kp;
-#endif
   fwd_pass1_core_k(v, kp);
 }
 SPF_HD void fwd_pass1(C2 (&v)[16], int a, const C2* T1) {
@@ -348,34 +256,13 @@ SPF_HD void fwd_pass1(C2 (&v)[16], int a, const C2* T1) {
   for (int k1 = 0; k1 < 16; k1++) v[k1] = cmul(v[k1], T1[k1 * 64 + a]);
 }
 SPF_HD void fwd_x1_write(const C2 (&v)[16], C2* buf, int a) {
-  if (SPF_ABLATE(4)) return;
 #pragma unroll
   for (int k1 = 0; k1 < 16; k1++) buf[k1 * kXPad + a] = v[k1];
 }
 SPF_HD void fwd_x1_read(C2 (&v)[16], const C2* buf, int u) {
-  if (SPF_ABLATE(4)) return;
   const int k1 = u & 15, q = u >> 4;
 #pragma unroll
   for (int mp = 0; mp < 16; mp++) v[mp] = buf[k1 * kXPad + q + 4 * mp];
-}
-// ---- warp-local first exchange (pbs_kernel, Cx::kTmemX1) ------------------------------------------------------------
-// The first exchange moves data between the 16 threads a = q + 4 m', m' = 0..15, and the 16 threads (k1, q): with the
-// team's threads numbered so that each such group sits inside ONE warp it needs no shared memory at all (the device
-// transposes the 16 x 16 tile through tensor memory, kernels.cuh::DevPairCx::x1_fwd).  Physical thread p = 32 W + l
-// (warp W of the team, lane l) then plays two roles:
-//   time domain / pass 1:  a = x1_time_index(p) = 4 (l >> 1) + 2 W + (l & 1)      (group q = 2 W + (l & 1), member l >> 1)
-//   pass 2 and later:      u = p = k1 + 16 q,  k1 = l & 15,  q = 2 W + (l >> 4)   (unchanged)
-// Everything laid out per thread in shared memory (accumulator image, first-exchange buffer) is indexed by the
-// PHYSICAL thread, so consecutive lanes still touch consecutive addresses; x1_position maps a logical a to it.
-SPF_HD constexpr int x1_time_index(int p) { return 4 * ((p & 31) >> 1) + 2 * (p >> 5) + (p & 1); }
-SPF_HD constexpr int x1_position(int a) { return 32 * ((a >> 1) & 1) + 2 * (a >> 2) + (a & 1); }
-// fwd_x1_read for a buffer written at physical positions (buf[k1][p] = y_a[k1], a = x1_time_index(p)):
-// thread (k1, q) gathers a = q + 4 m' from position 32 (q >> 1) + (q & 1) + 2 m'.
-SPF_HD void fwd_x1_read_perm(C2 (&v)[16], const C2* buf, int u) {
-  if (SPF_ABLATE(4)) return;
-  const int k1 = u & 15, q = u >> 4;
-#pragma unroll
-  for (int mp = 0; mp < 16; mp++) v[mp] = buf[k1 * kXPad + 32 * (q >> 1) + (q & 1) + 2 * mp];
 }
 SPF_HD void fwd_pass2(C2 (&v)[16], int u, const C2* T2) {
   const int q = u >> 4;
@@ -388,13 +275,11 @@ SPF_HD void fwd_pass2(C2 (&v)[16], int u, const C2* T2) {
 // write (each thread only overwrites what it alone consumed).  The reader of pass 3, thread
 // (k1, q), finds z of thread (k1, q') for k2 = q + 4 j at column q' + 4 q + 16 j of row k1.
 SPF_HD void fwd_x2_write(const C2 (&v)[16], C2* buf, int u) {
-  if (SPF_ABLATE(4)) return;
   const int k1 = u & 15, q = u >> 4;
 #pragma unroll
   for (int k2 = 0; k2 < 16; k2++) buf[k1 * kXPad + q + 4 * k2] = v[k2];
 }
 SPF_HD void fwd_x2_read(C2 (&v)[16], const C2* buf, int u) {
-  if (SPF_ABLATE(4)) return;
   const int k1 = u & 15, q = u >> 4;
 #pragma unroll
   for (int j = 0; j < 4; j++) {
@@ -419,7 +304,6 @@ SPF_HD void inv_pass3(C2 (&v)[16]) {
 // Inverse direction, same in-place layout: inv_x2_read takes the 16 locations (row k1, column
 // q + 4 k2) that inv_x1_write of the same thread overwrites next, so no barrier separates them.
 SPF_HD void inv_x2_write(const C2 (&v)[16], C2* buf, int u) {
-  if (SPF_ABLATE(4)) return;
   const int k1 = u & 15, q = u >> 4;
 #pragma unroll
   for (int j = 0; j < 4; j++) {
@@ -428,7 +312,6 @@ SPF_HD void inv_x2_write(const C2 (&v)[16], C2* buf, int u) {
   }
 }
 SPF_HD void inv_x2_read(C2 (&v)[16], const C2* buf, int u) {
-  if (SPF_ABLATE(4)) return;
   const int k1 = u & 15, q = u >> 4;
 #pragma unroll
   for (int k2 = 0; k2 < 16; k2++) v[k2] = buf[k1 * kXPad + q + 4 * k2];
@@ -440,13 +323,11 @@ SPF_HD void inv_pass2(C2 (&v)[16], int u, const C2* T2) {
   dft16<true>(v);
 }
 SPF_HD void inv_x1_write(const C2 (&v)[16], C2* buf, int u) {
-  if (SPF_ABLATE(4)) return;
   const int k1 = u & 15, q = u >> 4;
 #pragma unroll
   for (int mp = 0; mp < 16; mp++) buf[k1 * kXPad + q + 4 * mp] = v[mp];
 }
 SPF_HD void inv_x1_read(C2 (&v)[16], const C2* buf, int a) {
-  if (SPF_ABLATE(4)) return;
 #pragma unroll
   for (int k1 = 0; k1 < 16; k1++) v[k1] = buf[k1 * kXPad + a];
 }
@@ -460,14 +341,10 @@ SPF_HD void inv_pass1_core_s_k(C2 (&v)[16], double (&s)[16], KP& kp) {
 #pragma unroll
   for (int m = 1; m < 16; m++) rot_s(v[m], s[m], 64 - m, kp);
 #pragma unroll
-  for (int m = 1; m < 16; m++) s[m] = kp(s[m]);  // the output scales are constants of the pool too (consumed as FMA factors)
+  for (int m = 1; m < 16; m++) s[m] = kp(s[m]);  // the output scales come from the provider too (consumed as FMA factors)
 }
 SPF_HD void inv_pass1_core_s(C2 (&v)[16], double (&s)[16]) {
-#if defined(__CUDA_ARCH__) && SPF_KPOOL
-  KDev<1> kp;
-#else
   KLit kp;
-#endif
   inv_pass1_core_s_k(v, s, kp);
 }
 SPF_HD void inv_pass1_core(C2 (&v)[16]) {
@@ -486,21 +363,19 @@ SPF_HD void inv_pass1(C2 (&v)[16], int a, const C2* T1) {
 // scalar conversions
 // ------------------------------------------------------------------------------------------
 
-// int32 -> f64.  Host (and -DSPF_NO_I2F): without a conversion, 2^52 + 2^31 + x is exact, subtract the bias.
+// int32 -> f64
 SPF_HD double i32_to_f64(int32_t x) {
-#if defined(__CUDA_ARCH__) && !defined(SPF_NO_I2F)
+#if defined(__CUDA_ARCH__)
   // the conversion pipe is idle in these kernels while the FP64 pipe and the issue slots are not: one I2F.F64.S32 instead of
   // an integer op, a move and a DADD (same value)
   return __int2double_rn(x);
-#endif
+#else
+  // without a conversion: 2^52 + 2^31 + x is exact, subtract the bias
   uint64_t bits = 0x4330000000000000ull | (uint64_t)((uint32_t)x ^ 0x80000000u);
   double d;
-#if defined(__CUDA_ARCH__)
-  d = __longlong_as_double((long long)bits);
-#else
   __builtin_memcpy(&d, &bits, 8);
-#endif
   return d - 4503601774854144.0;  // 2^52 + 2^31
+#endif
 }
 
 // int64 -> f64, round to nearest even (what `as f64` does; entities/polynomial.rs:264-268).
@@ -558,7 +433,6 @@ SPF_HD int64_t f64_to_i64_sat(double x) {
 constexpr uint32_t kTorusCornerMag = 0x43E00000u;  // high word of 2^63
 template <bool SCALED, bool CORNER>
 SPF_HD uint64_t f64_to_torus_impl(double xs, double sc, uint32_t* mag_max) {
-  if (SPF_ABLATE(64)) return f64_bits(xs);
   const double magic = 124615124604835863084731911901282304.0;  // 1.5 * 2^116
   const double hq = (SCALED ? spf_fma(sc, xs, magic) : xs + magic) - magic;
   const double lo = SCALED ? spf_fma(sc, xs, -hq) : xs - hq;
@@ -589,51 +463,6 @@ SPF_HD uint64_t f64_to_torus(double x) { return f64_to_torus_impl<false, true>(x
 SPF_HD uint64_t f64_to_torus_s(double xs, double sc) { return f64_to_torus_impl<true, true>(xs, sc, nullptr); }
 SPF_HD uint64_t f64_to_torus_s_fast(double xs, double sc, uint32_t& mag_max) {
   return f64_to_torus_impl<true, false>(xs, sc, &mag_max);
-}
-
-// f64 -> torus of y = fl(sc * xs) with the ROUND-TO-INTEGRAL conversion instruction: t = y / 2^64 (the factor is folded into the
-// compile-time scale, so t is one DMUL), r = rint(t) on the conversion pipe, frac = t - r exactly (|frac| <= 1/2), and
-// lo = frac * 2^64 (an exponent-field add) is y reduced modulo 2^64 into [-2^63, 2^63]: an integer whenever |y| >= 2^52, so the
-// final F2I is exact.  Two FP64 instructions per value instead of four; the conversion pipe is idle in these kernels.
-// `small` tracks the minimum exponent word of t (|y| < 2^52 may carry a fraction: round-half-away needed) and `corner` the
-// maximum of frac (|frac| = 1/2 is the saturating-cast corner of f64_to_torus_impl): the caller redoes such (rare) groups with
-// f64_to_torus(sc * xs), which has the same semantics for every double.
-constexpr uint32_t kTorusSmallMag = 0x3F300000u;   // high word of 2^-12: |t| below it <=> |y| < 2^52
-constexpr uint32_t kTorusHalfMag = 0x3FE00000u;    // high word of 1/2
-SPF_HD uint64_t f64_to_torus_frnd(double xs, double sc, uint32_t& small_min, uint32_t& corner_max) {
-  if (SPF_ABLATE(64)) return f64_bits(xs);
-  const double t = (sc * 5.421010862427522e-20 /* 2^-64 */) * xs;
-#if defined(__CUDA_ARCH__)
-  double r;
-  asm("cvt.rni.f64.f64 %0, %1;" : "=d"(r) : "d"(t));
-#else
-  const double r = __builtin_nearbyint(t);  // round to nearest even, the default mode
-#endif
-  const double frac = t - r;
-  const uint64_t fb = f64_bits(frac);
-  const uint32_t th = (uint32_t)(f64_bits(t) >> 32) & 0x7FFFFFFFu, fh = (uint32_t)(fb >> 32) & 0x7FFFFFFFu;
-  small_min = th < small_min ? th : small_min;
-  corner_max = fh > corner_max ? fh : corner_max;
-  const double lo = bits_f64(fb + (64ull << 52));  // frac * 2^64 (frac = +-0 becomes +-2^-959: converts to 0)
-  return (uint64_t)f64_to_i64_sat(lo);
-}
-
-// f64 -> torus of y = fl(sc * xs) with INTEGER arithmetic: a double of magnitude >= 2^52 is an integer M * 2^s (M the 53-bit
-// significand, s >= 0), so round() is the identity and the reduction mod 2^64 is a shift of M -- one FP64 instruction (the product)
-// instead of four plus a conversion.  Smaller magnitudes (probability ~2^-33 per coefficient of a blind rotation) and the
-// saturating-cast corner (|y| = 2^63 mod 2^64, see f64_to_torus_impl) only raise `slow`: the caller redoes its values with
-// f64_to_torus(sc * xs), which has the same semantics for every double.
-SPF_HD uint64_t f64_to_torus_int(double xs, double sc, uint32_t& slow) {
-  if (SPF_ABLATE(64)) return f64_bits(xs);
-  const double y = sc * xs;
-  const uint64_t b = f64_bits(y);
-  const uint32_t hi = (uint32_t)(b >> 32);
-  const int s = (int)((hi >> 20) & 0x7FFu) - 1075;
-  const uint64_t M = (b & 0x000FFFFFFFFFFFFFull) | 0x0010000000000000ull;
-  const uint64_t m = (uint32_t)s < 64u ? M << (s & 63) : 0ull;                    // s >= 64: a multiple of 2^64 (s < 0: redone)
-  const uint64_t neg = (uint64_t)((int64_t)b >> 63);
-  slow |= (uint32_t)(s < 0) | (uint32_t)(m == 0x8000000000000000ull);
-  return (m ^ neg) - neg;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -134,13 +134,6 @@ struct spf_b200_graph {
   std::atomic<int> status{0};
   std::string status_msg;
   DevBuf ks_states;
-  // runs of consecutive narrow CMux levels executed by ONE cooperative launch each (cmux_chain_kernel): planned at the
-  // first run of a rank, the stage lists live in d_chain
-  struct Chain { size_t first, last; size_t stage_off; int n_stages; int grid; };
-  std::vector<Chain> chains;
-  int chain_rank = -1;          // rank the plan was made for (-1: not planned yet)
-  ChainStage* d_chain = nullptr;
-  unsigned long long* d_chain_bar = nullptr;
   bool poisoned = false;  // a failed peer-mode run leaves the ranks' barrier epochs out of step: rebuild the graphs
   // rank that writes the Output* nodes every rank holds (output rank -1); -1 = every rank writes them (one process per
   // rank: each has its own host buffers).  A box (box.cuh) runs all ranks into the same host buffers: rank 0 only.
@@ -237,7 +230,6 @@ unsigned long long alloc_base_of(const void* p, size_t* size_out = nullptr) {
 // Returns the io kind (see spf_b200_graph::io_kind).  `may_register`: page-lock an unpinned host buffer (graph build);
 // otherwise (set_io on a built graph) unpinned buffers are staged through the graph's slab.
 int pin_io(spf_b200_graph* g, void* p, size_t bytes, bool may_register = true) {
-  static const bool no_pin = getenv("SPF_B200_NO_PIN") != nullptr;
   if (!p) return 0;
   // both ends: a buffer that merely shares its first page with a neighbour's registration is not page-locked
   cudaPointerAttributes attr, attr_end;
@@ -248,7 +240,6 @@ int pin_io(spf_b200_graph* g, void* p, size_t bytes, bool may_register = true) {
   }
   cudaGetLastError();
   if (!may_register) return 1;
-  if (no_pin) return 0;  // plain pageable cudaMemcpyAsync (diagnostics)
   if (cudaHostRegister(p, bytes, cudaHostRegisterDefault) == cudaSuccess) { g->pinned.push_back(p); return 0; }
   cudaGetLastError();  // clear the sticky-free error
   return 1;
@@ -796,77 +787,6 @@ int stage_slot(spf_b200_graph* g, int id, size_t bytes, char** out) {
   return 0;
 }
 
-// Runs of consecutive MUX-tree levels for cmux_chain_kernel.  Eligible: CMux / MultiplyGgswGlwe groups whose share for this
-// rank fits the wide kernel's regime (at most two outputs per SM); groups that launch nothing (inputs, outputs, constants)
-// are transparent; anything else ends the run.  A run needs at least two levels to be worth a cooperative launch.
-int plan_chains(spf_b200_graph* g, int rank) {
-  spf_b200_ctx* ctx = g->ctx;
-  g->chains.clear();
-  g->chain_rank = rank;
-  if (ctx->p.cbs.count != 4) return 0;
-  const size_t wide_max = 2 * (size_t)ctx->sm_count;
-  auto launches_nothing = [](uint32_t op) {
-    return op <= SPF_OP_INPUT_GLEV1 || (op >= SPF_OP_ZERO_LWE0 && op <= SPF_OP_ONE_GLEV1) || (op >= SPF_OP_OUTPUT_LWE0 && op <= SPF_OP_OUTPUT_GLEV1) ||
-           op == SPF_OP_RETIRE || op == SPF_OP_NOP;
-  };
-  std::vector<ChainStage> stages;
-  std::vector<int> stage_level;
-  size_t i = 0;
-  const size_t ng = g->groups.size();
-  while (i < ng) {
-    const size_t stage0 = stages.size();
-    size_t first = ng, last = 0, widest = 0;
-    int levels = 0, prev_level = -1;
-    size_t j = i;
-    for (; j < ng; j++) {
-      const Group& G = g->groups[j];
-      if (launches_nothing(G.op)) continue;
-      if (!(G.op == SPF_OP_CMUX || G.op == SPF_OP_MULTIPLY_GGSW_GLWE) || !G.slot_outputs) break;
-      const size_t mine = G.all_cnt + G.r_cnt[rank];
-      if (mine > wide_max) break;
-      const void* const* base = reinterpret_cast<const void* const*>(g->d_ptrs + G.ptr_off);
-      void* const* outs = reinterpret_cast<void* const*>(g->d_ptrs + G.ptr_off + 3 * G.ids.size());
-      const size_t starts[2] = {G.all_start, G.r_start[rank]}, cnts[2] = {G.all_cnt, G.r_cnt[rank]};
-      for (int k = 0; k < 2; k++) {
-        if (cnts[k] == 0) continue;
-        if (G.level != prev_level) { levels++; prev_level = G.level; }
-        stages.push_back(ChainStage{base + 3 * starts[k], outs + starts[k], (int)cnts[k], 0});
-        stage_level.push_back(G.level);
-        widest = std::max(widest, cnts[k]);
-        first = std::min(first, j);
-        last = j;
-      }
-    }
-    if (levels >= 2) {
-      for (size_t k = stage0; k + 1 < stages.size(); k++) stages[k].barrier_after = stage_level[k + 1] != stage_level[k];
-      g->chains.push_back({first, last, stage0, (int)(stages.size() - stage0), (int)std::min<size_t>(widest, (size_t)ctx->sm_count)});
-    } else {
-      stages.resize(stage0);
-      stage_level.resize(stage0);
-    }
-    i = std::max(j, i) + 1;  // j stopped at a group that breaks the run (or at the end)
-  }
-  if (g->chains.empty()) return 0;
-  CU(cudaSetDevice(ctx->device));
-  if (g->d_chain) { cudaFree(g->d_chain); g->d_chain = nullptr; }
-  CU(cudaMalloc(&g->d_chain, stages.size() * sizeof(ChainStage)));
-  CU(cudaMemcpy(g->d_chain, stages.data(), stages.size() * sizeof(ChainStage), cudaMemcpyHostToDevice));
-  if (!g->d_chain_bar) CU(cudaMalloc(&g->d_chain_bar, sizeof(unsigned long long)));
-  return 0;
-}
-
-int launch_chain(spf_b200_graph* g, const spf_b200_graph::Chain& c, cudaStream_t s) {
-  spf_b200_ctx* ctx = g->ctx;
-  CU(cudaMemsetAsync(g->d_chain_bar, 0, sizeof(unsigned long long), s));
-  ChainBatch P{g->d_chain + c.stage_off, c.n_stages, g->d_chain_bar, (int)ctx->p.cbs.radix_log, (int)ctx->p.cbs.count};
-  DevTables T = tabs(ctx);
-  void* args[] = {&P, &T};
-  const cudaError_t e = cudaLaunchCooperativeKernel(reinterpret_cast<void*>(cmux_chain_kernel), dim3((unsigned)c.grid), dim3(kWideTeams * kTeam), args,
-                                                    (size_t)kWideSmem, s);
-  if (e != cudaSuccess) return fail(ctx, SPF_E_CUDA, std::string("cmux_chain_kernel: ") + cudaGetErrorString(e));
-  return check_launch(ctx, "cmux_chain_kernel");
-}
-
 // Whether `rank` writes Output* node `id` into its io buffer: outputs of a MUX tree live on the tree's owner.
 bool writes_output(const spf_b200_graph* g, size_t id, int rank) {
   const int r = spf_b200_graph_output_rank(g, id);
@@ -949,24 +869,9 @@ int enqueue_run(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange
                 std::vector<cudaEvent_t>* timing_events) {
   if (int rc = enqueue_inputs(g, world > 1 && !exchange, s)) return rc;
   if (timing_events) cudaEventRecord((*timing_events)[0], s);
-  // SPF_B200_CHAIN=1: runs of narrow CMux levels as one cooperative launch each (cmux_chain_kernel; measured slower than
-  // programmatic dependent launches, so opt-in)
-  const char* chain_env = getenv("SPF_B200_CHAIN");
-  const bool use_chains = !timing_events && chain_env && chain_env[0] == '1';
-  if (use_chains && g->chain_rank != rank)
-    if (int rc = plan_chains(g, rank)) return rc;
-  size_t next_chain = 0;
   size_t gi = 0;
-  for (size_t gidx = 0; gidx < g->groups.size(); gidx++) {
-    const Group& G = g->groups[gidx];
-    if (use_chains && next_chain < g->chains.size() && gidx == g->chains[next_chain].first) {
-      const spf_b200_graph::Chain& c = g->chains[next_chain++];
-      if (int rc = launch_chain(g, c, s)) return rc;
-      gidx = c.last;  // the groups in between launch nothing or were part of the run
-      continue;
-    }
+  for (const Group& G : g->groups)
     if (int rc = enqueue_group(g, G, rank, world, exchange, user, s, timing_events ? (*timing_events)[++gi] : nullptr)) return rc;
-  }
   return enqueue_outputs(g, rank, s);
 }
 
@@ -1214,8 +1119,6 @@ void spf_b200_graph_destroy(spf_b200_graph* g) {
   cudaFree(g->d_gather);
   cudaFree(g->d_gather_tab);
   cudaFree(g->ks_states.p);
-  cudaFree(g->d_chain);
-  cudaFree(g->d_chain_bar);
   if (g->h_stage) cudaFreeHost(g->h_stage);
   for (void* q : g->pinned) cudaHostUnregister(q);
   if (g->done) cudaEventDestroy(g->done);

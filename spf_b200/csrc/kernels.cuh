@@ -72,62 +72,28 @@ __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefe
 // each owned by a PAIR of teams (128 threads, see pbs_pair_team), one persistent CTA per SM:
 // 12 warps, <= 168 registers.  Resident pairs walk the 637 BSK rows roughly in step, so a row is
 // fetched from HBM once per sweep and then served from L2 to all CTAs.  The per-thread constants
-// and parked values of a pair live in TENSOR MEMORY (tcgen05.ld/st): the switches below exist for
-// A/B measurements (DESIGN.md section 7 lists what each is worth).
+// and parked values of a pair live in TENSOR MEMORY (tcgen05.ld/st); DESIGN.md section 7 lists the
+// alternatives that were measured and what each was worth.
 // ------------------------------------------------------------------------------------------
-#ifndef SPF_PBS_PAIRS
-#define SPF_PBS_PAIRS 3
-#endif
-#ifndef SPF_PBS_TRANSIENT
-#define SPF_PBS_TRANSIENT 1  // accumulator image in the exchange buffer (pbs_pair_team, Cx::kTransient): 33 KB per pair
-#endif
-#ifndef SPF_PBS_TWOBUF
-#define SPF_PBS_TWOBUF 0  // two exchange buffers per half: both digit levels' transforms in flight together (team_ops.cuh, Cx::kTwoBuf); needs SPF_PBS_RING=0
-#endif
-constexpr int kPbsPairs = SPF_PBS_PAIRS;
-constexpr int kPbsPairBytes = (SPF_PBS_TRANSIENT ? 0 : 2 * kN * 8) + (SPF_PBS_TWOBUF ? 4 : 2) * kXBuf * 16;  // [acc +] 2 (4) exchange buffers
+constexpr int kPbsPairs = 3;
+// Per pair: the two exchange buffers (one per half).  The accumulator image lives in the half's exchange buffer
+// (pbs_pair_team), so a pair needs no persistent accumulator in shared memory: the BSK ring lives in what that frees.
+constexpr int kPbsPairBytes = 2 * kXBuf * 16;
 // tensor-memory columns: [0,64) T1 | own coefficients 64 per pair | parked accumulators 64 per pair while they fit
-// in the 512 columns (| T2 block when SPF_PBS_TMEM_T2); pairs beyond that park their accumulators in shared memory
+// in the 512 columns | [448,512) reader-side pass-2 twiddles; pairs beyond that park their accumulators in shared memory
 constexpr int kPbsTmemOwn0 = 64;
 constexpr int kPbsTmemF0 = kPbsTmemOwn0 + 64 * kPbsPairs;
 constexpr int kPbsTmemFPairs = (512 - kPbsTmemF0) / 64 < kPbsPairs ? (512 - kPbsTmemF0) / 64 : kPbsPairs;
 constexpr int kPbsFParkBytes = (kPbsPairs - kPbsTmemFPairs) * 2 * kTeam * 16 * 16;  // 32 KiB per pair parked in smem
-#ifndef SPF_PBS_RING
-#define SPF_PBS_RING (!SPF_PBS_TWOBUF)  // bootstrapping key staged through a shared-memory ring by bulk copies, one copy per chunk and CTA
-#endif
-static_assert(!SPF_PBS_RING || SPF_PBS_TRANSIENT, "the BSK ring lives in the shared memory the transient accumulator frees");
-#ifndef SPF_PBS_RING_STAGES
-#define SPF_PBS_RING_STAGES 3
-#endif
-constexpr int kRingStages = SPF_PBS_RING_STAGES;
+// The bootstrapping key is staged through a shared-memory ring by bulk copies, one copy per chunk and CTA.
+constexpr int kRingStages = 3;
 constexpr int kRingChunkElems = 2 * kM;                  // one (row, level) GLEV row of the BSK: [p][bin]
 constexpr int kRingChunkBytes = kRingChunkElems * 16;    // 32768
-// Four stages: the twiddle tables are only read while tensor memory is filled, so they are loaded into the LAST stage's
-// place (behind the other three) and that stage joins the ring afterwards; with three stages they sit in front as before.
-constexpr bool kPbsTablesInRing = SPF_PBS_RING && kRingStages == 4;
-#ifndef SPF_PBS_PAIR_SHIFT
-#define SPF_PBS_PAIR_SHIFT 0  // experiment: extra byte offset of the pairs' exchange buffers
-#endif
-constexpr int kPbsPairOff = (kPbsTablesInRing ? 0 : kTableBytes) + SPF_PBS_PAIR_SHIFT;
+constexpr int kPbsPairOff = kTableBytes;
 constexpr int kPbsRingOff = kPbsPairOff + kPbsPairs * kPbsPairBytes + kPbsFParkBytes;
-constexpr int kPbsTablesOff = kPbsTablesInRing ? kPbsRingOff + 3 * kRingChunkBytes : 0;
-constexpr int kPbsRingBytes = SPF_PBS_RING ? kRingStages * kRingChunkBytes + 64 : 0;  // + full barriers, release counters
+constexpr int kPbsRingBytes = kRingStages * kRingChunkBytes + 64;  // + full barriers, release counters
 constexpr int kPbsSmem = kPbsRingOff + kPbsRingBytes;
 static_assert(kPbsSmem <= 232448, "pbs_kernel shared memory");
-
-#ifndef SPF_PBS_TMEM_T1
-#define SPF_PBS_TMEM_T1 1   // pass-1 twiddles (per thread) in tensor memory
-#endif
-#ifndef SPF_PBS_TMEM_T2
-#define SPF_PBS_TMEM_T2 1   // pass-2 twiddles in tensor memory: round 1 measured this slower (9.2 vs 8.6 ms per wave, 255-register
-                            // build); with the kernel bound by shared-memory wavefronts it is worth 2.6 % (7.39 -> 7.19 ms, r2)
-#endif
-#ifndef SPF_PBS_TMEM_F
-#define SPF_PBS_TMEM_F 1    // accumulators parked in tensor memory while the second digit level is transformed
-#endif
-#ifndef SPF_PBS_TMEM_OWN
-#define SPF_PBS_TMEM_OWN 1  // private copy of the thread's own accumulator coefficients in tensor memory
-#endif
 
 // tensor-memory helpers (32x32b shape: thread i of a warp <-> TMEM lane 32*(warp%4)+i, one
 // 32-bit word per column)
@@ -173,13 +139,8 @@ __device__ __forceinline__ void mbar_wait_trap(uint32_t bar, uint32_t parity) {
   unsigned long long t_start = 0;
   for (int spin = 0;; spin++) {
     uint32_t ok;
-#if SPF_MBAR_HINT
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(bar), "r"(parity), "r"((uint32_t)SPF_MBAR_HINT) : "memory");
-#else
     asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
                  : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-#endif
     if (ok) return;
     if ((spin & 1023) == 1023) {  // a chunk that has not landed after 2 s will never land
       unsigned long long now;
@@ -189,212 +150,8 @@ __device__ __forceinline__ void mbar_wait_trap(uint32_t bar, uint32_t parity) {
     }
   }
 }
-static_assert(!SPF_PBS_TRANSIENT || SPF_PBS_TMEM_OWN, "the transient accumulator image needs the tensor-memory own copy");
-static_assert(!kPbsTablesInRing || SPF_PBS_TMEM_T1, "four ring stages overlay the twiddle tables: the twiddles must live in tensor memory");
-
-#ifndef SPF_PBS_CHUNKED
-#define SPF_PBS_CHUNKED 1  // own coefficients / twiddles fetched from tensor memory in small chunks (needed by the 128-register
-                           // 4-pair build; worth 2.7 % at 3 pairs too: shorter live ranges, better schedule)
-#endif
-#ifndef SPF_PBS_READER_T2
-#define SPF_PBS_READER_T2 1  // pass-2 twiddles applied by the consumers of the second exchange (team_ops.cuh: rt2_fwd_consts)
-#endif
-#ifndef SPF_PBS_INT_CONV
-#define SPF_PBS_INT_CONV 0  // accumulator update: f64 -> torus by integer arithmetic on the rounded product (fft16.cuh: f64_to_torus_int)
-#endif
-#ifndef SPF_PBS_FST2
-#define SPF_PBS_FST2 1  // accumulators parked with one tcgen05.st per double instead of four 16-register stores
-#endif
-#ifndef SPF_PBS_EARLY_REL
-#define SPF_PBS_EARLY_REL 0  // BSK ring: per-warp release right behind the last read of a chunk
-#endif
-#ifndef SPF_PBS_RING_FENCE
-#define SPF_PBS_RING_FENCE 1  // fence.proxy.async in front of every refill of a ring stage
-#endif
-#ifndef SPF_MBAR_HINT
-#define SPF_MBAR_HINT 0  // suspend-time hint (ns) of the mbarrier waits; 0: the hardware default
-#endif
-#ifndef SPF_PBS_FRND_CONV
-#define SPF_PBS_FRND_CONV 0  // accumulator update: f64 -> torus through the round-to-integral conversion (fft16.cuh: f64_to_torus_frnd)
-#endif
-#ifndef SPF_PBS_TW_PIPE
-#define SPF_PBS_TW_PIPE 0  // twiddle chunks software-pipelined: the tensor-memory load of chunk g + 1 overlaps the products of chunk g
-#endif
-#ifndef SPF_PBS_FUSED_ST
-#define SPF_PBS_FUSED_ST 0  // twiddle products stored to the exchange buffer one by one (interleaved STS)
-#endif
-#ifndef SPF_PBS_TMEM_X1
-#define SPF_PBS_TMEM_X1 0  // first exchange of a transform inside the warp, through tensor memory (fft16.cuh: x1_time_index):
-                           // bit-exact, but measured SLOWER (7.36 vs 7.24 ms per 444-ciphertext wave, profiles/r2_j_x1_ab.txt): the
-                           // two store -> wait -> load -> wait round trips cost more exposed latency than the 50 pipe clocks
-                           // per warp they save (tcgen05.st runs at 256 B/clk/SM on the same pipe as ld/st.shared)
-#endif
-// 16x256b shape: thread t of a warp <-> lanes base + t/4 and base + 8 + t/4, the 64-bit unit (t % 4) + 4 cg of each
-// 256-bit column group cg; register w + 2 eh + 4 cg = word w of that unit in lane base + 8 eh + t/4 (cute: SM100_TMEM_LOAD_16dp256b4x;
-// checked in both directions by tools/probes/tmem_xchg_probe.cu).  "Store 32x32b, load 16x256b" therefore moves two lane-index bits
-// into the register index and two column-index bits into the lane index.
-__device__ __forceinline__ void tmem_ld256x4(uint32_t* r, uint32_t taddr) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.16x256b.x4.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_st256x4(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.16x256b.x4.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld16p(uint32_t* r, uint32_t taddr) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_st16p(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-// Register / column bookkeeping of the two-round 16 x 16 transpose (all indices are compile-time after unrolling).
-// Round 1 (pass-1 thread, lane (i3 i2 i1 i0 g), doubles D(k, c), c = re / im):  32x32b unit = (k >> 2) + 4 (c + 2 (k & 3));
-//   its 16x256b read hands thread (i1 i0 g | k3 k2) the doubles E(e = (i3 i2), klo = k & 3, c);
-// round 2: 32x32b unit = klo + 4 (c + 2 e); its 16x256b read hands thread (g | k3 k2 k1 k0) = lane 16 g + k1 the doubles
-//   F(e, e' = (i1 i0), c) = y_{a}[k1].c of the group member m' = 4 e + e'.
-__device__ __forceinline__ constexpr int x1_unit1(int k, int c) { return (k >> 2) + 4 * (c + 2 * (k & 3)); }
-__device__ __forceinline__ constexpr int x1_unit2(int e, int klo, int c) { return klo + 4 * (c + 2 * e); }
-// register of word w in the four 16x256b.x4 accesses (block 2 b + ch: lane base 16 b, column offset 32 ch)
-__device__ __forceinline__ constexpr int x1_reg256(int b, int eh, int ch, int cg, int w) { return 16 * (2 * b + ch) + w + 2 * eh + 4 * cg; }
-__device__ __forceinline__ constexpr int x1_reg_r1(int e, int klo, int c, int w) {  // E(e, klo, c): j1 = c + 2 klo = cg + 4 ch
-  return x1_reg256(e >> 1, e & 1, klo >> 1, c + 2 * (klo & 1), w);
-}
-__device__ __forceinline__ constexpr int x1_reg_r2(int e, int ep, int c, int w) {   // F(e, e', c): j2 = c + 2 e = cg + 4 ch
-  return x1_reg256(ep >> 1, ep & 1, e >> 1, c + 2 * (e & 1), w);
-}
-__device__ __forceinline__ void x1_ld256(uint32_t (&r)[64], uint32_t ta) {
-  tmem_ld256x4(r, ta); tmem_ld256x4(r + 16, ta + 32); tmem_ld256x4(r + 32, ta + (16u << 16)); tmem_ld256x4(r + 48, ta + 32 + (16u << 16));
-}
-__device__ __forceinline__ void x1_st256(uint32_t ta, const uint32_t (&r)[64]) {
-  tmem_st256x4(ta, r); tmem_st256x4(ta + 32, r + 16); tmem_st256x4(ta + (16u << 16), r + 32); tmem_st256x4(ta + 32 + (16u << 16), r + 48);
-}
-__device__ __forceinline__ void x1_ld32(uint32_t (&r)[64], uint32_t ta) {
-  tmem_ld16p(r, ta); tmem_ld16p(r + 16, ta + 16); tmem_ld16p(r + 32, ta + 32); tmem_ld16p(r + 48, ta + 48);
-}
-__device__ __forceinline__ void x1_st32(uint32_t ta, const uint32_t (&r)[64]) {
-  tmem_st16p(ta, r); tmem_st16p(ta + 16, r + 16); tmem_st16p(ta + 32, r + 32); tmem_st16p(ta + 48, r + 48);
-}
 struct DevPairCx {
-  static constexpr bool kTransient = SPF_PBS_TRANSIENT != 0;
-  static constexpr bool kChunked = SPF_PBS_CHUNKED != 0;
-  static constexpr bool kFusedStores = SPF_PBS_FUSED_ST != 0;
-  // ordered store: a volatile asm keeps its place among the twiddle multiplies
-  static __device__ __forceinline__ void sts_c2(C2* p, C2 v) {
-    asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"((uint32_t)__cvta_generic_to_shared(p)), "d"(v.x), "d"(v.y) : "memory");
-  }
-  __device__ __forceinline__ void sts(C2* p, C2 v) const { sts_c2(p, v); }
-  template <bool CONJ>
-  __device__ __forceinline__ void t1_mul_store(C2 (&v)[16], const C2* T1, C2* buf) const {
-#pragma unroll
-    for (int g = 0; g < 4; g++) {
-      uint32_t r[16];
-      tmem_ld16(r, t1_taddr + 16 * g);
-      tmem_wait_ld();
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const C2 w{__hiloint2double((int)r[4 * i + 1], (int)r[4 * i]), __hiloint2double((int)r[4 * i + 3], (int)r[4 * i + 2])};
-        const int k = 4 * g + i;
-        v[k] = CONJ ? cmul_conj(v[k], w) : cmul(v[k], w);
-        sts_c2(buf + k * kXPad + u, v[k]);
-      }
-    }
-  }
-  template <bool CONJ>
-  __device__ __forceinline__ void t2_mul_store(C2 (&v)[16], const C2* T2, C2* buf) const {
-    const int k1 = u & 15, q = u >> 4;
-#pragma unroll
-    for (int k2 = 0; k2 < 16; k2++) {
-      if (k2) v[k2] = CONJ ? cmul_conj(v[k2], T2[q * kT2Pad + k2]) : cmul(v[k2], T2[q * kT2Pad + k2]);
-      sts_c2(buf + k1 * kXPad + q + 4 * k2, v[k2]);
-    }
-  }
-  // ---- first exchange through tensor memory (SPF_PBS_TMEM_X1) ----
-  static constexpr bool kTmemX1 = SPF_PBS_TMEM_X1 != 0;
-  __device__ __forceinline__ int time_index() const { return kTmemX1 ? x1_time_index(u) : u; }
-  // forward: v[k1] of pass-1 thread a  ->  v[m'] = y_{q + 4 m'}[k1] of pass-2 thread (k1, q).  The 64 scratch columns are the
-  // warp's parking place of the accumulators (f_taddr), which is free whenever this is called (pbs_pair_team).
-  __device__ __forceinline__ void x1_fwd(C2 (&v)[16]) const {
-    uint32_t r[64], s[64];
-#pragma unroll
-    for (int k = 0; k < 16; k++) {
-      r[2 * x1_unit1(k, 0)] = (uint32_t)__double2loint(v[k].x); r[2 * x1_unit1(k, 0) + 1] = (uint32_t)__double2hiint(v[k].x);
-      r[2 * x1_unit1(k, 1)] = (uint32_t)__double2loint(v[k].y); r[2 * x1_unit1(k, 1) + 1] = (uint32_t)__double2hiint(v[k].y);
-    }
-    x1_st32(f_taddr, r);
-    tmem_wait_st();
-    x1_ld256(s, f_taddr);
-    tmem_wait_ld();
-#pragma unroll
-    for (int e = 0; e < 4; e++)
-#pragma unroll
-      for (int klo = 0; klo < 4; klo++)
-#pragma unroll
-        for (int c = 0; c < 2; c++)
-#pragma unroll
-          for (int w = 0; w < 2; w++) r[2 * x1_unit2(e, klo, c) + w] = s[x1_reg_r1(e, klo, c, w)];
-    x1_st32(f_taddr, r);
-    tmem_wait_st();
-    x1_ld256(s, f_taddr);
-    tmem_wait_ld();
-#pragma unroll
-    for (int e = 0; e < 4; e++)
-#pragma unroll
-      for (int ep = 0; ep < 4; ep++) {
-        v[4 * e + ep].x = __hiloint2double((int)s[x1_reg_r2(e, ep, 0, 1)], (int)s[x1_reg_r2(e, ep, 0, 0)]);
-        v[4 * e + ep].y = __hiloint2double((int)s[x1_reg_r2(e, ep, 1, 1)], (int)s[x1_reg_r2(e, ep, 1, 0)]);
-      }
-  }
-  // inverse: w[m'] of thread (k1, q)  ->  w[k1] of thread a = q + 4 m' (the same two rounds backwards, shapes swapped)
-  __device__ __forceinline__ void x1_inv(C2 (&v)[16]) const {
-    uint32_t r[64], s[64];
-#pragma unroll
-    for (int e = 0; e < 4; e++)
-#pragma unroll
-      for (int ep = 0; ep < 4; ep++) {
-        s[x1_reg_r2(e, ep, 0, 0)] = (uint32_t)__double2loint(v[4 * e + ep].x); s[x1_reg_r2(e, ep, 0, 1)] = (uint32_t)__double2hiint(v[4 * e + ep].x);
-        s[x1_reg_r2(e, ep, 1, 0)] = (uint32_t)__double2loint(v[4 * e + ep].y); s[x1_reg_r2(e, ep, 1, 1)] = (uint32_t)__double2hiint(v[4 * e + ep].y);
-      }
-    x1_st256(f_taddr, s);
-    tmem_wait_st();
-    x1_ld32(r, f_taddr);
-    tmem_wait_ld();
-#pragma unroll
-    for (int e = 0; e < 4; e++)
-#pragma unroll
-      for (int klo = 0; klo < 4; klo++)
-#pragma unroll
-        for (int c = 0; c < 2; c++)
-#pragma unroll
-          for (int w = 0; w < 2; w++) s[x1_reg_r1(e, klo, c, w)] = r[2 * x1_unit2(e, klo, c) + w];
-    x1_st256(f_taddr, s);
-    tmem_wait_st();
-    x1_ld32(r, f_taddr);
-    tmem_wait_ld();
-#pragma unroll
-    for (int k = 0; k < 16; k++) {
-      v[k].x = __hiloint2double((int)r[2 * x1_unit1(k, 0) + 1], (int)r[2 * x1_unit1(k, 0)]);
-      v[k].y = __hiloint2double((int)r[2 * x1_unit1(k, 1) + 1], (int)r[2 * x1_unit1(k, 1)]);
-    }
-  }
   // ---- reader-side pass-2 twiddles: 12 + 12 doubles of this thread in the columns [448, 496) (pair_tmem_init) ----
-  static constexpr bool kReaderT2 = SPF_PBS_READER_T2 != 0;
-  static constexpr bool kTwoBuf = SPF_PBS_TWOBUF != 0;
-  static constexpr bool kIntConv = SPF_PBS_INT_CONV != 0;
-  static constexpr bool kFrndConv = SPF_PBS_FRND_CONV != 0;
   __device__ __forceinline__ void rt2_fwd(double (&tw)[12], const C2*) const {
     uint32_t a[16], b[8];
     tmem_ld16(a, t1_taddr + 448);
@@ -421,8 +178,7 @@ struct DevPairCx {
   uint32_t own_taddr;  // this warp's private 64 columns (own coefficients)
   uint32_t f_taddr;    // this warp's 64 columns for the parked accumulators (unused when fpark != nullptr)
   C2* fpark;           // shared-memory parking [16][128] of a pair whose accumulators do not fit in tensor memory
-  // ---- BSK ring (SPF_PBS_RING; protocol in team_ops.cuh above pbs_pair_team) ----
-  static constexpr bool kBskRing = SPF_PBS_RING != 0;
+  // ---- BSK ring (protocol in team_ops.cuh above pbs_pair_team) ----
   uint32_t ring_s = 0, full_s = 0;  // shared addresses of stage 0 / of full[0]
   unsigned* rel = nullptr;          // per-stage count of pairs that are done with the resident chunk
   const C2* bsk = nullptr;
@@ -432,101 +188,52 @@ struct DevPairCx {
   __device__ __forceinline__ void ring_issue(int Gn) const {
     const int i = (Gn >> 2) % lwe_n, k = Gn & 3, c = (k & 1) * 2 + (1 - (k >> 1)), st = Gn % kRingStages;
     const C2* src = bsk + ((size_t)i * 4 + c) * kRingChunkElems;
-#if SPF_PBS_RING_FENCE
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-#endif
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // in front of every refill of a ring stage
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full_s + 8 * st), "r"((uint32_t)kRingChunkBytes) : "memory");
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(ring_s + st * kRingChunkBytes), "l"(src), "r"((uint32_t)kRingChunkBytes), "r"(full_s + 8 * st) : "memory");
   }
-  // returns the chunk's address: a shared-window address in a pointer's clothes when the ring is on (bsk_load)
-  __device__ __forceinline__ const C2* bsk_acquire(int G, const C2* g) const {
-#if SPF_PBS_RING
+  // returns the chunk's address: a shared-window address in a pointer's clothes (bsk_load)
+  __device__ __forceinline__ const C2* bsk_acquire(int G, const C2*) const {
     const int st = G % kRingStages;
     mbar_wait_trap(full_s + 8 * st, (uint32_t)(G / kRingStages) & 1u);
     return reinterpret_cast<const C2*>((size_t)(ring_s + st * kRingChunkBytes));
-#else
-    return g;
-#endif
   }
   __device__ __forceinline__ C2 bsk_load(const C2* p) const {
-#if SPF_PBS_RING
-    if (SPF_ABLATE(16)) return C2{1.5, (double)((size_t)p & 0xFF)};
     C2 r;
     asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "r"((uint32_t)(size_t)p) : "memory");
     return r;
-#else
-    if (SPF_ABLATE(16)) return C2{1.5, (double)((size_t)p & 0xFF)};
-    return ldg_c2_pinned(p);
-#endif
-  }
-  // SPF_PBS_EARLY_REL: every WARP counts itself off a chunk right after its last read of it (bsk_release_early, called behind the
-  // multiply-accumulate that consumed the chunk) instead of one thread per pair at the next pair barrier, which can be thousands of
-  // clocks later: the refill of the stage starts as soon as the twelfth warp is done, the pairs wait less for the next chunk.
-  static constexpr bool kEarlyRel = SPF_PBS_EARLY_REL != 0;
-  __device__ __forceinline__ void bsk_release_early(int G) const {
-#if SPF_PBS_RING && SPF_PBS_EARLY_REL
-    __syncwarp();
-    release_one(G);
-#endif
   }
   __device__ __forceinline__ void bsk_release(int G) const {
-#if SPF_PBS_RING && !SPF_PBS_EARLY_REL
-    release_one(G);
-#endif
-  }
-  __device__ __forceinline__ void release_one(int G) const {
-#if SPF_PBS_RING
     if (elected) {
       const int st = G % kRingStages;
       __threadfence_block();
-      if (atomicAdd(rel + st, 1u) == (unsigned)npairs - 1u) {  // last pair (warp) out re-arms the stage
+      if (atomicAdd(rel + st, 1u) == (unsigned)npairs - 1u) {  // last pair out re-arms the stage
         atomicExch(rel + st, 0u);
         __threadfence_block();
         if (G + kRingStages < total) ring_issue(G + kRingStages);
       }
     }
-#endif
   }
   __device__ __forceinline__ void bsk_skip(int G) const {  // a step whose rotation is the identity: count off unread chunks
-#if SPF_PBS_RING
     if (elected) {
 #pragma unroll 1
       for (int k = 0; k < 4; k++) {
         mbar_wait_trap(full_s + 8 * ((G + k) % kRingStages), (uint32_t)((G + k) / kRingStages) & 1u);  // the copy has landed
-        release_one(G + k);
+        bsk_release(G + k);
       }
     }
-#endif
   }
-  __device__ __forceinline__ void sync() const { if (!SPF_ABLATE(8)) asm volatile("bar.sync %0, 64;" ::"r"(bar_half) : "memory"); }
-  __device__ __forceinline__ void pair_sync() const { if (!SPF_ABLATE(8)) asm volatile("bar.sync %0, 128;" ::"r"(bar_pair) : "memory"); }
+  __device__ __forceinline__ void sync() const { asm volatile("bar.sync %0, 64;" ::"r"(bar_half) : "memory"); }
+  __device__ __forceinline__ void pair_sync() const { asm volatile("bar.sync %0, 128;" ::"r"(bar_pair) : "memory"); }
   // v[k1] *= T1[k1][u] (or its conjugate).  The 16 twiddles of a thread never change, so they sit
   // in the thread's tensor-memory columns instead of a shared-memory table: 16 LDS.128 per
   // transform (12 % of the kernel's shared-memory wavefronts) become 4 tcgen05.ld on a path the
-  // LSU pipe does not see.
+  // LSU pipe does not see.  Four twiddles (16 registers) at a time: shorter live ranges, a better schedule.
   template <bool CONJ>
-  __device__ __forceinline__ void t1_mul(C2 (&v)[16], const C2* T1) const {
-#if SPF_PBS_TMEM_T1 && SPF_PBS_CHUNKED && SPF_PBS_TW_PIPE
-    // the load of chunk g + 1 is in flight while chunk g is multiplied: one exposed tensor-memory round trip per call, not four
-    uint32_t r[2][16];
-    tmem_ld16(r[0], t1_taddr);
-    tmem_wait_ld();
+  __device__ __forceinline__ void t1_mul(C2 (&v)[16], const C2*) const {
 #pragma unroll
     for (int g = 0; g < 4; g++) {
-      if (g < 3) tmem_ld16(r[(g + 1) & 1], t1_taddr + 16 * (g + 1));
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const uint32_t* rr = r[g & 1];
-        const C2 w{__hiloint2double((int)rr[4 * i + 1], (int)rr[4 * i]), __hiloint2double((int)rr[4 * i + 3], (int)rr[4 * i + 2])};
-        const int k = 4 * g + i;
-        v[k] = CONJ ? cmul_conj(v[k], w) : cmul(v[k], w);
-      }
-      if (g < 3) tmem_wait_ld();
-    }
-#elif SPF_PBS_TMEM_T1 && SPF_PBS_CHUNKED
-#pragma unroll
-    for (int g = 0; g < 4; g++) {  // 4 twiddles (16 registers) at a time
       uint32_t r[16];
       tmem_ld16(r, t1_taddr + 16 * g);
       tmem_wait_ld();
@@ -537,82 +244,14 @@ struct DevPairCx {
         v[k] = CONJ ? cmul_conj(v[k], w) : cmul(v[k], w);
       }
     }
-#elif SPF_PBS_TMEM_T1
-#pragma unroll
-    for (int half = 0; half < 2; half++) {
-      uint32_t r0[16], r1[16];
-      tmem_ld16(r0, t1_taddr + 32 * half);
-      tmem_ld16(r1, t1_taddr + 32 * half + 16);
-      tmem_wait_ld();
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const C2 w0{__hiloint2double((int)r0[4 * i + 1], (int)r0[4 * i]), __hiloint2double((int)r0[4 * i + 3], (int)r0[4 * i + 2])};
-        const C2 w1{__hiloint2double((int)r1[4 * i + 1], (int)r1[4 * i]), __hiloint2double((int)r1[4 * i + 3], (int)r1[4 * i + 2])};
-        const int ka = 8 * half + i, kb = 8 * half + 4 + i;
-        v[ka] = CONJ ? cmul_conj(v[ka], w0) : cmul(v[ka], w0);
-        v[kb] = CONJ ? cmul_conj(v[kb], w1) : cmul(v[kb], w1);
-      }
-    }
-#else
-#pragma unroll
-    for (int k1 = 0; k1 < 16; k1++) v[k1] = CONJ ? cmul_conj(v[k1], T1[k1 * 64 + u]) : cmul(v[k1], T1[k1 * 64 + u]);
-#endif
   }
-  // v[k2] *= T2[q][k2], k2 = 1..15
-  template <bool CONJ>
-  __device__ __forceinline__ void t2_mul(C2 (&v)[16], const C2* T2) const {
-#if SPF_PBS_TMEM_T2 && SPF_PBS_TW_PIPE
-    uint32_t r[2][16];
-    tmem_ld16(r[0], t1_taddr + 448);
-    tmem_wait_ld();
-#pragma unroll
-    for (int g = 0; g < 4; g++) {
-      if (g < 3) tmem_ld16(r[(g + 1) & 1], t1_taddr + 448 + 16 * (g + 1));
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const uint32_t* rr = r[g & 1];
-        const C2 w{__hiloint2double((int)rr[4 * i + 1], (int)rr[4 * i]), __hiloint2double((int)rr[4 * i + 3], (int)rr[4 * i + 2])};
-        const int k = 4 * g + i;
-        if (k != 0) v[k] = CONJ ? cmul_conj(v[k], w) : cmul(v[k], w);
-      }
-      if (g < 3) tmem_wait_ld();
-    }
-#elif SPF_PBS_TMEM_T2
-#pragma unroll
-    for (int half = 0; half < 2; half++) {
-      uint32_t r0[16], r1[16];
-      tmem_ld16(r0, t1_taddr + 448 + 32 * half);
-      tmem_ld16(r1, t1_taddr + 448 + 32 * half + 16);
-      tmem_wait_ld();
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const C2 w0{__hiloint2double((int)r0[4 * i + 1], (int)r0[4 * i]), __hiloint2double((int)r0[4 * i + 3], (int)r0[4 * i + 2])};
-        const C2 w1{__hiloint2double((int)r1[4 * i + 1], (int)r1[4 * i]), __hiloint2double((int)r1[4 * i + 3], (int)r1[4 * i + 2])};
-        const int ka = 8 * half + i, kb = 8 * half + 4 + i;
-        if (ka != 0) v[ka] = CONJ ? cmul_conj(v[ka], w0) : cmul(v[ka], w0);
-        v[kb] = CONJ ? cmul_conj(v[kb], w1) : cmul(v[kb], w1);
-      }
-    }
-#else
-    const int q = u >> 4;
-#pragma unroll
-    for (int k2 = 1; k2 < 16; k2++) v[k2] = CONJ ? cmul_conj(v[k2], T2[q * kT2Pad + k2]) : cmul(v[k2], T2[q * kT2Pad + k2]);
-#endif
-  }
+  // accumulators parked in tensor memory while the second digit level is transformed
   __device__ __forceinline__ void f_store(const C2 (&f)[2][8]) const {
-#if SPF_PBS_TMEM_F
     if (fpark) {
 #pragma unroll
       for (int c = 0; c < 16; c++) fpark[c * 2 * kTeam + h * kTeam + u] = f[c >> 3][c & 7];
       return;
     }
-#if SPF_PBS_FST2 == 2
-#pragma unroll
-    for (int c = 0; c < 16; c++) {
-      const C2 x = f[c >> 3][c & 7];
-      tmem_st4(f_taddr + 4 * c, (uint32_t)__double2loint(x.x), (uint32_t)__double2hiint(x.x), (uint32_t)__double2loint(x.y), (uint32_t)__double2hiint(x.y));
-    }
-#elif SPF_PBS_FST2
     // one double per store: a 16-register store makes ptxas gather the 64 words into consecutive registers first (64 moves)
 #pragma unroll
     for (int c = 0; c < 16; c++) {
@@ -620,24 +259,9 @@ struct DevPairCx {
       tmem_st2(f_taddr + 4 * c, (uint32_t)__double2loint(x.x), (uint32_t)__double2hiint(x.x));
       tmem_st2(f_taddr + 4 * c + 2, (uint32_t)__double2loint(x.y), (uint32_t)__double2hiint(x.y));
     }
-#else
-#pragma unroll
-    for (int c = 0; c < 4; c++) {
-      uint32_t r[16];
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const C2 x = f[c >> 1][4 * (c & 1) + i];
-        r[4 * i] = (uint32_t)__double2loint(x.x); r[4 * i + 1] = (uint32_t)__double2hiint(x.x);
-        r[4 * i + 2] = (uint32_t)__double2loint(x.y); r[4 * i + 3] = (uint32_t)__double2hiint(x.y);
-      }
-      tmem_st16(f_taddr + 16 * c, r);
-    }
-#endif
     tmem_wait_st();
-#endif
   }
   __device__ __forceinline__ void f_load(C2 (&f)[2][8]) const {
-#if SPF_PBS_TMEM_F
     if (fpark) {
 #pragma unroll
       for (int c = 0; c < 16; c++) f[c >> 3][c & 7] = fpark[c * 2 * kTeam + h * kTeam + u];
@@ -654,23 +278,8 @@ struct DevPairCx {
         f[c >> 1][4 * (c & 1) + i] = C2{__hiloint2double((int)r[c][4 * i + 1], (int)r[c][4 * i]),
                                         __hiloint2double((int)r[c][4 * i + 3], (int)r[c][4 * i + 2])};
     }
-#endif
   }
-  __device__ __forceinline__ void own_load(uint64_t (&own)[32], const uint64_t* pa) const {
-#if SPF_PBS_TMEM_OWN
-    uint32_t r[4][16];
-#pragma unroll
-    for (int c = 0; c < 4; c++) tmem_ld16(r[c], own_taddr + 16 * c);
-    tmem_wait_ld();  // one wait for all four loads
-#pragma unroll
-    for (int c = 0; c < 4; c++)
-#pragma unroll
-      for (int i = 0; i < 8; i++) own[8 * c + i] = ((uint64_t)r[c][2 * i + 1] << 32) | r[c][2 * i];
-#else
-#pragma unroll
-    for (int i2 = 0; i2 < 32; i2++) own[i2] = pa[u + 64 * i2];
-#endif
-  }
+  // the thread's own accumulator coefficients: a private copy in tensor memory, fetched 8 (gather) or 4 + 4 (update) at a time
   __device__ __forceinline__ void own_ld8(uint64_t (&o)[8], int c) const {
     uint32_t r[16];
     tmem_ld16(r, own_taddr + 16 * c);
@@ -701,7 +310,6 @@ struct DevPairCx {
   }
   __device__ __forceinline__ void own_st_wait() const { tmem_wait_st(); }
   __device__ __forceinline__ void own_store(const uint64_t (&own)[32]) const {
-#if SPF_PBS_TMEM_OWN
 #pragma unroll
     for (int c = 0; c < 4; c++) {
       uint32_t r[16];
@@ -710,19 +318,14 @@ struct DevPairCx {
       tmem_st16(own_taddr + 16 * c, r);
     }
     tmem_wait_st();
-#endif
   }
 };
-
-static_assert(!SPF_PBS_TMEM_X1 || (SPF_PBS_TMEM_T1 && SPF_PBS_TMEM_F && !SPF_PBS_FUSED_ST && kPbsTmemFPairs == kPbsPairs),
-              "the tensor-memory first exchange needs the per-thread twiddles and a parking block per pair in tensor memory");
 
 // Tensor-memory scratchpad of the pair / quad team kernels: one 512-column allocation per CTA.
 // Columns [0,64) pass-1 twiddles of the thread (shared by the warps of a lane quarter, which have the same
 // thread-in-team index), then the per-pair blocks of pbs_kernel (kPbsTmemOwn0, kPbsTmemF0); [448,512) pass-2
-// twiddles when SPF_PBS_TMEM_T2.  Returns this warp's lane-quarter base address.
-__device__ __forceinline__ uint32_t pair_tmem_init(const C2* sT1, const C2* sT2, uint32_t& alloc_base, bool time_remap = false,
-                                                   bool reader_t2 = false) {
+// twiddles.  Returns this warp's lane-quarter base address.
+__device__ __forceinline__ uint32_t pair_tmem_init(const C2* sT1, const C2* sT2, uint32_t& alloc_base, bool reader_t2 = false) {
   __shared__ uint32_t tmem_base;
   const int warp = threadIdx.x >> 5;
   if (warp == 0) {
@@ -737,10 +340,9 @@ __device__ __forceinline__ uint32_t pair_tmem_init(const C2* sT1, const C2* sT2,
   const uint32_t t1_taddr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16);
   if (warp < 4) {  // every lane quarter is shared by warps w, w+4, w+8, which have the same u
     const int uu = (warp & 1) * 32 + (threadIdx.x & 31);
-    const int ua = time_remap ? x1_time_index(uu) : uu;  // pass-1 identity of this thread (SPF_PBS_TMEM_X1)
 #pragma unroll
     for (int k1 = 0; k1 < 16; k1++) {
-      const C2 w = sT1[k1 * 64 + ua];
+      const C2 w = sT1[k1 * 64 + uu];
       tmem_st4(t1_taddr + 4 * k1, (uint32_t)__double2loint(w.x), (uint32_t)__double2hiint(w.x),
                (uint32_t)__double2loint(w.y), (uint32_t)__double2hiint(w.y));
     }
@@ -759,14 +361,13 @@ __device__ __forceinline__ uint32_t pair_tmem_init(const C2* sT1, const C2* sT2,
         tmem_st4(t1_taddr + 448 + 24 + 4 * i, (uint32_t)__double2loint(wi[i].x), (uint32_t)__double2hiint(wi[i].x),
                  (uint32_t)__double2loint(wi[i].y), (uint32_t)__double2hiint(wi[i].y));
     } else {
-#if SPF_PBS_TMEM_T2
+      // pbs_quad_kernel: the table row of pass-2 twiddles (it writes its reader-side constants over it)
 #pragma unroll
-    for (int k2 = 0; k2 < 16; k2++) {
-      const C2 w = k2 ? sT2[(uu >> 4) * kT2Pad + k2] : C2{1.0, 0.0};
-      tmem_st4(t1_taddr + 448 + 4 * k2, (uint32_t)__double2loint(w.x), (uint32_t)__double2hiint(w.x),
-               (uint32_t)__double2loint(w.y), (uint32_t)__double2hiint(w.y));
-    }
-#endif
+      for (int k2 = 0; k2 < 16; k2++) {
+        const C2 w = k2 ? sT2[(uu >> 4) * kT2Pad + k2] : C2{1.0, 0.0};
+        tmem_st4(t1_taddr + 448 + 4 * k2, (uint32_t)__double2loint(w.x), (uint32_t)__double2hiint(w.x),
+                 (uint32_t)__double2loint(w.y), (uint32_t)__double2hiint(w.y));
+      }
     }
     tmem_wait_st();
   }
@@ -795,24 +396,21 @@ struct PbsBatch {
 
 __global__ void __launch_bounds__(kPbsPairs * 2 * kTeam, 1) pbs_kernel(PbsBatch P, DevTables tabs) {
   extern __shared__ __align__(16) unsigned char smem[];
-  C2* sT1 = reinterpret_cast<C2*>(smem + kPbsTablesOff);
+  C2* sT1 = reinterpret_cast<C2*>(smem);
   C2* sT2 = sT1 + kT1Elems;
   load_tables(sT1, sT2, tabs);
   uint32_t tmem_alloc;
-  const uint32_t t1_taddr = pair_tmem_init(sT1, sT2, tmem_alloc, DevPairCx::kTmemX1, DevPairCx::kReaderT2);
+  const uint32_t t1_taddr = pair_tmem_init(sT1, sT2, tmem_alloc, true);
   const int pair = threadIdx.x / (2 * kTeam);
   const int npairs = blockDim.x / (2 * kTeam);  // 1..kPbsPairs pairs per CTA (fewer for small batches)
   const int h = (threadIdx.x / kTeam) & 1;
-  unsigned char* base = smem + kPbsPairOff + pair * kPbsPairBytes;
-  uint64_t* acc = reinterpret_cast<uint64_t*>(base);  // unused when SPF_PBS_TRANSIENT
-  C2* xb = reinterpret_cast<C2*>(base + (SPF_PBS_TRANSIENT ? 0 : 2 * kN * 8));
+  C2* xb = reinterpret_cast<C2*>(smem + kPbsPairOff + pair * kPbsPairBytes);
   C2* fpark = pair < kPbsTmemFPairs ? nullptr
                                     : reinterpret_cast<C2*>(smem + kPbsPairOff + kPbsPairs * kPbsPairBytes) + (pair - kPbsTmemFPairs) * 2 * kTeam * 16;
   DevPairCx cx{(int)(threadIdx.x % kTeam), h, 1 + pair * 3 + h, 3 + pair * 3, t1_taddr, t1_taddr + kPbsTmemOwn0 + 64 * pair,
                t1_taddr + kPbsTmemF0 + 64 * (pair < kPbsTmemFPairs ? pair : 0), fpark};
   int G = 0;        // chunk position of this pair in the CTA-wide BSK chunk sequence
   int rounds = 0;   // ciphertexts the busiest pair (pair 0) of this CTA processes
-#if SPF_PBS_RING
   {
     uint64_t* full = reinterpret_cast<uint64_t*>(smem + kPbsRingOff + kRingStages * kRingChunkBytes);
     cx.ring_s = smem_u32(smem + kPbsRingOff);
@@ -820,8 +418,8 @@ __global__ void __launch_bounds__(kPbsPairs * 2 * kTeam, 1) pbs_kernel(PbsBatch 
     cx.rel = reinterpret_cast<unsigned*>(full + kRingStages);
     cx.bsk = P.bsk;
     cx.lwe_n = P.lwe_n;
-    cx.npairs = DevPairCx::kEarlyRel ? 4 * npairs : npairs;                       // participants that count themselves off a chunk
-    cx.elected = (threadIdx.x % (DevPairCx::kEarlyRel ? 32 : 2 * kTeam)) == 0;  // one thread per warp / per pair
+    cx.npairs = npairs;                             // participants that count themselves off a chunk
+    cx.elected = (threadIdx.x % (2 * kTeam)) == 0;  // one thread per pair
     if ((int)blockIdx.x < P.batch) rounds = (P.batch - (int)blockIdx.x + (int)gridDim.x * npairs - 1) / ((int)gridDim.x * npairs);
     cx.total = rounds * 4 * P.lwe_n;
     if (threadIdx.x == 0) {
@@ -835,7 +433,6 @@ __global__ void __launch_bounds__(kPbsPairs * 2 * kTeam, 1) pbs_kernel(PbsBatch 
     if (threadIdx.x == 0)
       for (int g0 = 0; g0 < kRingStages && g0 < cx.total; g0++) cx.ring_issue(g0);
   }
-#endif
   // Persistent pairs: slot (pair, CTA) takes ciphertexts slot, slot + slots, ...  Slots are numbered
   // pair-major so that a trailing partial round leaves at most one busy pair on as many SMs as
   // possible (a pair alone on an SM runs ~1.3x faster than one sharing it with two others).
@@ -850,16 +447,14 @@ __global__ void __launch_bounds__(kPbsPairs * 2 * kTeam, 1) pbs_kernel(PbsBatch 
     A.log_v = P.log_v;
     A.cbs_radix_log = P.cbs_radix_log;
     A.cbs_count = P.cbs_count;
-    pbs_pair_team(cx, A, acc, xb, sT1, sT2, G);
+    pbs_pair_team(cx, A, xb, sT1, sT2, G);
   }
-#if SPF_PBS_RING
   // a pair with fewer ciphertexts than pair 0 (the tail of the batch) still counts itself off the remaining chunks
   if (cx.elected)
     for (; G < cx.total; G++) {
       mbar_wait_trap(cx.full_s + 8 * (G % kRingStages), (uint32_t)(G / kRingStages) & 1u);
-      cx.release_one(G);
+      cx.bsk_release(G);
     }
-#endif
   pair_tmem_free(tmem_alloc);
 }
 
@@ -874,17 +469,8 @@ constexpr int kQuadRowBytes = 8 * kM * 16;                                      
 constexpr int kQuadSmem = kQuadT2Bytes + 2 * kN * 8 + 4 * kXBuf * 16 + kQuadRowBytes + 16;  // 231504
 
 
-#ifndef SPF_QUAD_TMEM_T2
-#define SPF_QUAD_TMEM_T2 1
-#endif
-#ifndef SPF_QUAD_SPLIT_GATHER
-#define SPF_QUAD_SPLIT_GATHER 1  // the two teams of a polynomial gather half of the rounded differences each and swap digits
-#endif
-#ifndef SPF_QUAD_READER_T2
-#define SPF_QUAD_READER_T2 1  // pass-2 twiddles applied by the consumers of the second exchange, as in pbs_kernel (3.52 -> 3.36 ms at batch 1, 3.39 -> 3.31 at 64)
-#endif
 struct DevQuadCx {
-  static constexpr bool kSplitGather = SPF_QUAD_SPLIT_GATHER != 0;
+  // Split gather: the two teams of a polynomial gather half of the rounded differences each and swap digits.
   // Teams (h, 0) and (h, 1) are warps {2h, 2h+1} and {4 + 2h, 5 + 2h}: thread u of both sits on the same tensor-memory lane,
   // so 16 packed digits change hands through eight columns of that lane (columns [64, 72) written by t = 0, [72, 80) by
   // t = 1) and one 128-thread barrier -- no shared memory (the kernel has none left) and no second gather.
@@ -896,8 +482,8 @@ struct DevQuadCx {
     tmem_wait_ld();
   }
   // reader-side pass-2 twiddles (team_ops.cuh: rt2_group_consts): 12 doubles per thread in the columns [448 + 24 t, 472 + 24 t)
-  // of its lane (warps w and w + 4 share a lane quarter and differ in t)
-  static constexpr bool kReaderT2 = SPF_QUAD_READER_T2 != 0;
+  // of its lane (warps w and w + 4 share a lane quarter and differ in t).  Measured against the producer-side twiddles: 3.52 -> 3.36 ms
+  // at batch 1, 3.39 -> 3.31 at 64.
   __device__ __forceinline__ void rt2(double (&tw)[6], C2 (&wi)[3], const C2*) const {
     uint32_t a[16], b[8];
     tmem_ld16(a, t1_taddr + 448 + 24 * t);
@@ -960,32 +546,6 @@ struct DevQuadCx {
       }
     }
   }
-  template <bool CONJ>
-  __device__ __forceinline__ void t2_mul(C2 (&v)[16], const C2* T2) const {
-#if SPF_PBS_TMEM_T2 && SPF_QUAD_TMEM_T2
-    // the thread's 15 pass-2 twiddles from its tensor-memory columns [448, 512) (filled by pair_tmem_init): tcgen05.ld
-    // costs next to nothing on the load / store pipe, the 15 broadcast LDS.128 it replaces sat on the critical path
-#pragma unroll
-    for (int half = 0; half < 2; half++) {
-      uint32_t r0[16], r1[16];
-      tmem_ld16(r0, t1_taddr + 448 + 32 * half);
-      tmem_ld16(r1, t1_taddr + 448 + 32 * half + 16);
-      tmem_wait_ld();
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const C2 w0{__hiloint2double((int)r0[4 * i + 1], (int)r0[4 * i]), __hiloint2double((int)r0[4 * i + 3], (int)r0[4 * i + 2])};
-        const C2 w1{__hiloint2double((int)r1[4 * i + 1], (int)r1[4 * i]), __hiloint2double((int)r1[4 * i + 3], (int)r1[4 * i + 2])};
-        const int ka = 8 * half + i, kb = 8 * half + 4 + i;
-        if (ka != 0) v[ka] = CONJ ? cmul_conj(v[ka], w0) : cmul(v[ka], w0);
-        v[kb] = CONJ ? cmul_conj(v[kb], w1) : cmul(v[kb], w1);
-      }
-    }
-#else
-    const int q = u >> 4;
-#pragma unroll
-    for (int k2 = 1; k2 < 16; k2++) v[k2] = CONJ ? cmul_conj(v[k2], T2[q * kT2Pad + k2]) : cmul(v[k2], T2[q * kT2Pad + k2]);
-#endif
-  }
 };
 
 __global__ void __launch_bounds__(4 * kTeam, 1) pbs_quad_kernel(PbsBatch P, DevTables tabs) {
@@ -1004,7 +564,6 @@ __global__ void __launch_bounds__(4 * kTeam, 1) pbs_quad_kernel(PbsBatch P, DevT
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
-#if SPF_QUAD_READER_T2
   {  // every thread's reader-side pass-2 constants over the table row pair_tmem_init left in [448, 512)
     const int tm = threadIdx.x / kTeam, uu = threadIdx.x % kTeam;
     double tw[6];
@@ -1024,7 +583,6 @@ __global__ void __launch_bounds__(4 * kTeam, 1) pbs_quad_kernel(PbsBatch P, DevT
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   }
-#endif
   const int team = threadIdx.x / kTeam;
   // team w = (h, t) with h = w & 1, t = w >> 1: the two teams that run the inverse transforms (t = 0) are warps
   // 0..3, one per SM sub-partition (warp % 4) -- with h = w >> 1 they were warps 0,1,4,5, i.e. the FP64-issue-bound
@@ -1051,47 +609,11 @@ __global__ void __launch_bounds__(4 * kTeam, 1) pbs_quad_kernel(PbsBatch P, DevT
 // ------------------------------------------------------------------------------------------
 // K5+K6: trace (+ CBS pre-processing) and scheme switch, one team per (ciphertext, level).
 // ------------------------------------------------------------------------------------------
-#ifndef SPF_TR_TEAMS
-#define SPF_TR_TEAMS 4
-#endif
-#ifndef SPF_TR_MIN_BLOCKS
-#define SPF_TR_MIN_BLOCKS 1
-#endif
-#ifndef SPF_TR_TMEM_TW
-#define SPF_TR_TMEM_TW 1  // trace / scheme-switch kernel: twiddles of both passes in tensor memory
-#endif
 // DevCx of the trace / scheme-switch kernel: tensor-memory columns [0,64) T1 | [64,128) T2 (per lane quarter, shared by the
 // two warps of the quarter: warps w and w + 4 have the same thread-in-team index) | 64 columns per warp of parked states
-#ifndef SPF_TR_TW_PIPE
-#define SPF_TR_TW_PIPE 0  // twiddle chunks software-pipelined (the tensor-memory load of chunk g + 1 overlaps the products of chunk g)
-#endif
 struct DevTrCx : DevCx {
-  static constexpr bool kTmemTwiddles = SPF_TR_TMEM_TW != 0;
+  static constexpr bool kTmemTwiddles = true;  // twiddles of both passes in tensor memory
   uint32_t tw_taddr;
-#if SPF_TR_TW_PIPE
-  template <bool CONJ, bool SKIP0>
-  __device__ __forceinline__ void tw_mul(C2 (&v)[16], uint32_t base) const {
-    uint32_t r[2][16];
-    tmem_ld16(r[0], base);
-    tmem_wait_ld();
-#pragma unroll
-    for (int g = 0; g < 4; g++) {
-      if (g < 3) tmem_ld16(r[(g + 1) & 1], base + 16 * (g + 1));
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const uint32_t* rr = r[g & 1];
-        const C2 w{__hiloint2double((int)rr[4 * i + 1], (int)rr[4 * i]), __hiloint2double((int)rr[4 * i + 3], (int)rr[4 * i + 2])};
-        const int k = 4 * g + i;
-        if (!SKIP0 || k) v[k] = CONJ ? cmul_conj(v[k], w) : cmul(v[k], w);
-      }
-      if (g < 3) tmem_wait_ld();
-    }
-  }
-  template <bool CONJ>
-  __device__ __forceinline__ void t1_mul(C2 (&v)[16]) const { tw_mul<CONJ, false>(v, tw_taddr); }
-  template <bool CONJ>
-  __device__ __forceinline__ void t2_mul(C2 (&v)[16]) const { tw_mul<CONJ, true>(v, tw_taddr + 64); }
-#else
   template <bool CONJ>
   __device__ __forceinline__ void t1_mul(C2 (&v)[16]) const {
 #pragma unroll
@@ -1122,10 +644,9 @@ struct DevTrCx : DevCx {
       }
     }
   }
-#endif
 };
-constexpr int kTrTmemCols = SPF_TR_TMEM_TW ? 256 : 128;
-constexpr int kTrTeams = SPF_TR_TEAMS;
+constexpr int kTrTmemCols = 256;  // [0,128) twiddles | [128,256) parked states, 64 columns per warp of a lane quarter
+constexpr int kTrTeams = 4;  // teams (ciphertext levels) per CTA: four fit the shared memory of one CTA per SM
 constexpr int kTrTeamBytes = 2 * kN * 8 + kXBuf * 16;                 // g + xbuf = 49408 (digits are stateless)
 constexpr int kTrSmem = kTableBytes + kTrTeams * kTrTeamBytes;        // 215104
 
@@ -1153,7 +674,7 @@ struct TraceSsBatch {
 };
 
 template <bool PEERS>
-__global__ void __launch_bounds__(kTrTeams * kTeam, SPF_TR_MIN_BLOCKS) trace_ss_kernel(const __grid_constant__ TraceSsBatch P, DevTables tabs) {
+__global__ void __launch_bounds__(kTrTeams * kTeam, 1) trace_ss_kernel(const __grid_constant__ TraceSsBatch P, DevTables tabs) {
   extern __shared__ __align__(16) unsigned char smem[];
   C2* sT1 = reinterpret_cast<C2*>(smem);
   C2* sT2 = sT1 + kT1Elems;
@@ -1171,7 +692,6 @@ __global__ void __launch_bounds__(kTrTeams * kTeam, SPF_TR_MIN_BLOCKS) trace_ss_
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_alloc = tmem_base;
   const uint32_t tw_taddr = tmem_alloc + ((uint32_t)((warp & 3) * 32) << 16);
-#if SPF_TR_TMEM_TW
   if (warp < 4) {  // twiddles of thread-in-team index uu = 32 (warp & 1) + lane, for both warps of this lane quarter
     const int uu = (warp & 1) * 32 + (threadIdx.x & 31);
 #pragma unroll
@@ -1188,7 +708,6 @@ __global__ void __launch_bounds__(kTrTeams * kTeam, SPF_TR_MIN_BLOCKS) trace_ss_
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#endif
   const int team = threadIdx.x / kTeam;
   const int item = blockIdx.x * (blockDim.x / kTeam) + team;
   if (item < P.batch * P.levels) {  // no early return: every thread must reach the deallocation barrier
@@ -1199,7 +718,7 @@ __global__ void __launch_bounds__(kTrTeams * kTeam, SPF_TR_MIN_BLOCKS) trace_ss_
     DevTrCx cx;
     cx.u = (int)(threadIdx.x % kTeam);
     cx.bar = team + 1;
-    cx.rp_taddr = tw_taddr + (SPF_TR_TMEM_TW ? 128u : 0u) + (uint32_t)(warp >> 2) * 64;
+    cx.rp_taddr = tw_taddr + 128u + (uint32_t)(warp >> 2) * 64;
     cx.tw_taddr = tw_taddr;
     TraceSsArgs A;
     const size_t glwe = 2 * kN;
@@ -1373,57 +892,10 @@ constexpr int kWideGlweBytes = 2 * kN * 8;
 constexpr int kWideSmem = kTableBytes + kWideTeams * kXBuf * 16 + 2 * kWideGlweBytes + 16;  // 216144
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity);
 
-#ifndef SPF_WIDE_STAGE_G
-#define SPF_WIDE_STAGE_G 0  // selector GGSW staged in tensor memory while the forward transforms run: bit-exact, the
-                            // multiply-accumulate phase drops from 5.6 k to 3.1 k clocks, but the transforms that now share the
-                            // SM's 45 B/clk L2 port with the 256 KiB transfer lose 3.3 k (profiles/r2_m_wide_phases.txt):
-                            // 19.78 vs 19.58 ms for the mul32 + compare program -- the port, not its placement, is the floor
-#endif
 struct DevWideCx {
   int u, team;
   __device__ __forceinline__ void sync() const { asm volatile("bar.sync %0, 64;" ::"r"(team + 1) : "memory"); }
   __device__ __forceinline__ void cta_sync() const { __syncthreads(); }
-  // ---- GGSW staging (team_ops.cuh::cmux_wide, g_stage) ----
-  // Tensor memory is exactly one GGSW: 512 columns x 128 lanes x 4 B = 256 KiB.  Thread (p, k1, k2) of the multiply-accumulate
-  // phase owns the bins k1 + 16 k2 + 256 k3 of output p over the 8 spectra j: 32 complex values = 128 columns of its lane;
-  // the four warps of a lane quarter take the four 128-column blocks.  Batch j = the four values of spectrum j (k3 = 0..3).
-  static constexpr bool kStageG = SPF_WIDE_STAGE_G != 0;
-  const C2* gbase = nullptr;  // ggsw + p * kM + k1 + 16 k2 of this thread
-  uint32_t g_taddr = 0;       // this warp's lane quarter and 128-column block
-  int count = 4;
-  C2 stg[4];
-  template <int I>
-  __device__ __forceinline__ void g_stage() {
-    if constexpr (kStageG) {
-      if constexpr (I > 0) {
-        uint32_t r[16];
-#pragma unroll
-        for (int k3 = 0; k3 < 4; k3++) {
-          r[4 * k3] = (uint32_t)__double2loint(stg[k3].x); r[4 * k3 + 1] = (uint32_t)__double2hiint(stg[k3].x);
-          r[4 * k3 + 2] = (uint32_t)__double2loint(stg[k3].y); r[4 * k3 + 3] = (uint32_t)__double2hiint(stg[k3].y);
-        }
-        tmem_st16(g_taddr + 16 * (I - 1), r);
-        if constexpr (I == 8) tmem_wait_st();
-      }
-      if constexpr (I < 8) {
-        const int rr = I / 4, tt = I % 4;  // spectrum j = I: digit tt of polynomial rr <-> GGSW level count - 1 - tt (count == 4)
-        const C2* grow = gbase + (size_t)(rr * 4 + (3 - tt)) * 2 * kM;
-#pragma unroll
-        for (int k3 = 0; k3 < 4; k3++) stg[k3] = ldg_c2_pinned(grow + 256 * k3);
-      }
-    }
-  }
-  __device__ __forceinline__ void g_read16(C2 (&g)[4][4], int jb) const {
-    uint32_t r[4][16];
-#pragma unroll
-    for (int jj = 0; jj < 4; jj++) tmem_ld16(r[jj], g_taddr + 16 * (jb + jj));
-    tmem_wait_ld();
-#pragma unroll
-    for (int jj = 0; jj < 4; jj++)
-#pragma unroll
-      for (int k3 = 0; k3 < 4; k3++)
-        g[jj][k3] = C2{__hiloint2double((int)r[jj][4 * k3 + 1], (int)r[jj][4 * k3]), __hiloint2double((int)r[jj][4 * k3 + 3], (int)r[jj][4 * k3 + 2])};
-  }
 };
 
 __global__ void __launch_bounds__(kWideTeams * kTeam, 1) cmux_wide_kernel(CmuxBatch P, DevTables tabs) {
@@ -1446,20 +918,6 @@ __global__ void __launch_bounds__(kWideTeams * kTeam, 1) cmux_wide_kernel(CmuxBa
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   load_tables(sT1, sT2, tabs);  // ends with a CTA barrier: the mbarrier is initialised for everyone
-#if SPF_WIDE_STAGE_G
-  uint32_t tmem_alloc;
-  {
-    __shared__ uint32_t tmem_base;
-    if ((threadIdx.x >> 5) == 0) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(&tmem_base)), "n"(kPbsTmemCols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    tmem_alloc = tmem_base;
-  }
-#endif
   const size_t glwe = 2 * kN;
   const int item = c / P.glwe_per_item;
   const size_t off = P.ptrs ? (size_t)(c % P.glwe_per_item) * glwe : (size_t)c * glwe;
@@ -1477,131 +935,9 @@ __global__ void __launch_bounds__(kWideTeams * kTeam, 1) cmux_wide_kernel(CmuxBa
                    ::"r"(smem_u32(sd0)), "l"(d0 + off), "r"((uint32_t)kWideGlweBytes), "r"(smem_u32(mbar)) : "memory");
   }
   DevWideCx cx{(int)(threadIdx.x % kTeam), (int)(threadIdx.x / kTeam)};
-#if SPF_WIDE_STAGE_G
-  {
-    const int tid = threadIdx.x, warp = tid >> 5;
-    cx.gbase = ggsw + (size_t)(tid >> 8) * kM + (tid & 255);  // p * kM + k1 + 16 k2
-    cx.g_taddr = tmem_alloc + ((uint32_t)((warp & 3) * 32) << 16) + 128 * (warp >> 2);
-    cx.count = P.count;
-  }
-#endif
   mbar_wait(smem_u32(mbar), 0);
   cmux_wide(cx, P.out_ptrs ? static_cast<uint64_t*>(P.out_ptrs[c]) : P.out + (size_t)c * glwe, d0 ? sd0 : nullptr, sd1, ggsw, xb, sT1, sT2,
             P.radix_log, P.count);
-#if SPF_WIDE_STAGE_G
-  pair_tmem_free(tmem_alloc);
-#endif
-}
-
-// ------------------------------------------------------------------------------------------
-// K2c `cmux_chain_kernel`: a RUN of consecutive MUX-tree levels in ONE cooperative launch.
-// A MUX tree is a chain of narrow levels (the 32-bit multiplier: 621 levels, mean width 73): launched one kernel per
-// level, every level pays the dependent-launch gap (~4 us even with programmatic launch) on top of the 9.7 us the wide
-// CMUX kernel works.  Here the CTAs stay resident, walk the levels of the run from a device-side list (the graph
-// executor's own per-group pointer tables) and separate two levels by a grid-wide barrier -- a release / acquire counter
-// in global memory -- instead of a kernel boundary; twiddle tables and the mbarrier are set up once.  The per-item body is
-// cmux_wide, unchanged (bit-identical results).  Cooperative launch guarantees that all CTAs are co-resident (other
-// graphs of the asynchronous executor may be in flight on other streams), so the spin barrier cannot deadlock.
-// MEASURED (profiles/r2_r_chain_ab.txt): 637 -> 19 launches for the mul32 + compare program, and 19.96 instead of
-// 19.44 ms -- the release / acquire round trips through L2 cost ~4.2 us per level where a programmatic dependent launch,
-// whose successor has its tables loaded and its selector on the way before the predecessor ends, costs ~3.3 us.  Kept
-// as an opt-in (SPF_B200_CHAIN=1): the executor stays on one launch per level.
-// ------------------------------------------------------------------------------------------
-struct ChainStage {
-  const void* const* ptrs;  // {selector GGSW, d0 (may be null), d1} per item
-  void* const* out_ptrs;    // output GLWE per item
-  int n;                    // items of this stage
-  int barrier_after;        // the next stage belongs to a later level
-};
-struct ChainBatch {
-  const ChainStage* stages;
-  int n_stages;
-  unsigned long long* bar;  // zeroed before the launch
-  int radix_log, count;
-};
-struct DevChainCx {
-  static constexpr bool kStageG = false;
-  int u, team;
-  __device__ __forceinline__ void sync() const { asm volatile("bar.sync %0, 64;" ::"r"(team + 1) : "memory"); }
-  __device__ __forceinline__ void cta_sync() const { __syncthreads(); }
-  template <int I> __device__ __forceinline__ void g_stage() const {}
-  __device__ __forceinline__ void g_read16(C2 (&)[4][4], int) const {}
-};
-__global__ void __launch_bounds__(kWideTeams * kTeam, 1) cmux_chain_kernel(ChainBatch P, DevTables tabs) {
-  extern __shared__ __align__(16) unsigned char smem[];
-  C2* sT1 = reinterpret_cast<C2*>(smem);
-  C2* sT2 = sT1 + kT1Elems;
-  C2* xb = reinterpret_cast<C2*>(smem + kTableBytes);
-  uint64_t* sd1 = reinterpret_cast<uint64_t*>(smem + kTableBytes + kWideTeams * kXBuf * 16);
-  uint64_t* sd0 = sd1 + 2 * kN;
-  uint64_t* mbar = sd0 + 2 * kN;
-  if (threadIdx.x == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mbar)) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  load_tables(sT1, sT2, tabs);  // ends with a CTA barrier
-  DevChainCx cx{(int)(threadIdx.x % kTeam), (int)(threadIdx.x / kTeam)};
-  unsigned long long target = 0;
-  uint32_t phase = 0;
-  // the stage list and the pointer tables are written before the launch: the next stage's descriptor and this CTA's first
-  // item of it are fetched BEFORE the grid barrier, so the two dependent global round trips are off the path between levels
-  ChainStage S = P.n_stages > 0 ? P.stages[0] : ChainStage{nullptr, nullptr, 0, 0};
-  const void* nx[4] = {nullptr, nullptr, nullptr, nullptr};
-  auto fetch_first = [&](const ChainStage& T) {
-    if ((int)blockIdx.x < T.n) {
-      nx[0] = T.ptrs[3 * blockIdx.x]; nx[1] = T.ptrs[3 * blockIdx.x + 1]; nx[2] = T.ptrs[3 * blockIdx.x + 2]; nx[3] = T.out_ptrs[blockIdx.x];
-    }
-  };
-  fetch_first(S);
-  for (int st = 0; st < P.n_stages; st++) {
-    ChainStage Snext = st + 1 < P.n_stages ? P.stages[st + 1] : ChainStage{nullptr, nullptr, 0, 0};
-    for (int c = blockIdx.x; c < S.n; c += gridDim.x) {
-      const bool firsti = c == (int)blockIdx.x;
-      const C2* ggsw = static_cast<const C2*>(firsti ? nx[0] : S.ptrs[3 * c]);
-      const uint64_t* d0 = static_cast<const uint64_t*>(firsti ? nx[1] : S.ptrs[3 * c + 1]);
-      const uint64_t* d1 = static_cast<const uint64_t*>(firsti ? nx[2] : S.ptrs[3 * c + 2]);
-      uint64_t* outp = static_cast<uint64_t*>(firsti ? const_cast<void*>(nx[3]) : S.out_ptrs[c]);
-      if (threadIdx.x == 0) {
-        // the inputs may have been written by other CTAs of this launch (generic proxy, before the grid barrier): order
-        // this thread's acquire of the barrier before the bulk copies' reads (async proxy)
-        asm volatile("fence.proxy.async;" ::: "memory");
-        const uint32_t bytes = d0 ? 2 * kWideGlweBytes : kWideGlweBytes;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(mbar)), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(smem_u32(sd1)), "l"(d1), "r"((uint32_t)kWideGlweBytes), "r"(smem_u32(mbar)) : "memory");
-        if (d0)
-          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                       ::"r"(smem_u32(sd0)), "l"(d0), "r"((uint32_t)kWideGlweBytes), "r"(smem_u32(mbar)) : "memory");
-      }
-      mbar_wait_trap(smem_u32(mbar), phase);
-      phase ^= 1u;
-      cmux_wide(cx, outp, d0 ? sd0 : nullptr, sd1, ggsw, xb, sT1, sT2, P.radix_log, P.count);
-      __syncthreads();  // the staged inputs and the exchange buffers are free for the next item
-    }
-    fetch_first(Snext);
-    if (S.barrier_after) {
-      __syncthreads();  // every thread's output stores precede thread 0's release
-      if (threadIdx.x == 0) {
-        target += gridDim.x;
-        __threadfence();
-        atomicAdd(P.bar, 1ull);
-        unsigned long long seen;
-        unsigned long long t_start = 0;
-        for (int spin = 0;; spin++) {
-          asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(seen) : "l"(P.bar) : "memory");
-          if (seen >= target) break;
-          if ((spin & 4095) == 4095) {  // a CTA that never arrives: trap instead of hanging the GPU
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            if (t_start == 0) t_start = now;
-            else if (now - t_start > 2000000000ull) __trap();
-          }
-        }
-      }
-      __syncthreads();
-    }
-    S = Snext;
-  }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1739,58 +1075,16 @@ __global__ void __launch_bounds__(kKsThreads) keyswitch_kernel(KsBatch P) {
 }
 
 // ------------------------------------------------------------------------------------------
-// K4t: the keyswitch as a dense integer contraction on the tensor cores.
+// K4u: the keyswitch as a dense integer contraction on the 5th-generation tensor cores (tcgen05.mma kind::i8,
+// TMEM accumulators).
 //   out[b][c] = (0, body_b) - sum_{k=(i,t)} d[b][k] * KSK[k][c]   is   [B x 12288] x [12288 x 638] mod 2^64.
 // With unsigned digits u = d + B/2 in {0..B-1} (see K4) and the KSK split into its 8 BYTE PLANES,
 //   sum_k u[b][k] * KSK[k][c] = sum_j 2^(8j) * (U x P_j)[b][c],   P_j[k][c] = byte j of KSK[k][c],
 // every U x P_j is an exact u8 x u8 -> s32 GEMM (12288 * 3 * 255 < 2^24), i.e. 8 int8 tensor-core
 // GEMMs whose results are recombined with shifts in the epilogue; the surplus (B/2) * sum_k KSK[k][c]
-// is the same per-key constant as in K4.  mma.sync.m16n8k32.u8.u8.s32 (IMMA.16832: measured 572 T
-// MAC/s on this part); the KSK planes are stored fragment-major (ks_tc_prepare_kernel) so a warp
-// streams 2 KiB of B fragments per k-step with four 16-byte loads per lane.
-// CTA tile: 128 ciphertexts x 32 columns, 8 warps = 2 (rows) x 4 (n-tiles), warp tile 64 x 8 x 8 planes
-// (128 s32 accumulators per thread).  K is walked in chunks of (512 mask elements, one digit level);
-// the chunk's rounded states sit in shared memory as u16 and the u8 A fragments are cut out of them
-// with two shifts, two masks and one byte permute per register.  grid.z splits K; partial results
-// are combined with u64 atomics (wrapping adds commute: bit-exact).
+// is the same per-key constant as in K4.  K is walked in chunks of (kKtIC mask elements, one digit level).
 // ------------------------------------------------------------------------------------------
-constexpr int kKtM = 128, kKtN = 32, kKtIC = 512;
-constexpr int kKtRow = kKtIC + 8;                          // u16 per smem row (+16 B: conflict-free LDS.64)
-constexpr int kKtSmem = kKtM * kKtRow * 2;                 // 133120
-
-struct KsTcBatch {
-  uint64_t* out;            // [B][n0+1], zero-initialised when gridDim.z > 1
-  const uint64_t* in;       // [B][n1+1]
-  const void* const* ptrs;  // optional: ptrs[b] = L1 LWE input of item b
-  const uint16_t* st16;     // [B][n1] rounded + offset states (ks_tc_states_kernel)
-  const uint4* bfrag;       // [n_tiles][k_steps][32 lanes][4] : per lane 8 planes x (b0, b1)
-  const uint64_t* colsum;   // [chunks][n0+1]: sum over the chunk's (i, t) of ksk, chunk = c * L + t
-  int batch, n1, n0, radix_log, count;
-  int chunks_per_cta;       // (i-chunk, level) pairs per grid.z slice
-};
-
-// bfrag[(nt * KS + ks) * 32 + lane] = {plane 0: b0, b1, plane 1: b0, b1}, ... 4 x uint4 per lane; k-step ks covers
-// k = ks * 32 .. +31 with k = t * n1 + i (digit t <-> KSK level L-1-t); b0 holds rows k = 4 (lane % 4) .. +3
-// of column nt * 8 + lane / 4, b1 the rows 16 further (PTX ISA, m16n8k32 B fragment).
-__global__ void ks_tc_prepare_kernel(uint4* bfrag, const uint64_t* ksk, int n1, int levels, int cols, int n_tiles) {
-  const int ks_total = n1 * levels / 32;
-  const size_t lane_slot = blockIdx.x * (size_t)blockDim.x + threadIdx.x;  // (nt, ks, lane)
-  if (lane_slot >= (size_t)n_tiles * ks_total * 32) return;
-  const int lane = (int)(lane_slot & 31), ks = (int)((lane_slot >> 5) % ks_total), nt = (int)((lane_slot >> 5) / ks_total);
-  const int col = nt * 8 + (lane >> 2);
-  uint32_t w[16];
-#pragma unroll
-  for (int x = 0; x < 16; x++) w[x] = 0;
-  if (col < cols) {
-    for (int r = 0; r < 2; r++)
-      for (int e = 0; e < 4; e++) {
-        const int k = ks * 32 + 4 * (lane & 3) + 16 * r + e, t = k / n1, i = k % n1;
-        const uint64_t v = ksk[((size_t)i * levels + (levels - 1 - t)) * cols + col];
-        for (int j = 0; j < 8; j++) w[2 * j + r] |= (uint32_t)((v >> (8 * j)) & 0xFF) << (8 * e);
-      }
-  }
-  for (int x = 0; x < 4; x++) bfrag[lane_slot * 4 + x] = make_uint4(w[4 * x], w[4 * x + 1], w[4 * x + 2], w[4 * x + 3]);
-}
+constexpr int kKtIC = 512;
 
 // colsum[c * levels + t][col] = sum_{i in chunk c} ksk[i][levels-1-t][col]
 __global__ void ks_tc_colsum_kernel(uint64_t* colsum, const uint64_t* ksk, int n1, int levels, int cols) {
@@ -1802,7 +1096,7 @@ __global__ void ks_tc_colsum_kernel(uint64_t* colsum, const uint64_t* ksk, int n
   colsum[(size_t)chunk * cols + col] = acc;
 }
 
-// st16[b][i] = round(a_i of input b) + radix_offset: the digit source of K4t, computed once per
+// st16[b][i] = round(a_i of input b) + radix_offset: the digit source of K4u, computed once per
 // launch instead of once per column block
 __global__ void ks_tc_states_kernel(uint16_t* st16, const uint64_t* in, const void* const* ptrs, int batch, int n1,
                                     int radix_log, int count) {
@@ -1816,110 +1110,6 @@ __global__ void ks_tc_states_kernel(uint16_t* st16, const uint64_t* in, const vo
   }
 }
 
-__device__ __forceinline__ void imma_16832_u8(int (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-__global__ void __launch_bounds__(256, 1) keyswitch_tc_kernel(KsTcBatch P) {
-  extern __shared__ __align__(16) unsigned char smem[];
-  uint16_t* st = reinterpret_cast<uint16_t*>(smem);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, q4 = lane & 3;
-  const int wm = warp >> 2, wn = warp & 3;
-  const int b0 = blockIdx.x * kKtM;
-  const int nt = blockIdx.y * (kKtN / 8) + wn;
-  const int L = P.count, chunks_per_t = P.n1 / kKtIC, total_chunks = chunks_per_t * L;
-  const int ks_per_t = P.n1 / 32, ks_total = ks_per_t * L;
-  const int kc_begin = blockIdx.z * P.chunks_per_cta, kc_end = min(kc_begin + P.chunks_per_cta, total_chunks);
-  const uint32_t off = (uint32_t)radix_offset(P.radix_log, L);
-  const uint32_t dmask = ((1u << P.radix_log) - 1) * 0x00010001u;
-  int acc[4][8][4];
-#pragma unroll
-  for (int mt = 0; mt < 4; mt++)
-#pragma unroll
-    for (int j = 0; j < 8; j++)
-#pragma unroll
-      for (int x = 0; x < 4; x++) acc[mt][j][x] = 0;
-  int staged_c = -1;
-  for (int kc = kc_begin; kc < kc_end; kc++) {
-    const int c = kc / L, t = kc % L;  // chunk order: mask-element chunk outer, digit level inner
-    if (c != staged_c) {
-      __syncthreads();  // previous chunk's fragments have been read
-      // 128 rows x 1 KiB: 16 bytes per thread and step, rows beyond the batch get all digits = B/2
-      for (int idx = threadIdx.x; idx < kKtM * (kKtIC / 8); idx += blockDim.x) {
-        const int b = idx / (kKtIC / 8), i8 = idx % (kKtIC / 8);
-        uint4 v = make_uint4(off * 0x00010001u, off * 0x00010001u, off * 0x00010001u, off * 0x00010001u);
-        if (b0 + b < P.batch) v = __ldg(reinterpret_cast<const uint4*>(P.st16 + (size_t)(b0 + b) * P.n1 + c * kKtIC) + i8);
-        *reinterpret_cast<uint4*>(st + b * kKtRow + 8 * i8) = v;
-      }
-      __syncthreads();
-      staged_c = c;
-    }
-    const int shift = P.radix_log * t;
-    const uint4* bp = P.bfrag + ((size_t)nt * ks_total + (size_t)t * ks_per_t + (size_t)c * (kKtIC / 32)) * 32 * 4 + lane * 4;
-    uint4 bq[4];
-#pragma unroll
-    for (int x = 0; x < 4; x++) bq[x] = __ldg(bp + x);
-#pragma unroll 1
-    for (int ks = 0; ks < kKtIC / 32; ks++) {
-      uint4 bn[4];
-      if (ks + 1 < kKtIC / 32) {
-#pragma unroll
-        for (int x = 0; x < 4; x++) bn[x] = __ldg(bp + (size_t)(ks + 1) * 32 * 4 + x);
-      }
-      const uint32_t bw[16] = {bq[0].x, bq[0].y, bq[0].z, bq[0].w, bq[1].x, bq[1].y, bq[1].z, bq[1].w,
-                               bq[2].x, bq[2].y, bq[2].z, bq[2].w, bq[3].x, bq[3].y, bq[3].z, bq[3].w};
-#pragma unroll
-      for (int mt = 0; mt < 4; mt++) {
-        // A fragment: a0 (row g, k 4 q4..+3), a1 (row g+8), a2 (row g, k + 16), a3 (row g+8, k + 16)
-        uint32_t a[4];
-#pragma unroll
-        for (int x = 0; x < 4; x++) {
-          const int row = wm * 64 + mt * 16 + g + 8 * (x & 1);
-          const uint2 w = *reinterpret_cast<const uint2*>(st + row * kKtRow + ks * 32 + 4 * q4 + 16 * (x >> 1));
-          a[x] = __byte_perm((w.x >> shift) & dmask, (w.y >> shift) & dmask, 0x6420);
-        }
-#pragma unroll
-        for (int j = 0; j < 8; j++) imma_16832_u8(acc[mt][j], a, bw[2 * j], bw[2 * j + 1]);
-      }
-      if (ks + 1 < kKtIC / 32) {
-#pragma unroll
-        for (int x = 0; x < 4; x++) bq[x] = bn[x];
-      }
-    }
-  }
-  // ---- epilogue: recombine the byte planes, remove the digit offset, subtract from (0, body) ----
-  const int cols = P.n0 + 1;
-  const bool split = gridDim.z > 1;
-#pragma unroll
-  for (int x = 0; x < 4; x++) {  // c0: (row g, col 2 q4), c1: (g, 2 q4 + 1), c2: (g + 8, 2 q4), c3: (g + 8, 2 q4 + 1)
-    const int col = nt * 8 + 2 * q4 + (x & 1);
-    if (col >= cols) continue;
-    uint64_t surplus = 0;
-    for (int kc = kc_begin; kc < kc_end; kc++) surplus += P.colsum[(size_t)kc * cols + col];
-    surplus <<= P.radix_log - 1;
-#pragma unroll
-    for (int mt = 0; mt < 4; mt++) {
-      const int b = b0 + wm * 64 + mt * 16 + g + 8 * (x >> 1);
-      if (b >= P.batch) continue;
-      uint64_t sum = 0;
-#pragma unroll
-      for (int j = 0; j < 8; j++) sum += (uint64_t)(uint32_t)acc[mt][j][x] << (8 * j);
-      uint64_t body = 0;
-      if (col == P.n0 && blockIdx.z == 0)
-        body = (P.ptrs ? static_cast<const uint64_t*>(P.ptrs[b]) : P.in + (size_t)b * (P.n1 + 1))[P.n1];
-      const uint64_t v = body - (sum - surplus);
-      uint64_t* o = P.out + (size_t)b * cols + col;
-      if (split) atomicAdd(reinterpret_cast<unsigned long long*>(o), (unsigned long long)v);
-      else *o = v;
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------
-// K4u: the keyswitch contraction on the 5th-generation tensor cores (tcgen05.mma kind::i8, TMEM
-// accumulators), same mathematics as K4t: eight exact u8 x u8 -> s32 byte-plane GEMMs.
 // CTA tile 128 ciphertexts x 64 columns x 8 planes = 8 accumulators of 64 TMEM columns (all 512).
 // Per k-step (32 digits): the 16 KiB of B (8 planes x 64 columns x 32 bytes, stored by
 // ks_umma_prepare_kernel in the canonical K-major core-matrix layout) arrive by ONE bulk copy
@@ -1928,7 +1118,6 @@ __global__ void __launch_bounds__(256, 1) keyswitch_tc_kernel(KsTcBatch P) {
 // "empty" barrier.  6-stage ring; warps 0-3 produce A and run the epilogue (TMEM lane = row),
 // warp 4 feeds B, warp 5 issues the MMAs.  Epilogue: recombine the planes with shifts, remove the
 // digit offset (per-key column sums), subtract from (0, body); grid.z splits K (u64 atomics).
-// ------------------------------------------------------------------------------------------
 constexpr int kKuM = 128, kKuN = 64, kKuStages = 6;
 constexpr int kKuATile = kKuM * 32, kKuBPlane = kKuN * 32, kKuBTile = 8 * kKuBPlane;   // 4096, 2048, 16384
 constexpr int kKuSmem = kKuStages * (kKuATile + kKuBTile) + 1024;                      // + barriers, surplus table
@@ -1939,7 +1128,7 @@ struct KsUBatch {
   const void* const* ptrs;
   const uint16_t* st16;     // [B][n1] rounded + offset states
   const uint8_t* btiles;    // [n_blocks][k_steps][8 planes][2 kc][8 col-groups][8 cols][16 B]
-  const uint64_t* colsum;   // [chunks][n0+1], chunk = c * L + t  (as K4t)
+  const uint64_t* colsum;   // [chunks][n0+1], chunk = c * L + t  (ks_tc_colsum_kernel)
   int batch, n1, n0, radix_log, count;
   int chunks_per_cta;
 };

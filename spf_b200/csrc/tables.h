@@ -25,20 +25,6 @@ inline void fill_twiddle_tables(C2* T1, C2* T2) {
     }
 }
 
-// The constants of the deferred-scale transforms in the order the device code asks for them (fft16.cuh: KDev / KRec); returns
-// false if a pool overflows.
-inline bool fill_kpools(double (*pool)[kPoolLen]) {
-  C2 v[16];
-  double s[16];
-  for (int i = 0; i < 16; i++) v[i] = C2{1.0 + i, 0.5 - i};
-  KRec r0{pool[0], 0}, r1{pool[1], 0}, r2{pool[2], 0}, r3{pool[3], 0};
-  fwd_pass1_core_k(v, r0);
-  inv_pass1_core_s_k(v, s, r1);
-  dft16_k<false>(v, r2);
-  dft16_k<true>(v, r3);
-  return r0.i <= kPoolLen && r1.i <= kPoolLen && r2.i <= kPoolLen && r3.i <= kPoolLen;
-}
-
 // inverse of k_r = N / 2^r + 1 modulo 2N, r = 0..10 (ops/automorphisms/mod.rs:72-73)
 inline void fill_kinv(uint32_t* kinv) {
   for (int r = 0; r < 11; r++) {

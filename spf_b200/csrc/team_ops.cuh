@@ -28,19 +28,6 @@ SPF_HD C2 ldg_c2(const C2* p) {
   return *p;
 #endif
 }
-// Same load as ldg_c2 but ordered: a volatile asm with a memory clobber and a plain (not .nc)
-// ld.global, which neither nvcc nor ptxas moves across a bar.sync.  __ldg loads of the BSK get sunk
-// (together with the arithmetic that consumes them) below the next two barriers, which delays
-// their issue and costs ~20 % per CMUX step (measured 10.98 vs 9.1 ms per 444-ciphertext wave).
-SPF_HD C2 ldg_c2_pinned(const C2* p) {
-#if defined(__CUDA_ARCH__)
-  C2 r;
-  asm volatile("ld.global.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p) : "memory");
-  return r;
-#else
-  return *p;
-#endif
-}
 SPF_HD C2 cscale(C2 a, double f) { return C2{a.x * f, a.y * f}; }
 SPF_HD uint64_t ldg_u64(const uint64_t* p) {
 #if defined(__CUDA_ARCH__)
@@ -312,19 +299,13 @@ SPF_HD double digit16_to_f64(uint32_t d) {
   return x - 4503599627403264.0;  // 2^52 + 2^15
 }
 
-// Signed 16-bit digit sitting in the LOW half of d (upper half ignored) -> f64 with one IMAD and one
-// DADD: the low word (d << 16) + 2^31 of a double with exponent 2^36 (ulp 2^-16) reads as
-// 2^36 + 2^15 + sext16(d).
-// SPF_DIGIT_I2F (device): one conversion instruction (I2F.F64.S16 on the conversion pipe, which selects the half word itself)
-// instead of an integer op, a move for the exponent word and a DADD on the FP64 pipe; the values are identical.
-#ifndef SPF_GATHER_SEL
-#define SPF_GATHER_SEL 0  // pbs_pair_team: rotated gather with two base pointers / sign masks chosen by one comparison per coefficient
-#endif
-#ifndef SPF_DIGIT_I2F
-#define SPF_DIGIT_I2F 1  // measured: 6.96 -> 6.73 ms per 444-ciphertext wave of pbs_kernel (profiles/r2_zz_i2f_ab.txt)
-#endif
+// Signed 16-bit digit sitting in the LOW half of d (upper half ignored) -> f64.  Host: one IMAD and one DADD: the low
+// word (d << 16) + 2^31 of a double with exponent 2^36 (ulp 2^-16) reads as 2^36 + 2^15 + sext16(d).  Device: one
+// conversion instruction (I2F.F64.S16 on the conversion pipe, which selects the half word itself) instead of an integer
+// op, a move for the exponent word and a DADD on the FP64 pipe; the values are identical (measured: 6.96 -> 6.73 ms per
+// 444-ciphertext wave of pbs_kernel, profiles/r2_zz_i2f_ab.txt).
 SPF_HD double digit_lo16_to_f64(uint32_t d) {
-#if defined(__CUDA_ARCH__) && SPF_DIGIT_I2F
+#if defined(__CUDA_ARCH__)
   double r;
   asm("{\n\t.reg .b16 lo, hi;\n\tmov.b32 {lo, hi}, %1;\n\tcvt.rn.f64.s16 %0, lo;\n\t}" : "=d"(r) : "r"(d));
   return r;
@@ -332,9 +313,9 @@ SPF_HD double digit_lo16_to_f64(uint32_t d) {
   return bits_f64(0x4230000000000000ull | (uint64_t)(uint32_t)(d * 65536u + 0x80000000u)) - 68719509504.0;  // 2^36 + 2^15
 #endif
 }
-// the same for a digit sitting in the HIGH half of d (lower half ignored): one LOP3 and one DADD
+// the same for a digit sitting in the HIGH half of d (lower half ignored); host: one LOP3 and one DADD
 SPF_HD double digit_hi16_to_f64(uint32_t d) {
-#if defined(__CUDA_ARCH__) && SPF_DIGIT_I2F
+#if defined(__CUDA_ARCH__)
   double r;
   asm("{\n\t.reg .b16 lo, hi;\n\tmov.b32 {lo, hi}, %1;\n\tcvt.rn.f64.s16 %0, hi;\n\t}" : "=d"(r) : "r"(d));
   return r;
@@ -362,36 +343,9 @@ SPF_HD double digit_hi16_to_f64(uint32_t d) {
 // Register slot s' = 4 jj + k3 of thread u in half h holds bin u + 64 * (2h + jj + 4 k3).
 SPF_HD constexpr int split_bin(int u, int h, int s) { return u + 64 * (2 * h + (s >> 2) + 4 * (s & 3)); }
 
-// final forward radix-4 pass on this half's bins of digit polynomial b (spectrum-in-progress in
-// xb[b]), then f[p] (+)= D * G[b][level][p] for both output polynomials p.  Written as two
-// independent 4-bin batches: the compiler hoists the second batch's BSK loads above the first
-// batch's arithmetic (measured: explicit earlier prefetching only costs registers and spills).
-template <bool INIT, class Cx>
-SPF_HD void mad_split(Cx& cx, C2 (&f)[2][8], const C2* xbb, const C2* g /* GGSW row b, level: [p][bin] */, int u, int h) {
-  const int k1 = u & 15, q = u >> 4;
-#pragma unroll
-  for (int jj = 0; jj < 2; jj++) {
-    C2 d[4], g0[4], g1[4];
-#pragma unroll
-    for (int qp = 0; qp < 4; qp++) d[qp] = SPF_ABLATE(4) ? C2{1.0 + qp, 2.0 + jj} : xbb[k1 * kXPad + qp + 4 * q + 16 * (2 * h + jj)];
-#pragma unroll
-    for (int k3 = 0; k3 < 4; k3++) {
-      g0[k3] = cx.bsk_load(g + split_bin(u, h, 4 * jj + k3));
-      g1[k3] = cx.bsk_load(g + kM + split_bin(u, h, 4 * jj + k3));
-    }
-    bfly4<false>(d[0], d[1], d[2], d[3]);
-#pragma unroll
-    for (int k3 = 0; k3 < 4; k3++) {
-      const int s = 4 * jj + k3;
-      if (INIT) { f[0][s] = cmul(d[k3], g0[k3]); f[1][s] = cmul(d[k3], g1[k3]); }
-      else { cmad(f[0][s], d[k3], g0[k3]); cmad(f[1][s], d[k3], g1[k3]); }
-    }
-  }
-}
-
-// ---- reader-side pass-2 twiddles (Cx::kReaderT2) --------------------------------------------------------------------
+// ---- reader-side pass-2 twiddles -----------------------------------------------------------------------------------
 // The pass-2 -> pass-3 twiddle W64^(q' k2) of a forward transform does not have to be applied by the thread that produced
-// z[k2] (15 complex multiplies per transform): the thread that CONSUMES the value in mad_split knows q' (its loop index)
+// z[k2] (15 complex multiplies per transform): the thread that CONSUMES the value in mad_split_rt knows q' (its loop index)
 // and k2 = q + 4 (2 h + jj) (its own bins), needs only 3 twiddles per radix-4 group -- the same 6 for all four spectra of a
 // step -- and can apply them in the tan form  w = c (1 + i t):  two FMAs per value, the factored-out c riding into the
 // butterfly as scale ratios (bfly4_r; the same instruction count as the plain butterfly).  4 x 2 x 3 x 2 = 48 FP64
@@ -433,15 +387,19 @@ SPF_HD void rt2_group_consts(const C2* T2, int q, int grp, double (&tw)[6], C2 (
   tw[4] = c[2];
   tw[5] = c[3] / c[1];
 }
-// mad_split for spectra whose pass-2 twiddles have NOT been applied yet (tw from rt2_fwd_consts)
+// final forward radix-4 pass on this half's bins of digit polynomial b (spectrum-in-progress in xbb, its pass-2 twiddles NOT
+// applied yet: tw from rt2_fwd_consts), then f[p] (+)= D * G[b][level][p] for both output polynomials p.  Written as two
+// independent 4-bin batches: the compiler hoists the second batch's BSK loads above the first batch's arithmetic
+// (measured: explicit earlier prefetching only costs registers and spills).
 template <bool INIT, class Cx>
-SPF_HD void mad_split_rt(Cx& cx, C2 (&f)[2][8], const C2* xbb, const C2* g, int u, int h, const double (&tw)[12]) {
+SPF_HD void mad_split_rt(Cx& cx, C2 (&f)[2][8], const C2* xbb, const C2* g /* GGSW row b, level: [p][bin] */, int u, int h,
+                         const double (&tw)[12]) {
   const int k1 = u & 15, q = u >> 4;
 #pragma unroll
   for (int jj = 0; jj < 2; jj++) {
     C2 d[4], g0[4], g1[4];
 #pragma unroll
-    for (int qp = 0; qp < 4; qp++) d[qp] = SPF_ABLATE(4) ? C2{1.0 + qp, 2.0 + jj} : xbb[k1 * kXPad + qp + 4 * q + 16 * (2 * h + jj)];
+    for (int qp = 0; qp < 4; qp++) d[qp] = xbb[k1 * kXPad + qp + 4 * q + 16 * (2 * h + jj)];
 #pragma unroll
     for (int k3 = 0; k3 < 4; k3++) {
       g0[k3] = cx.bsk_load(g + split_bin(u, h, 4 * jj + k3));
@@ -450,8 +408,7 @@ SPF_HD void mad_split_rt(Cx& cx, C2 (&f)[2][8], const C2* xbb, const C2* g, int 
 #pragma unroll
     for (int qp = 1; qp < 4; qp++) {
       const double t = tw[6 * jj + qp - 1];
-      if (SPF_ABLATE(2)) d[qp] = abl_mix(d[qp], C2{t, t});
-      else d[qp] = C2{spf_fma(-t, d[qp].y, d[qp].x), spf_fma(t, d[qp].x, d[qp].y)};  // d (1 + i t); the factor c rides in the ratios
+      d[qp] = C2{spf_fma(-t, d[qp].y, d[qp].x), spf_fma(t, d[qp].x, d[qp].y)};  // d (1 + i t); the factor c rides in the ratios
     }
     bfly4_r<false>(d[0], d[1], d[2], d[3], tw[6 * jj + 3], tw[6 * jj + 4], tw[6 * jj + 5]);
 #pragma unroll
@@ -463,33 +420,25 @@ SPF_HD void mad_split_rt(Cx& cx, C2 (&f)[2][8], const C2* xbb, const C2* g, int 
   }
 }
 
-// BSK ring (Cx::kBskRing, device only): the key is consumed in CHUNKS of one (row, level) GLEV row [p][bin] = 32 KiB, four
+// BSK ring (device only): the key is consumed in CHUNKS of one (row, level) GLEV row [p][bin] = 32 KiB, four
 // per CMUX step in the order (row 0, level 1), (row 1, level 1), (row 0, level 0), (row 1, level 0).  All pairs of a
 // CTA walk the same chunk sequence G = 4 i + k (continuing over the ciphertexts they process: the key repeats), so
 // ONE bulk copy per chunk (cp.async.bulk -> mbarrier, kernels.cuh) serves all of them from a small shared-memory ring:
 // bsk_acquire waits until chunk G has landed, bsk_release (one thread per pair, after a pair barrier that follows the
 // last read) counts the pair off; the last pair to release a stage re-arms it with chunk G + stages.
 template <class Cx>
-SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const C2* T1, const C2* T2, int& G) {
+SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, C2* xb, const C2* T1, const C2* T2, int& G) {
   const int u = cx.u, h = cx.h;
   const int k1 = u & 15, q = u >> 4;
   const int n = A.lwe_n;
   const bool cbs = A.lut == nullptr;
   const int log2n = 12;  // log2(2N)
   C2* xown = xb + h * kXBuf;
-  // Cx::kTmemX1 (device): the first exchange of a transform stays inside the warp (fft16.cuh: x1_time_index).  The thread
-  // then owns the coefficients j = ua + 64 i of its polynomial in the time domain while everything it keeps per thread in
-  // shared memory (the accumulator image pa[u + 64 i]) stays indexed by the physical thread u; from pass 2 on it is
-  // thread (k1, q) = u as before.
-  constexpr bool kX1 = Cx::kTmemX1;
-  const int ua = cx.time_index();
-  // Cx::kTransient: the accumulator polynomial of this half lives ONLY in the threads' own-coefficient copies
-  // (device: tensor memory); the shared-memory image the rotated gather reads is written into the half's exchange
-  // buffer at the end of a step and is dead once the digits have been taken, so a pair needs no persistent 32 KiB
-  // accumulator in shared memory (two more half-barriers per step: gather -> first exchange write, last exchange
-  // read -> image write).
-  constexpr bool kTr = Cx::kTransient;
-  uint64_t* pa = kTr ? reinterpret_cast<uint64_t*>(xown) : acc + h * kN;  // the polynomial this half owns
+  // The accumulator polynomial of this half lives ONLY in the threads' own-coefficient copies (device: tensor memory);
+  // the shared-memory image the rotated gather reads is written into the half's exchange buffer at the end of a step
+  // and is dead once the digits have been taken, so a pair needs no persistent 32 KiB accumulator in shared memory
+  // (two more half-barriers per step: gather -> first exchange write, last exchange read -> image write).
+  uint64_t* pa = reinterpret_cast<uint64_t*>(xown);  // the polynomial this half owns
   // 1. acc = LUT * X^{-b~}   (programmable_bootstrapping.rs:378-390)
   {
     uint64_t b = ldg_u64(A.lwe_in + n);
@@ -498,7 +447,7 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
     const int rot = (2 * kN - bt) & (2 * kN - 1);
     const int v = 1 << A.log_v;
     for (int i = 0; i < 32; i++) {
-      const int j = ua + 64 * i;
+      const int j = u + 64 * i;
       int idx = j - rot;
       bool neg = false;
       if (idx < 0) { idx += kN; neg = true; }
@@ -512,21 +461,14 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
   cx.sync();
   // 2. 637 CMUXes (programmable_bootstrapping.rs:396-409)
   uint64_t a_next = n > 0 ? ldg_u64(A.lwe_in) : 0;
-  // own[i2] = pa[u + 64 i2]: the thread's own coefficients stay in registers from the accumulator
-  // update of one step to the gather of the next (they are dead while the transforms run).
-  // Cx::kChunked (the 4-pairs-per-CTA build, 128 registers): they are instead fetched from the tensor-memory copy
-  // 8 (gather) or 4 + 4 (update) at a time, so neither phase holds all 32 next to a 16-point transform.
-  constexpr bool kCh = Cx::kChunked;
-  uint64_t own[kCh ? 8 : 32];
+  // own[]: the thread's own coefficients pa[u + 64 i2], fetched from the thread's tensor-memory copy 8 (gather) or
+  // 4 + 4 (update) at a time, so neither phase holds all 32 next to a 16-point transform.
+  uint64_t own[8];
   {
     uint64_t o0[32];
 #pragma unroll
     for (int i2 = 0; i2 < 32; i2++) o0[i2] = pa[u + 64 * i2];
     cx.own_store(o0);
-    if constexpr (!kCh) {
-#pragma unroll
-      for (int i2 = 0; i2 < 32; i2++) own[i2] = o0[i2];
-    }
   }
 #pragma unroll 1
   for (int i = 0; i < n; i++) {
@@ -546,76 +488,23 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
       // signed 16-bit digits, LSB first (math/radix.rs:81-113 for logB=16, l=2).  The source index
       // of coefficient j = u + 64 i2 is (u - a~ + 64 i2) mod 2N: bit 11 = negacyclic sign.
       {
-        const int base = (ua - at) & (2 * kN - 1);
+        const int base = (u - at) & (2 * kN - 1);
         // byte address of source row tt = (base >> 6) + i2 (mod 32) of this thread's column:
         // rows are 512 B apart, so the row index lives in bits 9..13 of the offset
-        const char* col = reinterpret_cast<const char*>(pa) + 8 * (kX1 ? x1_position(base & 63) : (base & 63));
+        const char* col = reinterpret_cast<const char*>(pa) + 8 * (base & 63);
         const uint32_t bh9 = (uint32_t)(base >> 6) << 9;
-#if SPF_GATHER_SEL
-        // The row index (base >> 6) + i2 wraps past row 31 exactly once over i2 = 0..31, and the negacyclic sign flips at the
-        // same place: two base pointers and two sign masks per thread, chosen by ONE comparison per coefficient -- the row offset
-        // 512 i2 is then an immediate of the load and the conditional negation is (x ^ m) - m with m = 0 / ~0.
-        const int rb = (base >> 6) & 31;
-        const int wrap = 32 - rb;                                 // i2 >= wrap: wrapped
-        const char* pU = col + 512 * rb;
-        const char* pW = pU - 32 * 512;
-        const uint32_t mU = 0u - (uint32_t)(base >> 11), mW = ~mU;  // base bit 11: the sign before the wrap
-#endif
 #pragma unroll
         for (int i2 = 0; i2 < 32; i2++) {
-          if constexpr (kCh) {
-            if ((i2 & 7) == 0) cx.own_ld8(own, i2 >> 3);  // own[0..7] = coefficients 8c .. 8c + 7
-          }
-#if SPF_GATHER_SEL
-          const bool wr = i2 >= wrap;
-          const uint64_t xr = *reinterpret_cast<const uint64_t*>((wr ? pW : pU) + 512 * i2);
-          const uint32_t m = wr ? mW : mU;
-          const uint64_t mm = ((uint64_t)m << 32) | m;
-          const uint64_t diff = ((xr ^ mm) - mm) - own[kCh ? (i2 & 7) : i2];
-#else
+          if ((i2 & 7) == 0) cx.own_ld8(own, i2 >> 3);  // own[0..7] = coefficients 8c .. 8c + 7
           const uint32_t t9 = bh9 + 512u * i2;  // bit 14 = negacyclic sign
-          const uint64_t x = SPF_ABLATE(32) ? (uint64_t)t9 * 0x9E3779B97F4A7C15ull : *reinterpret_cast<const uint64_t*>(col + (t9 & 0x3E00u));
-          const uint64_t diff = ((t9 & 0x4000u) ? 0 - x : x) - own[kCh ? (i2 & 7) : i2];
-#endif
+          const uint64_t x = *reinterpret_cast<const uint64_t*>(col + (t9 & 0x3E00u));
+          const uint64_t diff = ((t9 & 0x4000u) ? 0 - x : x) - own[i2 & 7];
           const uint32_t w = (uint32_t)(diff >> 32) + ((uint32_t)diff >> 31);
           const uint32_t w1 = w + 0x8000u;  // high half = second digit: (w >> 16) + carry of the first
           if (i2 < 16) { v[i2].x = digit_lo16_to_f64(w); pk[i2] = w1 >> 16; }
           else { v[i2 - 16].y = digit_lo16_to_f64(w); pk[i2 - 16] |= w1 & 0xFFFF0000u; }
         }
       }
-      if constexpr (Cx::kTwoBuf) {
-        // Two exchange buffers per half (Cx::kTwoBuf: xb + h kXBuf for digit level 0, xb + (2 + h) kXBuf for digit level 1): both
-        // forward transforms of the half are in flight together -- pass 1 of the second level is computed while the first
-        // level's products sit in shared memory, ONE half-barrier covers both first exchanges and ONE pair-barrier both
-        // second exchanges, and the multiply-accumulate of all four spectra follows in one piece: the accumulators are never
-        // parked, three barriers per step disappear.
-        static_assert(!Cx::kBskRing && !Cx::kTmemX1 && !Cx::kFusedStores && Cx::kReaderT2, "two-buffer form: LDG key, reader-side pass-2 twiddles");
-        C2* xown2 = xb + (2 + h) * kXBuf;
-        fwd_pass1_core(v);
-        cx.template t1_mul<false>(v, T1);
-        if (kTr) cx.sync();  // every thread of the half has gathered from the accumulator image in xown
-        fwd_x1_write(v, xown, u);
-#pragma unroll
-        for (int m = 0; m < 16; m++) { v[m].x = digit_lo16_to_f64(pk[m]); v[m].y = digit_hi16_to_f64(pk[m]); }
-        fwd_pass1_core(v);
-        cx.template t1_mul<false>(v, T1);
-        fwd_x1_write(v, xown2, u);
-        cx.sync();
-        fwd_x1_read(v, xown, u);
-        dft16<false>(v);
-        fwd_x2_write(v, xown, u);  // in place
-        fwd_x1_read(v, xown2, u);
-        dft16<false>(v);
-        fwd_x2_write(v, xown2, u);
-        cx.pair_sync();
-        double tw[12];
-        cx.rt2_fwd(tw, T2);
-        // the same accumulation order as the one-buffer form: (row 0, level 1), (row 1, level 1), (row 0, level 0), (row 1, level 0)
-        mad_split_rt<true>(cx, f, xb, ggsw + (size_t)((0 * 2 + 1) * 2) * kM, u, h, tw);
-        mad_split_rt<false>(cx, f, xb + kXBuf, ggsw + (size_t)((1 * 2 + 1) * 2) * kM, u, h, tw);
-        mad_split_rt<false>(cx, f, xb + 2 * kXBuf, ggsw + (size_t)((0 * 2 + 0) * 2) * kM, u, h, tw);
-        mad_split_rt<false>(cx, f, xb + 3 * kXBuf, ggsw + (size_t)((1 * 2 + 0) * 2) * kM, u, h, tw);
-      } else {
 #pragma unroll
       for (int t = 0; t < 2; t++) {
         const int level = 1 - t;  // LSB digit <-> last GLEV level (fft_ops.rs:92)
@@ -624,68 +513,24 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
           for (int m = 0; m < 16; m++) { v[m].x = digit_lo16_to_f64(pk[m]); v[m].y = digit_hi16_to_f64(pk[m]); }
         }
         fwd_pass1_core(v);
-        if constexpr (Cx::kFusedStores) {
-          // every product goes to the exchange buffer as soon as it exists: the stores overlap the remaining
-          // multiplies instead of queueing up behind them in front of the barrier
-          if (t == 1) { cx.pair_sync(); cx.bsk_release(G); cx.bsk_release(G + 1); }
-          else if (kTr) cx.sync();
-          cx.template t1_mul_store<false>(v, T1, xown);  // v[k1] *= T1[k1][u]; xown[k1][u] = v[k1]
-          cx.sync();
-          fwd_x1_read(v, xown, u);
-          dft16<false>(v);
-          if constexpr (Cx::kReaderT2) fwd_x2_write(v, xown, u);  // the twiddles are applied by the readers (mad_split_rt)
-          else cx.template t2_mul_store<false>(v, T2, xown);  // v[k2] *= W64^(q k2); in-place second exchange
-        } else {
-          cx.template t1_mul<false>(v, T1);  // v[k1] *= T1[k1][ua]
-          if constexpr (kX1) {
-            if (t == 0) {
-              // first digit level: the accumulators are not live, their tensor-memory columns carry the exchange
-              cx.x1_fwd(v);
-              dft16<false>(v);
-              if constexpr (!Cx::kReaderT2) cx.template t2_mul<false>(v, T2);
-              if (kTr) cx.sync();  // every thread of the half has gathered from the accumulator image in xown
-            } else {
-              // second digit level (the accumulators are parked in those columns): shared memory, per-thread slots
-              cx.pair_sync(); cx.bsk_release(G); cx.bsk_release(G + 1);
-              fwd_x1_write(v, xown, u);
-              cx.sync();
-              fwd_x1_read_perm(v, xown, u);
-              dft16<false>(v);
-              if constexpr (!Cx::kReaderT2) cx.template t2_mul<false>(v, T2);
-              cx.sync();  // the slots read above are not the ones fwd_x2_write overwrites: wait for the other readers of the row
-            }
-            fwd_x2_write(v, xown, u);
-          } else {
-          if (t == 1) { cx.pair_sync(); cx.bsk_release(G); cx.bsk_release(G + 1); }  // both halves have consumed the level-0 spectra (and the key chunks)
-          else if (kTr) cx.sync();     // every thread of the half has gathered from the accumulator image in xown
-          fwd_x1_write(v, xown, u);
-          cx.sync();
-          fwd_x1_read(v, xown, u);
-          dft16<false>(v);
-          if constexpr (!Cx::kReaderT2) cx.template t2_mul<false>(v, T2);  // v[k2] *= W64^(q k2) (else: by the readers, mad_split_rt)
-          fwd_x2_write(v, xown, u);  // in place: no barrier after fwd_x1_read
-          }
-        }
+        cx.template t1_mul<false>(v, T1);  // v[k1] *= T1[k1][u]
+        if (t == 1) { cx.pair_sync(); cx.bsk_release(G); cx.bsk_release(G + 1); }  // both halves have consumed the level-0 spectra (and the key chunks)
+        else cx.sync();  // every thread of the half has gathered from the accumulator image in xown
+        fwd_x1_write(v, xown, u);
+        cx.sync();
+        fwd_x1_read(v, xown, u);
+        dft16<false>(v);
+        fwd_x2_write(v, xown, u);  // in place: no barrier after fwd_x1_read; the pass-2 twiddles are applied by the readers
         if (t == 1) cx.f_load(f);
         cx.pair_sync();
         const C2* g0 = cx.bsk_acquire(G + 2 * t, ggsw + (size_t)((0 * 2 + level) * 2) * kM);
-        if constexpr (Cx::kReaderT2) {
-          double tw[12];
-          cx.rt2_fwd(tw, T2);
-          if (t == 0) mad_split_rt<true>(cx, f, xb, g0, u, h, tw);
-          else mad_split_rt<false>(cx, f, xb, g0, u, h, tw);
-          cx.bsk_release_early(G + 2 * t);
-          const C2* g1 = cx.bsk_acquire(G + 2 * t + 1, ggsw + (size_t)((1 * 2 + level) * 2) * kM);
-          mad_split_rt<false>(cx, f, xb + kXBuf, g1, u, h, tw);
-          cx.bsk_release_early(G + 2 * t + 1);
-        } else {
-        if (t == 0) mad_split<true>(cx, f, xb, g0, u, h);
-        else mad_split<false>(cx, f, xb, g0, u, h);
+        double tw[12];
+        cx.rt2_fwd(tw, T2);
+        if (t == 0) mad_split_rt<true>(cx, f, xb, g0, u, h, tw);
+        else mad_split_rt<false>(cx, f, xb, g0, u, h, tw);
         const C2* g1 = cx.bsk_acquire(G + 2 * t + 1, ggsw + (size_t)((1 * 2 + level) * 2) * kM);
-        mad_split<false>(cx, f, xb + kXBuf, g1, u, h);
-        }
+        mad_split_rt<false>(cx, f, xb + kXBuf, g1, u, h, tw);
         if (t == 0) cx.f_store(f);  // device: parked in tensor memory while the second transform runs
-      }
       }
     }
     // first inverse pass on this half's bins of both output polynomials, hand them to their owners
@@ -694,7 +539,7 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
       bfly4<true>(f[p][0], f[p][1], f[p][2], f[p][3]);
       bfly4<true>(f[p][4], f[p][5], f[p][6], f[p][7]);
     }
-    if constexpr (Cx::kReaderT2) {  // the conjugate pass-2 twiddles of the inverse transform, applied by the bin owner
+    {  // the conjugate pass-2 twiddles of the inverse transform, applied by the bin owner
       C2 wi[6];
       cx.rt2_inv(wi, T2);
 #pragma unroll
@@ -704,14 +549,13 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
 #pragma unroll
           for (int qp = 1; qp < 4; qp++) f[p][4 * jj + qp] = cmul_conj(f[p][4 * jj + qp], wi[3 * jj + qp - 1]);
     }
-    // in place: every thread overwrites exactly the 8 locations per buffer it read in mad_split
+    // in place: every thread overwrites exactly the 8 locations per buffer it read in mad_split_rt
 #pragma unroll
     for (int p = 0; p < 2; p++) {
 #pragma unroll
       for (int jj = 0; jj < 2; jj++) {
 #pragma unroll
-        for (int qp = 0; qp < 4; qp++)
-          if (!SPF_ABLATE(4)) xb[p * kXBuf + k1 * kXPad + qp + 4 * q + 16 * (2 * h + jj)] = f[p][4 * jj + qp];
+        for (int qp = 0; qp < 4; qp++) xb[p * kXBuf + k1 * kXPad + qp + 4 * q + 16 * (2 * h + jj)] = f[p][4 * jj + qp];
       }
     }
     cx.pair_sync();
@@ -722,61 +566,20 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
     {
       C2 w[16];
       inv_x2_read(w, xown, u);
-      if constexpr (!Cx::kReaderT2) cx.template t2_mul<true>(w, T2);
-      if constexpr (Cx::kFusedStores) {
-        dft16_emit<true>(w, [&](int mp, C2 val) { cx.sts(xown + k1 * kXPad + q + 4 * mp, val); });  // = inv_x1_write
-      } else if constexpr (kX1) {
-        dft16<true>(w);
-        cx.x1_inv(w);  // w[k1] of thread ua; the accumulators' tensor-memory columns are free again
-      } else {
-        dft16<true>(w);
-        inv_x1_write(w, xown, u);  // in place: no barrier after inv_x2_read
-      }
-      if constexpr (!kX1) {
-        cx.sync();
-        inv_x1_read(w, xown, u);
-      }
-      if (kTr) cx.sync();  // xown becomes the accumulator image again (every thread has read its inverse-pass inputs)
+      dft16<true>(w);
+      inv_x1_write(w, xown, u);  // in place: no barrier after inv_x2_read
+      cx.sync();
+      inv_x1_read(w, xown, u);
+      cx.sync();  // xown becomes the accumulator image again (every thread has read its inverse-pass inputs)
       cx.template t1_mul<true>(w, T1);  // w[k1] *= conj(T1[k1][u])
       double ws[16];
       inv_pass1_core_s(w, ws);  // true value ws[m] * w[m]: the untwist's real factor rides into the conversion
-      if constexpr (!kCh) cx.own_load(own, pa);  // own[i2] = pa[u + 64 i2] (device: from the thread's tensor-memory copy)
       // The saturating-cast corner of the conversion (probability ~2^-53 per value) is tested once
       // per 8 values: the fast conversion only tracks the largest exponent word it saw.
 #pragma unroll
       for (int m4 = 0; m4 < 16; m4 += 4) {
         uint32_t mag_max = 0;
         uint64_t r[8];
-        if constexpr (Cx::kFrndConv) {
-          // round-to-integral conversion of fl(ws * w): two FP64 instructions per value instead of four (fft16.cuh: f64_to_torus_frnd)
-          uint32_t small_min = 0x7FFFFFFFu;
-#pragma unroll
-          for (int i = 0; i < 4; i++) {
-            r[2 * i] = f64_to_torus_frnd(w[m4 + i].x, ws[m4 + i], small_min, mag_max);
-            r[2 * i + 1] = f64_to_torus_frnd(w[m4 + i].y, ws[m4 + i], small_min, mag_max);
-          }
-          if (__builtin_expect(small_min < kTorusSmallMag || mag_max >= kTorusHalfMag, 0)) {
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-              r[2 * i] = f64_to_torus(ws[m4 + i] * w[m4 + i].x);
-              r[2 * i + 1] = f64_to_torus(ws[m4 + i] * w[m4 + i].y);
-            }
-          }
-        } else if constexpr (Cx::kIntConv) {
-          // integer conversion of fl(ws * w): one FP64 instruction per value instead of four (fft16.cuh: f64_to_torus_int)
-#pragma unroll
-          for (int i = 0; i < 4; i++) {
-            r[2 * i] = f64_to_torus_int(w[m4 + i].x, ws[m4 + i], mag_max);
-            r[2 * i + 1] = f64_to_torus_int(w[m4 + i].y, ws[m4 + i], mag_max);
-          }
-          if (__builtin_expect(mag_max != 0, 0)) {
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-              r[2 * i] = f64_to_torus(ws[m4 + i] * w[m4 + i].x);
-              r[2 * i + 1] = f64_to_torus(ws[m4 + i] * w[m4 + i].y);
-            }
-          }
-        } else {
 #pragma unroll
         for (int i = 0; i < 4; i++) {
           r[2 * i] = f64_to_torus_s_fast(w[m4 + i].x, ws[m4 + i], mag_max);
@@ -789,37 +592,24 @@ SPF_HD void pbs_pair_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
             r[2 * i + 1] = f64_to_torus_s(w[m4 + i].y, ws[m4 + i]);
           }
         }
-        }
-        if constexpr (kCh) {
-          cx.own_ld4x2(own, m4);  // own[0..3] = coefficients m4 .. m4 + 3, own[4..7] = m4 + 16 .. m4 + 19
+        cx.own_ld4x2(own, m4);  // own[0..3] = coefficients m4 .. m4 + 3, own[4..7] = m4 + 16 .. m4 + 19
 #pragma unroll
-          for (int i = 0; i < 4; i++) {
-            const int j = u + 64 * (m4 + i);
-            own[i] += r[2 * i];
-            own[4 + i] += r[2 * i + 1];
-            pa[j] = own[i];
-            pa[j + kM] = own[4 + i];
-          }
-          cx.own_st4x2(own, m4);
-        } else {
-#pragma unroll
-          for (int i = 0; i < 4; i++) {
-            const int m = m4 + i, j = u + 64 * m;
-            own[m] += r[2 * i];
-            own[m + 16] += r[2 * i + 1];
-            pa[j] = own[m];
-            pa[j + kM] = own[m + 16];
-          }
+        for (int i = 0; i < 4; i++) {
+          const int j = u + 64 * (m4 + i);
+          own[i] += r[2 * i];
+          own[4 + i] += r[2 * i + 1];
+          pa[j] = own[i];
+          pa[j + kM] = own[4 + i];
         }
+        cx.own_st4x2(own, m4);
       }
-      if constexpr (kCh) cx.own_st_wait();
-      else cx.own_store(own);
+      cx.own_st_wait();
     }
     cx.sync();  // next step gathers rotated coefficients written by other threads of this half
   }
   // 3. result
-  for (int i = 0; i < 32; i++) A.glwe_out[h * kN + ua + 64 * i] = pa[u + 64 * i];
-  if (kTr) cx.sync();  // the next ciphertext of this pair overwrites the image
+  for (int i = 0; i < 32; i++) A.glwe_out[h * kN + u + 64 * i] = pa[u + 64 * i];
+  cx.sync();  // the next ciphertext of this pair overwrites the image
 }
 
 // QUAD-TEAM blind rotation (latency mode, batches of at most one ciphertext per SM): one ciphertext
@@ -896,46 +686,33 @@ SPF_HD void pbs_quad_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
       const int base = (u - at) & (2 * kN - 1);
       const char* col = reinterpret_cast<const char*>(pa) + 8 * (base & 63);
       const uint32_t bh9 = (uint32_t)(base >> 6) << 9;
-      if constexpr (Cx::kSplitGather) {
-        // The two teams of a polynomial need the same 32 rounded differences, one digit level each.  Each gathers HALF of
-        // them (team t the coefficients 16 t .. 16 t + 15 of its column), keeps its own digit and hands the other level's
-        // 16 digits, packed two to a word, to the partner thread (same u, other t) -- on the device through eight
-        // tensor-memory columns of the lane the two threads share.  Same bits as before: a 16-bit digit d is converted
-        // by digit_lo16_to_f64(d), which equals digit_hi16_to_f64(d << 16).
-        uint32_t pk[8];
-        auto gather_half = [&](auto tt) {  // the half is a compile-time constant: own[] stays in registers
-          constexpr int T = decltype(tt)::value;
-#pragma unroll
-          for (int k = 0; k < 16; k++) {
-            const int i2 = 16 * T + k;
-            const uint32_t t9 = bh9 + 512u * i2;
-            const uint64_t x = *reinterpret_cast<const uint64_t*>(col + (t9 & 0x3E00u));
-            const uint64_t diff = ((t9 & 0x4000u) ? 0 - x : x) - own[i2];
-            const uint32_t w = (uint32_t)(diff >> 32) + ((uint32_t)diff >> 31);
-            const uint32_t w1 = w + 0x8000u;
-            const uint32_t other = T ? (w & 0xFFFFu) : (w1 >> 16);  // the digit of level 1 - T
-            if (T) v[k].y = digit_hi16_to_f64(w1); else v[k].x = digit_lo16_to_f64(w);
-            if (k & 1) pk[k >> 1] |= other << 16; else pk[k >> 1] = other;
-          }
-        };
-        if (t) gather_half(std::integral_constant<int, 1>{}); else gather_half(std::integral_constant<int, 0>{});
-        cx.digit_xchg(pk);
+      // The two teams of a polynomial need the same 32 rounded differences, one digit level each.  Each gathers HALF of
+      // them (team t the coefficients 16 t .. 16 t + 15 of its column), keeps its own digit and hands the other level's
+      // 16 digits, packed two to a word, to the partner thread (same u, other t) -- on the device through eight
+      // tensor-memory columns of the lane the two threads share.  The digits are those of a full gather: a 16-bit digit d
+      // is converted by digit_lo16_to_f64(d), which equals digit_hi16_to_f64(d << 16).
+      uint32_t pk[8];
+      auto gather_half = [&](auto tt) {  // the half is a compile-time constant: own[] stays in registers
+        constexpr int T = decltype(tt)::value;
 #pragma unroll
         for (int k = 0; k < 16; k++) {
-          const double d = digit_lo16_to_f64(pk[k >> 1] >> (16 * (k & 1)));
-          if (t) v[k].x = d; else v[k].y = d;  // team 1 lacked the first half (real parts), team 0 the second
+          const int i2 = 16 * T + k;
+          const uint32_t t9 = bh9 + 512u * i2;
+          const uint64_t x = *reinterpret_cast<const uint64_t*>(col + (t9 & 0x3E00u));
+          const uint64_t diff = ((t9 & 0x4000u) ? 0 - x : x) - own[i2];
+          const uint32_t w = (uint32_t)(diff >> 32) + ((uint32_t)diff >> 31);
+          const uint32_t w1 = w + 0x8000u;
+          const uint32_t other = T ? (w & 0xFFFFu) : (w1 >> 16);  // the digit of level 1 - T
+          if (T) v[k].y = digit_hi16_to_f64(w1); else v[k].x = digit_lo16_to_f64(w);
+          if (k & 1) pk[k >> 1] |= other << 16; else pk[k >> 1] = other;
         }
-      } else {
+      };
+      if (t) gather_half(std::integral_constant<int, 1>{}); else gather_half(std::integral_constant<int, 0>{});
+      cx.digit_xchg(pk);
 #pragma unroll
-      for (int i2 = 0; i2 < 32; i2++) {
-        const uint32_t t9 = bh9 + 512u * i2;
-        const uint64_t x = *reinterpret_cast<const uint64_t*>(col + (t9 & 0x3E00u));
-        const uint64_t diff = ((t9 & 0x4000u) ? 0 - x : x) - own[i2];
-        const uint32_t w = (uint32_t)(diff >> 32) + ((uint32_t)diff >> 31);
-        // digit 0: low half of w; digit 1: high half of w + 0x8000 (math/radix.rs:81-113, logB = 16, l = 2)
-        const double d = t ? digit_hi16_to_f64(w + 0x8000u) : digit_lo16_to_f64(w);
-        if (i2 < 16) v[i2].x = d; else v[i2 - 16].y = d;
-      }
+      for (int k = 0; k < 16; k++) {
+        const double d = digit_lo16_to_f64(pk[k >> 1] >> (16 * (k & 1)));
+        if (t) v[k].x = d; else v[k].y = d;  // team 1 lacked the first half (real parts), team 0 the second
       }
       SPF_QT(0);
       fwd_pass1_core(v);
@@ -945,8 +722,7 @@ SPF_HD void pbs_quad_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
       SPF_QT(1);
       fwd_x1_read(v, xown, u);
       dft16<false>(v);
-      if constexpr (!Cx::kReaderT2) cx.template t2_mul<false>(v, T2);  // else: applied by the readers below (as in pbs_pair_team)
-      fwd_x2_write(v, xown, u);  // in place
+      fwd_x2_write(v, xown, u);  // in place; the pass-2 twiddles are applied by the readers below (as in pbs_pair_team)
       SPF_QT(2);
     }
     cx.quad_sync();
@@ -958,7 +734,7 @@ SPF_HD void pbs_quad_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
     C2 f[2][4];
     double rtw[6];
     C2 rwi[3];
-    if constexpr (Cx::kReaderT2) cx.rt2(rtw, rwi, T2);  // this thread's pass-2 twiddles in the tan form (rt2_group_consts)
+    cx.rt2(rtw, rwi, T2);  // this thread's pass-2 twiddles in the tan form (rt2_group_consts)
 #pragma unroll
     for (int b = 0; b < 4; b++) {  // spectrum of team b = (hb, tb): digit tb <-> GLEV level 1 - tb
       const C2* grow = staged + (size_t)(((b >> 1) * 2 + (1 - (b & 1))) * 2) * kM;
@@ -970,13 +746,9 @@ SPF_HD void pbs_quad_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
         g0[k3] = cx.row_load(grow + u + 64 * (g + 4 * k3));
         g1[k3] = cx.row_load(grow + kM + u + 64 * (g + 4 * k3));
       }
-      if constexpr (Cx::kReaderT2) {
 #pragma unroll
-        for (int qp = 1; qp < 4; qp++) d[qp] = C2{spf_fma(-rtw[qp - 1], d[qp].y, d[qp].x), spf_fma(rtw[qp - 1], d[qp].x, d[qp].y)};
-        bfly4_r<false>(d[0], d[1], d[2], d[3], rtw[3], rtw[4], rtw[5]);
-      } else {
-        bfly4<false>(d[0], d[1], d[2], d[3]);
-      }
+      for (int qp = 1; qp < 4; qp++) d[qp] = C2{spf_fma(-rtw[qp - 1], d[qp].y, d[qp].x), spf_fma(rtw[qp - 1], d[qp].x, d[qp].y)};
+      bfly4_r<false>(d[0], d[1], d[2], d[3], rtw[3], rtw[4], rtw[5]);
 #pragma unroll
       for (int k3 = 0; k3 < 4; k3++) {
         if (b == 0) { f[0][k3] = cmul(d[k3], g0[k3]); f[1][k3] = cmul(d[k3], g1[k3]); }
@@ -987,10 +759,8 @@ SPF_HD void pbs_quad_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
 #pragma unroll
     for (int p = 0; p < 2; p++) {
       bfly4<true>(f[p][0], f[p][1], f[p][2], f[p][3]);
-      if constexpr (Cx::kReaderT2) {  // the inverse transform's conjugate pass-2 twiddles, applied by the bin owner
 #pragma unroll
-        for (int qp = 1; qp < 4; qp++) f[p][qp] = cmul_conj(f[p][qp], rwi[qp - 1]);
-      }
+      for (int qp = 1; qp < 4; qp++) f[p][qp] = cmul_conj(f[p][qp], rwi[qp - 1]);  // the inverse transform's conjugate pass-2 twiddles
 #pragma unroll
       for (int qp = 0; qp < 4; qp++) xb[2 * p * kXBuf + k1 * kXPad + qp + 4 * q + 16 * g] = f[p][qp];
     }
@@ -1005,7 +775,6 @@ SPF_HD void pbs_quad_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
       C2 w[16];
       double ws[16];
       inv_x2_read(w, xown, u);
-      if constexpr (!Cx::kReaderT2) cx.template t2_mul<true>(w, T2);
       dft16<true>(w);
       inv_x1_write(w, xown, u);  // in place
       cx.sync();
@@ -1046,7 +815,7 @@ SPF_HD void pbs_quad_team(Cx& cx, const PbsArgs& A, uint64_t* acc, C2* xb, const
     cx.quad_sync();
     if (t == 1) {
 #pragma unroll
-      for (int i2 = Cx::kSplitGather ? 16 : 0; i2 < 32; i2++) own[i2] = pa[u + 64 * i2];
+      for (int i2 = 16; i2 < 32; i2++) own[i2] = pa[u + 64 * i2];
     }
   }
 #if defined(SPF_QUAD_TRACE) && defined(__CUDA_ARCH__)
@@ -1248,7 +1017,6 @@ SPF_HD void cmux_wide(Cx& cx, uint64_t* out, const uint64_t* d0, const uint64_t*
     const uint64_t off = radix_offset(radix_log, count);
     const uint64_t dmask = (1ull << radix_log) - 1;
     const int32_t half = 1 << (radix_log - 1);
-    cx.template g_stage<0>();
     C2 v[16];
     const int shift = 64 - radix_log * count;
     if (shift >= 33) {
@@ -1258,7 +1026,6 @@ SPF_HD void cmux_wide(Cx& cx, uint64_t* out, const uint64_t* d0, const uint64_t*
       const int sh = shift - 32 + t * radix_log;
 #pragma unroll
       for (int m = 0; m < 16; m++) {
-        if (m == 8) cx.template g_stage<1>();
         const int j = r * kN + u + 64 * m;
         const uint64_t x0 = d0 ? d1[j] - d0[j] : d1[j];  // d0 / d1 may be shared-memory copies (cmux_wide_kernel)
         const uint64_t x1 = d0 ? d1[j + kM] - d0[j + kM] : d1[j + kM];
@@ -1266,7 +1033,6 @@ SPF_HD void cmux_wide(Cx& cx, uint64_t* out, const uint64_t* d0, const uint64_t*
         v[m].y = i32_to_f64((int32_t)((((uint32_t)(x1 >> 32) + c1) >> sh) & (uint32_t)dmask) - half);
       }
     } else {
-      cx.template g_stage<1>();
 #pragma unroll
       for (int m = 0; m < 16; m++) {
         const int j = r * kN + u + 64 * m;
@@ -1278,31 +1044,20 @@ SPF_HD void cmux_wide(Cx& cx, uint64_t* out, const uint64_t* d0, const uint64_t*
       }
     }
     SPF_WT(1);
-    // cx.g_stage<i>: device only -- the selector GGSW (256 KiB, each element used once, by one thread) is brought into the
-    // thread's tensor-memory columns in 8 batches WHILE the digits are taken and the forward transforms run (batch i is
-    // requested at point i and parked at point i + 1), so the multiply-accumulate phase below no longer waits for
-    // 256 KiB to come through one SM's L2 port (6.5 k of the kernel's 20 k clocks)
-    cx.template g_stage<2>();
     fwd_pass1_core(v);
-    cx.template g_stage<3>();
 #pragma unroll
     for (int k1i = 0; k1i < 16; k1i++) v[k1i] = cmul(v[k1i], T1[k1i * 64 + u]);
-    cx.template g_stage<4>();
     fwd_x1_write(v, xown, u);
     cx.sync();
     SPF_WT(2);
     fwd_x1_read(v, xown, u);
-    cx.template g_stage<5>();
     dft16<false>(v);
-    cx.template g_stage<6>();
     {
       const int qq = u >> 4;
 #pragma unroll
       for (int k2i = 1; k2i < 16; k2i++) v[k2i] = cmul(v[k2i], T2[qq * kT2Pad + k2i]);
     }
-    cx.template g_stage<7>();
     fwd_x2_write(v, xown, u);  // in place
-    cx.template g_stage<8>();
   }
   cx.cta_sync();
   SPF_WT(3);
@@ -1313,15 +1068,12 @@ SPF_HD void cmux_wide(Cx& cx, uint64_t* out, const uint64_t* d0, const uint64_t*
 #pragma unroll
   for (int jb = 0; jb < 2 * 4; jb += 4) {  // 4 spectra per batch: their GGSW values are requested together
     C2 g[4][4], d[4][4];
-    if constexpr (Cx::kStageG) cx.g_read16(g, jb);  // parked by g_stage: the same sixteen values
 #pragma unroll
     for (int jj = 0; jj < 4; jj++) {
       const int j = jb + jj, rr = j / count, tt = j % count;  // digit tt <-> GGSW level count-1-tt (fft_ops.rs:92)
       const C2* grow = ggsw + ((size_t)(rr * count + (count - 1 - tt)) * 2 + p) * kM;
-      if constexpr (!Cx::kStageG) {
 #pragma unroll
-        for (int k3 = 0; k3 < 4; k3++) g[jj][k3] = ldg_c2(grow + k1 + 16 * k2 + 256 * k3);
-      }
+      for (int k3 = 0; k3 < 4; k3++) g[jj][k3] = ldg_c2(grow + k1 + 16 * k2 + 256 * k3);
 #pragma unroll
       for (int qp = 0; qp < 4; qp++) d[jj][qp] = xb[j * kXBuf + k1 * kXPad + qp + 4 * k2];
     }

@@ -476,28 +476,3 @@ def test_multiply_then_compare_32bit(keys, client, proc):
         g.run()
         _check_multiply(client, [v], w, out_prod, out_gt)
         g.close()
-
-
-def test_chained_mux_levels_match_per_level_launches(keys, client, proc, monkeypatch):
-    """SPF_B200_CHAIN=1: runs of consecutive narrow CMux levels execute as ONE cooperative launch (cmux_chain_kernel, levels
-    separated by a grid barrier).  The per-item body is the wide CMUX kernel's, so the outputs must equal those of the
-    one-launch-per-level form bit for bit -- a missed barrier or a stale staged input would change them -- and far fewer
-    kernels are launched.  (Opt-in: measured 2.7 % slower than programmatic dependent launches.)"""
-    w = 8
-    vals = [(201, 57, 90), (255, 255, 0)]
-    circ, out_prod, out_gt = _multiply_program(client, keys, w, vals)
-    g = proc.compile(circ)
-    monkeypatch.setenv("SPF_B200_CHAIN", "0")
-    g.run()
-    per_level = g.launches
-    want = [np.array(x, copy=True) for p in out_prod for x in p] + [np.array(x, copy=True) for x in out_gt]
-    _check_multiply(client, vals, w, out_prod, out_gt)
-    for x in [x for p in out_prod for x in p] + list(out_gt):
-        x[:] = 0
-    monkeypatch.setenv("SPF_B200_CHAIN", "1")
-    for _ in range(2):  # the second run reuses the plan
-        g.run()
-        got = [x for p in out_prod for x in p] + list(out_gt)
-        assert all(np.array_equal(a, b) for a, b in zip(want, got))
-        assert g.launches < per_level // 4
-    g.close()

@@ -72,8 +72,7 @@ rows.append({"op": "keyswitch_l1_l0", "batch": B, "ms": ms, "ops_per_s": B / ms 
              "int8_tmac_per_s": B * 2048 * 6 * 640 * 8 / ms / 1e9, "tcgen05_i8_nominal_tmac_per_s": 2250.0,
              "tensor_frac": B * 2048 * 6 * 640 * 8 / ms / 1e9 / 2250.0,
              "note": "8 u8 x u8 -> s32 byte-plane GEMMs on tcgen05.mma kind::i8 (TMEM accumulators); peak = nominal dense "
-                     "int8 rate of the part (4.5 POPS); the kernel is bound by the L2 -> SM stream of the key planes; "
-                     "SPF_B200_KS_IMPL=mma selects the legacy mma.sync kernel (measured IMMA rate 572 T MAC/s)"})
+                     "int8 rate of the part (4.5 POPS); the kernel is bound by the L2 -> SM stream of the key planes"})
 # ---- sample extract ----
 g = rand_u64(B, ev.len_glwe)
 l1o = torch.empty(B * ev.len_lwe_l1, dtype=torch.int64, device=dev)
