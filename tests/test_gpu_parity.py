@@ -9,7 +9,10 @@ Bars (DESIGN.md "Parity contract"):
     CBS): decryptions bit-exact, phase (b - a.s) distance <= 4 x the measured maximum (PBS 3.8e-6, CBS 2.4e-6,
     trace 1.9e-7 of the torus; tests/test_gpu_distances.py) -- ciphertext bytes are not comparable between any
     two FFT implementations (see test_emu.test_pbs_first_steps...); against the host emulator, which
-    rounds identically, every kernel is BIT-EXACT (tests/test_gpu_bitexact.py).
+    rounds identically, every kernel is BIT-EXACT (tests/test_gpu_bitexact.py);
+  * exact regime (integer-polynomial keys, tests/exact_keys.py): PBS, trace, CMUX and the CBS stages BIT-EXACT against
+    the oracle on arbitrary u64 inputs, every item; CBS and scheme-switch outputs FFT-domain <= 1e-14 relative
+    (tests/test_gpu_exact.py).
 """
 import ctypes as C
 
@@ -42,8 +45,10 @@ def test_keyswitch_ragged_batches(oracle, keys, evaluation, batch):
     rng = np.random.default_rng(batch)
     l1 = rng.integers(0, 1 << 64, (batch, keys.lwe1_len), dtype=np.uint64)
     got = evaluation.keyswitch_lwe_l1_lwe_l0(l1)
-    for i in (0, batch // 2, batch - 1):
-        assert np.array_equal(got[i], oracle.keyswitch_lwe(keys, l1[i]))
+    want = np.zeros_like(got)
+    oracle.lib().orc_keyswitch_lwe_batch(want, l1, batch, keys.ksk, C.byref(keys.params), oracle.hw_threads())
+    bad = [i for i in range(batch) if not np.array_equal(got[i], want[i])]
+    assert not bad, bad
 
 
 def test_sample_extract_bit_exact(oracle, keys, evaluation):
@@ -54,7 +59,13 @@ def test_sample_extract_bit_exact(oracle, keys, evaluation):
     for i, h in enumerate(idx):
         assert np.array_equal(got[i], oracle.sample_extract(keys, g[i], int(h)))
     got0 = evaluation.sample_extract_l1(g, 0)
-    assert np.array_equal(got0[3], oracle.sample_extract(keys, g[3], 0))
+    for i in range(len(g)):
+        assert np.array_equal(got0[i], oracle.sample_extract(keys, g[i], 0)), i
+    # every index once, one per item
+    g = rng.integers(0, 1 << 64, (2048, keys.glwe_len), dtype=np.uint64)
+    got = evaluation.sample_extract_l1(g, np.arange(2048, dtype=np.uint32))
+    bad = [h for h in range(2048) if not np.array_equal(got[h], oracle.sample_extract(keys, g[h], h))]
+    assert not bad, bad
 
 
 def test_not_xor_mul_xn_bit_exact(oracle, keys, evaluation):
