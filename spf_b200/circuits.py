@@ -157,11 +157,59 @@ def multiply_then_greater_than(a_bits, b_bits, c_bits, out_prod, out_gt, program
     return M.prune(c, keep)[0]
 
 
+def _instruction_graph(operands, out_bits, body) -> tuple[FheCircuit, list[int], list[int]]:
+    """One instruction as a graph: an InputGlwe1 per operand bit, `body(c, input_nodes)` -> the GLWE node behind every
+    result bit, an OutputGlwe1 per result bit, pruned to what the results read (fhe_circuit.rs:516-555).  operands: lists
+    of bit ciphertexts; input_nodes has the same shape.  Returns (graph, operand-bit nodes, result-bit nodes), both in
+    the flattened order of operands / out_bits; an operand bit no result reads has node -1."""
+    from . import mux_circuits as M
+
+    c = FheCircuit()
+    ins = [[c.add("InputGlwe1", io=x) for x in op] for op in operands]
+    res = body(c, ins)
+    assert len(res) == len(out_bits)
+    outs = [c.add("OutputGlwe1", n, io=buf) for n, buf in zip(res, out_bits)]
+    c, ren = M.prune(c, outs)
+    return c, [ren.get(n, -1) for op in ins for n in op], [ren[n] for n in outs]
+
+
+def _fronts(c: FheCircuit, inputs: list[list[int]]) -> list[list[int]]:
+    """The front end of fhe_circuit.rs:473-494 on every input node: one circuit bootstrap per operand bit."""
+    return [[_refresh(c, x) for x in op] for op in inputs]
+
+
+_COMPARE = {"gt": (True, False), "ge": (True, True), "lt": (False, False), "le": (False, True)}  # (greater, or_equal)
+_SHIFT_MODES = ("logical", "rotation", "arithmetic")
+# The barrel shifter's BDD orders the value bits above the amount bits (bitshift.rs), so its size grows as 2^w: 16 bits
+# is 196 588 multiplexers, 20 bits 3.2 million, 32 bits cannot be built.
+SHIFT_MAX_WIDTH = 16
+
+
+def _operands(name: str, *ops, equal: bool = True) -> list[list]:
+    ops = [list(op) for op in ops]
+    if any(not op for op in ops):
+        raise ValueError(f"InstructionCache.{name}: empty operand")
+    if equal and len({len(op) for op in ops}) > 1:
+        raise ValueError(f"InstructionCache.{name}: operand widths differ ({', '.join(str(len(op)) for op in ops)})")
+    return ops
+
+
+def _results(name: str, out_bits, *allowed: int) -> list:
+    out = list(out_bits)
+    if len(out) not in allowed:
+        raise ValueError(f"InstructionCache.{name}: {len(out)} result bits, expected {' or '.join(map(str, allowed))}")
+    return out
+
+
 class InstructionCache:
     """Graph-generation cache (SURVEY.md 8(f).3): one compiled, levelised, device-resident graph per
-    (instruction, width), re-bound to the operands of each invocation with CompiledGraph.set_io
+    (instruction, widths, flags), re-bound to the operands of each invocation with CompiledGraph.set_io
     instead of rebuilding the MUX circuit and re-levelising it per dispatch as
-    FheCircuit::insert_mux_circuit_and_connect_inputs (fhe_circuit.rs:473-494) does."""
+    FheCircuit::insert_mux_circuit_and_connect_inputs (fhe_circuit.rs:473-494) does.
+
+    Operands and results are lists of L1 GLWE bit ciphertexts, least significant bit first: host arrays, or
+    BoxCiphertext handles on a BoxEvaluation.  Every method checks its widths before anything is built (ValueError),
+    runs blocking and returns the graph it ran."""
 
     def __init__(self, evaluation):
         from . import BoxEvaluation, BoxGraph, CompiledGraph
@@ -170,40 +218,41 @@ class InstructionCache:
         self._ev, self._cache = evaluation, {}
         self.hits = self.misses = 0
 
-    def _run(self, key, build, in_bufs, out_bufs):
+    def _run(self, key, body, operands, out_bits):
+        """Build (on a miss) _instruction_graph(operands, out_bits, body), bind it to these operands and results and run
+        it.  Binding goes through the operand-bit / result-bit node maps recorded at build time: pruning may have removed
+        operand bits, and a rewired result may read an operand bit directly."""
         if key not in self._cache:
             self.misses += 1
-            c = build()
-            ins = [i for i, n in enumerate(c.nodes) if n[0] == 2]    # InputGlwe1, in operand order
-            outs = [i for i, n in enumerate(c.nodes) if n[0] == 7]   # OutputGlwe1, in result-bit order
-            assert len(ins) == len(in_bufs) and len(outs) == len(out_bufs)
+            c, ins, outs = _instruction_graph(operands, out_bits, body)
             self._cache[key] = (self._compile(self._ev, c), ins, outs)
         else:
             self.hits += 1
         g, ins, outs = self._cache[key]
-        for node, buf in zip(ins + outs, list(in_bufs) + list(out_bufs)):
-            g.set_io(node, buf)
+        for node, buf in zip(ins + outs, [x for op in operands for x in op] + list(out_bits)):
+            if node >= 0:
+                g.set_io(node, buf)
         g.run()
         return g
 
-    def add(self, a_bits, b_bits, out_bits):
-        """out = a + b (w-bit operands as L1 GLWE bit ciphertexts, w + 1 result bits), blocking."""
-        a_bits, b_bits, out_bits = list(a_bits), list(b_bits), list(out_bits)
-        return self._run(("add", len(a_bits)), lambda: ripple_carry_adder(a_bits, b_bits, out_bits), a_bits + b_bits, out_bits)
-
     def _mux_instruction(self, key, mux_builder, operands, out_bits, interleave):
-        """One ISA instruction = front end (fhe_circuit.rs:473-494) + one BDD-derived MUX circuit + outputs."""
+        """One ISA instruction = front end (fhe_circuit.rs:473-494) + one BDD-derived MUX circuit whose first
+        len(out_bits) outputs are the results.  MUX inputs: the operands' selectors one operand after the other, or
+        interleaved a0 b0 a1 b1 ..."""
         from . import mux_circuits as M
 
-        def build():
-            c = FheCircuit()
-            sels = [[_front(c, x) for x in op] for op in operands]
+        def body(c, ins):
+            sels = _fronts(c, ins)
             order = [x for grp in zip(*sels) for x in grp] if interleave else [x for op in sels for x in op]
-            for node, buf in zip(M.insert_mux_circuit(c, mux_builder(), order), out_bits):
-                c.add("OutputGlwe1", node, io=buf)
-            return M.prune(c, [i for i, n in enumerate(c.nodes) if n[0] == 7])[0]
+            return M.insert_mux_circuit(c, mux_builder(), order)[:len(out_bits)]
 
-        return self._run(key, build, [x for op in operands for x in op], out_bits)
+        return self._run(key, body, operands, out_bits)
+
+    def add(self, a_bits, b_bits, out_bits):
+        """out = a + b (w-bit operands, w + 1 result bits: the last is the carry)."""
+        a, b = _operands("add", a_bits, b_bits)
+        out = _results("add", out_bits, len(a) + 1)
+        return self._run(("add", len(a)), lambda c, ins: _adder_nodes(c, *_fronts(c, ins)), [a, b], out)
 
     def multiply(self, a_bits, b_bits, out_bits):
         """out = low w bits of a * b, w <= 16 (one multiplier block, parasol_cpu/src/proc/ops/mul.rs:75-117)."""
@@ -222,9 +271,192 @@ class InstructionCache:
         """out = (a > b), unsigned (comparisons.rs:62-98 with compare_or_maybe_equal(w, true, false))."""
         from . import mux_circuits as M
 
-        a_bits, b_bits = list(a_bits), list(b_bits)
+        a_bits, b_bits = _operands("greater_than", a_bits, b_bits)
         w = len(a_bits)
         return self._mux_instruction(("gt", w), lambda: M.compare_or_maybe_equal(w, True, False), [a_bits, b_bits], [out_bit], interleave=True)
+
+    # ---- MUX-circuit instructions: one circuit bootstrap per operand bit, then one CMUX level per MUX depth ----
+    def sub(self, a_bits, b_bits, out_bits):
+        """out = (a - b) mod 2^w; with w + 1 result bits the last one is the borrow (sub.rs:12-49)."""
+        from . import mux_circuits as M
+
+        a, b = _operands("sub", a_bits, b_bits)
+        w = len(a)
+        out = _results("sub", out_bits, w, w + 1)
+        return self._mux_instruction(("sub", w, len(out)), lambda: M.full_subtractor(w), [a, b], out, interleave=True)
+
+    def neg(self, a_bits, out_bits):
+        """out = -a mod 2^w, two's complement (neg.rs:7-27)."""
+        from . import mux_circuits as M
+
+        (a,) = _operands("neg", a_bits)
+        w = len(a)
+        out = _results("neg", out_bits, w)
+        return self._mux_instruction(("neg", w), lambda: M.negator(w), [a], out, interleave=False)
+
+    def compare(self, a_bits, b_bits, out_bit, op: str, signed: bool = False):
+        """out = (a op b) for op in "gt" "ge" "lt" "le", unsigned or two's complement (comparisons.rs:79-141)."""
+        from . import mux_circuits as M
+
+        if op not in _COMPARE:
+            raise ValueError(f"InstructionCache.compare: op {op!r}, expected one of {sorted(_COMPARE)}")
+        a, b = _operands("compare", a_bits, b_bits)
+        w, signed = len(a), bool(signed)
+        gen = M.compare_or_maybe_equal_signed if signed else M.compare_or_maybe_equal
+        return self._mux_instruction(("cmp", w, op, signed), lambda: gen(w, *_COMPARE[op]), [a, b], [out_bit], interleave=True)
+
+    def equal(self, a_bits, b_bits, out_bit):
+        """out = (a == b) (comparisons.rs, compare_equal)."""
+        from . import mux_circuits as M
+
+        a, b = _operands("equal", a_bits, b_bits)
+        w = len(a)
+        return self._mux_instruction(("eq", w), lambda: M.compare_equal(w), [a, b], [out_bit], interleave=True)
+
+    def not_equal(self, a_bits, b_bits, out_bit):
+        """out = (a != b) (comparisons.rs, compare_not_equal)."""
+        from . import mux_circuits as M
+
+        a, b = _operands("not_equal", a_bits, b_bits)
+        w = len(a)
+        return self._mux_instruction(("ne", w), lambda: M.compare_not_equal(w), [a, b], [out_bit], interleave=True)
+
+    def and_(self, a_bits, b_bits, out_bits):
+        """out = a & b (make_and_circuit)."""
+        from . import mux_circuits as M
+
+        a, b = _operands("and_", a_bits, b_bits)
+        w = len(a)
+        out = _results("and_", out_bits, w)
+        return self._mux_instruction(("and", w), lambda: M.make_and_circuit(w), [a, b], out, interleave=True)
+
+    def or_(self, a_bits, b_bits, out_bits):
+        """out = a | b (make_or_circuit)."""
+        from . import mux_circuits as M
+
+        a, b = _operands("or_", a_bits, b_bits)
+        w = len(a)
+        out = _results("or_", out_bits, w)
+        return self._mux_instruction(("or", w), lambda: M.make_or_circuit(w), [a, b], out, interleave=True)
+
+    def shift(self, a_bits, amount_bits, out_bits, right: bool, mode: str = "logical"):
+        """out = a shifted by the encrypted amount (bitshift.rs:49-157).  mode "logical" clears the bits shifted in (an
+        amount >= w gives 0), "rotation" wraps (power-of-two w; the amount counts mod w), "arithmetic" fills a right
+        shift with the sign bit.  w <= 16 (SHIFT_MAX_WIDTH); the amount needs at least ceil(log2(w)) bits (at least 1)."""
+        from . import mux_circuits as M
+
+        a, amt = _operands("shift", a_bits, amount_bits, equal=False)
+        w, k, right = len(a), len(amt), bool(right)
+        out = _results("shift", out_bits, w)
+        if w > SHIFT_MAX_WIDTH:
+            raise ValueError(f"InstructionCache.shift: widths up to {SHIFT_MAX_WIDTH} bits, got {w} "
+                             "(a constant amount has no such limit: shift_const)")
+        if mode not in _SHIFT_MODES:
+            raise ValueError(f"InstructionCache.shift: mode {mode!r}, expected one of {_SHIFT_MODES}")
+        if mode == "arithmetic" and not right:
+            raise ValueError("InstructionCache.shift: an arithmetic shift is a right shift")
+        if mode == "rotation" and w & (w - 1):
+            raise ValueError(f"InstructionCache.shift: rotation needs a power-of-two width, got {w}")
+        if k < max(1, (w - 1).bit_length()):
+            raise ValueError(f"InstructionCache.shift: a {w}-bit value needs at least {max(1, (w - 1).bit_length())} amount bits, got {k}")
+        # the barrel shifter takes value and amount bits most significant first, and gives its results so
+        return self._mux_instruction(("shift", w, k, right, mode), lambda: M.bitshift(w, k, right, mode),
+                                     [a[::-1], amt[::-1]], out[::-1], interleave=False)
+
+    def multiply_signed(self, a_bits, b_bits, out_bits):
+        """out = low w bits of the two's-complement product a * b, w <= 16 (circuits/mul.rs:19-73: |a|, |b|, one
+        multiplier block, conditional negate; three bootstrap levels)."""
+        from . import mux_circuits as M
+
+        a, b = _operands("multiply_signed", a_bits, b_bits)
+        w = len(a)
+        if w > M.CIRCUIT_CUTOFF:
+            raise ValueError(f"InstructionCache.multiply_signed: widths up to {M.CIRCUIT_CUTOFF} bits, got {w}")
+        out = _results("multiply_signed", out_bits, w)
+        return self._run(("mul_signed", w), lambda c, ins: M.append_int_multiply(c, *_fronts(c, ins))[0], [a, b], out)
+
+    # ---- no MUX circuit ----
+    def select(self, cond, a_bits, b_bits, out_bits):
+        """out = cond ? b : a, for one encrypted bit `cond`: cond is bootstrapped to a selector, then one CMux per bit."""
+        a, b = _operands("select", a_bits, b_bits)
+        out = _results("select", out_bits, len(a))
+
+        def body(c, ins):
+            (sel,), a_, b_ = ins
+            sel = _refresh(c, sel)
+            return [c.add("CMux", sel, lo, hi) for lo, hi in zip(a_, b_)]
+
+        return self._run(("select", len(a)), body, [[cond], a, b], out)
+
+    def xor(self, a_bits, b_bits, out_bits):
+        """out = a ^ b: one GlweAdd per bit (KeylessEvaluation::xor), no bootstrap."""
+        a, b = _operands("xor", a_bits, b_bits)
+        out = _results("xor", out_bits, len(a))
+        return self._run(("xor", len(a)), lambda c, ins: [c.add("GlweAdd", x, y) for x, y in zip(*ins)], [a, b], out)
+
+    def not_(self, a_bits, out_bits):
+        """out = ~a: one Not per bit (KeylessEvaluation::not), no bootstrap."""
+        (a,) = _operands("not_", a_bits)
+        out = _results("not_", out_bits, len(a))
+        return self._run(("not", len(a)), lambda c, ins: [c.add("Not", x) for x in ins[0]], [a], out)
+
+    def shift_const(self, a_bits, k: int, out_bits, right: bool, mode: str = "logical"):
+        """out = a shifted by the plaintext amount k, 0 <= k <= w: pure rewiring, no bootstrap.  Vacated bits are an
+        encrypted-constant zero ("logical"), the sign bit ("arithmetic", right shifts only), or the bits shifted out
+        ("rotation")."""
+        (a,) = _operands("shift_const", a_bits)
+        w, k, right = len(a), int(k), bool(right)
+        out = _results("shift_const", out_bits, w)
+        if mode not in _SHIFT_MODES:
+            raise ValueError(f"InstructionCache.shift_const: mode {mode!r}, expected one of {_SHIFT_MODES}")
+        if mode == "arithmetic" and not right:
+            raise ValueError("InstructionCache.shift_const: an arithmetic shift is a right shift")
+        if not 0 <= k <= w:
+            raise ValueError(f"InstructionCache.shift_const: amount {k} outside 0 .. {w}")
+
+        def body(c, ins):
+            x, zero = ins[0], None
+            res = []
+            for i in range(w):
+                src = i + k if right else i - k
+                if mode == "rotation":
+                    res.append(x[src % w])
+                elif 0 <= src < w:
+                    res.append(x[src])
+                elif mode == "arithmetic":
+                    res.append(x[w - 1])
+                else:
+                    zero = zero if zero is not None else c.add("ZeroGlwe1")
+                    res.append(zero)
+            return res
+
+        return self._run(("shift_const", w, k, right, mode), body, [a], out)
+
+    def zext(self, a_bits, out_bits):
+        """out = a zero-extended to len(out_bits) >= w bits: copies and encrypted-constant zeros, no bootstrap."""
+        return self._extend("zext", a_bits, out_bits)
+
+    def sext(self, a_bits, out_bits):
+        """out = a sign-extended to len(out_bits) >= w bits: copies of the bits and of the sign bit, no bootstrap."""
+        return self._extend("sext", a_bits, out_bits)
+
+    def trunc(self, a_bits, out_bits):
+        """out = the low len(out_bits) <= w bits of a: copies, no bootstrap."""
+        return self._extend("trunc", a_bits, out_bits)
+
+    def _extend(self, name, a_bits, out_bits):
+        (a,) = _operands(name, a_bits)
+        w = len(a)
+        out = list(out_bits)
+        if not (1 <= len(out) <= w if name == "trunc" else len(out) >= w):
+            raise ValueError(f"InstructionCache.{name}: {len(out)} result bits from a {w}-bit operand")
+
+        def body(c, ins):
+            x = ins[0]
+            fill = x[w - 1] if name == "sext" else c.add("ZeroGlwe1") if len(out) > w else None
+            return [x[i] if i < w else fill for i in range(len(out))]
+
+        return self._run((name, w, len(out)), body, [a], out)
 
 
 def _keep_outputs(mux, n_outputs: int):
