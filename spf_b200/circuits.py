@@ -8,6 +8,8 @@
   constructions (mux_circuits/src/*.rs), generated natively."""
 from __future__ import annotations
 
+import weakref
+
 import numpy as np
 
 from . import FheCircuit
@@ -71,12 +73,19 @@ def _front(c: FheCircuit, ct):
     return c.add("CircuitBootstrap", x)
 
 
+_SELECTORS: "weakref.WeakKeyDictionary[FheCircuit, dict[int, int]]" = weakref.WeakKeyDictionary()
+
+
 def _refresh(c: FheCircuit, glwe_node: int) -> int:
     """Turn a computed GLWE bit back into a selector: SampleExtract(0) -> KeyswitchL1toL0 ->
-    CircuitBootstrap, the hop between two dependency levels of a Parasol program."""
-    x = c.add("SampleExtract", glwe_node, arg=0)
-    x = c.add("KeyswitchL1toL0", x)
-    return c.add("CircuitBootstrap", x)
+    CircuitBootstrap, the hop between two dependency levels of a Parasol program.  Memoised per circuit: a GLWE node
+    read by several MUX circuits (a register bit read by several instructions of a Block) is bootstrapped once."""
+    memo = _SELECTORS.setdefault(c, {})
+    if glwe_node not in memo:
+        x = c.add("SampleExtract", glwe_node, arg=0)
+        x = c.add("KeyswitchL1toL0", x)
+        memo[glwe_node] = c.add("CircuitBootstrap", x)
+    return memo[glwe_node]
 
 
 def _adder_nodes(c: FheCircuit, sa: list[int], sb: list[int]) -> list[int]:
@@ -157,20 +166,37 @@ def multiply_then_greater_than(a_bits, b_bits, c_bits, out_prod, out_gt, program
     return M.prune(c, keep)[0]
 
 
-def _instruction_graph(operands, out_bits, body) -> tuple[FheCircuit, list[int], list[int]]:
-    """One instruction as a graph: an InputGlwe1 per operand bit, `body(c, input_nodes)` -> the GLWE node behind every
-    result bit, an OutputGlwe1 per result bit, pruned to what the results read (fhe_circuit.rs:516-555).  operands: lists
-    of bit ciphertexts; input_nodes has the same shape.  Returns (graph, operand-bit nodes, result-bit nodes), both in
-    the flattened order of operands / out_bits; an operand bit no result reads has node -1."""
+def _program_graph(inputs, program, outputs) -> tuple[FheCircuit, list[int], list[int]]:
+    """A straight-line program as one graph: an InputGlwe1 per input bit, then for every instruction
+    `body(c, operand_nodes)` -> the GLWE node behind each of its result bits, an OutputGlwe1 per output bit, pruned to
+    what the outputs read (fhe_circuit.rs:516-555).  Bits are any hashable names.  inputs / outputs: (bit, buffer)
+    pairs; program: (body, operand bits as a list of lists, result bits).  Returns (graph, input-bit nodes, output-bit
+    nodes) in the order of inputs / outputs; an input bit no output reads has node -1."""
     from . import mux_circuits as M
 
     c = FheCircuit()
-    ins = [[c.add("InputGlwe1", io=x) for x in op] for op in operands]
-    res = body(c, ins)
-    assert len(res) == len(out_bits)
-    outs = [c.add("OutputGlwe1", n, io=buf) for n, buf in zip(res, out_bits)]
+    ins = [c.add("InputGlwe1", io=buf) for _, buf in inputs]
+    node = {bit: n for (bit, _), n in zip(inputs, ins)}
+    for body, operands, results in program:
+        res = body(c, [[node[b] for b in op] for op in operands])
+        assert len(res) == len(results)
+        node.update(zip(results, res))
+    outs = [c.add("OutputGlwe1", node[bit], io=buf) for bit, buf in outputs]
     c, ren = M.prune(c, outs)
-    return c, [ren.get(n, -1) for op in ins for n in op], [ren[n] for n in outs]
+    return c, [ren.get(n, -1) for n in ins], [ren[n] for n in outs]
+
+
+def _instruction_graph(operands, out_bits, body) -> tuple[FheCircuit, list[int], list[int]]:
+    """One instruction as a graph: every operand bit is an input of its own (so the same buffer passed twice is read
+    through two InputGlwe1 nodes) and every result bit an output.  operands: lists of bit ciphertexts.  Returns (graph,
+    operand-bit nodes, result-bit nodes), both in the flattened order of operands / out_bits."""
+    names, k = [], 0
+    for op in operands:
+        names.append(list(range(k, k + len(op))))
+        k += len(op)
+    results = [("result", i) for i in range(len(out_bits))]
+    return _program_graph(list(zip(range(k), [x for op in operands for x in op])), [(body, names, results)],
+                          list(zip(results, out_bits)))
 
 
 def _fronts(c: FheCircuit, inputs: list[list[int]]) -> list[list[int]]:
@@ -201,39 +227,11 @@ def _results(name: str, out_bits, *allowed: int) -> list:
     return out
 
 
-class InstructionCache:
-    """Graph-generation cache (SURVEY.md 8(f).3): one compiled, levelised, device-resident graph per
-    (instruction, widths, flags), re-bound to the operands of each invocation with CompiledGraph.set_io
-    instead of rebuilding the MUX circuit and re-levelising it per dispatch as
-    FheCircuit::insert_mux_circuit_and_connect_inputs (fhe_circuit.rs:473-494) does.
-
-    Operands and results are lists of L1 GLWE bit ciphertexts, least significant bit first: host arrays, or
-    BoxCiphertext handles on a BoxEvaluation.  Every method checks its widths before anything is built (ValueError),
-    runs blocking and returns the graph it ran."""
-
-    def __init__(self, evaluation):
-        from . import BoxEvaluation, BoxGraph, CompiledGraph
-
-        self._compile = BoxGraph if isinstance(evaluation, BoxEvaluation) else CompiledGraph
-        self._ev, self._cache = evaluation, {}
-        self.hits = self.misses = 0
-
-    def _run(self, key, body, operands, out_bits):
-        """Build (on a miss) _instruction_graph(operands, out_bits, body), bind it to these operands and results and run
-        it.  Binding goes through the operand-bit / result-bit node maps recorded at build time: pruning may have removed
-        operand bits, and a rewired result may read an operand bit directly."""
-        if key not in self._cache:
-            self.misses += 1
-            c, ins, outs = _instruction_graph(operands, out_bits, body)
-            self._cache[key] = (self._compile(self._ev, c), ins, outs)
-        else:
-            self.hits += 1
-        g, ins, outs = self._cache[key]
-        for node, buf in zip(ins + outs, [x for op in operands for x in op] + list(out_bits)):
-            if node >= 0:
-                g.set_io(node, buf)
-        g.run()
-        return g
+class _Instructions:
+    """The Parasol integer instructions, shared by InstructionCache (one graph per call) and Block (one graph per
+    block).  Each method checks its arguments (ValueError), then hands `self._run(key, body, operands, out_bits)` the
+    cache key of its shape and flags, its body -- body(c, operand_nodes) -> the GLWE node behind every result bit -- and
+    its operand and result bits."""
 
     def _mux_instruction(self, key, mux_builder, operands, out_bits, interleave):
         """One ISA instruction = front end (fhe_circuit.rs:473-494) + one BDD-derived MUX circuit whose first
@@ -457,6 +455,161 @@ class InstructionCache:
             return [x[i] if i < w else fill for i in range(len(out))]
 
         return self._run((name, w, len(out)), body, [a], out)
+
+
+class InstructionCache(_Instructions):
+    """Graph-generation cache (SURVEY.md 8(f).3): one compiled, levelised, device-resident graph per
+    (instruction, widths, flags), re-bound to the operands of each invocation with CompiledGraph.set_io
+    instead of rebuilding the MUX circuit and re-levelising it per dispatch as
+    FheCircuit::insert_mux_circuit_and_connect_inputs (fhe_circuit.rs:473-494) does.
+
+    Operands and results are lists of L1 GLWE bit ciphertexts, least significant bit first: host arrays, or
+    BoxCiphertext handles on a BoxEvaluation.  Every method checks its widths before anything is built (ValueError),
+    runs blocking and returns the graph it ran.  block() records several instructions and runs them as one graph."""
+
+    def __init__(self, evaluation):
+        from . import BoxEvaluation, BoxGraph, CompiledGraph
+
+        self._compile = BoxGraph if isinstance(evaluation, BoxEvaluation) else CompiledGraph
+        self._ev, self._cache = evaluation, {}
+        self.hits = self.misses = 0
+
+    def block(self) -> "Block":
+        """An empty Block whose graphs are cached here."""
+        return Block(self)
+
+    def _run(self, key, body, operands, out_bits):
+        return self._cached(key, lambda: _instruction_graph(operands, out_bits, body),
+                            [x for op in operands for x in op] + list(out_bits))
+
+    def _cached(self, key, build, bufs):
+        """Build (on a miss) the graph of `key` with build() -> (graph, input-bit nodes, output-bit nodes), bind it to
+        `bufs` (input bits then output bits) and run it.  Binding goes through the node maps recorded at build time:
+        pruning may have removed input bits, and a rewired output may read an input bit directly."""
+        if key not in self._cache:
+            self.misses += 1
+            c, ins, outs = build()
+            self._cache[key] = (self._compile(self._ev, c), ins, outs)
+        else:
+            self.hits += 1
+        g, ins, outs = self._cache[key]
+        for node, buf in zip(ins + outs, bufs):
+            if node >= 0:
+                g.set_io(node, buf)
+        g.run()
+        return g
+
+
+class Bit:
+    """One bit of a Block register (`reg[i]`): pass it where an instruction takes `out_bit` or `cond`."""
+
+    __slots__ = ("block", "reg", "index")
+
+    def __init__(self, block: "Block", reg: int, index: int):
+        self.block, self.reg, self.index = block, reg, index
+
+    def __repr__(self) -> str:
+        return f"r{self.reg}[{self.index}]"
+
+
+class Reg:
+    """A Block register: an ordered list of bits, least significant first.  Slicing gives a view over the same bits (an
+    operand or result of an instruction, not a key of Block.run), indexing gives a Bit."""
+
+    __slots__ = ("bits", "index")
+
+    def __init__(self, bits, index: int | None = None):
+        self.bits, self.index = tuple(bits), index   # index: creation order; None for a view
+
+    def __len__(self) -> int:
+        return len(self.bits)
+
+    def __iter__(self):
+        return iter(self.bits)
+
+    def __getitem__(self, i):
+        return Reg(self.bits[i]) if isinstance(i, slice) else self.bits[i]
+
+    def __repr__(self) -> str:
+        return f"Reg({list(self.bits)})"
+
+
+class Block(_Instructions):
+    """A straight-line sequence of instructions over registers, run as ONE graph (InstructionCache.block()).
+
+    The instruction methods are InstructionCache's -- same names, argument order, flags and checks -- with registers or
+    register views in place of buffer lists; they record the instruction and return nothing.  Every bit is written at
+    most once, and an instruction may not write a bit that it or an earlier instruction reads: program order is the
+    only order.  run() lowers the whole block into one graph, so the planner batches the bootstraps of independent
+    instructions into one launch per stage, intermediates stay in device memory, and a bit read by several
+    instructions is bootstrapped once.  A result read by a later instruction goes through the same SampleExtract ->
+    KeyswitchL1toL0 -> CircuitBootstrap refresh it would after a round trip through the host."""
+
+    def __init__(self, cache: InstructionCache):
+        self._icache, self._regs, self._program = cache, [], []
+        self._read, self._written = set(), set()
+
+    def reg(self, width: int) -> Reg:
+        """A new register of `width` >= 1 bits."""
+        width = int(width)
+        if width < 1:
+            raise ValueError(f"Block.reg: width {width}, expected at least 1")
+        r = len(self._regs)
+        self._regs.append(Reg([Bit(self, r, i) for i in range(width)], index=r))
+        return self._regs[-1]
+
+    def _run(self, key, body, operands, out_bits):
+        reads, out = [b for op in operands for b in op], list(out_bits)
+        for b in reads + out:
+            if not isinstance(b, Bit) or b.block is not self:
+                raise ValueError(f"Block {key[0]}: {b!r} is not a bit of this block's registers")
+        if len(set(out)) < len(out) or self._written.intersection(out):
+            raise ValueError(f"Block {key[0]}: writes a bit a second time")
+        if self._read.intersection(out) or set(reads).intersection(out):
+            raise ValueError(f"Block {key[0]}: writes a bit that this or an earlier instruction reads")
+        self._program.append((key, body, operands, out))
+        self._read.update(reads)
+        self._written.update(out)
+
+    def _binding(self, name: str, regs) -> list:
+        """{Reg: buffers} -> [(register, buffer list)] in register creation order."""
+        bound = []
+        for r, bufs in dict(regs).items():
+            if not isinstance(r, Reg) or r.index is None or r.bits[0].block is not self:
+                raise ValueError(f"Block.run: {name} keys must be registers of this block (from reg(), not views)")
+            bufs = list(bufs)
+            if len(bufs) != len(r):
+                raise ValueError(f"Block.run: {name} register r{r.index} has {len(r)} bits, bound to {len(bufs)} buffers")
+            bound.append((r, bufs))
+        return sorted(bound, key=lambda rb: rb[0].index)
+
+    def run(self, inputs, outputs):
+        """Run the block: inputs / outputs are {register: list of L1 GLWE bit ciphertexts} -- host arrays, or
+        BoxCiphertext handles on a BoxEvaluation.  Every register read and never written must be an input, every output
+        register must be written in full; written registers that are not outputs are intermediates.  The graph is
+        built on the cache's first sight of this block's structure and rebound afterwards; returns it."""
+        if not self._program:
+            raise ValueError("Block.run: empty block")
+        ins, outs = self._binding("inputs", inputs), self._binding("outputs", outputs)
+        in_regs = {r.index for r, _ in ins}
+        for r, _ in ins:
+            if self._written.intersection(r):
+                raise ValueError(f"Block.run: input register r{r.index} is written by an instruction")
+        unbound = sorted({b.reg for b in self._read - self._written} - in_regs)
+        if unbound:
+            raise ValueError(f"Block.run: registers {['r%d' % r for r in unbound]} are read and never written: bind them in inputs")
+        for r, _ in outs:
+            if not self._written.issuperset(r):
+                raise ValueError(f"Block.run: output register r{r.index} is not written in full")
+        name = lambda b: (b.reg, b.index)
+        key = ("block",
+               tuple((k, tuple(tuple(map(name, op)) for op in operands), tuple(map(name, res))) for k, _, operands, res in self._program),
+               tuple(len(r) for r in self._regs), tuple(r.index for r, _ in ins), tuple(r.index for r, _ in outs))
+        in_bits = [(b, buf) for r, bufs in ins for b, buf in zip(r, bufs)]
+        out_bits = [(b, buf) for r, bufs in outs for b, buf in zip(r, bufs)]
+        program = [(body, operands, res) for _, body, operands, res in self._program]
+        return self._icache._cached(key, lambda: _program_graph(in_bits, program, out_bits),
+                                    [buf for _, buf in in_bits + out_bits])
 
 
 def _keep_outputs(mux, n_outputs: int):

@@ -206,6 +206,22 @@ int create_common(const spf_params* params, const double* bsk, size_t bsk_len, c
       default: break;
     }
   }
+  // Load the small kernels of a graph run now as well (the ones above are loaded by their attribute calls).  Under lazy
+  // module loading, the CUDA 12 default, a kernel's first launch may wait for the device to drain.  In a box run the
+  // host enqueues rank after rank while earlier ranks' streams spin in peer barriers; a first launch there would wait
+  // behind a barrier whose other side is not enqueued yet, and the run would stall until the barrier times out.
+  {
+    cudaFuncAttributes fa;
+    CUB(cudaFuncGetAttributes(&fa, peer_barrier_kernel));
+    CUB(cudaFuncGetAttributes(&fa, peer_bcast_kernel));
+    CUB(cudaFuncGetAttributes(&fa, box_copy_kernel<kBoxCopySmall>));
+    CUB(cudaFuncGetAttributes(&fa, box_copy_kernel<kBoxCopyLarge>));
+    CUB(cudaFuncGetAttributes(&fa, gather_outputs_kernel));
+    CUB(cudaFuncGetAttributes(&fa, sample_extract_kernel));
+    CUB(cudaFuncGetAttributes(&fa, glwe_elementwise_kernel));
+    CUB(cudaFuncGetAttributes(&fa, ks_tc_states_kernel));
+    CUB(cudaFuncGetAttributes(&fa, fft_scale_kernel));
+  }
   // constant tables
   {
     std::vector<C2> T1(kT1Elems), T2(kT2Elems);
