@@ -243,7 +243,7 @@ typedef void (*spf_completion_fn)(void *user, int status, const char *message);
 int spf_b200_graph_spawn(spf_b200_graph *graph, spf_b200_graph *const *after, size_t n_after,
                          spf_completion_fn on_complete, void *user);
 int spf_b200_graph_wait(spf_b200_graph *graph);
-const char *spf_b200_graph_status_message(const spf_b200_graph *graph); /* error message of the last spawned run, "" if none */
+const char *spf_b200_graph_status_message(const spf_b200_graph *graph); /* error of the last run (spawned or blocking), "" if none */
 int spf_b200_set_max_in_flight(spf_b200_ctx *ctx, int n);
 /* Page-locked host memory for ciphertext buffers.  Input and Output node buffers that are already page-locked (this
  * allocator, cudaHostAlloc, a cudaHostRegister done by the caller) are used as they are; any other buffer is registered

@@ -792,6 +792,30 @@ class CircuitProcessor:
         return g
 
 
+def _spawn(graph, spawn_fn, after, on_complete) -> None:
+    """One asynchronous run of a CompiledGraph or BoxGraph through its spawn entry point: `after` and `on_complete` as
+    in CompiledGraph.spawn."""
+    deps = [d for d in after if d is not None]
+    arr = (_vp * max(len(deps), 1))(*[d._h for d in deps])
+
+    def _done(user, status, message):
+        try:
+            if on_complete is not None:
+                on_complete(None if status == 0 else SpfError(int(status), (message or b"").decode()))
+        except Exception:  # never let an exception cross the C ABI
+            pass
+
+    graph._spawn_cb = COMPLETION_FN(_done)  # kept alive until the next spawn / close
+    graph.ev._check(spawn_fn(graph._h, arr, len(deps), C.cast(graph._spawn_cb, _vp), None))
+
+
+def _wait(graph, wait_fn, message_fn) -> None:
+    """Blocks until the graph's last run is over; raises its error, if any."""
+    rc = wait_fn(graph._h)
+    if rc:
+        raise SpfError(int(rc), (message_fn(graph._h) or b"").decode() or "the graph's last run failed")
+
+
 class CompiledGraph:
     """A levelised graph resident on one GPU.  With world > 1 the graph is laid out for a sharded
     run (spf_b200_graph_build_sharded): every CircuitBootstrap level is split into `world` chunks,
@@ -854,24 +878,11 @@ class CompiledGraph:
         the first SpfError of the run; it must not call into spf_b200 or CUDA."""
         if self.world != 1:
             raise SpfError(-1, "sharded graphs are not spawned")
-        deps = [d for d in after if d is not None]
-        arr = (_vp * max(len(deps), 1))(*[d._h for d in deps])
-
-        def _done(user, status, message):
-            try:
-                if on_complete is not None:
-                    on_complete(None if status == 0 else SpfError(int(status), (message or b"").decode()))
-            except Exception:  # never let an exception cross the C ABI
-                pass
-
-        self._spawn_cb = COMPLETION_FN(_done)  # kept alive until the next spawn / close
-        self.ev._check(lib().spf_b200_graph_spawn(self._h, arr, len(deps), C.cast(self._spawn_cb, _vp), None))
+        _spawn(self, lib().spf_b200_graph_spawn, after, on_complete)
 
     def wait(self) -> None:
         """Block until the last run (spawned or blocking) is over; raises its error, if any."""
-        rc = lib().spf_b200_graph_wait(self._h)
-        if rc:
-            raise SpfError(int(rc), (lib().spf_b200_graph_status_message(self._h) or b"").decode() or "the graph's last run failed")
+        _wait(self, lib().spf_b200_graph_wait, lib().spf_b200_graph_status_message)
 
     # ---- peer-memory exchange (no exchange callable): every rank maps every other rank's arena ----
     @property
@@ -1122,23 +1133,10 @@ class BoxGraph:
     def spawn(self, after=(), on_complete=None) -> None:
         """One asynchronous run over all ranks; on_complete(error) fires once, after every rank has retired, from a CUDA
         callback thread (it must not call into spf_b200 or CUDA).  `after`: BoxGraphs of the same box."""
-        deps = [d for d in after if d is not None]
-        arr = (_vp * max(len(deps), 1))(*[d._h for d in deps])
-
-        def _done(user, status, message):
-            try:
-                if on_complete is not None:
-                    on_complete(None if status == 0 else SpfError(int(status), (message or b"").decode()))
-            except Exception:  # never let an exception cross the C ABI
-                pass
-
-        self._spawn_cb = COMPLETION_FN(_done)
-        self.ev._check(lib().spf_b200_box_graph_spawn(self._h, arr, len(deps), C.cast(self._spawn_cb, _vp), None))
+        _spawn(self, lib().spf_b200_box_graph_spawn, after, on_complete)
 
     def wait(self) -> None:
-        rc = lib().spf_b200_box_graph_wait(self._h)
-        if rc:
-            raise SpfError(int(rc), (lib().spf_b200_box_graph_status_message(self._h) or b"").decode() or "the graph's last run failed")
+        _wait(self, lib().spf_b200_box_graph_wait, lib().spf_b200_box_graph_status_message)
 
     @property
     def levels(self) -> int:

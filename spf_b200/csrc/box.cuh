@@ -18,10 +18,7 @@ struct spf_b200_box {
   double replication_ms = 0;
   // lifetime: box graphs keep the box alive (its flow control and error slot), as graphs keep their context
   std::atomic<int> refs{1};
-  // flow control of spawned box runs (spf_b200_box_graph_spawn), per box
-  std::mutex fc_mu;
-  std::condition_variable fc_cv;
-  int in_flight = 0, max_in_flight = 4;
+  FlowControl fc;  // of the spawned runs of this box's graphs
   // one worker thread per rank for the host-pointer ops: created with the box, joined by spf_b200_box_destroy
   std::vector<std::thread> workers;
   std::mutex w_mu;
@@ -50,10 +47,7 @@ struct spf_b200_box_graph {
   std::vector<spf_b200_box_ciphertext*> bound;  // per node: the box ciphertext handle bound to it (a reference), or NULL
   std::vector<void*> pinned;       // host io buffers page-locked (portable: every device DMAs them) by this box graph
   int* h_err = nullptr;            // page-locked copy of every member's barrier error word, read by the completion
-  std::atomic<int> status{0};
-  std::string status_msg;
-  std::atomic<bool> poisoned{false};
-  uint64_t launches_per_run = 0;
+  RunState run;
 };
 
 namespace {
@@ -218,14 +212,6 @@ int enqueue_handle_copies(spf_b200_box_graph* bg, int i, bool outputs) {
   return launch_box_copy(g->ctx, items, g->stream);
 }
 
-// Whether some handle-bound output is written by one member into the replicas of the others (with two or more
-// members; the replicas of non-members written by member 0 are not read by this graph).
-bool has_owned_handle_outputs(const spf_b200_graph* g) {
-  for (int id : g->outputs)
-    if (g->io_kind[id] == 3 && spf_b200_graph_output_rank(g, id) >= 0) return true;
-  return false;
-}
-
 int box_create_impl(const spf_params* params, const double* bsk, size_t bsk_len, const uint64_t* ksk, size_t ksk_len,
                     const double* ssk, size_t ssk_len, const double* ak, size_t ak_len, const int* devices, int n,
                     spf_b200_box** out) {
@@ -354,118 +340,9 @@ void settle_all_io(spf_b200_graph* g) {
   for (size_t v = 0; v < g->nodes.size(); v++) settle_io(g, v);
 }
 
-// Everything of a run that could wait on the device, done before any rank enqueues: the staging slab of pageable io
-// buffers (its growth synchronises the stream) and the keyswitch digit-state scratch at the size of the largest
-// keyswitch group (growing it frees the old buffer, which synchronises the device).  Afterwards the enqueue_* parts only
-// enqueue: copies from page-locked memory, kernel launches, event records.
-int prepare_run(spf_b200_graph* g, int rank) {
-  spf_b200_ctx* ctx = g->ctx;
-  CU(cudaSetDevice(ctx->device));
-  for (size_t id = 0; id < g->nodes.size(); id++) {
-    if (g->io_kind[id] != 1) continue;
-    char* dummy = nullptr;
-    if (int rc = stage_slot(g, (int)id, 0, &dummy)) return rc;
-  }
-  size_t ks = 0;
-  for (const Group& G : g->groups)
-    if (G.op == SPF_OP_KEYSWITCH_L1_TO_L0) ks = std::max(ks, std::max(G.all_cnt, G.r_cnt[rank]));
-  if (ks) if (int rc = ensure(ctx, g->ks_states, ks * (size_t)ctx->p.glwe_k * ctx->p.glwe_n * 2)) return rc;
-  return 0;
-}
-
-struct BoxSpawn {
-  spf_b200_box_graph* bg;
-  spf_completion_fn cb;
-  void* user;
-  int status;
-  std::string msg;
-  std::atomic<int> remaining;
-  std::atomic<int> barrier_failed{0};
-};
-struct BoxRankDone {
-  BoxSpawn* rec;
-  int rank;
-};
-
-// Host function behind rank r's share of a spawned box run; the last rank to retire delivers the completion.
-void CUDART_CB box_rank_done(void* arg) {
-  BoxRankDone* d = static_cast<BoxRankDone*>(arg);
-  BoxSpawn* rec = d->rec;
-  spf_b200_box_graph* bg = rec->bg;
-  const int r = d->rank;
-  delete d;
-  const bool peer = bg->g.size() > 1;
-  if (peer && bg->h_err[r]) rec->barrier_failed.store(1);
-  if (rec->status == 0 && !(peer && bg->h_err[r])) copy_out_staged(bg->g[r], r);
-  if (rec->remaining.fetch_sub(1) != 1) return;
-  if (rec->status == 0 && rec->barrier_failed.load()) {
-    rec->status = SPF_E_GRAPH;
-    rec->msg = "peer barrier timed out: a rank of the box run did not arrive";
-  }
-  if (rec->status && peer) bg->poisoned.store(true);
-  if (rec->status) {
-    bg->status_msg = rec->msg;
-    bg->status.store(rec->status);
-  }
-  spf_b200_box* b = bg->box;
-  {
-    std::lock_guard<std::mutex> lk(b->fc_mu);
-    b->in_flight--;
-  }
-  b->fc_cv.notify_all();
-  if (rec->cb) rec->cb(rec->user, rec->status, rec->status ? rec->msg.c_str() : nullptr);
-  delete rec;
-}
-
-// Enqueues one run on every member from the calling thread, level-interleaved: the inputs of every member, then group k
-// of every member for k = 0, 1, ..., then the outputs of every member.  So when the host has to wait for a member's
-// stream (its launch queue is full), every other member's work up to the same level -- and so to the same peer barrier
-// -- is enqueued already, and the wait ends.  Returns the first error; members after a failed one are not enqueued
-// further.  Box ciphertext handles: each member reads its own replica right after its other inputs.  When an owner
-// writes the replicas of other members at the end, a barrier after the inputs first makes sure that every member has
-// read its replica (a graph may read and write the same handle, and need not have a bootstrap level, whose barrier
-// would do); the start-of-run barrier keeps these writes ahead of the next run's reads.
-int box_enqueue(spf_b200_box_graph* bg) {
-  spf_b200_box* b = bg->box;
-  const int n = (int)bg->g.size();
-  auto rank_fail = [&](int r, int rc) { return box_fail(b, rc, "rank " + std::to_string(bg->rank[r]) + ": " + bg->g[r]->ctx->err); };
-  for (int r = 0; r < n; r++)
-    if (int rc = prepare_run(bg->g[r], r)) return rank_fail(r, rc);
-  for (int r = 0; r < n; r++) {
-    BCU(b, cudaSetDevice(bg->g[r]->ctx->device));
-    if (int rc = enqueue_inputs(bg->g[r], n > 1, bg->g[r]->stream)) return rank_fail(r, rc);
-    if (int rc = enqueue_handle_copies(bg, r, false)) return rank_fail(r, rc);
-  }
-  if (n > 1 && has_owned_handle_outputs(bg->g[0]))
-    for (int r = 0; r < n; r++) {
-      BCU(b, cudaSetDevice(bg->g[r]->ctx->device));
-      if (int rc = peer_barrier(bg->g[r], bg->g[r]->stream)) return rank_fail(r, rc);
-    }
-  for (size_t k = 0; k < bg->g[0]->groups.size(); k++)
-    for (int r = 0; r < n; r++) {
-      spf_b200_graph* g = bg->g[r];
-      BCU(b, cudaSetDevice(g->ctx->device));
-      if (int rc = enqueue_group(g, g->groups[k], r, n, nullptr, nullptr, g->stream, nullptr)) return rank_fail(r, rc);
-    }
-  for (int r = 0; r < n; r++) {
-    BCU(b, cudaSetDevice(bg->g[r]->ctx->device));
-    if (int rc = enqueue_outputs(bg->g[r], r, bg->g[r]->stream)) return rank_fail(r, rc);
-    if (int rc = enqueue_handle_copies(bg, r, true)) return rank_fail(r, rc);
-  }
-  return 0;
-}
-
-bool box_graph_poisoned(const spf_b200_box_graph* bg) {
-  if (bg->poisoned.load()) return true;
-  for (const spf_b200_graph* g : bg->g)
-    if (g->poisoned) return true;
-  return false;
-}
-
-uint64_t box_launches(const spf_b200_box* b) {
-  uint64_t s = 0;
-  for (const spf_b200_ctx* c : b->ctx) s += c->launches.load();
-  return s;
+// A run of a box graph: member i runs shard i on box rank rank[i]; errors go to the box's slot, prefixed with that rank.
+Run box_run(spf_b200_box_graph* bg) {
+  return Run{bg->g, 0, nullptr, nullptr, bg, &bg->rank, bg->h_err, &bg->run, &bg->box->fc, &bg->box->err};
 }
 
 }  // namespace
@@ -590,11 +467,7 @@ int spf_b200_box_cmux(spf_b200_box* b, uint64_t* glwe_out, const double* sel_ggs
 int spf_b200_box_set_max_in_flight(spf_b200_box* b, int n) {
   if (!b) return SPF_E_INVALID;
   if (n < 1) return box_fail(b, SPF_E_INVALID, "max_in_flight must be at least 1");
-  {
-    std::lock_guard<std::mutex> lk(b->fc_mu);
-    b->max_in_flight = n;
-  }
-  b->fc_cv.notify_all();
+  b->fc.set(n);
   return 0;
 }
 
@@ -700,131 +573,41 @@ int spf_b200_box_graph_ranks(const spf_b200_box_graph* bg, int* ranks_out) {
   return (int)bg->rank.size();
 }
 
-int spf_b200_box_graph_run(spf_b200_box_graph* bg) {
-  if (!bg) return SPF_E_INVALID;
-  spf_b200_box* b = bg->box;
-  if (box_graph_poisoned(bg))
-    return box_fail(b, SPF_E_GRAPH, "an earlier run of this box graph failed: the ranks' barrier epochs disagree, rebuild the graph");
-  const int n = (int)bg->g.size();
-  // a spawned run still in flight finishes first (the staging slabs and the barrier epochs are per graph)
-  for (spf_b200_graph* g : bg->g) {
-    BCU(b, cudaSetDevice(g->ctx->device));
-    BCU(b, cudaEventSynchronize(g->done));
-  }
-  const uint64_t l0 = box_launches(b);
-  int rc = box_enqueue(bg);
-  const std::string msg = rc ? b->err : std::string();
-  cudaError_t se = cudaSuccess;
-  for (spf_b200_graph* g : bg->g) {  // also on failure: nothing of this run is in flight afterwards
-    cudaSetDevice(g->ctx->device);
-    const cudaError_t e = cudaStreamSynchronize(g->stream);
-    if (se == cudaSuccess) se = e;
-    cudaEventRecord(g->done, g->stream);
-  }
-  if (rc == 0 && se != cudaSuccess) rc = box_fail(b, SPF_E_CUDA, std::string("box graph run: ") + cudaGetErrorString(se));
-  else if (rc) b->err = msg;
-  if (rc == 0 && n > 1) {
-    for (int r = 0; r < n && rc == 0; r++) {
-      int err = 0;
-      cudaSetDevice(bg->g[r]->ctx->device);
-      if (cudaMemcpy(&err, bg->g[r]->arena + 2048, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) err = 1;
-      if (err) rc = box_fail(b, SPF_E_GRAPH, "peer barrier timed out: a rank of the box run did not arrive");
-    }
-  }
-  if (rc == 0)
-    for (int r = 0; r < n; r++) copy_out_staged(bg->g[r], r);
-  if (rc && n > 1) bg->poisoned.store(true);
-  bg->status_msg = rc ? b->err : std::string();
-  bg->status.store(rc);
-  bg->launches_per_run = box_launches(b) - l0;
-  return rc;
-}
+int spf_b200_box_graph_run(spf_b200_box_graph* bg) { return bg ? run_blocking(box_run(bg)) : SPF_E_INVALID; }
 
 int spf_b200_box_graph_spawn(spf_b200_box_graph* bg, spf_b200_box_graph* const* after, size_t n_after,
                              spf_completion_fn on_complete, void* user) {
   if (!bg) return SPF_E_INVALID;
   spf_b200_box* b = bg->box;
   if (n_after && !after) return box_fail(b, SPF_E_INVALID, "spawn: NULL dependency list");
-  const int n = (int)bg->g.size();
-  {
-    std::unique_lock<std::mutex> lk(b->fc_mu);
-    b->fc_cv.wait(lk, [&] { return b->in_flight < b->max_in_flight; });
-    b->in_flight++;
+  const Run run = box_run(bg);
+  spawn_begin(run);
+  int status = 0;
+  std::string msg;
+  if (poisoned(run)) {
+    status = SPF_E_GRAPH;
+    msg = kPoisoned;
   }
-  for (spf_b200_graph* g : bg->g) {  // the staging slab of pageable io buffers is reused by this run
-    bool staged = false;
-    for (char k : g->io_kind) staged |= k == 1;
-    if (staged) {
-      cudaSetDevice(g->ctx->device);
-      cudaEventSynchronize(g->done);
-    }
-  }
-  BoxSpawn* rec = new BoxSpawn{bg, on_complete, user, 0, std::string(), {n}};
-  if (box_graph_poisoned(bg)) {
-    rec->status = SPF_E_GRAPH;
-    rec->msg = "an earlier run of this box graph failed: the ranks' barrier epochs disagree, rebuild the graph";
-  }
-  for (size_t i = 0; i < n_after && rec->status == 0; i++) {
+  std::vector<std::vector<spf_b200_graph*>> deps;
+  for (size_t i = 0; i < n_after && status == 0; i++) {
     spf_b200_box_graph* d = after[i];
     if (!d || d == bg) continue;
     if (d->box != b) {
-      rec->status = SPF_E_INVALID;
-      rec->msg = "spawn: a dependency belongs to another box";
-    } else if (const int ds = d->status.load()) {
-      rec->status = ds;
-      rec->msg = "a dependency of this graph failed: " + d->status_msg;
+      status = SPF_E_INVALID;
+      msg = "spawn: a dependency belongs to another box";
+    } else if (const int ds = d->run.status.load()) {
+      status = ds;
+      msg = "a dependency of this graph failed: " + d->run.msg;
     } else {
-      // every member waits for every member of the dependency, whichever ranks either runs on (a cross-device wait
-      // when they differ): an output is written by one member into every replica, read by all
-      for (int r = 0; r < n && rec->status == 0; r++) {
-        cudaSetDevice(bg->g[r]->ctx->device);
-        for (size_t q = 0; q < d->g.size() && rec->status == 0; q++)
-          if (cudaStreamWaitEvent(bg->g[r]->stream, d->g[q]->done, 0) != cudaSuccess) {
-            rec->status = SPF_E_CUDA;
-            rec->msg = "cudaStreamWaitEvent on a dependency failed";
-          }
-      }
+      deps.push_back(d->g);
     }
   }
-  const uint64_t l0 = box_launches(b);
-  if (rec->status == 0) {
-    if (const int rc = box_enqueue(bg)) {
-      rec->status = rc;
-      rec->msg = b->err;
-    }
-  }
-  bg->launches_per_run = box_launches(b) - l0;
-  bg->status.store(rec->status);
-  bg->status_msg = rec->msg;
-  for (int r = 0; r < n; r++) {
-    spf_b200_graph* g = bg->g[r];
-    cudaSetDevice(g->ctx->device);
-    cudaError_t e = cudaSuccess;
-    if (n > 1) e = cudaMemcpyAsync(&bg->h_err[r], g->arena + 2048, sizeof(int), cudaMemcpyDeviceToHost, g->stream);
-    if (e == cudaSuccess) e = cudaLaunchHostFunc(g->stream, box_rank_done, new BoxRankDone{rec, r});
-    cudaEventRecord(g->done, g->stream);
-    if (e != cudaSuccess) {  // could not enqueue this rank's completion: retire the rank here
-      cudaStreamSynchronize(g->stream);
-      if (rec->status == 0) {
-        rec->status = SPF_E_CUDA;
-        rec->msg = std::string("box spawn: ") + cudaGetErrorString(e);
-      }
-      box_rank_done(new BoxRankDone{rec, r});
-    }
-  }
-  return 0;
+  return spawn(run, deps, status, msg, on_complete, user);
 }
 
-int spf_b200_box_graph_wait(spf_b200_box_graph* bg) {
-  if (!bg) return SPF_E_INVALID;
-  for (spf_b200_graph* g : bg->g) {
-    BCU(bg->box, cudaSetDevice(g->ctx->device));
-    BCU(bg->box, cudaEventSynchronize(g->done));
-  }
-  return bg->status.load();
-}
+int spf_b200_box_graph_wait(spf_b200_box_graph* bg) { return bg ? wait_run(box_run(bg)) : SPF_E_INVALID; }
 
-const char* spf_b200_box_graph_status_message(const spf_b200_box_graph* bg) { return bg ? bg->status_msg.c_str() : ""; }
+const char* spf_b200_box_graph_status_message(const spf_b200_box_graph* bg) { return bg ? bg->run.msg.c_str() : ""; }
 
 int spf_b200_box_graph_set_io(spf_b200_box_graph* bg, size_t node, void* io) {
   if (!bg) return SPF_E_INVALID;
@@ -932,6 +715,6 @@ int spf_b200_box_ciphertext_read(spf_b200_box_ciphertext* h, int rank, void* hos
 }
 
 int spf_b200_box_graph_levels(const spf_b200_box_graph* bg) { return bg && !bg->g.empty() ? bg->g[0]->n_levels : -1; }
-uint64_t spf_b200_box_graph_launches(const spf_b200_box_graph* bg) { return bg ? bg->launches_per_run : 0; }
+uint64_t spf_b200_box_graph_launches(const spf_b200_box_graph* bg) { return bg ? bg->run.launches : 0; }
 
 }  // extern "C"

@@ -32,6 +32,31 @@ struct DevBuf {
   size_t cap = 0;
 };
 
+// Flow control of spawned graph runs (graph.cuh: spawn_begin): at most max_in_flight runs between dispatch and
+// completion, as the bounded channel of CircuitProcessor::new (circuit_processor/mod.rs:95-123).  A run takes one slot,
+// whatever its number of member graphs.
+struct FlowControl {
+  std::mutex mu;
+  std::condition_variable cv;
+  int in_flight = 0, max_in_flight = 4;
+
+  void acquire() {
+    std::unique_lock<std::mutex> lk(mu);
+    cv.wait(lk, [&] { return in_flight < max_in_flight; });
+    in_flight++;
+  }
+  void release() {
+    std::lock_guard<std::mutex> lk(mu);
+    in_flight--;
+    cv.notify_all();
+  }
+  void set(int n) {
+    std::lock_guard<std::mutex> lk(mu);
+    max_in_flight = n;
+    cv.notify_all();
+  }
+};
+
 }  // namespace
 
 struct spf_b200_ctx {
@@ -55,11 +80,7 @@ struct spf_b200_ctx {
   int sm_count = 148;
   // lifetime: graphs built on this context keep it alive (spf_b200_destroy only drops the owner's reference)
   std::atomic<int> refs{1};
-  // flow control of the asynchronous executor (graph.cuh: spf_b200_graph_spawn): at most max_in_flight spawned graphs
-  // between dispatch and completion, as the bounded channel of CircuitProcessor::new (circuit_processor/mod.rs:95-123)
-  std::mutex fc_mu;
-  std::condition_variable fc_cv;
-  int in_flight = 0, max_in_flight = 4;
+  FlowControl fc;  // of the spawned runs of this context's graphs
   // device constants for the graph executor's Zero*/One* nodes (graph.cuh::ensure_constants)
   void* consts = nullptr;
   char *c_lwe0[2] = {nullptr, nullptr}, *c_glwe[2] = {nullptr, nullptr}, *c_glev[2] = {nullptr, nullptr},

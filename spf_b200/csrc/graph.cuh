@@ -83,6 +83,14 @@ struct Group {
   bool slot_outputs = false;  // CMux / MultiplyGgswGlwe: every output has its own recycled GLWE slot (out pointer table)
 };
 
+// What the last run of a context graph or box graph left: the first error latched by the run (spawned or blocking) and
+// its message, and the kernel launches the run enqueued.
+struct RunState {
+  std::atomic<int> status{0};
+  std::string msg;
+  uint64_t launches = 0;
+};
+
 }  // namespace
 
 struct spf_b200_graph {
@@ -104,7 +112,6 @@ struct spf_b200_graph {
   std::vector<size_t> gather_off;  // byte offset of output k in d_gather, (size_t)-1 for GGSW outputs
   size_t gather_items = 0;
   int n_levels = 0;
-  uint64_t launches_per_run = 0;
   int world = 1;  // CircuitBootstrap groups are laid out as `world` equal chunks (spf_b200_graph_build_sharded)
   std::vector<int> owner;  // rank that computes the node's ciphertext, -1 = every rank holds it
   std::vector<int> slot;   // CMux outputs: index of the node's GLWE slot in the recycled pool, -1 otherwise
@@ -127,26 +134,17 @@ struct spf_b200_graph {
   char* h_stage = nullptr;        // page-locked staging slab for kind-1 buffers
   size_t h_stage_bytes = 0;
   std::vector<size_t> stage_off;  // per node: offset of its ciphertext in h_stage (kind 1), (size_t)-1 otherwise
-  // asynchronous execution (spf_b200_graph_spawn): the graph's own stream, an event recorded behind every run, the first
-  // error latched by the current / last run, the digit-state scratch of its keyswitch levels
+  // asynchronous execution (spf_b200_graph_spawn): the graph's own stream, an event recorded behind every run, the state
+  // of the last run as a context graph, the digit-state scratch of its keyswitch levels
   cudaStream_t stream = nullptr;
   cudaEvent_t done = nullptr;
-  std::atomic<int> status{0};
-  std::string status_msg;
+  RunState run;
   DevBuf ks_states;
-  bool poisoned = false;  // a failed peer-mode run leaves the ranks' barrier epochs out of step: rebuild the graphs
+  // a failed peer-mode run leaves the ranks' barrier epochs out of step: rebuild the graphs (set by a completion thread)
+  std::atomic<bool> poisoned{false};
   // rank that writes the Output* nodes every rank holds (output rank -1); -1 = every rank writes them (one process per
   // rank: each has its own host buffers).  A box (box.cuh) runs all ranks into the same host buffers: rank 0 only.
   int replicated_writer = -1;
-};
-
-// one spawned run between dispatch and completion
-struct SpawnRecord {
-  spf_b200_graph* g;
-  spf_completion_fn cb;
-  void* user;
-  int status;
-  std::string msg;
 };
 
 namespace {
@@ -787,13 +785,33 @@ int stage_slot(spf_b200_graph* g, int id, size_t bytes, char** out) {
   return 0;
 }
 
+// Everything of a run that could wait on the device, done for every member before any member enqueues: the staging
+// slab of pageable io buffers (its growth synchronises the stream) and the keyswitch digit-state scratch at the size of
+// the largest keyswitch group (growing it frees the old buffer, which synchronises the device).  Afterwards the
+// enqueue_* parts only enqueue: copies from page-locked memory, kernel launches, event records.
+int prepare_run(spf_b200_graph* g, int rank) {
+  spf_b200_ctx* ctx = g->ctx;
+  CU(cudaSetDevice(ctx->device));
+  for (const std::vector<int>* io : {&g->inputs, &g->outputs})  // not every node: a graph may have a million
+    for (int id : *io) {
+      if (g->io_kind[id] != 1) continue;
+      char* dummy = nullptr;
+      if (int rc = stage_slot(g, id, 0, &dummy)) return rc;
+    }
+  size_t ks = 0;
+  for (const Group& G : g->groups)
+    if (G.op == SPF_OP_KEYSWITCH_L1_TO_L0) ks = std::max(ks, std::max(G.all_cnt, G.r_cnt[rank]));
+  if (ks) if (int rc = ensure(ctx, g->ks_states, ks * (size_t)ctx->p.glwe_k * ctx->p.glwe_n * 2)) return rc;
+  return 0;
+}
+
 // Whether `rank` writes Output* node `id` into its io buffer: outputs of a MUX tree live on the tree's owner.
 bool writes_output(const spf_b200_graph* g, size_t id, int rank) {
   const int r = spf_b200_graph_output_rank(g, id);
   return r == rank || (r < 0 && (g->replicated_writer < 0 || g->replicated_writer == rank));
 }
 
-// The parts of one run that are ENQUEUED on stream s (enqueue_run: inputs, every group in order, outputs).  Each
+// The parts of one run that are ENQUEUED on stream s (enqueue: inputs, every group in order, outputs).  Each
 // returns the first error (message in ctx->err); work already enqueued keeps running -- the caller drains the stream.
 // Input copies (and, in peer mode, the start-of-run barrier).
 int enqueue_inputs(spf_b200_graph* g, bool peer_mode, cudaStream_t s) {
@@ -861,18 +879,6 @@ int enqueue_group(spf_b200_graph* g, const Group& G, int rank, int world, spf_ex
     }
   }
   return 0;
-}
-
-int enqueue_outputs(spf_b200_graph* g, int rank, cudaStream_t s);
-
-int enqueue_run(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange, void* user, cudaStream_t s,
-                std::vector<cudaEvent_t>* timing_events) {
-  if (int rc = enqueue_inputs(g, world > 1 && !exchange, s)) return rc;
-  if (timing_events) cudaEventRecord((*timing_events)[0], s);
-  size_t gi = 0;
-  for (const Group& G : g->groups)
-    if (int rc = enqueue_group(g, G, rank, world, exchange, user, s, timing_events ? (*timing_events)[++gi] : nullptr)) return rc;
-  return enqueue_outputs(g, rank, s);
 }
 
 // Gathered and GGSW output copies of this rank.
@@ -944,18 +950,289 @@ void copy_out_staged(spf_b200_graph* g, int rank) {
   }
 }
 
-void CUDART_CB spawn_done(void* arg) {
-  SpawnRecord* rec = static_cast<SpawnRecord*>(arg);
-  spf_b200_graph* g = rec->g;
-  if (rec->status == 0) copy_out_staged(g, 0);
-  spf_b200_ctx* ctx = g->ctx;
-  {
-    std::lock_guard<std::mutex> lk(ctx->fc_mu);
-    ctx->in_flight--;
+// Whether some handle-bound output is written by one member into the replicas of the others (with two or more
+// members; the replicas of non-members written by member 0 are not read by this graph).
+bool has_owned_handle_outputs(const spf_b200_graph* g) {
+  for (int id : g->outputs)
+    if (g->io_kind[id] == 3 && spf_b200_graph_output_rank(g, id) >= 0) return true;
+  return false;
+}
+
+int enqueue_handle_copies(spf_b200_box_graph* bg, int i, bool outputs);  // box.cuh
+
+// ---- the executor: one run of a compiled graph over its member graphs ---------------------------------------------
+// A context graph has one member: shard `rank` of its world, in a process of its own, exchanging through an exchange
+// callback or peer memory.  A box graph has one member per member rank, all driven from the calling thread: member i
+// runs shard i of the graph sharded over the members, exchanging through peer memory (box.cuh).  No two fields share a
+// type, so a positional initialisation (context_run, box_run) that swaps two of them does not compile.
+struct Run {
+  std::vector<spf_b200_graph*> g;
+  int rank = 0;                        // shard rank of member 0; member i runs shard rank + i
+  spf_exchange_fn exchange = nullptr;  // context graphs only
+  void* user = nullptr;
+  spf_b200_box_graph* box = nullptr;   // the box graph of the run (box ciphertext handle copies), NULL for a context graph
+  const std::vector<int>* box_rank = nullptr;  // member i's box rank, the prefix of its errors in the box's slot
+  int* h_err = nullptr;                // page-locked copy of member i's barrier error word (spawned peer-mode runs)
+  RunState* state = nullptr;
+  FlowControl* fc = nullptr;
+  std::string* err = nullptr;          // the error slot: the context's, or the box's
+
+  bool peer() const { return g[0]->world > 1 && !exchange; }
+};
+
+const char* const kPoisoned =
+    "an earlier peer-memory run of this graph failed: the ranks' barrier epochs disagree, rebuild the graphs";
+const char* const kBarrierTimeout = "peer barrier timed out: a rank of the sharded run did not arrive";
+
+int run_fail(const Run& run, int code, const std::string& msg) {
+  *run.err = msg;
+  return code;
+}
+
+// Member i's error, whose message is in its context.
+int member_fail(const Run& run, int i, int code) {
+  return run_fail(run, code, (run.box_rank ? "rank " + std::to_string((*run.box_rank)[i]) + ": " : std::string()) + run.g[i]->ctx->err);
+}
+
+uint64_t launches(const Run& run) {
+  uint64_t s = 0;
+  for (const spf_b200_graph* g : run.g) s += g->ctx->launches.load();
+  return s;
+}
+
+// Waits for the `done` event of every member: the end of its last run, completion included.
+int wait_done(const Run& run) {
+  for (spf_b200_graph* g : run.g) {
+    cudaError_t e = cudaSetDevice(g->ctx->device);
+    if (e == cudaSuccess) e = cudaEventSynchronize(g->done);
+    if (e != cudaSuccess) return run_fail(run, SPF_E_CUDA, std::string("graph wait: ") + cudaGetErrorString(e));
   }
-  ctx->fc_cv.notify_all();
+  return 0;
+}
+
+bool poisoned(const Run& run) {
+  for (const spf_b200_graph* g : run.g)
+    if (g->poisoned) return true;
+  return false;
+}
+
+// Enqueues one run on every member from the calling thread, level-interleaved: the inputs of every member, then group k
+// of every member for k = 0, 1, ..., then the outputs of every member.  So when the host has to wait for a member's
+// stream (its launch queue is full), every other member's work up to the same level -- and so to the same peer barrier
+// -- is enqueued already, and the wait ends.  Returns the first error; members after a failed one are not enqueued
+// further.  Box ciphertext handles: each member reads its own replica right after its other inputs.  When an owner
+// writes the replicas of other members at the end, a barrier after the inputs first makes sure that every member has
+// read its replica (a graph may read and write the same handle, and need not have a bootstrap level, whose barrier
+// would do); the start-of-run barrier keeps these writes ahead of the next run's reads.  `timing`: events recorded on
+// member 0's stream (with its device current) after its input copies and after each of its groups.
+int enqueue(const Run& run, const std::vector<cudaEvent_t>* timing) {
+  const int n = (int)run.g.size();
+  for (int i = 0; i < n; i++)
+    if (int rc = prepare_run(run.g[i], run.rank + i)) return member_fail(run, i, rc);
+  // step(i, g) for every member i, on its device
+  auto each = [&](auto step) {
+    for (int i = 0; i < n; i++) {
+      const cudaError_t e = cudaSetDevice(run.g[i]->ctx->device);
+      if (e != cudaSuccess) return run_fail(run, SPF_E_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+      if (int rc = step(i, run.g[i])) return member_fail(run, i, rc);
+    }
+    return 0;
+  };
+  if (int rc = each([&](int i, spf_b200_graph* g) {
+        if (int rc = enqueue_inputs(g, run.peer(), g->stream)) return rc;
+        if (timing && i == 0) cudaEventRecord((*timing)[0], g->stream);
+        return run.box ? enqueue_handle_copies(run.box, i, false) : 0;
+      }))
+    return rc;
+  if (n > 1 && has_owned_handle_outputs(run.g[0]))
+    if (int rc = each([&](int, spf_b200_graph* g) { return peer_barrier(g, g->stream); })) return rc;
+  for (size_t k = 0; k < run.g[0]->groups.size(); k++)
+    if (int rc = each([&](int i, spf_b200_graph* g) {
+          return enqueue_group(g, g->groups[k], run.rank + i, g->world, run.exchange, run.user, g->stream,
+                               timing && i == 0 ? (*timing)[k + 1] : nullptr);
+        }))
+      return rc;
+  return each([&](int i, spf_b200_graph* g) {
+    if (int rc = enqueue_outputs(g, run.rank + i, g->stream)) return rc;
+    return run.box ? enqueue_handle_copies(run.box, i, true) : 0;
+  });
+}
+
+// Executes the run once and returns when the outputs are valid.  A failure after the first enqueue drains every
+// member's stream before returning (the caller's io buffers are not touched afterwards); in peer mode it also leaves
+// the ranks' barrier epochs out of step, so the members are marked poisoned and the graph must be rebuilt.
+int run_blocking(const Run& run) {
+  if (poisoned(run)) return run_fail(run, SPF_E_GRAPH, kPoisoned);
+  // a spawned run still in flight finishes first (the staging slabs and the barrier epochs are per graph)
+  if (int rc = wait_done(run)) return rc;
+  const uint64_t l0 = launches(run);
+  // SPF_B200_GRAPH_TIMING=1: CUDA events around every group of member 0, per-op totals on stderr (diagnostics only;
+  // the events serialise nothing but do defeat the programmatic overlap between CMUX levels)
+  static const bool timing = getenv("SPF_B200_GRAPH_TIMING") != nullptr;
+  const spf_b200_graph* g0 = run.g[0];
+  std::vector<cudaEvent_t> ev;
+  if (timing) {
+    cudaSetDevice(g0->ctx->device);
+    ev.resize(g0->groups.size() + 1);
+    for (auto& e : ev) cudaEventCreate(&e);
+  }
+  int rc = enqueue(run, timing ? &ev : nullptr);
+  cudaError_t se = cudaSuccess;
+  for (spf_b200_graph* g : run.g) {  // also on failure: nothing of this run is in flight afterwards
+    cudaSetDevice(g->ctx->device);
+    const cudaError_t e = cudaStreamSynchronize(g->stream);
+    if (se == cudaSuccess) se = e;
+    cudaEventRecord(g->done, g->stream);
+  }
+  if (rc == 0 && se != cudaSuccess) rc = run_fail(run, SPF_E_CUDA, std::string("graph run: ") + cudaGetErrorString(se));
+  const bool peer = run.peer();
+  for (size_t i = 0; i < run.g.size() && peer && rc == 0; i++) {
+    int err = 0;
+    cudaSetDevice(run.g[i]->ctx->device);
+    if (cudaMemcpy(&err, run.g[i]->arena + 2048, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) err = 1;
+    if (err) rc = run_fail(run, SPF_E_GRAPH, kBarrierTimeout);
+  }
+  if (rc == 0)
+    for (size_t i = 0; i < run.g.size(); i++) copy_out_staged(run.g[i], run.rank + (int)i);
+  if (rc && peer)
+    for (spf_b200_graph* g : run.g) g->poisoned = true;
+  if (timing && rc == 0) {
+    std::map<uint32_t, std::pair<double, size_t>> per_op;
+    std::map<uint32_t, size_t> groups_of;
+    for (size_t k = 0; k < g0->groups.size(); k++) {
+      float ms = 0;
+      cudaEventElapsedTime(&ms, ev[k], ev[k + 1]);
+      per_op[g0->groups[k].op].first += ms;
+      per_op[g0->groups[k].op].second += g0->groups[k].ids.size();
+      groups_of[g0->groups[k].op]++;
+    }
+    for (auto& kv : per_op)
+      fprintf(stderr, "[spf_b200 graph] %-18s %6zu groups %8zu nodes %9.3f ms\n", kOpNames[kv.first], groups_of[kv.first], kv.second.second, kv.second.first);
+  }
+  for (auto& e : ev) cudaEventDestroy(e);
+  run.state->msg = rc ? *run.err : std::string();
+  run.state->status.store(rc);
+  run.state->launches = launches(run) - l0;
+  return rc;
+}
+
+// ---- asynchronous execution: CircuitProcessor::spawn_graph + CompletionHandler + flow control -------------------------
+// (circuit_processor/mod.rs:130-253,573-623; completion_handler.rs:14-56).  The whole run is enqueued on the members'
+// own streams and the call returns; `on_complete(user, status, message)` fires exactly once when every member has
+// retired, with the FIRST error of the run (0 = none).  A run whose dependency failed retires as a no-op with that
+// error, as tasks do after CompletionHandler::error is set.  At most max_in_flight runs per context or box are between
+// dispatch and completion: further spawns block in the caller, as dispatch() blocks on the flow-control channel.
+
+// One spawned run between dispatch and completion: every member retires in a host function of its own stream, and
+// the last one delivers the completion.
+struct SpawnRecord {
+  Run run;
+  spf_completion_fn cb;
+  void* user;
+  std::atomic<int> status;  // read by every member's host function, set on this thread when one cannot be enqueued
+  std::string msg;
+  std::atomic<int> remaining;
+  std::atomic<int> barrier_failed{0};
+};
+struct MemberDone {
+  SpawnRecord* rec;
+  int i;
+};
+
+void CUDART_CB member_done(void* arg) {
+  MemberDone* d = static_cast<MemberDone*>(arg);
+  SpawnRecord* rec = d->rec;
+  const int i = d->i;
+  delete d;
+  const Run& run = rec->run;
+  const bool peer = run.peer();
+  const bool barrier_failed = peer && run.h_err[i];
+  if (barrier_failed) rec->barrier_failed.store(1);
+  if (rec->status == 0 && !barrier_failed) copy_out_staged(run.g[i], run.rank + i);
+  if (rec->remaining.fetch_sub(1) != 1) return;
+  if (rec->status == 0 && rec->barrier_failed.load()) {  // the one error only the completion can see
+    rec->status = SPF_E_GRAPH;
+    rec->msg = kBarrierTimeout;
+    run.state->msg = rec->msg;
+    run.state->status.store(rec->status);
+  }
+  if (rec->status && peer)
+    for (spf_b200_graph* g : run.g) g->poisoned = true;
+  run.fc->release();
   if (rec->cb) rec->cb(rec->user, rec->status, rec->status ? rec->msg.c_str() : nullptr);
   delete rec;
+}
+
+// First half of a spawn, before the caller decides whether the run can start: takes the run's flow-control slot, then
+// waits for the previous run of every member whose page-locked staging slab (pageable io buffers) this run reuses.
+void spawn_begin(const Run& run) {
+  run.fc->acquire();
+  for (spf_b200_graph* g : run.g) {
+    bool staged = false;
+    for (char k : g->io_kind) staged |= k == 1;
+    if (staged) {
+      cudaSetDevice(g->ctx->device);
+      cudaEventSynchronize(g->done);
+    }
+  }
+}
+
+// Second half: every member's stream waits for every member of each dependency in `deps` (a cross-device wait when
+// they differ: an output of a box graph is written by one member into every replica, read by all), then the run is
+// enqueued -- unless `status`, the caller's verdict, says it cannot start: then it retires as a no-op with that error.
+int spawn(const Run& run, const std::vector<std::vector<spf_b200_graph*>>& deps, int status, const std::string& msg,
+          spf_completion_fn on_complete, void* user) {
+  const int n = (int)run.g.size();
+  SpawnRecord* rec = new SpawnRecord{run, on_complete, user, status, msg, {n}};
+  for (const std::vector<spf_b200_graph*>& d : deps)
+    for (spf_b200_graph* g : run.g) {
+      cudaSetDevice(g->ctx->device);
+      for (spf_b200_graph* q : d)
+        if (cudaStreamWaitEvent(g->stream, q->done, 0) != cudaSuccess && rec->status == 0) {
+          rec->status = SPF_E_CUDA;
+          rec->msg = "cudaStreamWaitEvent on a dependency failed";
+        }
+    }
+  const uint64_t l0 = launches(run);
+  if (rec->status == 0) {
+    if (const int rc = enqueue(run, nullptr)) {
+      rec->status = rc;
+      rec->msg = *run.err;
+    }
+  }
+  run.state->launches = launches(run) - l0;
+  run.state->status.store(rec->status);
+  run.state->msg = rec->msg;
+  for (int i = 0; i < n; i++) {
+    spf_b200_graph* g = run.g[i];
+    cudaSetDevice(g->ctx->device);
+    cudaError_t e = cudaSuccess;
+    if (run.peer()) e = cudaMemcpyAsync(&run.h_err[i], g->arena + 2048, sizeof(int), cudaMemcpyDeviceToHost, g->stream);
+    MemberDone* d = new MemberDone{rec, i};
+    if (e == cudaSuccess) e = cudaLaunchHostFunc(g->stream, member_done, d);
+    cudaEventRecord(g->done, g->stream);
+    if (e != cudaSuccess) {  // could not enqueue this member's completion: retire the member here
+      cudaStreamSynchronize(g->stream);
+      if (rec->status == 0) {
+        rec->status = SPF_E_CUDA;
+        rec->msg = std::string("spawn: ") + cudaGetErrorString(e);
+        run.state->msg = rec->msg;
+        run.state->status.store(rec->status);
+      }
+      member_done(d);
+    }
+  }
+  return 0;
+}
+
+// Blocks until the last run (spawned or blocking) has completed on every member, callback included; returns its status.
+int wait_run(const Run& run) {
+  if (int rc = wait_done(run)) return rc;
+  return run.state->status.load();
+}
+
+Run context_run(spf_b200_graph* g, int rank, spf_exchange_fn exchange, void* user) {
+  return Run{{g}, rank, exchange, user, nullptr, nullptr, nullptr, &g->run, &g->ctx->fc, &g->ctx->err};
 }
 
 }  // namespace
@@ -969,140 +1246,52 @@ extern "C" {
 // inputs): each CircuitBootstrap group -- the only expensive ops -- is split into `world` equal
 // chunks, rank r bootstraps chunk r, then `exchange` (an all-gather over NVLink, see
 // spf_b200/multi.py) or the peer-memory stores complete the group's GGSWs on every rank; MUX trees run on their
-// owner ranks.  A failure after the first enqueue drains the stream before returning (the caller's io buffers are
-// not touched afterwards); in peer mode it also leaves the ranks' barrier epochs out of step, so the graph is
-// marked poisoned and must be rebuilt.
+// owner ranks.
 int spf_b200_graph_run_sharded(spf_b200_graph* g, int rank, int world, spf_exchange_fn exchange, void* user) {
   if (!g) return SPF_E_INVALID;
   spf_b200_ctx* ctx = g->ctx;
   if (world != g->world || rank < 0 || rank >= world)
     return fail(ctx, SPF_E_INVALID, "rank/world do not match the graph's sharded layout");
-  const bool peer_mode = world > 1 && !exchange;
-  if (peer_mode && (!g->peers_set || g->peer_rank != rank))
+  if (world > 1 && !exchange && (!g->peers_set || g->peer_rank != rank))
     return fail(ctx, SPF_E_INVALID, "a sharded run needs an exchange callback or opened peer arenas (spf_b200_graph_open_peers)");
-  if (g->poisoned)
-    return fail(ctx, SPF_E_GRAPH, "an earlier peer-memory run of this graph failed: the ranks' barrier epochs disagree, rebuild the graphs");
-  CU(cudaSetDevice(ctx->device));
-  cudaStream_t s = g->stream;
-  const uint64_t l0 = ctx->launches.load();
-  // SPF_B200_GRAPH_TIMING=1: CUDA events around every group, per-op totals on stderr (diagnostics only;
-  // the events serialise nothing but do defeat the programmatic overlap between CMUX levels)
-  static const bool timing = getenv("SPF_B200_GRAPH_TIMING") != nullptr;
-  std::vector<cudaEvent_t> ev;
-  if (timing) {
-    ev.resize(g->groups.size() + 1);
-    for (auto& e : ev) cudaEventCreate(&e);
-  }
-  int rc = enqueue_run(g, rank, world, exchange, user, s, timing ? &ev : nullptr);
-  const std::string msg = rc ? ctx->err : std::string();
-  const cudaError_t se = cudaStreamSynchronize(s);  // also on failure: nothing of this run is in flight afterwards
-  cudaEventRecord(g->done, s);
-  if (rc == 0 && se != cudaSuccess) rc = fail(ctx, SPF_E_CUDA, std::string("graph run: ") + cudaGetErrorString(se));
-  else if (rc) ctx->err = msg;
-  if (rc == 0) copy_out_staged(g, rank);
-  if (rc == 0 && peer_mode) {
-    int err = 0;
-    if (cudaMemcpy(&err, g->arena + 2048, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) err = 1;
-    if (err) {
-      cudaMemset(g->arena + 2048, 0, sizeof(int));
-      rc = fail(ctx, SPF_E_GRAPH, "peer barrier timed out: a rank of the sharded run did not arrive");
-    }
-  }
-  if (rc && peer_mode) g->poisoned = true;
-  if (timing && rc == 0) {
-    std::map<uint32_t, std::pair<double, size_t>> per_op;
-    std::map<uint32_t, size_t> groups_of;
-    for (size_t k = 0; k < g->groups.size(); k++) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, ev[k], ev[k + 1]);
-      per_op[g->groups[k].op].first += ms;
-      per_op[g->groups[k].op].second += g->groups[k].ids.size();
-      groups_of[g->groups[k].op]++;
-    }
-    for (auto& kv : per_op)
-      fprintf(stderr, "[spf_b200 graph] %-18s %6zu groups %8zu nodes %9.3f ms\n", kOpNames[kv.first], groups_of[kv.first], kv.second.second, kv.second.first);
-  }
-  for (auto& e : ev) cudaEventDestroy(e);
-  g->status.store(rc);
-  g->launches_per_run = ctx->launches.load() - l0;
-  return rc;
+  return run_blocking(context_run(g, rank, exchange, user));
 }
 
-// ---- asynchronous execution: CircuitProcessor::spawn_graph + CompletionHandler + flow control -------------------------
-// (circuit_processor/mod.rs:130-253,573-623; completion_handler.rs:14-56).  The whole run is enqueued on the graph's own
-// stream and the call returns; `on_complete(user, status, message)` fires exactly once when every op has retired, with
-// the FIRST error of the run (0 = none).  A run whose dependency failed retires as a no-op with that error, as tasks
-// do after CompletionHandler::error is set.  At most spf_b200_set_max_in_flight graphs are between dispatch and
-// completion: further spawns block in the caller, as dispatch() blocks on the flow-control channel.  `after`: graphs
-// whose LAST spawned run must complete first (stream-ordered on the device, no host wait) -- with device handles as
-// io buffers (see spf_b200_graph_set_io) graph k + 1 consumes graph k's outputs without leaving HBM.
+// `after`: graphs whose LAST spawned run must complete first (stream-ordered on the device, no host wait) -- with device
+// handles as io buffers (see spf_b200_graph_set_io) graph k + 1 consumes graph k's outputs without leaving HBM.
 // The callback runs on a CUDA-internal thread: it must not call CUDA or spf_b200 functions.
 int spf_b200_graph_spawn(spf_b200_graph* g, spf_b200_graph* const* after, size_t n_after, spf_completion_fn on_complete, void* user) {
   if (!g) return SPF_E_INVALID;
   spf_b200_ctx* ctx = g->ctx;
   if (g->world != 1) return fail(ctx, SPF_E_INVALID, "spawn: sharded graphs run through spf_b200_graph_run_sharded");
   if (n_after && !after) return fail(ctx, SPF_E_INVALID, "spawn: NULL dependency list");
-  CU(cudaSetDevice(ctx->device));
-  {
-    std::unique_lock<std::mutex> lk(ctx->fc_mu);
-    ctx->fc_cv.wait(lk, [&] { return ctx->in_flight < ctx->max_in_flight; });
-    ctx->in_flight++;
-  }
-  // the staging slab of pageable io buffers is reused by the next run: wait for the previous one
-  bool staged = false;
-  for (char k : g->io_kind) staged |= k == 1;
-  if (staged) cudaEventSynchronize(g->done);
-  SpawnRecord* rec = new SpawnRecord{g, on_complete, user, 0, std::string()};
-  for (size_t i = 0; i < n_after && rec->status == 0; i++) {
+  const Run run = context_run(g, 0, nullptr, nullptr);
+  spawn_begin(run);
+  int status = 0;
+  std::string msg;
+  std::vector<std::vector<spf_b200_graph*>> deps;
+  for (size_t i = 0; i < n_after && status == 0; i++) {
     spf_b200_graph* d = after[i];
     if (!d || d == g) continue;
-    if (const int ds = d->status.load()) {
-      rec->status = ds;
-      rec->msg = "a dependency of this graph failed: " + d->status_msg;
-    } else if (cudaStreamWaitEvent(g->stream, d->done, 0) != cudaSuccess) {
-      rec->status = SPF_E_CUDA;
-      rec->msg = "cudaStreamWaitEvent on a dependency failed";
+    if (const int ds = d->run.status.load()) {
+      status = ds;
+      msg = "a dependency of this graph failed: " + d->run.msg;
+    } else {
+      deps.push_back({d});
     }
   }
-  if (rec->status == 0) {
-    if (const int rc = enqueue_run(g, 0, 1, nullptr, nullptr, g->stream, nullptr)) {
-      rec->status = rc;
-      rec->msg = ctx->err;
-    }
-  }
-  g->status.store(rec->status);
-  g->status_msg = rec->msg;
-  const cudaError_t e = cudaLaunchHostFunc(g->stream, spawn_done, rec);
-  cudaEventRecord(g->done, g->stream);
-  if (e != cudaSuccess) {  // could not even enqueue the completion: deliver it here
-    cudaStreamSynchronize(g->stream);
-    rec->status = rec->status ? rec->status : SPF_E_CUDA;
-    if (rec->msg.empty()) rec->msg = std::string("cudaLaunchHostFunc: ") + cudaGetErrorString(e);
-    spawn_done(rec);
-  }
-  return 0;
+  return spawn(run, deps, status, msg, on_complete, user);
 }
 
-// Blocks until the last run of the graph (spawned or blocking) has completed, callback included; returns its status.
-int spf_b200_graph_wait(spf_b200_graph* g) {
-  if (!g) return SPF_E_INVALID;
-  spf_b200_ctx* ctx = g->ctx;
-  CU(cudaSetDevice(ctx->device));
-  CU(cudaEventSynchronize(g->done));
-  return g->status.load();
-}
+int spf_b200_graph_wait(spf_b200_graph* g) { return g ? wait_run(context_run(g, 0, nullptr, nullptr)) : SPF_E_INVALID; }
 
-// message of the error latched by the graph's last spawned run ("" when it succeeded)
-const char* spf_b200_graph_status_message(const spf_b200_graph* g) { return g ? g->status_msg.c_str() : ""; }
+// message of the error latched by the graph's last run, spawned or blocking ("" when it succeeded)
+const char* spf_b200_graph_status_message(const spf_b200_graph* g) { return g ? g->run.msg.c_str() : ""; }
 
 int spf_b200_set_max_in_flight(spf_b200_ctx* ctx, int n) {
   if (!ctx) return SPF_E_INVALID;
   if (n < 1) return fail(ctx, SPF_E_INVALID, "max_in_flight must be at least 1");
-  {
-    std::lock_guard<std::mutex> lk(ctx->fc_mu);
-    ctx->max_in_flight = n;
-  }
-  ctx->fc_cv.notify_all();
+  ctx->fc.set(n);
   return 0;
 }
 
@@ -1287,7 +1476,7 @@ static int graph_plan_impl(const spf_params* params, const spf_node* nodes, size
 }
 
 int spf_b200_graph_levels(const spf_b200_graph* g) { return g ? g->n_levels : -1; }
-uint64_t spf_b200_graph_launches(const spf_b200_graph* g) { return g ? g->launches_per_run : 0; }
+uint64_t spf_b200_graph_launches(const spf_b200_graph* g) { return g ? g->run.launches : 0; }
 
 int spf_b200_run_graph(spf_b200_ctx* ctx, const spf_node* nodes, size_t n) {
   spf_b200_graph* g = nullptr;
