@@ -464,8 +464,10 @@ typedef enum {
   SPF_MUX_BITWISE = 6,            /* and.rs / or.rs; flags bit0 = or (else and) */
   SPF_MUX_UNSIGNED_MULTIPLIER = 7,/* mul.rs:30-141, n x m -> n + m bits; inputs a[0..n) then b[0..m) */
   SPF_MUX_GRADESCHOOL_REDUCE = 8, /* mul.rs:428-586; inputs ordered by encode_gradeschool_reduction */
-  SPF_MUX_BITSHIFT = 9            /* bitshift.rs:49-157; n value bits + m shift bits, both big-endian; flags bit0 = right,
+  SPF_MUX_BITSHIFT = 9,           /* bitshift.rs:49-157; n value bits + m shift bits, both big-endian; flags bit0 = right,
                                      bits1-2 = mode (0 logical, 1 rotation, 2 arithmetic) */
+  SPF_MUX_CONST_MULTIPLIER = 10   /* low n bits of x * flags (the plaintext constant), n <= 32, m = 0; inputs x[0..n)
+                                     least significant first, in natural order: depth <= n */
 } spf_mux_kind;
 /* *out is malloc'ed; release with spf_b200_mux_free.  SPF_E_INVALID for bad sizes. */
 int spf_b200_mux_circuit(uint32_t kind, uint32_t n, uint32_t m, uint32_t flags, spf_mux_node **out, size_t *count);

@@ -166,37 +166,102 @@ def multiply_then_greater_than(a_bits, b_bits, c_bits, out_prod, out_gt, program
     return M.prune(c, keep)[0]
 
 
+class PlainBit:
+    """One plaintext bit (`value` 0 or 1): a bit of a Plain operand or of a Block.const register."""
+
+    __slots__ = ("value",)
+
+    def __init__(self, value: int):
+        self.value = value
+
+    def __repr__(self) -> str:
+        return f"plain({self.value})"
+
+
+_PLAIN_BITS = (PlainBit(0), PlainBit(1))
+
+
+class Plain:
+    """A plaintext operand: `value` as `width` bits, least significant first like every other operand.  Every instruction
+    takes it in place of an operand bit list (a one-bit Plain also as select's cond); its bits enter the graph as
+    trivial ZeroGlwe1 / OneGlwe1 and are folded out of the circuit (mux_circuits.fold_constants), so they are never
+    bootstrapped and the multiplexers they decide disappear.  value: 0 <= value < 2^width, or a two's-complement
+    negative value >= -2^(width - 1)."""
+
+    __slots__ = ("value", "width", "bits")
+
+    def __init__(self, value: int, width: int):
+        value, width = int(value), int(width)
+        if width < 1:
+            raise ValueError(f"Plain: width {width}, expected at least 1")
+        if not -(1 << (width - 1)) <= value < 1 << width:
+            raise ValueError(f"Plain: value {value} does not fit in {width} bits")
+        self.value, self.width = value % (1 << width), width
+        self.bits = tuple(_PLAIN_BITS[(self.value >> i) & 1] for i in range(width))
+
+    def __len__(self) -> int:
+        return self.width
+
+    def __iter__(self):
+        return iter(self.bits)
+
+    def __getitem__(self, i):
+        return self.bits[i]
+
+    def __repr__(self) -> str:
+        return f"Plain({self.value}, {self.width})"
+
+
+def _is_plain(bits) -> bool:
+    """Whether every bit of an operand is plaintext."""
+    return all(isinstance(b, PlainBit) for b in bits)
+
+
+def _plain_value(bits) -> int:
+    return sum(b.value << i for i, b in enumerate(bits))
+
+
 def _program_graph(inputs, program, outputs) -> tuple[FheCircuit, list[int], list[int]]:
     """A straight-line program as one graph: an InputGlwe1 per input bit, then for every instruction
     `body(c, operand_nodes)` -> the GLWE node behind each of its result bits, an OutputGlwe1 per output bit, pruned to
-    what the outputs read (fhe_circuit.rs:516-555).  Bits are any hashable names.  inputs / outputs: (bit, buffer)
-    pairs; program: (body, operand bits as a list of lists, result bits).  Returns (graph, input-bit nodes, output-bit
-    nodes) in the order of inputs / outputs; an input bit no output reads has node -1."""
+    what the outputs read (fhe_circuit.rs:516-555).  Bits are any hashable names; a PlainBit operand enters as a
+    ZeroGlwe1 / OneGlwe1, and a graph with such bits is constant-folded before it is pruned.  inputs / outputs: (bit,
+    buffer) pairs; program: (body, operand bits as a list of lists, result bits).  Returns (graph, input-bit nodes,
+    output-bit nodes) in the order of inputs / outputs; an input bit no output reads has node -1."""
     from . import mux_circuits as M
 
     c = FheCircuit()
     ins = [c.add("InputGlwe1", io=buf) for _, buf in inputs]
     node = {bit: n for (bit, _), n in zip(inputs, ins)}
+    plain = False
     for body, operands, results in program:
+        for b in (b for op in operands for b in op if isinstance(b, PlainBit) and b not in node):
+            node[b], plain = c.add("OneGlwe1" if b.value else "ZeroGlwe1"), True
         res = body(c, [[node[b] for b in op] for op in operands])
         assert len(res) == len(results)
         node.update(zip(results, res))
     outs = [c.add("OutputGlwe1", node[bit], io=buf) for bit, buf in outputs]
+    if plain:
+        c, ren = M.fold_constants(c)
+        ins, outs = [ren[n] for n in ins], [ren[n] for n in outs]
     c, ren = M.prune(c, outs)
     return c, [ren.get(n, -1) for n in ins], [ren[n] for n in outs]
 
 
 def _instruction_graph(operands, out_bits, body) -> tuple[FheCircuit, list[int], list[int]]:
-    """One instruction as a graph: every operand bit is an input of its own (so the same buffer passed twice is read
-    through two InputGlwe1 nodes) and every result bit an output.  operands: lists of bit ciphertexts.  Returns (graph,
-    operand-bit nodes, result-bit nodes), both in the flattened order of operands / out_bits."""
-    names, k = [], 0
+    """One instruction as a graph: every encrypted operand bit is an input of its own (so the same buffer passed twice
+    is read through two InputGlwe1 nodes) and every result bit an output.  operands: lists of bit ciphertexts or
+    PlainBits.  Returns (graph, encrypted operand-bit nodes, result-bit nodes), both in the flattened order of operands
+    / out_bits."""
+    names, inputs = [], []
     for op in operands:
-        names.append(list(range(k, k + len(op))))
-        k += len(op)
+        names.append([])
+        for x in op:
+            if not isinstance(x, PlainBit):
+                inputs.append((len(inputs), x))
+            names[-1].append(x if isinstance(x, PlainBit) else len(inputs) - 1)
     results = [("result", i) for i in range(len(out_bits))]
-    return _program_graph(list(zip(range(k), [x for op in operands for x in op])), [(body, names, results)],
-                          list(zip(results, out_bits)))
+    return _program_graph(inputs, [(body, names, results)], list(zip(results, out_bits)))
 
 
 def _fronts(c: FheCircuit, inputs: list[list[int]]) -> list[list[int]]:
@@ -227,6 +292,27 @@ def _results(name: str, out_bits, *allowed: int) -> list:
     return out
 
 
+def _check_results(name: str, out_bits) -> None:
+    if any(isinstance(b, (Plain, PlainBit)) for b in out_bits):
+        raise ValueError(f"{name}: a plaintext (Plain or a const register) cannot take a result")
+
+
+def _bit(name: str, bit):
+    """A single-bit operand: a ciphertext, a register bit, a PlainBit, or a one-bit Plain."""
+    if isinstance(bit, Plain):
+        if bit.width != 1:
+            raise ValueError(f"InstructionCache.{name}: a {bit.width}-bit Plain where one bit is expected")
+        return bit.bits[0]
+    return bit
+
+
+def _plain_key(key, operands):
+    """The cache key of a call: with plaintext operand bits, which bits they are and their values are part of it."""
+    if not any(isinstance(b, PlainBit) for op in operands for b in op):
+        return key
+    return key + (tuple(tuple(b.value if isinstance(b, PlainBit) else None for b in op) for op in operands),)
+
+
 class _Instructions:
     """The Parasol integer instructions, shared by InstructionCache (one graph per call) and Block (one graph per
     block).  Each method checks its arguments (ValueError), then hands `self._run(key, body, operands, out_bits)` the
@@ -253,14 +339,22 @@ class _Instructions:
         return self._run(("add", len(a)), lambda c, ins: _adder_nodes(c, *_fronts(c, ins)), [a, b], out)
 
     def multiply(self, a_bits, b_bits, out_bits):
-        """out = low w bits of a * b, w <= 16 (one multiplier block, parasol_cpu/src/proc/ops/mul.rs:75-117)."""
+        """out = low w bits of a * b, w <= 16 (one multiplier block, parasol_cpu/src/proc/ops/mul.rs:75-117).  With a
+        Plain operand, w <= 32 and the circuit is the constant multiplier (mux_circuits.const_multiplier, depth <= w) on
+        the other operand."""
         from . import mux_circuits as M
 
         a_bits, b_bits, out_bits = list(a_bits), list(b_bits), list(out_bits)
         w = len(a_bits)
-        if w > M.CIRCUIT_CUTOFF or len(b_bits) != w or len(out_bits) != w:
-            raise ValueError("InstructionCache.multiply: equal widths up to 16 bits (wider products span two bootstrap levels: "
-                             "use circuits.multiply_then_greater_than / mux_circuits.append_uint_multiply)")
+        plain = _is_plain(a_bits) or _is_plain(b_bits)
+        if w > (32 if plain else M.CIRCUIT_CUTOFF) or len(b_bits) != w or len(out_bits) != w:
+            raise ValueError("InstructionCache.multiply: equal widths up to 16 bits, 32 with a Plain operand (wider products "
+                             "span two bootstrap levels: use circuits.multiply_then_greater_than / mux_circuits.append_uint_multiply)")
+        if plain:
+            # the constant is b when b is plaintext (a then enters the circuit, and folds if it is plaintext too)
+            e, k = (0, _plain_value(b_bits)) if _is_plain(b_bits) else (1, _plain_value(a_bits))
+            body = lambda c, ins: M.insert_mux_circuit(c, M.const_multiplier(w, k), _fronts(c, [ins[e]])[0])
+            return self._run(("mul", w), body, [a_bits, b_bits], out_bits)
         full = lambda: M.unsigned_multiplier(w, w)
         low = lambda: _keep_outputs(full(), w)
         return self._mux_instruction(("mul", w), low, [a_bits, b_bits], out_bits, interleave=False)
@@ -340,11 +434,16 @@ class _Instructions:
     def shift(self, a_bits, amount_bits, out_bits, right: bool, mode: str = "logical"):
         """out = a shifted by the encrypted amount (bitshift.rs:49-157).  mode "logical" clears the bits shifted in (an
         amount >= w gives 0), "rotation" wraps (power-of-two w; the amount counts mod w), "arithmetic" fills a right
-        shift with the sign bit.  w <= 16 (SHIFT_MAX_WIDTH); the amount needs at least ceil(log2(w)) bits (at least 1)."""
+        shift with the sign bit.  w <= 16 (SHIFT_MAX_WIDTH); the amount needs at least ceil(log2(w)) bits (at least 1).
+        A Plain amount k is shift_const(a, k) -- min(k, w), or k mod w for a rotation -- with shift_const's rules (any
+        width) and its cached graph."""
         from . import mux_circuits as M
 
         a, amt = _operands("shift", a_bits, amount_bits, equal=False)
         w, k, right = len(a), len(amt), bool(right)
+        if _is_plain(amt):
+            amount = _plain_value(amt)
+            return self.shift_const(a, amount % w if mode == "rotation" else min(amount, w), out_bits, right, mode)
         out = _results("shift", out_bits, w)
         if w > SHIFT_MAX_WIDTH:
             raise ValueError(f"InstructionCache.shift: widths up to {SHIFT_MAX_WIDTH} bits, got {w} "
@@ -363,20 +462,30 @@ class _Instructions:
 
     def multiply_signed(self, a_bits, b_bits, out_bits):
         """out = low w bits of the two's-complement product a * b, w <= 16 (circuits/mul.rs:19-73: |a|, |b|, one
-        multiplier block, conditional negate; three bootstrap levels)."""
+        multiplier block, conditional negate; three bootstrap levels).  With a Plain operand c, w <= 32: |a| times |c|
+        through the constant multiplier, negated by a's sign (mux_circuits.append_int_multiply_const)."""
         from . import mux_circuits as M
 
         a, b = _operands("multiply_signed", a_bits, b_bits)
         w = len(a)
-        if w > M.CIRCUIT_CUTOFF:
-            raise ValueError(f"InstructionCache.multiply_signed: widths up to {M.CIRCUIT_CUTOFF} bits, got {w}")
+        plain = _is_plain(a) or _is_plain(b)
+        if w > (32 if plain else M.CIRCUIT_CUTOFF):
+            raise ValueError(f"InstructionCache.multiply_signed: widths up to {M.CIRCUIT_CUTOFF} bits (32 with a Plain "
+                             f"operand), got {w}")
         out = _results("multiply_signed", out_bits, w)
+        if plain:
+            e, k = (0, _plain_value(b)) if _is_plain(b) else (1, _plain_value(a))
+            k -= (k >> (w - 1)) << w   # two's complement
+            body = lambda c, ins: M.append_int_multiply_const(c, _fronts(c, [ins[e]])[0], k)
+            return self._run(("mul_signed", w), body, [a, b], out)
         return self._run(("mul_signed", w), lambda c, ins: M.append_int_multiply(c, *_fronts(c, ins))[0], [a, b], out)
 
     # ---- no MUX circuit ----
     def select(self, cond, a_bits, b_bits, out_bits):
-        """out = cond ? b : a, for one encrypted bit `cond`: cond is bootstrapped to a selector, then one CMux per bit."""
+        """out = cond ? b : a, for one encrypted bit `cond`: cond is bootstrapped to a selector, then one CMux per bit.
+        A plaintext cond (a one-bit Plain) makes out a copy of a or b."""
         a, b = _operands("select", a_bits, b_bits)
+        cond = _bit("select", cond)
         out = _results("select", out_bits, len(a))
 
         def body(c, ins):
@@ -464,8 +573,11 @@ class InstructionCache(_Instructions):
     FheCircuit::insert_mux_circuit_and_connect_inputs (fhe_circuit.rs:473-494) does.
 
     Operands and results are lists of L1 GLWE bit ciphertexts, least significant bit first: host arrays, or
-    BoxCiphertext handles on a BoxEvaluation.  Every method checks its widths before anything is built (ValueError),
-    runs blocking and returns the graph it ran.  block() records several instructions and runs them as one graph."""
+    BoxCiphertext handles on a BoxEvaluation.  Any operand may be a Plain instead: its bits are constants of the graph,
+    folded out of the circuit.  The cache key then records which operand bits are plaintext and their values, so every
+    distinct constant builds (and caches) a graph of its own, and a call with the same constants in the same places
+    hits.  Every method checks its widths before anything is built (ValueError), runs blocking and returns the graph it
+    ran.  block() records several instructions and runs them as one graph."""
 
     def __init__(self, evaluation):
         from . import BoxEvaluation, BoxGraph, CompiledGraph
@@ -479,8 +591,9 @@ class InstructionCache(_Instructions):
         return Block(self)
 
     def _run(self, key, body, operands, out_bits):
-        return self._cached(key, lambda: _instruction_graph(operands, out_bits, body),
-                            [x for op in operands for x in op] + list(out_bits))
+        _check_results(f"InstructionCache.{key[0]}", out_bits)
+        return self._cached(_plain_key(key, operands), lambda: _instruction_graph(operands, out_bits, body),
+                            [x for op in operands for x in op if not isinstance(x, PlainBit)] + list(out_bits))
 
     def _cached(self, key, build, bufs):
         """Build (on a miss) the graph of `key` with build() -> (graph, input-bit nodes, output-bit nodes), bind it to
@@ -543,7 +656,9 @@ class Block(_Instructions):
     only order.  run() lowers the whole block into one graph, so the planner batches the bootstraps of independent
     instructions into one launch per stage, intermediates stay in device memory, and a bit read by several
     instructions is bootstrapped once.  A result read by a later instruction goes through the same SampleExtract ->
-    KeyswitchL1toL0 -> CircuitBootstrap refresh it would after a round trip through the host."""
+    KeyswitchL1toL0 -> CircuitBootstrap refresh it would after a round trip through the host.  Operands may also be
+    const registers (const()) or Plain values: the block's graph is then constant-folded as a whole, so a result that
+    depends on constants only is a constant for the instructions after it; the cache key records the constants."""
 
     def __init__(self, cache: InstructionCache):
         self._icache, self._regs, self._program = cache, [], []
@@ -558,23 +673,31 @@ class Block(_Instructions):
         self._regs.append(Reg([Bit(self, r, i) for i in range(width)], index=r))
         return self._regs[-1]
 
+    def const(self, width: int, value: int) -> Reg:
+        """A read-only register of plaintext bits holding `value` (the range of Plain(value, width)): instructions read
+        it like Plain(value, width); writing it, or binding it in run(), raises ValueError."""
+        return Reg(Plain(value, width).bits)
+
     def _run(self, key, body, operands, out_bits):
         reads, out = [b for op in operands for b in op], list(out_bits)
+        _check_results(f"Block {key[0]}", out)
         for b in reads + out:
-            if not isinstance(b, Bit) or b.block is not self:
+            if not isinstance(b, PlainBit) and (not isinstance(b, Bit) or b.block is not self):
                 raise ValueError(f"Block {key[0]}: {b!r} is not a bit of this block's registers")
         if len(set(out)) < len(out) or self._written.intersection(out):
             raise ValueError(f"Block {key[0]}: writes a bit a second time")
         if self._read.intersection(out) or set(reads).intersection(out):
             raise ValueError(f"Block {key[0]}: writes a bit that this or an earlier instruction reads")
         self._program.append((key, body, operands, out))
-        self._read.update(reads)
+        self._read.update(b for b in reads if isinstance(b, Bit))
         self._written.update(out)
 
     def _binding(self, name: str, regs) -> list:
         """{Reg: buffers} -> [(register, buffer list)] in register creation order."""
         bound = []
         for r, bufs in dict(regs).items():
+            if isinstance(r, Reg) and r.bits and isinstance(r.bits[0], PlainBit):
+                raise ValueError(f"Block.run: a const register is plaintext, it cannot be bound in {name}")
             if not isinstance(r, Reg) or r.index is None or r.bits[0].block is not self:
                 raise ValueError(f"Block.run: {name} keys must be registers of this block (from reg(), not views)")
             bufs = list(bufs)
@@ -601,7 +724,7 @@ class Block(_Instructions):
         for r, _ in outs:
             if not self._written.issuperset(r):
                 raise ValueError(f"Block.run: output register r{r.index} is not written in full")
-        name = lambda b: (b.reg, b.index)
+        name = lambda b: ("plain", b.value) if isinstance(b, PlainBit) else (b.reg, b.index)
         key = ("block",
                tuple((k, tuple(tuple(map(name, op)) for op in operands), tuple(map(name, res))) for k, _, operands, res in self._program),
                tuple(len(r) for r in self._regs), tuple(r.index for r, _ in ins), tuple(r.index for r, _ in outs))

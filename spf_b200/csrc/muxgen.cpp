@@ -349,6 +349,37 @@ Fns build_gradeschool_reduce(BddManager& M, uint32_t n, uint32_t m) {
   return result;
 }
 
+// Multiplication by a plaintext constant k: the low n bits of x * k, inputs x0 .. x(n-1) least significant first, in
+// their natural order (no duplicated copies as in build_multiplier), so output bit i is an ROBDD over x0 .. xi and
+// every path tests each variable at most once: depth <= n.  The function is the ripple sum of the shifted copies
+// x << j for every set bit j of k; its ROBDD is built directly from the states of that sum read least significant bit
+// first instead of through apply() on the partial sums (which takes a minute at 32 bits):
+// after x0 .. x(t-1), bit t + d of the product is bit d of C + k * (xt + 2 x(t+1) + ...), where the carry C =
+// (k * (x0 .. x(t-1))) >> t < k matters only mod 2^(d+1).  Testing xt adds k * xt to C and shifts one bit out.
+struct ConstMultiplier {
+  BddManager& M;
+  uint64_t k;
+  std::unordered_map<uint64_t, uint32_t> memo;  // (t, d, C mod 2^(d+1)) -> BDD node
+  uint32_t bit(uint32_t t, uint32_t d, uint64_t carry) {
+    carry &= (2ull << d) - 1;  // d <= 31
+    const uint64_t key = (uint64_t)t << 58 | (uint64_t)d << 52 | carry;
+    auto it = memo.find(key);
+    if (it != memo.end()) return it->second;
+    const uint64_t lo = carry, hi = carry + k;
+    const uint32_t r = d == 0 ? M.mk(t, (uint32_t)(lo & 1), (uint32_t)(hi & 1))
+                              : M.mk(t, bit(t + 1, d - 1, lo >> 1), bit(t + 1, d - 1, hi >> 1));
+    memo.emplace(key, r);
+    return r;
+  }
+};
+
+Fns build_const_multiplier(BddManager& M, uint32_t n, uint32_t k) {
+  ConstMultiplier cm{M, k, {}};
+  Fns out(n);
+  for (uint32_t i = 0; i < n; i++) out[i] = cm.bit(0, i, 0);
+  return out;
+}
+
 // ---- BDD -> multiplexer list ----------------------------------------------------------------------
 // MuxCircuit::from(&[Bdd]) + remap_inputs + optimize (lib.rs:249-341,355-451): a BDD node testing
 // variable v with children (lo, hi) is the multiplexer sel = input(v), low = lo, high = hi.  With a
@@ -474,6 +505,11 @@ static int mux_circuit_impl(uint32_t kind, uint32_t n, uint32_t m, uint32_t flag
       if (m == 0 || n < m) return SPF_E_INVALID;  // mul.rs:431
       BddManager M(2 * (n + m));
       return emit(M, build_gradeschool_reduce(M, n, m), 2 * (n + m), nullptr, out, count);
+    }
+    case SPF_MUX_CONST_MULTIPLIER: {  // n input bits, flags = the constant (its low n bits count)
+      if (n > 32 || m != 0) return SPF_E_INVALID;
+      BddManager M(n);
+      return emit(M, build_const_multiplier(M, n, n == 32 ? flags : flags & ((1u << n) - 1)), n, nullptr, out, count);
     }
     default:
       return SPF_E_INVALID;
