@@ -274,6 +274,12 @@ _SHIFT_MODES = ("logical", "rotation", "arithmetic")
 # The barrel shifter's BDD orders the value bits above the amount bits (bitshift.rs), so its size grows as 2^w: 16 bits
 # is 196 588 multiplexers, 20 bits 3.2 million, 32 bits cannot be built.
 SHIFT_MAX_WIDTH = 16
+# lookup: a k-bit index reads 2^k table entries, one polynomial of N = 2048 coefficients per 2^11 entries and result
+# bit above 11 index bits, so 16 index bits with 16 result bits copy 16 MiB of table per run
+LOOKUP_MAX_INDEX_BITS = 16
+LOOKUP_MAX_RESULT_BITS = 64
+# select_n: one CMux tree of 2^k - 1 multiplexers per result bit over 2^k encrypted entries
+SELECT_N_MAX_INDEX_BITS = 8
 
 
 def _operands(name: str, *ops, equal: bool = True) -> list[list]:
@@ -311,6 +317,83 @@ def _plain_key(key, operands):
     if not any(isinstance(b, PlainBit) for op in operands for b in op):
         return key
     return key + (tuple(tuple(b.value if isinstance(b, PlainBit) else None for b in op) for op in operands),)
+
+
+def _table_values(table, m: int) -> np.ndarray:
+    """A lookup table's entries as uint64 values mod 2^m; every entry must be an integer in Plain(value, m)'s range."""
+    lo, hi = -(1 << (m - 1)), 1 << m
+    arr = table if isinstance(table, np.ndarray) else np.asarray(table)
+    if arr.ndim != 1:
+        raise ValueError(f"InstructionCache.lookup: the table must be a sequence of integers, got shape {arr.shape}")
+    if arr.dtype.kind in "iub":   # vectorised: the 2^16 entries of a 16-bit table are checked in well under a millisecond
+        if len(arr) and not (lo <= int(arr.min()) and int(arr.max()) < hi):
+            bad = next(v for v in arr.tolist() if not lo <= v < hi)
+            raise ValueError(f"InstructionCache.lookup: entry {bad} does not fit in {m} bits")
+        return arr.astype(np.uint64) & np.uint64((1 << m) - 1)
+    if isinstance(table, np.ndarray):
+        raise ValueError(f"InstructionCache.lookup: table entries must be integers, got dtype {arr.dtype}")
+    values = []
+    for v in table:   # entries numpy cannot hold in one integer dtype (2^63 and over next to negative values)
+        if not isinstance(v, (int, np.integer)):
+            raise ValueError(f"InstructionCache.lookup: table entry {v!r} is not an integer")
+        if not lo <= int(v) < hi:
+            raise ValueError(f"InstructionCache.lookup: entry {int(v)} does not fit in {m} bits")
+        values.append(int(v) % (1 << m))
+    return np.array(values, np.uint64)
+
+
+def _lookup_layout(k: int, m: int, log_n: int) -> tuple[int, int, int]:
+    """(stride s, groups, polynomials per group) of a k-bit -> m-bit table in polynomials of 2^log_n coefficients: entry
+    i, result bit g * s + r is coefficient i * s + r of group g's polynomial, with s the smallest power of two >= m when
+    k + log2(s) <= log_n, else the largest that fits; above log_n index bits s = 1 and each of the m groups (result bits)
+    takes 2^(k - log_n) polynomials, polynomial h holding entries [h * 2^log_n, (h + 1) * 2^log_n)."""
+    s = 1 << (m - 1).bit_length()
+    if k + s.bit_length() - 1 > log_n:
+        s = 1 << max(0, log_n - k)
+    return s, -(-m // s), 1 << max(0, k - log_n)
+
+
+def _table_bodies(values: np.ndarray, k: int, m: int, s: int, groups: int, per_group: int) -> np.ndarray:
+    """The body coefficients (bits, 0 / 1) of every table polynomial, [groups * per_group, entries per polynomial * s] in
+    the order group, then polynomial of the group; entries past len(values) read as 0."""
+    padded = np.zeros(1 << k, np.uint64)
+    padded[:len(values)] = values
+    bits = np.zeros((1 << k, groups * s), np.uint64)
+    bits[:, :m] = (padded[:, None] >> np.arange(m, dtype=np.uint64)) & np.uint64(1)
+    e = (1 << k) // per_group
+    return bits.reshape(per_group, e, groups, s).transpose(2, 0, 1, 3).reshape(groups * per_group, e * s)
+
+
+_TABLES: "weakref.WeakKeyDictionary[FheCircuit, dict[tuple, list[int]]]" = weakref.WeakKeyDictionary()
+
+
+def _lookup_nodes(c: FheCircuit, key, values: np.ndarray, sels: list[int], m: int, params, zeros) -> list[int]:
+    """Vertical packing of a plaintext table behind the selectors `sels` (index bits, LSB first): the table as trivial
+    GLWE polynomials (InputGlwe1 nodes whose buffers, from zeros(shape), the graph owns; memoised per circuit by `key`,
+    so two lookups of one table in a block share them), a CMux tree on the index bits above log2 N, then per index bit j
+    acc = CMux(x_j, acc, acc * X^(-2^j s)), and every result bit rotated to coefficient 0.  The coefficient read never
+    wraps, and at the q/2 bit encoding a negacyclic sign flip is the identity anyway.  Returns the GLWE nodes of the m
+    result bits."""
+    n, gk = params.glwe_n, params.glwe_k
+    log_n, k = n.bit_length() - 1, len(sels)
+    s, groups, per_group = _lookup_layout(k, m, log_n)
+    memo = _TABLES.setdefault(c, {})
+    if key not in memo:
+        bodies = _table_bodies(values, k, m, s, groups, per_group)
+        polys = zeros((groups * per_group, (gk + 1) * n))
+        polys[:, gk * n:gk * n + bodies.shape[1]] = bodies << np.uint64(63)
+        memo[key] = [c.add("InputGlwe1", io=p) for p in polys]
+    polys = memo[key]
+    res = []
+    for g in range(groups):
+        level = polys[g * per_group:(g + 1) * per_group]
+        for sel in sels[log_n:]:   # polynomial h = x >> log_n: index bit log_n at the leaves
+            level = [c.add("CMux", sel, level[i], level[i + 1]) for i in range(0, len(level), 2)]
+        acc = level[0]
+        for j, sel in enumerate(sels[:log_n]):
+            acc = c.add("CMux", sel, acc, c.add("MulXN", acc, arg=2 * n - (s << j)))
+        res += [acc if r == 0 else c.add("MulXN", acc, arg=2 * n - r) for r in range(min(s, m - g * s))]
+    return res
 
 
 class _Instructions:
@@ -495,6 +578,73 @@ class _Instructions:
 
         return self._run(("select", len(a)), body, [[cond], a, b], out)
 
+    # ---- table reads: one circuit bootstrap per index bit, then one CMUX level per index bit ----
+    def lookup(self, table, index_bits, out_bits):
+        """out = table[x] for the encrypted k-bit index x (LSB first) and a plaintext table: a sequence of Python ints
+        or a 1-D integer numpy array, 1 <= len(table) <= 2^k, entries in Plain(value, m)'s range for m = len(out_bits)
+        (1 <= m <= 64), entries past len(table) reading as 0; k <= 16 (LOOKUP_MAX_INDEX_BITS).  Circuit bootstrapping
+        and vertical packing: the table is packed into trivial GLWE polynomials of N = glwe_n coefficients (the
+        evaluation's params, DEFAULT_128 without one), m result bits side by side per entry where k + log2(m) <=
+        log2(N), otherwise in groups of result bits with a polynomial each; the index bits are bootstrapped to selectors
+        and blind-rotate each polynomial by x, one CMux per index bit -- above log2(N) index bits after a CMux tree that
+        picks the polynomial holding x.  Whatever the function: k bootstraps, ceil(m / s) * k CMux nodes for k <= 11
+        (s the entries' stride), m * (2^(k - 11) - 1 + 11) above.  The graph owns the table polynomials and copies them
+        to the device on every run (32 KiB each: 16 MiB for a 16-bit -> 16-bit table); the cache key holds the table,
+        so every table builds a graph of its own.  A Plain index makes the results constants (no bootstrap, no table);
+        the plaintext bits of a partly Plain index fold into fixed rotations.  Result bits carry their bit in
+        coefficient 0, as every instruction reads it, but their other coefficients hold other table bits: refresh them
+        (any instruction does) before they go to circuits.pack."""
+        (idx,) = _operands("lookup", index_bits)
+        out = list(out_bits)
+        k, m = len(idx), len(out)
+        if k > LOOKUP_MAX_INDEX_BITS:
+            raise ValueError(f"InstructionCache.lookup: index widths up to {LOOKUP_MAX_INDEX_BITS} bits, got {k}")
+        if not 1 <= m <= LOOKUP_MAX_RESULT_BITS:
+            raise ValueError(f"InstructionCache.lookup: {m} result bits, expected 1 .. {LOOKUP_MAX_RESULT_BITS}")
+        if not 1 <= len(table) <= 1 << k:
+            raise ValueError(f"InstructionCache.lookup: a table of {len(table)} entries for a {k}-bit index (1 .. {1 << k})")
+        values = _table_values(table, m)
+        key = ("lookup", k, m, values.tobytes())
+        if _is_plain(idx):
+            x = _plain_value(idx)
+            v = int(values[x]) if x < len(values) else 0
+            body = lambda c, ins: [c.add("OneGlwe1" if (v >> i) & 1 else "ZeroGlwe1") for i in range(m)]
+        else:
+            params, zeros = self._params(), self._host_zeros
+            body = lambda c, ins: _lookup_nodes(c, key, values, [_refresh(c, x) for x in ins[0]], m, params, zeros)
+        return self._run(key, body, [idx], out)
+
+    def select_n(self, entries, index_bits, out_bits):
+        """out = entries[x] for the encrypted k-bit index x (LSB first), k <= 8 (SELECT_N_MAX_INDEX_BITS): entries are
+        1 .. 2^k operands of len(out_bits) bits each -- bit lists, registers, Plain values or const registers -- and an
+        index past the last entry reads 0.  The index bits are bootstrapped to selectors, the entries are not: one CMux
+        tree per result bit with index bit 0 at the leaves (2^k - 1 CMux nodes, k levels).  Missing and Plain entries
+        are constants and fold out of the tree."""
+        (idx,) = _operands("select_n", index_bits)
+        out = list(out_bits)
+        k, m = len(idx), len(out)
+        if k > SELECT_N_MAX_INDEX_BITS:
+            raise ValueError(f"InstructionCache.select_n: index widths up to {SELECT_N_MAX_INDEX_BITS} bits, got {k}")
+        if m < 1:
+            raise ValueError("InstructionCache.select_n: no result bits")
+        entries = [list(e) for e in entries]
+        if not 1 <= len(entries) <= 1 << k:
+            raise ValueError(f"InstructionCache.select_n: {len(entries)} entries for a {k}-bit index (1 .. {1 << k})")
+        if any(len(e) != m for e in entries):
+            raise ValueError(f"InstructionCache.select_n: entry widths {[len(e) for e in entries]}, expected {m}")
+        missing = [[_PLAIN_BITS[0]] * m] * ((1 << k) - len(entries))
+
+        def body(c, ins):
+            sels, res = [_refresh(c, x) for x in ins[0]], []
+            for b in range(m):
+                level = [e[b] for e in ins[1:]]
+                for sel in sels:
+                    level = [c.add("CMux", sel, level[i], level[i + 1]) for i in range(0, len(level), 2)]
+                res.append(level[0])
+            return res
+
+        return self._run(("select_n", k, m), body, [idx] + entries + missing, out)
+
     def xor(self, a_bits, b_bits, out_bits):
         """out = a ^ b: one GlweAdd per bit (KeylessEvaluation::xor), no bootstrap."""
         a, b = _operands("xor", a_bits, b_bits)
@@ -590,6 +740,19 @@ class InstructionCache(_Instructions):
         """An empty Block whose graphs are cached here."""
         return Block(self)
 
+    def _params(self):
+        """The evaluation's params (DEFAULT_128 without an evaluation)."""
+        from . import default_128
+
+        return self._ev.params if self._ev is not None else default_128()
+
+    def _host_zeros(self, shape) -> np.ndarray:
+        """Zeroed uint64 host memory for buffers a graph owns (lookup tables): one page-locked slab when there is an
+        evaluation, so that their copies are DMAs without a registration per buffer."""
+        from . import pinned_zeros
+
+        return pinned_zeros(shape) if self._ev is not None else np.zeros(shape, np.uint64)
+
     def _run(self, key, body, operands, out_bits):
         _check_results(f"InstructionCache.{key[0]}", out_bits)
         return self._cached(_plain_key(key, operands), lambda: _instruction_graph(operands, out_bits, body),
@@ -677,6 +840,12 @@ class Block(_Instructions):
         """A read-only register of plaintext bits holding `value` (the range of Plain(value, width)): instructions read
         it like Plain(value, width); writing it, or binding it in run(), raises ValueError."""
         return Reg(Plain(value, width).bits)
+
+    def _params(self):
+        return self._icache._params()
+
+    def _host_zeros(self, shape) -> np.ndarray:
+        return self._icache._host_zeros(shape)
 
     def _run(self, key, body, operands, out_bits):
         reads, out = [b for op in operands for b in op], list(out_bits)
